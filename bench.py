@@ -2,7 +2,7 @@
 """Benchmark of the warp-and-fuse hot path (BASELINE.json metric: SR frames/s, 4x, 1080p out; projection+warp
 GB/s vs HBM peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload, identical in both arms) = configs[1] "C2": 4x VSR 480x270 -> 1920x1080, 7-frame window
@@ -22,6 +22,10 @@ One JSON line on stdout (rank 0):
             GB/s and fractions of the measured copy peak and of the nominal 8 TB/s
   c4, c5    the other BASELINE configurations, driver-visible (N=1 only; skip with --no-extras)
   cpu_baseline  the CPU oracle on a bounded sample with all host cores (rank 0, N=1)
+--dump-outputs DIR writes the u8 frames (1080x1920x3) of the last timed step, one per rank in rank order as the gather
+hands them to the caller, as DIR/frames.npy in float32.  Past 64 MB (N > 2) it writes the same fixed, seeded sample of
+pixels of every frame instead: DIR/frames_sample.npy (N, pixels, 3) and their flat indices, DIR/frames_sample_pixels.npy.
+The inputs and weights are seeded, so two builds run with the same arguments can be compared frame for frame.
 `--impl reference` times the CPU restatement (oracle/; the reference's ops on this path are CUDA-only) with all host
 threads: one step = the full-size front + the conv stack (both passes) on one quarter-height band (68x480 LR pixels)
 of one of the 20 maps -- a bounded sample, scaled by pixel-maps and labelled `extrapolated`.
@@ -348,6 +352,26 @@ def sub_c5(dev, rank, world, frames=300):
             "gathered_bytes": int(allf.numel())}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_frames(out_dir, frames):
+    """frames (N,H,W,C) u8 -> out_dir/frames.npy in float32, or, past DUMP_LIMIT_BYTES, the same fixed, seeded sample
+    of pixels of every frame (frames_sample.npy, (N,pixels,C)) with their flat indices (frames_sample_pixels.npy)."""
+    import numpy as np
+    import torch
+    n, h, w, c = frames.shape
+    os.makedirs(out_dir, exist_ok=True)
+    if frames.numel() * 4 <= DUMP_LIMIT_BYTES:
+        np.save(os.path.join(out_dir, "frames.npy"), frames.float().cpu().numpy())
+        return
+    k = DUMP_LIMIT_BYTES // (n * c * 4 + 8)                   # float32 values of every frame + one float64 index
+    pix = np.sort(np.random.default_rng(0).choice(h * w, size=k, replace=False))
+    sample = frames.reshape(n, h * w, c)[:, torch.from_numpy(pix).to(frames.device)]
+    np.save(os.path.join(out_dir, "frames_sample.npy"), sample.float().cpu().numpy())
+    np.save(os.path.join(out_dir, "frames_sample_pixels.npy"), pix.astype(np.float64))
+
+
 def _gained(sr, gain=2.3):
     """x2.3 so that a 40-layer random net keeps O(1) activations (the reference's default initialisers decay)."""
     import torch
@@ -395,7 +419,7 @@ def run_b200(args, rank, world, local_rank):
     host = [{k: v.pin_memory() for k, v in make_inputs(seed=100 * (s + 1) + rank).items()} for s in range(SEEDS)]
     res = [{k: v.to(dev) for k, v in hs.items()} for hs in host]
     h2d = sum(v.numel() * v.element_size() for v in host[0].values())
-    frames_u8 = torch.empty((max(args.steps, 1),) + HW3, dtype=torch.uint8, device=dev)   # this rank's output frames
+    frames_u8 = torch.empty((args.steps,) + HW3, dtype=torch.uint8, device=dev)   # this rank's output frames
     d2h = frames_u8[0].numel()
     counters = {"k": 0}
 
@@ -403,8 +427,9 @@ def run_b200(args, rank, world, local_rank):
         k = counters["k"]
         counters["k"] = k + 1
         r = res[k % SEEDS]
-        return pipe.step(r["frames"], r["flows"], r["inv_depth"], r["logits_a"], r["logits_b"],
-                         out_u8=frames_u8[k % frames_u8.shape[0]], want_f32=False)
+        counters["last"] = pipe.step(r["frames"], r["flows"], r["inv_depth"], r["logits_a"], r["logits_b"],
+                                     out_u8=frames_u8[k % frames_u8.shape[0]], want_f32=False)
+        return counters["last"]
 
     # End-to-end loop: every step's inputs come from pinned host memory and every step's u8 frame goes back to the
     # host, inside the timed region -- double-buffered on a copy stream, so that the H2D of step k+1 and the D2H of
@@ -497,6 +522,11 @@ def run_b200(args, rank, world, local_rank):
     _lib.launch_count_reset()
     ms_total = timed(step_resident, args.steps)
     launches = _lib.launch_count()
+    if args.dump_outputs:
+        # every rank's frame of the last timed step, gathered before the e2e loop reuses its buffer
+        last = gather_frames(counters["last"].unsqueeze(0))
+        if rank == 0:
+            dump_frames(args.dump_outputs, last)
     ms_e2e = timed(step_e2e, args.steps)
     clocks = sampler.stop() if rank == 0 else None
 
@@ -509,7 +539,7 @@ def run_b200(args, rank, world, local_rank):
                          "'frames': the T frame maps (video_super_resolution.py:62 feeds `data` unchanged); 'unchanged': all "
                          "but the estimate slot (this pipeline's flow / depth maps are inputs, not re-estimated). "
                          "maps_convolved_per_frame counts both passes (headline: 2 M)."}
-        n_re = max(min(args.steps, 10), 2)
+        n_re = args.steps
         for mode, n_maps in (("frames", 2 * M_MAPS - T_WIN), ("unchanged", M_MAPS + 1)):
             pipe_r = WarpFusePipeline(T_WIN, H_LR, W_LR, sr, SCALE, device=dev, max_disp=MAX_DISP, reuse=mode)
 
@@ -647,7 +677,14 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the front_c3 / c4 / c5 sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write every rank's output frame of the last timed step to DIR/frames.npy (float32, values "
+                         "0..255; a seeded pixel sample past 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the frames of the b200 arm; the reference arm computes a sample of a frame")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

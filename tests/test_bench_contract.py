@@ -37,16 +37,45 @@ def test_non_zero_ranks_of_the_reference_arm_exit_quietly():
     assert r.returncode == 0 and r.stdout.strip() == ""
 
 
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bad_arguments_are_refused(argv, tmp_path):
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True,
+                       timeout=120, cwd=tmp_path)
+    assert r.returncode == 2 and r.stdout == "" and "error" in r.stderr
+    assert not os.path.exists(tmp_path / "out")
+
+
+def test_dump_frames_samples_the_same_pixels_of_every_frame_past_the_limit(tmp_path, monkeypatch):
+    import numpy as np
+    import torch
+    import bench
+    frames = torch.randint(0, 256, (3, 40, 50, 3), dtype=torch.uint8, generator=torch.Generator().manual_seed(0))
+    bench.dump_frames(str(tmp_path / "all"), frames)
+    assert np.array_equal(np.load(tmp_path / "all" / "frames.npy"), frames.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 3 * 40 * 50 * 3 * 4 // 2)
+    bench.dump_frames(str(tmp_path / "sample"), frames)
+    assert sorted(os.listdir(tmp_path / "sample")) == ["frames_sample.npy", "frames_sample_pixels.npy"]
+    sample, pix = np.load(tmp_path / "sample" / "frames_sample.npy"), np.load(tmp_path / "sample" / "frames_sample_pixels.npy")
+    assert sample.dtype == np.float32 and pix.dtype == np.float64 and sample.nbytes + pix.nbytes <= bench.DUMP_LIMIT_BYTES
+    assert sample.shape == (3, pix.size, 3) and pix.size > 0 and np.unique(pix).size == pix.size
+    assert np.array_equal(sample, frames.float().numpy().reshape(3, -1, 3)[:, pix.astype(np.int64)])
+
+
 @pytest.mark.gpu
-def test_b200_arm_prints_one_contract_line():
+def test_b200_arm_prints_one_contract_line(tmp_path):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-cpu-baseline",
-                        "--no-extras"], capture_output=True, text=True, timeout=900)
+                        "--no-extras", "--dump-outputs", str(tmp_path / "dump")], capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [l for l in r.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
     d = json.loads(lines[0])
     assert (REQUIRED - {"cpu_baseline"}) <= set(d)
-    assert d["gpu_launches"] > 0 and d["dtype"] == "bf16" and d["n_gpus"] == 1
+    assert d["gpu_launches"] > 0 and d["dtype"] == "bf16" and d["n_gpus"] == 1 and d["steps"] == 2
+    import numpy as np
+    assert os.listdir(tmp_path / "dump") == ["frames.npy"]
+    frames = np.load(tmp_path / "dump" / "frames.npy")
+    assert frames.dtype == np.float32 and frames.shape == (1, 1080, 1920, 3)
+    assert np.array_equal(frames, np.round(frames)) and 0 <= frames.min() and frames.max() <= 255 and frames.std() > 1
     import bench
     assert d["config"]["workload"] == bench.WORKLOAD
     roof = d["roofline"]
