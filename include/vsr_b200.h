@@ -319,18 +319,13 @@ int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* plan, const float* x, float* y,
  * forward and returns, per kernel class, the summed device time (ms), the number of launches, and
  * the layers' specified 2*MAC FLOPs and compulsory bytes (inputs + outputs of each launch, once).
  * Arrays have VSR_SRFBN_KERNEL_CLASSES entries, in the order of vsr_srfbn_kernel_class_name(). */
-#define VSR_SRFBN_KERNEL_CLASSES 11
+#define VSR_SRFBN_KERNEL_CLASSES 10
 const char* vsr_srfbn_kernel_class_name(int k);
 int vsr_srfbn_profile_enable(vsr_srfbn_plan* plan, int enable);
 int vsr_srfbn_profile_read(vsr_srfbn_plan* plan, double* ms, int32_t* launches, double* flops, double* bytes);
 /* per-launch device time of the last profiled forward, in launch order; returns the number of
  * launches (<0 on error) and fills at most `capacity` entries */
 int vsr_srfbn_profile_launches(vsr_srfbn_plan* plan, float* ms, int32_t* kclass, int32_t capacity);
-
-/* Test hook (synchronises the stream): 1 if a role of a co-scheduled group launch gave up waiting for the other during
- * the forwards run so far (the output is then wrong), 0 if not, < 0 on error.  Group launches run the transposed conv
- * and the fused down kernel of a feedback group as two roles of one launch so that hr[i] is handed over through L2. */
-int vsr_srfbn_debug_group_error(const vsr_srfbn_plan* plan, vsr_stream_t stream);
 
 /* Test hook: per-map network output before the fc fuse, (M,3,s*h,s*w) f32 (SRProjectionModule.py:143);
  * valid after vsr_srfbn_forward on the same stream. */

@@ -31,6 +31,16 @@ def test_python_binding_covers_header():
     assert declared <= bound, declared - bound
 
 
+def test_shipped_library_reads_no_variant_switches():
+    """The shipped library reads one environment variable, VSR_CORR_GENERIC (it chooses between two live correlation
+    kernels): no switch changes which conv-stack kernels a process runs.  The timing-experiment switches exist only in
+    the -DVSR_KNOCKOUT build."""
+    from video_super_resolution_b200 import build
+    with open(build.build(), "rb") as f:
+        names = set(re.findall(rb"VSR_[A-Z0-9_]+", f.read()))
+    assert names == {b"VSR_CORR_GENERIC"}, sorted(names)
+
+
 def test_host_side_entry_points_without_gpu():
     from video_super_resolution_b200 import _lib
     L = _lib.lib()

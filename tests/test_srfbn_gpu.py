@@ -165,41 +165,6 @@ def test_full_stack_against_oracle(M, h, w, steps, scale):
         f"fused max err {(got - want).abs().max():.4f} at scale {scale:.2f}"
 
 
-def test_group_launch_matches_separate_launches_bit_for_bit(monkeypatch):
-    """The co-scheduled group launch (deconv role + fused-down role in one kernel, hr[i] handed over through L2 with
-    per-tile flags) runs the same arithmetic as the two separate launches: identical bits, no give-up flag, and the
-    result agrees with the fp32 oracle.  648 tiles: above the threshold from which the plan groups."""
-    M, h, w = 8, 64, 128
-    sd = so.init_state_dict(num_maps=M, seed=3, gain=2.3)
-    x = (torch.rand((M, 3, h, w), generator=torch.Generator().manual_seed(4)) * 255).to(DEV)
-    outs = {}
-    for mode in ("1", "0"):
-        monkeypatch.setenv("VSR_GROUP", mode)
-        mod = SRProjectionModule(num_maps=M)
-        mod.load_state_dict(sd)
-        maps = mod.premix(x)
-        y = mod(x)
-        mod.profile(True)
-        mod(x)
-        classes = {k for k, v in mod.profile_read().items() if v["launches"]}
-        mod.profile(False)
-        assert ("group(deconv8x8s4+fused_downtran_conv8x8s4)" in classes) == (mode == "1"), classes
-        assert not mod.group_error()
-        outs[mode] = (maps.clone(), y.clone())
-        del mod
-    assert torch.equal(outs["1"][0], outs["0"][0]) and torch.equal(outs["1"][1], outs["0"][1])
-    with torch.no_grad():
-        want = so.forward_maps(x.cpu(), sd)
-    assert _psnr(outs["1"][0].cpu(), want) > 50.0
-    # several forwards in a row: the flags are re-zeroed per forward, the epochs restart
-    monkeypatch.setenv("VSR_GROUP", "1")
-    mod = SRProjectionModule(num_maps=M)
-    mod.load_state_dict(sd)
-    for _ in range(3):
-        y = mod(x)
-    assert torch.equal(y, outs["1"][1]) and not mod.group_error()
-
-
 @pytest.mark.parametrize("scale", [4, 2])
 def test_workspace_cap_chunks_the_maps_bit_identically(scale):
     """vsr_srfbn_plan_set_workspace_cap: the plan sweeps its layers over chunks of maps (the largest divisor of M that

@@ -89,7 +89,6 @@ SIGNATURES = {
     "vsr_srfbn_profile_enable": (c_int, [c_void_p, c_int]),
     "vsr_srfbn_profile_read": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vsr_srfbn_profile_launches": (c_int, [c_void_p, c_void_p, c_void_p, c_int]),
-    "vsr_srfbn_debug_group_error": (c_int, [c_void_p, c_void_p]),
     "vsr_srfbn_debug_premix": (c_int, [c_void_p, c_void_p, c_void_p]),
     "vsr_test_pointwise": (c_int, [c_void_p, c_i64, c_int, c_void_p, c_void_p, c_float, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "vsr_test_deconv": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),

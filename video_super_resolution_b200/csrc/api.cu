@@ -2,20 +2,9 @@
 #include "common.cuh"
 
 #include <stdio.h>
-#include <stdlib.h>
 
 namespace vsr {
 std::atomic<uint64_t> g_launch_count{0};
-
-bool pdl_enabled() {
-  static const bool on = [] {
-    // measured on B200 at C2 (profiles/ab_pdl_r01.log): no gain with dependents released at CTA exit, 2.5 % slower
-    // with an early trigger (the waiting CTAs of the next layer compete for issue slots and power) -> off by default
-    const char* e = getenv("VSR_PDL");
-    return e && atoi(e) != 0;
-  }();
-  return on;
-}
 }
 
 extern "C" const char* vsr_version(void) { return "vsr_b200 0.1 (sm_100a)"; }

@@ -46,29 +46,12 @@ struct PerDeviceOnce {
   }
 };
 
-// Programmatic dependent launch: the next kernel of a stream may start its prologue (barrier init, TMEM
-// allocation, weight loads) on SMs the previous kernel has already left; it must not touch any
-// activation buffer before griddep_wait(), which returns once every earlier grid has completed and
-// flushed.  Without the launch attribute both instructions are no-ops.
+// Programmatic dependent launch: the next kernel of a stream may start its prologue on SMs the previous
+// kernel has already left; it must not touch any buffer an earlier kernel writes or reads before
+// griddep_wait(), which returns once every earlier grid has completed and flushed.  Without the launch
+// attribute both instructions are no-ops.
 __device__ __forceinline__ void griddep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void griddep_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-
-bool pdl_enabled();   // VSR_PDL=1 turns the attribute on (A/B timing; default off, see api.cu)
-
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t smem, cudaStream_t st, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid, 1, 1);
-  cfg.blockDim = dim3((unsigned)block, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
 
 constexpr int kNumSMs = 148;  // B200
 

@@ -53,8 +53,6 @@ struct alignas(64) FusedDownParams {
   int32_t num_stages;
   int32_t tiles_x, tiles_y, batch;
   int32_t lr_h, lr_w;
-  int32_t prefetch_ahead;             // L2 prefetch distance in half-tiles
-  int32_t wd_resident;                // 1: all 128 KB of conv weights stay in shared memory; 0: 2-deep ring per group
   int32_t debug;                      // timing experiments (results become wrong): bit0 skip phase-A MMAs, bit1 skip
                                       // the TMEM reads + conversion of phase A, bit2 skip the final TMEM reads/stores,
                                       // bit3 skip phase-B MMAs
@@ -63,32 +61,8 @@ struct alignas(64) FusedDownParams {
   float* part;                        // (B, h, w, 4 slots, 32) fp32 partial sums of the BOUNDARY pixels (see final epilogue)
   void* lr_out;                       // (B, h, w, 32) bf16: finished interior pixels
   long long* trace;                   // VSR_KNOCKOUT builds: clock64 stamps of CTA 0's roles, [tile][32]; nullptr = off
-  int32_t xchg;                       // 1: tile rows 1,3,5 are finished too (row partials exchanged between lane quarters
-                                      // through shared memory); 0: only the even tile rows
 };
 
-__device__ __forceinline__ void tma_load_5d(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1,
-                                            int c2, int c3, int c4) {
-  asm volatile(
-      "cp.async.bulk.tensor.5d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6, %7}], [%2];" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-      : "memory");
-}
-// TMA prefetch into L2 only (no shared memory, no barrier): lets the producer run far ahead of its
-// shared-memory ring, so that the ring's loads hit L2 instead of paying the full HBM latency.
-__device__ __forceinline__ void tma_prefetch_5d(const CUtensorMap* map, int c0, int c1, int c2, int c3, int c4) {
-  asm volatile("cp.async.bulk.prefetch.tensor.5d.L2.global.tile [%0, {%1, %2, %3, %4, %5}];" ::"l"(
-                   reinterpret_cast<uint64_t>(map)),
-               "r"(c0), "r"(c1), "r"(c2), "r"(c3), "r"(c4)
-               : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_4d(const CUtensorMap* map, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];" ::"l"(
-                   reinterpret_cast<uint64_t>(map)),
-               "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-               : "memory");
-}
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
@@ -104,18 +78,15 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
 #endif
 
 template <bool HAS_TRAN>
-inline size_t fused_down_smem_bytes(int nsrc, int num_stages, int wd_resident, int xchg) {
+inline size_t fused_down_smem_bytes(int nsrc, int num_stages) {
   size_t wt = HAS_TRAN ? ((size_t)nsrc * kWtChunkBytes + 1023) / 1024 * 1024 : 0;
   size_t stage = HAS_TRAN ? 16384 : 2 * 16384;
-  return 1024 + (wd_resident ? 4 * kWdGroupBytes : kWdRingBytes) + wt + (HAS_TRAN ? kHBytes : 0) +
-         (size_t)num_stages * stage + 1024 + (xchg ? kXchgBytes : 0);
+  return 1024 + kWdRingBytes + wt + (HAS_TRAN ? kHBytes : 0) + (size_t)num_stages * stage + 1024 + kXchgBytes;
 }
 
-// The kernel body as a device function: fused_down_kernel runs it over the whole grid; group_kernel below runs it on
-// the CTAs after the deconv role's, with the tile hand-off `gs` (the newest source map is read from L2 as soon as the
-// deconv role has published the tile).
 template <bool HAS_TRAN>
-__device__ __forceinline__ void fused_body(const FusedDownParams& p, const int cta, const int ncta, const GroupSync* gs) {
+__global__ void __launch_bounds__(kFusedThreads, 1)
+fused_down_kernel(const __grid_constant__ FusedDownParams p) {
   constexpr int kStageBytes = HAS_TRAN ? 16384 : 2 * 16384;
   constexpr int kTmemCols = HAS_TRAN ? 512 : 256;
   constexpr uint32_t kDB = HAS_TRAN ? 256 : 0;       // first column of the two D_B accumulators
@@ -123,7 +94,7 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   uint8_t* s_wd = smem;
-  uint8_t* s_wt = s_wd + (p.wd_resident ? 4 * kWdGroupBytes : kWdRingBytes);
+  uint8_t* s_wt = s_wd + kWdRingBytes;
   const int wt_region = HAS_TRAN ? ((p.nsrc * kWtChunkBytes + 1023) / 1024 * 1024) : 0;
   uint8_t* s_h = s_wt + wt_region;
   uint8_t* s_a = s_h + (HAS_TRAN ? kHBytes : 0);
@@ -144,11 +115,11 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
   float* s_down = s_bias + 36;                                 // 33 floats: strided-conv bias + slope
   float4* s_x = reinterpret_cast<float4*>(tail + 1024);        // kXchgBytes: final-epilogue row exchange
 
+  const int cta = blockIdx.x, ncta = gridDim.x;   // persistent CTAs: tiles cta, cta + ncta, ...
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int total_tiles = p.tiles_x * p.tiles_y * p.batch;
 
-  // (no early griddepcontrol.launch_dependents: dependents are released as CTAs exit)
   if (threadIdx.x == 0) {
     for (int s = 0; s < p.num_stages; ++s) {
       mbar_init(&full_bar[s], 1);
@@ -193,65 +164,24 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
         for (int j = 0; j < p.nsrc; ++j) tma_load_2d(s_wt + j * kWtChunkBytes, &p.wt_map, w_full, j * 32, 0);
       }
       __syncwarp();
-      griddep_wait();   // weights are static; the HR maps only after the previous layers have completed
       int s = 0;
       uint32_t phase = 0;
-      // L2 prefetch cursor: runs kAhead half-tiles (8 sub-positions of every source = 64 KB per source)
-      // ahead of the loads.  Unit of the linear order: (tile, half) with half = sub-positions 8*half..+7.
-      const int kAhead = p.prefetch_ahead;   // 0 disables
-      auto prefetch_half = [&](int tile, int half) {
-        if (tile >= total_tiles) return;
-        int px0, py0, pb;
-        tile_coord(tile, px0, py0, pb);
-        if (elect_one()) {
-          if (HAS_TRAN) {
-            for (int sp = half * 8; sp < half * 8 + 8; sp += 2)
-              for (int j = 0; j < p.nsrc; ++j) tma_prefetch_4d(&p.hr_maps[j], 0, px0, py0, pb * 8 + (sp >> 1));
-          } else {
-            for (int pr = half * 4; pr < half * 4 + 4; ++pr) tma_prefetch_4d(&p.h0_map, 0, px0, py0, pb * 8 + pr);
-          }
-        }
-        __syncwarp();
-      };
-      {
-        int t = cta, hf = 0;
-        for (int i = 0; i < kAhead; ++i) {
-          prefetch_half(t, hf);
-          if (++hf == 2) { hf = 0; t += ncta; }
-        }
-      }
       int tile_n = -1;
       for (int tile = cta; tile < total_tiles; tile += ncta) {
         ++tile_n;
         int x0, y0, b;
         tile_coord(tile, x0, y0, b);
-        bool newest_ready = false;
         VSR_TRACE(0);
         for (int half = 0; half < 2; ++half) {
-          if (kAhead > 0) {  // the half-tile kAhead units ahead of (tile, half)
-            const int u = half + kAhead;
-            prefetch_half(tile + (u >> 1) * ncta, u & 1);
-          }
           if (HAS_TRAN) {
             // one box = 2 sub-positions x 128 blocks x 32 ch (16 KB): a [128 x 64] K-major tile whose K
             // halves are the two sub-positions (box count, not bytes, limits a single-thread producer)
             for (int sp = half * 8; sp < half * 8 + 8; sp += 2) {
               for (int j = 0; j < p.nsrc; ++j) {
                 mbar_wait(&empty_bar[s], phase ^ 1);
-                // group launch: the newest map's tile comes from the deconv role of this launch (L2); the older
-                // maps stream from HBM and are marked evict-first so that they do not push it out
-                if (gs != nullptr && j == p.nsrc - 1 && !newest_ready) {
-                  spin_until_ge(gs->tile_flags + tile, 32 * gs->epoch, gs->error);
-                  fence_proxy_async_all();
-                  newest_ready = true;
-                }
                 if (elect_one()) {
                   mbar_expect_tx(&full_bar[s], kStageBytes);
-                  if (gs != nullptr)
-                    tma_load_4d_hint(s_a + s * kStageBytes, &p.hr_maps[j], &full_bar[s], 0, x0, y0, b * 8 + (sp >> 1),
-                                     kL2EvictFirst);
-                  else
-                    tma_load_4d(s_a + s * kStageBytes, &p.hr_maps[j], &full_bar[s], 0, x0, y0, b * 8 + (sp >> 1));
+                  tma_load_4d(s_a + s * kStageBytes, &p.hr_maps[j], &full_bar[s], 0, x0, y0, b * 8 + (sp >> 1));
                 }
                 __syncwarp();
                 if (++s == p.num_stages) { s = 0; phase ^= 1; }
@@ -261,11 +191,6 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
           } else {
             for (int g = half * 2; g < half * 2 + 2; ++g) {
               mbar_wait(&empty_bar[s], phase ^ 1);
-              if (gs != nullptr && !newest_ready) {
-                spin_until_ge(gs->tile_flags + tile, 32 * gs->epoch, gs->error);
-                fence_proxy_async_all();
-                newest_ready = true;
-              }
               if (elect_one()) {
                 mbar_expect_tx(&full_bar[s], kStageBytes);
                 tma_load_4d(s_a + s * kStageBytes, &p.h0_map, &full_bar[s], 0, x0, y0, b * 8 + 2 * g);
@@ -339,9 +264,8 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
         a0 = dA + (uint64_t)((s * kStageBytes) >> 4);
       }
       if (g == 0) mbar_wait(&db_empty[tb], (n_b[tb] & 1) ^ 1);
-      const int wslot = p.wd_resident ? g : (int)(n_wd & 1);
-      if (!p.wd_resident) mbar_wait(&wd_full[wslot], (n_wd >> 1) & 1);
-      else if (n_wd == 0) mbar_wait(&wd_full[0], 0);      // one-time load of all four groups
+      const int wslot = (int)(n_wd & 1);
+      mbar_wait(&wd_full[wslot], (n_wd >> 1) & 1);
       tc_fence_after();
       const uint32_t d = tmem_base + kDB + (uint32_t)(tb * 128);
       const uint64_t b0 = dWd + (uint64_t)((wslot * kWdGroupBytes) >> 4);
@@ -354,7 +278,7 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
               umma_bf16(d, a0 + (uint64_t)(kc * 1024 + k * 2), b0 + (uint64_t)(kc * 1024 + k * 2), idesc_b,
                         (uint32_t)((g | kc | k) != 0));
         }
-        if (!p.wd_resident) umma_commit(&wd_empty[wslot]);
+        umma_commit(&wd_empty[wslot]);
         if (HAS_TRAN) umma_commit(h_empty);
         else umma_commit(&empty_bar[s]);
         if (g == 3) umma_commit(&db_full[tb]);
@@ -388,31 +312,23 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
     // every tile needs the 128 KB of 8x8-s4 weights once, 32 KB per sub-position group; all SMs
     // stream the same bytes, so these are L2 hits.  A 2-deep ring instead of a resident copy frees
     // 64 KB of shared memory for the activation pipeline (HBM latency hiding).
-    if (p.wd_resident) {
-      if (elect_one()) {
-        mbar_expect_tx(&wd_full[0], 4 * kWdGroupBytes);
-        for (int kc = 0; kc < 8; ++kc) tma_load_2d(s_wd + kc * 16384, &p.wd_map, &wd_full[0], kc * 64, 0);
-      }
-    } else {
-      uint32_t n_wd = 0;
-      for (int tile = cta; tile < total_tiles; tile += ncta)
-        for (int g = 0; g < 4; ++g) {
-          const int slot = n_wd & 1;
-          mbar_wait(&wd_empty[slot], ((n_wd >> 1) & 1) ^ 1);
-          if (elect_one()) {
-            mbar_expect_tx(&wd_full[slot], kWdGroupBytes);
-            tma_load_2d(s_wd + slot * kWdGroupBytes, &p.wd_map, &wd_full[slot], (2 * g) * 64, 0);
-            tma_load_2d(s_wd + slot * kWdGroupBytes + 16384, &p.wd_map, &wd_full[slot], (2 * g + 1) * 64, 0);
-          }
-          __syncwarp();
-          ++n_wd;
+    uint32_t n_wd = 0;
+    for (int tile = cta; tile < total_tiles; tile += ncta)
+      for (int g = 0; g < 4; ++g) {
+        const int slot = n_wd & 1;
+        mbar_wait(&wd_empty[slot], ((n_wd >> 1) & 1) ^ 1);
+        if (elect_one()) {
+          mbar_expect_tx(&wd_full[slot], kWdGroupBytes);
+          tma_load_2d(s_wd + slot * kWdGroupBytes, &p.wd_map, &wd_full[slot], (2 * g) * 64, 0);
+          tma_load_2d(s_wd + slot * kWdGroupBytes + 16384, &p.wd_map, &wd_full[slot], (2 * g + 1) * 64, 0);
         }
-    }
+        __syncwarp();
+        ++n_wd;
+      }
   } else if (warp >= 2 && warp < 2 + kFusedEpiWarps) {
     // ===================== epilogue warps 2..17 =====================
     // warp -> TMEM lane quarter q = warp % 4 (hardware rule) and sub = which of the 4 column groups
     // (phase A: sub-position within the group; final: tap) this warp handles
-    griddep_wait();     // the partial-sum slots are read by the previous finalize launch
     const int q = warp & 3;
     const int sub = (warp - 2) >> 2;
     const int row = q * 32 + lane;
@@ -509,21 +425,21 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
         float below[8];
 #pragma unroll
         for (int k = 0; k < 8; ++k) below[k] = __shfl_down_sync(0xffffffffu, comb[1][k], 16);
-        if (p.xchg && half == 0 && q > 0) {
+        if (half == 0 && q > 0) {
           float4* x = s_x + (((q - 1) * 4 + sub) * 16 + xl) * 2;
           x[0] = make_float4(comb[1][0], comb[1][1], comb[1][2], comb[1][3]);
           x[1] = make_float4(comb[1][4], comb[1][5], comb[1][6], comb[1][7]);
         }
-        if (p.xchg) asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");     // the 16 epilogue warps only
-        if (p.xchg && half == 1 && q < 3) {
+        asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");     // the 16 epilogue warps only
+        if (half == 1 && q < 3) {
           const float4* x = s_x + ((q * 4 + sub) * 16 + xl) * 2;
           const float4 x0v = x[0], x1v = x[1];
           below[0] = x0v.x; below[1] = x0v.y; below[2] = x0v.z; below[3] = x0v.w;
           below[4] = x1v.x; below[5] = x1v.y; below[6] = x1v.z; below[7] = x1v.w;
         }
-        if (p.xchg) asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");     // reads done before the next tile's writes
+        asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");     // reads done before the next tile's writes
         const int rr = 2 * q + half;                                               // block row inside the tile
-        if ((p.xchg ? rr < 7 : half == 0) && xl < 15 && in_tensor && Yb < p.lr_h && Xb < p.lr_w) {   // interior pixel (Yb, Xb)
+        if (rr < 7 && xl < 15 && in_tensor && Yb < p.lr_h && Xb < p.lr_w) {   // interior pixel (Yb, Xb)
           const float slope = s_down[32];
           float r[8];
 #pragma unroll
@@ -536,8 +452,8 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
         for (int dy = 0; dy < 2; ++dy) {
           const int Y = Yb - dy;
           if (in_tensor && Y >= 0 && Y < p.lr_h) {
-            // row 7 of a tile (without the exchange: every odd row), or the tile's last column
-            const bool boundary = (p.xchg ? (((rr - dy) & 7) == 7) : (((rr - dy) & 1) == 1)) || (xl == 15);
+            // row 7 of a tile, or the tile's last column
+            const bool boundary = (((rr - dy) & 7) == 7) || (xl == 15);
             if (Xb < p.lr_w && boundary) {
               float4* dst = reinterpret_cast<float4*>(p.part + ((((int64_t)b * p.lr_h + Y) * p.lr_w + Xb) * 4 + 2 * dy) * 32 + sub * 8);
               dst[0] = make_float4(comb[dy][0], comb[dy][1], comb[dy][2], comb[dy][3]);
@@ -556,9 +472,6 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
       if (warp == 2 && lane == 0) VSR_TRACE(26);                                  // final epilogue of the tile done
       ++m_b[tb];
       tb ^= 1;
-      // group launch: progress counter the deconv role throttles on (this warp has read the tile's accumulators, so
-      // every load of the tile has long been consumed)
-      if (gs != nullptr && warp == 2 && lane == 0) red_release_gpu_add(gs->fused_done, 1);
     }
   }
 
@@ -570,40 +483,17 @@ __device__ __forceinline__ void fused_body(const FusedDownParams& p, const int c
   }
 }
 
-template <bool HAS_TRAN>
-__global__ void __launch_bounds__(kFusedThreads, 1)
-fused_down_kernel(const __grid_constant__ FusedDownParams p) {
-  fused_body<HAS_TRAN>(p, (int)blockIdx.x, (int)gridDim.x, nullptr);
-}
-
-// One launch for a feedback group's up-projection AND its HR half: CTAs [0, n_deconv) run the transposed conv
-// (igemm_body<EPI_DECONV>) and write hr[i]; the remaining CTAs run the fused downtran + strided conv over hr[0..i] in the
-// same tile order, a few hundred tiles behind, and find hr[i]'s tile in L2 (SURVEY.md 8 a6; SRProjectionModule.py:
-// 62-65 then :70-80).  Launched as two kernels every hr[i] is written to and read back from HBM: 6 of the 34 HR-map
-// transfers of a feedback step.  The roles also complement each other: alone, the deconv is bound by TMEM reads /
-// shared-memory traffic at 0.7 of the write bandwidth while the fused kernel is bound by HBM reads.
-template <bool HAS_TRAN>
-__global__ void __launch_bounds__(kFusedThreads, 1)
-group_kernel(const __grid_constant__ IgemmParams dp, const __grid_constant__ FusedDownParams fp,
-             const __grid_constant__ GroupSync gs) {
-  static_assert(kFusedThreads >= kDeconvThreads, "the launch is as wide as the wider role");
-  if ((int)blockIdx.x < gs.n_deconv)
-    igemm_body<EPI_DECONV, 32, 256>(dp, (int)blockIdx.x, gs.n_deconv, &gs);
-  else
-    fused_body<HAS_TRAN>(fp, (int)blockIdx.x - gs.n_deconv, (int)gridDim.x - gs.n_deconv, &gs);
-}
-
-// Boundary pixels (rows Y % 8 == 7 -- period 8; odd rows without the exchange -- period 2; columns X % 16 == 15;
-// see the fused kernel's final epilogue):
+// Boundary pixels (rows Y % 8 == 7 and columns X % 16 == 15; see the fused kernel's final epilogue):
 // lr_out[p, c] = bf16(PReLU(sum of the pixel's partial slots + bias[c])).  8 channels per thread.
 // Deterministic: every slot has one writer, the sum order is fixed.
+constexpr int kFinalizePeriod = 8;   // boundary rows: one per 8-row tile
 __global__ void __launch_bounds__(256)
 finalize_lr_kernel(const float4* __restrict__ part, const float* __restrict__ bias, uint4* __restrict__ out, int B, int h,
-                   int w, int period) {
+                   int w) {
   // Work items = boundary pixels only, enumerated arithmetically (the first version walked every pixel and skipped
-  // the interior ones): first the full rows Y = period*k + period-1, then, in the other rows, the columns X = 16*j + 15.
+  // the interior ones): first the full rows Y = 8*k + 7, then, in the other rows, the columns X = 16*j + 15.
+  constexpr int period = kFinalizePeriod;
   const float slope = __ldg(bias + 32);
-  griddep_wait();
   const int R = h / period, Cc = w / 16;
   const int64_t nA = (int64_t)B * R * w, nB = (int64_t)B * (h - R) * Cc;
   const int64_t n8 = (nA + nB) * 4;

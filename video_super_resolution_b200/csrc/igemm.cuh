@@ -413,63 +413,9 @@ inline size_t igemm_smem_bytes(int num_chunks, size_t ring_bytes, int extra = 0)
   return 1024 /*align slack*/ + b + ring_bytes + 1024 /*barriers + bias*/ + 2048 + extra;
 }
 
-
-// ------------------------------------------------------------------------------------------------
-// Producer -> consumer hand-off between two ROLES of one launch (group_kernel, fused_down.cuh): the CTAs of the
-// deconv role write hr[i] tile by tile and publish each tile; the CTAs of the fused-down role consume hr[0..i] in the
-// same tile order and take the newest map out of L2 instead of HBM.  All CTAs of the launch are co-resident (one per
-// SM, cooperative launch attribute), producers never wait for consumers' data -- only for their progress counter, a
-// throttle that keeps the published-but-unconsumed tiles inside the L2 -- so the waits cannot deadlock.  Every spin
-// is bounded: after kSpinLimit probes the waiter raises `error` and carries on (wrong output, reported by the host,
-// instead of a hung GPU).
-// ------------------------------------------------------------------------------------------------
-struct GroupSync {
-  int32_t* tile_flags;     // [spatial tiles]: += 1 per finished (epilogue warp, N half) store; complete at 32 * epoch
-  int32_t* fused_done;     // [1]: tiles the fused role has finished in this launch, + base
-  int32_t* error;          // [1]: set to 1 by a waiter that gave up
-  int32_t epoch;           // launch number since the flags were last zeroed (1-based)
-  int32_t done_base;       // value of *fused_done when this launch starts
-  int32_t n_deconv;        // CTAs [0, n_deconv) run the deconv role, the others the fused-down role
-  int32_t window;          // the deconv role stays at most this many tiles ahead of fused_done
-};
-constexpr uint32_t kSpinLimit = 1u << 22;      // x ~100-200 ns per probe: a second or so
-
-__device__ __forceinline__ int32_t ld_acquire_gpu(const int32_t* p) {
-  int32_t v;
-  asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ void red_release_gpu_add(int32_t* p, int32_t v) {
-  asm volatile("red.release.gpu.global.add.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-// generic <-> async proxy ordering for global memory written / read by TMA
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
-__device__ __forceinline__ void spin_until_ge(const int32_t* p, int32_t target, int32_t* error) {
-  uint32_t n = 0;
-  while (ld_acquire_gpu(p) < target) {
-    __nanosleep(64);
-    // once anybody has given up everybody stops waiting: the launch ends quickly (its output is lost either way)
-    if (++n > kSpinLimit || *reinterpret_cast<volatile int32_t*>(error) != 0) {
-      *reinterpret_cast<volatile int32_t*>(error) = 1;
-      break;
-    }
-  }
-}
-// L2 eviction-priority hints for TMA loads (the encodings cuTensorMap / CUTLASS use for createpolicy results)
-constexpr uint64_t kL2EvictFirst = 0x12F0000000000000ull, kL2EvictLast = 0x14F0000000000000ull;
-__device__ __forceinline__ void tma_load_4d_hint(void* smem_dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1,
-                                                 int c2, int c3, uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%3, %4, %5, %6}], [%2], %7;" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "l"(policy)
-      : "memory");
-}
-
-// The kernel body as a device function: igemm_kernel runs it over the whole grid; group_kernel (fused_down.cuh) runs
-// the EPI_DECONV instance on CTAs [0, n_deconv) of its grid, with the tile hand-off `gs`.
 template <int MODE, int CK, int BN>
-__device__ __forceinline__ void igemm_body(const IgemmParams& p, const int cta, const int ncta, const GroupSync* gs) {
+__global__ void __launch_bounds__(igemm_threads(MODE), 1)
+igemm_kernel(const __grid_constant__ IgemmParams p) {
   constexpr int kThreadsHere = igemm_threads(MODE);
   constexpr int kEpiThreads = kThreadsHere - 64;
   static_assert(CK == 32 || CK == 64, "K chunk is 32 (64B swizzle) or 64 (128B swizzle) BF16");
@@ -501,11 +447,11 @@ __device__ __forceinline__ void igemm_body(const IgemmParams& p, const int cta, 
   float* s_bias = reinterpret_cast<float*>(tail + 512);            // up to 384 floats
   uint8_t* s_stage = tail + 2048;                                  // EPI_DECONV store staging (64 KB)
 
+  const int cta = blockIdx.x, ncta = gridDim.x;   // persistent CTAs: tiles cta, cta + ncta, ...
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int total_tiles = p.n_tiles * p.tiles_x * p.tiles_y * p.batch;
 
-  // (no early griddepcontrol.launch_dependents: dependents are released as CTAs exit)
   if (threadIdx.x == 0) {
     for (int s = 0; s < p.num_stages; ++s) {
       mbar_init(&full_bar[s], 1);
@@ -537,15 +483,12 @@ __device__ __forceinline__ void igemm_body(const IgemmParams& p, const int cta, 
           tma_load_2d(smem_b + kc * kBBytes, &p.b_map, b_full, kc * CK, n_tile0 * BN);
       }
       __syncwarp();
-      griddep_wait();   // weights are static; activations only after the previous layers have completed
       int s = 0;
       uint32_t phase = 0;
       TileWalk walk;
       walk.init(p, cta, ncta);
       for (int tile = cta; tile < total_tiles; tile += ncta, walk.next(p)) {
         const TileCoord t = walk.coord(p);
-        if (MODE == EPI_DECONV && gs != nullptr)     // stay within `window` tiles of the consumer role: what is
-          spin_until_ge(gs->fused_done, gs->done_base + tile / p.n_tiles - gs->window, gs->error);   // published stays in L2
         for (int kc0 = 0; kc0 < p.num_chunks; kc0 += p.cps) {
           const int nk = min(p.cps, p.num_chunks - kc0);
           mbar_wait(&empty_bar[s], phase ^ 1);
@@ -652,12 +595,10 @@ __device__ __forceinline__ void igemm_body(const IgemmParams& p, const int cta, 
     }
   } else if (warp < 2 + kEpiThreads / 32) {
     // ===================== epilogue (warps 2..5; 2..17 for EPI_DECONV) =====================
-    griddep_wait();                         // output buffers may still be read by earlier layers
     const int q = warp & 3;                 // TMEM lane quarter this warp may read
     const int row = q * 32 + lane;          // row of the 128-pixel tile
     int as = 0;
     uint32_t acc_phase = 0;
-    int prev_tile = -1;                     // EPI_DECONV group launch: the tile whose store is still in flight
     TileWalk walk;
     walk.init(p, cta, ncta);
     for (int tile = cta; tile < total_tiles; tile += ncta, walk.next(p)) {
@@ -771,15 +712,7 @@ __device__ __forceinline__ void igemm_body(const IgemmParams& p, const int cta, 
             convert32(v, s_bias, pc, o);
             if (__builtin_expect(!inside, 0)) zero16(o);   // ring positions (tile border only) stay zero
             if (c2 == 0) {   // the previous tile's store must have read the staging tile before it is overwritten
-              if (elect_one()) {                      // (waited for here, after the TMEM read + conversion, not before)
-                if (gs != nullptr && prev_tile >= 0) {   // group launch: the store must have COMPLETED; publish the tile
-                  asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-                  fence_proxy_async_all();
-                  red_release_gpu_add(gs->tile_flags + prev_tile, 1);
-                } else {
-                  tma_store_wait_read();
-                }
-              }
+              if (elect_one()) tma_store_wait_read();   // (waited for here, after the TMEM read + conversion, not before)
               __syncwarp();
             }
             uint8_t* srow = stg + lane * 128;
@@ -800,7 +733,6 @@ __device__ __forceinline__ void igemm_body(const IgemmParams& p, const int cta, 
               tma_store_4d(&p.out_map, stg, 0, t.x0, t.y0 + 2 * q, t.b * 8 + t.n_tile * 4 + sub);
             tma_store_commit();
           }
-          prev_tile = tile / p.n_tiles;     // spatial tile index (both N halves publish into the same flag)
         }
       } else if constexpr (MODE == EPI_DECONV2) {
         // ConvTranspose2d k6 s2 p2 (SRFBN's x2 geometry): row = LR pixel (Y,X), the 3x3 LR taps are the
@@ -933,13 +865,7 @@ __device__ __forceinline__ void igemm_body(const IgemmParams& p, const int cta, 
     }
     __syncwarp();
     if (MODE == EPI_DECONV2 && elect_one()) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-    if (MODE == EPI_DECONV && elect_one()) {
-      asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");      // the last tile's store
-      if (gs != nullptr && prev_tile >= 0) {
-        fence_proxy_async_all();
-        red_release_gpu_add(gs->tile_flags + prev_tile, 1);
-      }
-    }
+    if (MODE == EPI_DECONV && elect_one()) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // the last tile's store
   }
 
   tc_fence_before();
@@ -948,12 +874,6 @@ __device__ __forceinline__ void igemm_body(const IgemmParams& p, const int cta, 
     tc_fence_after();
     tmem_dealloc<kTmemCols>(tmem_base);
   }
-}
-
-template <int MODE, int CK, int BN>
-__global__ void __launch_bounds__(igemm_threads(MODE), 1)
-igemm_kernel(const __grid_constant__ IgemmParams p) {
-  igemm_body<MODE, CK, BN>(p, (int)blockIdx.x, (int)gridDim.x, nullptr);
 }
 
 }  // namespace vsr

@@ -370,7 +370,7 @@ projection_pipeline_kernel(const ProjArgs a) {
 // are launched with programmatic stream serialization -- the next stage's CTAs may become resident while the last CTAs
 // of this one drain -- and every stage starts by letting its successor launch and then waiting for its predecessor to
 // have completed and flushed (griddepcontrol.wait).  (The layers of the conv stack, 0.1-2 ms each, measured no gain
-// from this: api.cu.)
+// from this: DESIGN.md section 6.)
 __device__ __forceinline__ void chain_enter() {
   griddep_launch_dependents();
   griddep_wait();

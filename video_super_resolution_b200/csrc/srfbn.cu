@@ -90,11 +90,11 @@ int make_w_map(CUtensorMap* m, const void* base, int64_t K, int64_t N, int ck, i
 // ------------------------------------------------------------------------------------------------
 // kernel variants
 // ------------------------------------------------------------------------------------------------
-enum Variant : int { V_PW32 = 0, V_PW128, V_DECONV, V_CONVOUT, V_FUSED_TRAN, V_FUSED_PLAIN, V_FINALIZE, V_DECONV2, V_GROUP_TRAN, V_GROUP_PLAIN, V_DOWN2, V_COUNT };
+enum Variant : int { V_PW32 = 0, V_PW128, V_DECONV, V_CONVOUT, V_FUSED_TRAN, V_FUSED_PLAIN, V_FINALIZE, V_DECONV2, V_DOWN2, V_COUNT };
 
 // kernel classes for the per-launch accounting bench.py reads (vsr_srfbn_profile_*)
-static_assert(VSR_SRFBN_KERNEL_CLASSES == 11, "header constant");
-enum KClass : int { KC_IM2COL = 0, KC_CONV_IN, KC_PW_LR, KC_PW_HR, KC_DECONV, KC_DOWNCONV, KC_CONV_OUT, KC_FC, KC_FUSED_DOWN, KC_FINALIZE, KC_GROUP, KC_COUNT };
+static_assert(VSR_SRFBN_KERNEL_CLASSES == 10, "header constant");
+enum KClass : int { KC_IM2COL = 0, KC_CONV_IN, KC_PW_LR, KC_PW_HR, KC_DECONV, KC_DOWNCONV, KC_CONV_OUT, KC_FC, KC_FUSED_DOWN, KC_FINALIZE, KC_COUNT };
 
 struct Layer {
   int variant;
@@ -104,9 +104,7 @@ struct Layer {
   const float* fin_bias;
   void* fin_out;
   int64_t fin_n8;
-  int fin_w, fin_h, fin_b, fin_period;   // fin_period: 8 (rows Y % 8 == 7) or 2 (odd rows), matching the fused kernel's xchg mode
-  GroupSync gs;          // V_GROUP_*: p = the deconv role, f = the fused-down role
-  int group_index;       // V_GROUP_*: i of the feedback group (selects the role split)
+  int fin_w, fin_h, fin_b;
   int grid;
   size_t smem;
   int kclass;
@@ -114,25 +112,9 @@ struct Layer {
   double bytes;   // compulsory HBM bytes of this launch: its inputs + outputs, each once
 };
 
-// VSR_GROUP=1: run a group's transposed conv and its fused down kernel as two ROLES of one launch (group_kernel), hr[i]
-// handed over through L2.  Off by default: measured on B200 at C2 it is SLOWER (48.8 vs 44.0 ms per pass for the 19 + 18
-// launches it replaces; profiles/group_launch_r02.log).  The fused kernel streams at ~38 GB/s per SM -- what ~112 KB of
-// TMA boxes in flight per SM yield at the loaded HBM latency -- so it only reaches the HBM roof with all 148 SMs pulling;
-// giving 30-116 SMs to the deconv role costs more read bandwidth than the L2 hits of the newest map return.  Kept
-// (bit-identical to the two launches, tests/test_srfbn_gpu.py) as the measured answer to "hand hr[i] over through L2".
 #ifdef VSR_KNOCKOUT
 long long* g_trace_buf = nullptr;
 #endif
-
-int group_enabled() {
-  const char* e = getenv("VSR_GROUP");
-  return e ? (atoi(e) != 0) : 0;
-}
-
-int fused_xchg() {   // tuning knob, see FusedDownParams::xchg
-  const char* e = getenv("VSR_FUSED_XCHG");
-  return e ? (atoi(e) != 0) : 1;
-}
 
 template <int MODE, int CK, int BN>
 int launch_variant(const Layer& L, cudaStream_t st) {
@@ -144,9 +126,7 @@ int launch_variant(const Layer& L, cudaStream_t st) {
     if (e != cudaSuccess) return cuda_status(e);
     once.mark(dev);
   }
-  cudaError_t e = launch_pdl(igemm_kernel<MODE, CK, BN>, L.grid, igemm_threads(MODE),
-                             L.smem, st, L.p);
-  if (e != cudaSuccess) return cuda_status(e);
+  igemm_kernel<MODE, CK, BN><<<L.grid, igemm_threads(MODE), L.smem, st>>>(L.p);
   return after_launch();
 }
 
@@ -160,50 +140,22 @@ int launch_fused(const Layer& L, cudaStream_t st) {
     if (e != cudaSuccess) return cuda_status(e);
     once.mark(dev);
   }
-  cudaError_t e = launch_pdl(fused_down_kernel<HAS_TRAN>, L.grid, kFusedThreads, L.smem, st, L.f);
-  if (e != cudaSuccess) return cuda_status(e);
-  return after_launch();
-}
-
-template <bool HAS_TRAN>
-int launch_group(const Layer& L, cudaStream_t st) {
-  static PerDeviceOnce once;
-  int dev;
-  if (once.needed(&dev)) {
-    cudaError_t e = cudaFuncSetAttribute(group_kernel<HAS_TRAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    if (e != cudaSuccess) return cuda_status(e);
-    once.mark(dev);
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)L.grid, 1, 1);
-  cfg.blockDim = dim3((unsigned)kFusedThreads, 1, 1);
-  cfg.dynamicSmemBytes = L.smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeCooperative;     // all CTAs co-resident or the launch fails: the roles wait on each other
-  attr[0].val.cooperative = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, group_kernel<HAS_TRAN>, L.p, L.f, L.gs);
-  if (e != cudaSuccess) return cuda_status(e);
+  fused_down_kernel<HAS_TRAN><<<L.grid, kFusedThreads, L.smem, st>>>(L.f);
   return after_launch();
 }
 
 int launch_layer(const Layer& L, cudaStream_t st) {
   switch (L.variant) {
-    case V_GROUP_TRAN: return launch_group<true>(L, st);
-    case V_GROUP_PLAIN: return launch_group<false>(L, st);
     case V_FUSED_TRAN: return launch_fused<true>(L, st);
     case V_FUSED_PLAIN: return launch_fused<false>(L, st);
     case V_FINALIZE: {
-      const int R = L.fin_h / L.fin_period;
+      const int R = L.fin_h / kFinalizePeriod;
       const int64_t items = ((int64_t)L.fin_b * R * L.fin_w + (int64_t)L.fin_b * (L.fin_h - R) * (L.fin_w / 16)) * 4;
       if (items == 0) return VSR_OK;
       int64_t blocks = ceil_div64(items, 256);
       if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
-      cudaError_t e = launch_pdl(finalize_lr_kernel, (int)blocks, 256, 0, st, reinterpret_cast<const float4*>(L.fin_acc),
-                                 L.fin_bias, reinterpret_cast<uint4*>(L.fin_out), L.fin_b, L.fin_h, L.fin_w, L.fin_period);
-      if (e != cudaSuccess) return cuda_status(e);
+      finalize_lr_kernel<<<(int)blocks, 256, 0, st>>>(reinterpret_cast<const float4*>(L.fin_acc), L.fin_bias,
+                                                      reinterpret_cast<uint4*>(L.fin_out), L.fin_b, L.fin_h, L.fin_w);
       return after_launch();
     }
     case V_PW32: return launch_variant<EPI_ROWS, 32, 32>(L, st);
@@ -344,15 +296,12 @@ int build_deconv(Layer& L, const void* x, int B, int h, int w, const void* w_dev
   p.lr_h = h;
   p.lr_w = w;
   p.deconv_nhwc = nhwc;
-  {
-    const char* e = nullptr;
 #ifdef VSR_KNOCKOUT
-    e = getenv("VSR_DECONV_DEBUG");
+  {
+    const char* e = getenv("VSR_DECONV_DEBUG");
     p.debug = e ? atoi(e) : 0;
-#endif
-    e = getenv("VSR_DECONV_STAGES");     // tuning knob: ring depth (18 KB per stage)
-    if (e && atoi(e) >= 1 && atoi(e) <= 5) p.num_stages = atoi(e);
   }
+#endif
   if (!nhwc) {
     EncodeTiledFn enc = encode_fn();
     if (!enc) return VSR_ERR_STATE;
@@ -532,10 +481,6 @@ int build_fused_down(Layer& L, const void* const* hr, int nsrc, int B, int h, in
   f.batch = B;
   f.lr_h = h;
   f.lr_w = w;
-  {
-    const char* e = getenv("VSR_PREFETCH_AHEAD");   // tuning knob (half-tiles of L2 prefetch distance)
-    f.prefetch_ahead = e ? atoi(e) : 0;   // measured: hurts (strided 64 B boxes over-fetch), see DESIGN.md
-  }
 #ifdef VSR_KNOCKOUT
   {
     const char* e = getenv("VSR_FUSED_DEBUG");
@@ -550,27 +495,15 @@ int build_fused_down(Layer& L, const void* const* hr, int nsrc, int B, int h, in
     }
   }
 #endif
-  {
-    const char* e = getenv("VSR_FUSED_STAGES");
-    if (e && atoi(e) > 0 && atoi(e) <= (tran ? 7 : 5)) f.num_stages = atoi(e);
-  }
-  f.xchg = fused_xchg();
   f.tran_bias = tran_bias_dev;
   f.down_bias = down_bias_dev;
   f.part = part;
   f.lr_out = lr_out;
-  {
-    // measured on B200 (C2 shape, nsrc = 6): weights resident + 3 x 16 KB activation stages 3.73 ms,
-    // weights streamed per group from L2 + 7 stages 3.22 ms -> streaming is the default
-    const char* e = getenv("VSR_FUSED_WD_RESIDENT");
-    f.wd_resident = e ? atoi(e) : 0;
-    if (f.wd_resident) f.num_stages = tran ? 3 : 2;
-  }
-  while (f.num_stages > 2 && (tran ? fused_down_smem_bytes<true>(nsrc, f.num_stages, f.wd_resident, f.xchg)
-                                   : fused_down_smem_bytes<false>(nsrc, f.num_stages, f.wd_resident, f.xchg)) > 227 * 1024)
+  // the deepest ring that fits: 4 stages for nsrc 1, 7 for nsrc 2-5, 6 for nsrc 6
+  while (f.num_stages > 2 && (tran ? fused_down_smem_bytes<true>(nsrc, f.num_stages)
+                                   : fused_down_smem_bytes<false>(nsrc, f.num_stages)) > 227 * 1024)
     --f.num_stages;
-  L.smem = tran ? fused_down_smem_bytes<true>(nsrc, f.num_stages, f.wd_resident, f.xchg)
-                : fused_down_smem_bytes<false>(nsrc, f.num_stages, f.wd_resident, f.xchg);
+  L.smem = tran ? fused_down_smem_bytes<true>(nsrc, f.num_stages) : fused_down_smem_bytes<false>(nsrc, f.num_stages);
   int64_t total = (int64_t)f.tiles_x * f.tiles_y * B;
   L.grid = (int)(total < kNumSMs ? total : kNumSMs);
   const double lrpx = (double)B * h * w;
@@ -590,58 +523,9 @@ int build_finalize(Layer& L, float* acc, const float* bias_dev, void* out, int64
   L.fin_w = w;
   L.fin_h = h;
   L.fin_b = (int)(pixels / ((int64_t)h * w));
-  L.fin_period = fused_xchg() ? 8 : 2;
   L.kclass = KC_FINALIZE;
   L.flops = 0;
   L.bytes = 0;   // the boundary-pixel pass moves no compulsory bytes (its pixels' output is counted in the fused launch)
-  return VSR_OK;
-}
-
-// Co-scheduled group launch (group_kernel): `d` = the group's deconv layer, `f` = its fused-down layer, both already
-// built.  Role split: the deconv role needs ~3.9 CTA-us per spatial tile (both N halves), the fused role ~0.7 (i = 0, its
-// only map comes from L2) to ~16 (i = 5) once the newest map is an L2 hit; n_deconv is the even number of CTAs that
-// balances the two (tunable: VSR_GROUP_ND="n0,n1,..,n5").
-int group_deconv_ctas(int i) {
-  static const int dflt[6] = {116, 64, 50, 42, 36, 30};
-  int nd = dflt[i < 0 ? 0 : (i > 5 ? 5 : i)];
-  if (const char* e = getenv("VSR_GROUP_ND")) {
-    int k = 0;
-    for (const char* q = e; *q && k <= i; ++k) {
-      const int v = atoi(q);
-      if (k == i && v >= 2) nd = v;
-      while (*q && *q != ',') ++q;
-      if (*q == ',') ++q;
-    }
-  }
-  nd &= ~1;
-  if (nd < 2) nd = 2;
-  if (nd > kNumSMs - 2) nd = kNumSMs - 2;
-  return nd;
-}
-
-int build_group(Layer& L, const Layer& d, const Layer& f, int group_index, int32_t* flags, int32_t epoch, int32_t n_spatial) {
-  memset(&L, 0, sizeof(L));
-  L.variant = f.variant == V_FUSED_TRAN ? V_GROUP_TRAN : V_GROUP_PLAIN;
-  L.p = d.p;
-  L.f = f.f;
-  L.group_index = group_index;
-  L.grid = kNumSMs;
-  L.smem = d.smem > f.smem ? d.smem : f.smem;
-  L.gs.tile_flags = flags + 64;          // [0] fused_done, [1] error, then the per-tile flags
-  L.gs.fused_done = flags;
-  L.gs.error = flags + 1;
-  L.gs.epoch = epoch;
-  L.gs.done_base = (epoch - 1) * n_spatial;
-  L.gs.n_deconv = group_deconv_ctas(group_index);
-  {
-    const char* e = getenv("VSR_GROUP_WINDOW");
-    L.gs.window = e && atoi(e) > 0 ? atoi(e) : kNumSMs + 64;
-  }
-  L.kclass = KC_GROUP;
-  L.flops = d.flops + f.flops;
-  // compulsory HBM bytes of the pair: LR in, hr[i] out (write-back), hr[0..i-1] in, LR out; hr[i] is not read back
-  const double lrpx = (double)d.p.batch * d.p.lr_h * d.p.lr_w;
-  L.bytes = d.bytes + f.bytes - lrpx * 64.0 * 16.0;
   return VSR_OK;
 }
 
@@ -809,7 +693,6 @@ fc_fuse_kernel(const float* __restrict__ maps, const float* __restrict__ fcw, fl
   __shared__ float s_w[32 * kMaxMaps + 65];
   const int nw = 32 * M + 65;
   for (int i = threadIdx.x; i < nw; i += blockDim.x) s_w[i] = fcw[i];
-  griddep_wait();   // weights above are static; the per-map images come from the previous launch
   __syncthreads();
   const float* w0 = s_w;
   const float* b0 = s_w + 32 * M;
@@ -909,8 +792,7 @@ struct vsr_srfbn_plan {
   size_t misc_off;        // fp32: sub_mean bias (3)
   size_t weight_bytes;
   // workspace offsets
-  size_t o_a0, o_c128, o_xfeat, o_hidden, o_lr[7], o_u, o_hr[6], o_hb, o_ht, o_acc, o_premix, o_flags, flags_bytes, ws_bytes;
-  bool grouped;           // group launches in the layer list: the flags are zeroed at the start of every forward
+  size_t o_a0, o_c128, o_xfeat, o_hidden, o_lr[7], o_u, o_hr[6], o_hb, o_ht, o_acc, o_premix, ws_bytes;
   int chunk_maps;         // maps processed per sweep over the layer list (a divisor of num_maps; == num_maps: no chunking)
   size_t ws_cap;          // caller's workspace cap in bytes (0 = none)
   bool bound;
@@ -922,7 +804,6 @@ struct vsr_srfbn_plan {
   // fewer maps; built by vsr_srfbn_prepare_refresh
   std::vector<Layer> refresh_layers;
   int refresh_first, refresh_conv_out_layer;
-  bool refresh_grouped;
   bool premix_valid;      // a full forward has filled the per-map images of every map
   std::vector<cudaEvent_t> events;   // profiling: one before every launch + one after the last
   bool profile;
@@ -981,9 +862,6 @@ static void layout_workspace(vsr_srfbn_plan* pl) {
   pl->o_ht = put(x2 ? P * s2 * 64 : 0);   // x2: downtran result (the x4 path keeps it on chip)
   pl->o_acc = put(x2 ? 0 : P * 512);   // fp32 partial slots of the fused down kernel
   pl->o_premix = put((size_t)c.num_maps * c.h * c.w * s2 * 3 * 4);
-  // hand-off flags of the group launches: fused_done, error, one counter per 16 x 8-block tile
-  pl->flags_bytes = x2 ? 0 : (64 + (size_t)pl->chunk_maps * ceil_div(c.h + 1, 8) * ceil_div(c.w + 1, 16)) * 4;
-  pl->o_flags = put(pl->flags_bytes);
   pl->ws_bytes = off;
 }
 
@@ -1005,7 +883,6 @@ extern "C" int vsr_srfbn_plan_create(const vsr_srfbn_config* cfg, vsr_srfbn_plan
   pl->conv_out_layer = -1;
   pl->refresh_first = -1;
   pl->refresh_conv_out_layer = -1;
-  pl->refresh_grouped = false;
   pl->premix_valid = false;
   pl->profile = false;
   pl->chunk_maps = cfg->num_maps;
@@ -1105,7 +982,7 @@ extern "C" int vsr_srfbn_pack_weights(const vsr_srfbn_plan* pl, const vsr_srfbn_
   return VSR_OK;
 }
 
-static int build_layer_list(vsr_srfbn_plan* pl, int M, std::vector<Layer>& layers, int& conv_out_layer, bool& grouped);
+static int build_layer_list(vsr_srfbn_plan* pl, int M, std::vector<Layer>& layers, int& conv_out_layer);
 
 extern "C" int vsr_srfbn_bind(vsr_srfbn_plan* pl, const void* dev_weights, void* dev_workspace,
                               size_t workspace_bytes) {
@@ -1119,7 +996,7 @@ extern "C" int vsr_srfbn_bind(vsr_srfbn_plan* pl, const void* dev_weights, void*
   pl->refresh_layers.clear();
   pl->refresh_first = -1;
   pl->premix_valid = false;
-  int rc = build_layer_list(pl, pl->chunk_maps, pl->layers, pl->conv_out_layer, pl->grouped);
+  int rc = build_layer_list(pl, pl->chunk_maps, pl->layers, pl->conv_out_layer);
   if (rc) return rc;
   pl->bound = true;
   return VSR_OK;
@@ -1127,7 +1004,7 @@ extern "C" int vsr_srfbn_bind(vsr_srfbn_plan* pl, const void* dev_weights, void*
 
 // The layer list of the stack for M maps at a time (M <= chunk_maps: the buffers are laid out for chunk_maps maps and a
 // list over fewer maps uses their heads).
-static int build_layer_list(vsr_srfbn_plan* pl, int M, std::vector<Layer>& layers, int& conv_out_layer, bool& grouped) {
+static int build_layer_list(vsr_srfbn_plan* pl, int M, std::vector<Layer>& layers, int& conv_out_layer) {
   layers.clear();
   const vsr_srfbn_config& c = pl->cfg;
   const int h = c.h, w = c.w;
@@ -1137,8 +1014,6 @@ static int build_layer_list(vsr_srfbn_plan* pl, int M, std::vector<Layer>& layer
   auto Bp = [&](int id) { return reinterpret_cast<const float*>(pl->dev_w + pl->we[id].b_off); };
   int rc;
   Layer L;
-  int32_t group_epoch = 0;
-  grouped = false;
 #define PUSH(expr)        \
   do {                    \
     rc = (expr);          \
@@ -1194,17 +1069,8 @@ static int build_layer_list(vsr_srfbn_plan* pl, int M, std::vector<Layer>& layer
                               i > 0 ? Bp(W_DOWNTRAN0 + i - 1) : nullptr, Wp(W_DOWN0 + i), Bp(W_DOWN0 + i),
                               reinterpret_cast<float*>(ws + pl->o_acc), ws + pl->o_lr[i + 1]);
         if (rc) return rc;
-        const int n_spatial = M * F.f.tiles_x * F.f.tiles_y;
-        if (group_enabled() && n_spatial >= 4 * kNumSMs) {
-          // one launch: the deconv role publishes hr[i] tile by tile, the fused role takes it from L2
-          PUSH(build_group(L, D, F, i, reinterpret_cast<int32_t*>(ws + pl->o_flags), ++group_epoch, n_spatial));
-          grouped = true;
-        } else {
-          L = D;
-          layers.push_back(L);
-          L = F;
-          layers.push_back(L);
-        }
+        layers.push_back(D);
+        layers.push_back(F);
         PUSH(build_finalize(L, reinterpret_cast<float*>(ws + pl->o_acc), Bp(W_DOWN0 + i), ws + pl->o_lr[i + 1], P, h, w));
       }
     }
@@ -1232,8 +1098,7 @@ extern "C" int vsr_srfbn_prepare_refresh(vsr_srfbn_plan* pl, int first_map) {
   if (pl->chunk_maps != pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;     // not with a workspace cap (chunked sweeps)
   if (pl->refresh_first == first_map) return VSR_OK;
   pl->refresh_first = -1;
-  const int rc = build_layer_list(pl, pl->cfg.num_maps - first_map, pl->refresh_layers, pl->refresh_conv_out_layer,
-                                  pl->refresh_grouped);
+  const int rc = build_layer_list(pl, pl->cfg.num_maps - first_map, pl->refresh_layers, pl->refresh_conv_out_layer);
   if (rc) return rc;
   pl->refresh_first = first_map;
   return VSR_OK;
@@ -1244,18 +1109,14 @@ extern "C" int vsr_srfbn_forward(vsr_srfbn_plan* pl, const float* x, float* y, v
 }
 
 // One sweep of a layer list over the maps [m0, m0 + Mc) of the stack x; the per-map images land in the premix buffer.
-static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_out_layer, bool grouped, const float* x,
-                      int m0, int Mc, cudaStream_t st, size_t* ev) {
+static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_out_layer, const float* x, int m0, int Mc,
+                      cudaStream_t st, size_t* ev) {
   const vsr_srfbn_config& c = pl->cfg;
   const int64_t P = (int64_t)Mc * c.h * c.w;
   auto mark = [&]() {
     if (ev && pl->profile && *ev < pl->events.size()) cudaEventRecord(pl->events[(*ev)++], st);
   };
   const float* xc = x + (int64_t)m0 * 3 * c.h * c.w;
-  if (grouped) {
-    cudaError_t e = cudaMemsetAsync(pl->ws + pl->o_flags, 0, pl->flags_bytes, st);
-    if (e != cudaSuccess) return cuda_status(e);
-  }
   mark();
   {
     int64_t blocks = ceil_div64(P, 256);
@@ -1284,9 +1145,8 @@ static int fuse_maps(vsr_srfbn_plan* pl, float* y, uint8_t* y_u8, cudaStream_t s
   const int64_t n = (int64_t)3 * c.upscale * c.upscale * c.h * c.w;
   int64_t blocks = ceil_div64(ceil_div64(n, 4), 256);
   if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
-  cudaError_t e = launch_pdl(fc_fuse_kernel, (int)blocks, 256, 0, st, reinterpret_cast<const float*>(pl->ws + pl->o_premix),
-                             reinterpret_cast<const float*>(pl->dev_w + pl->fc_off), y, y_u8, c.num_maps, n);
-  if (e != cudaSuccess) return cuda_status(e);
+  fc_fuse_kernel<<<(int)blocks, 256, 0, st>>>(reinterpret_cast<const float*>(pl->ws + pl->o_premix),
+                                              reinterpret_cast<const float*>(pl->dev_w + pl->fc_off), y, y_u8, c.num_maps, n);
   return after_launch();
 }
 
@@ -1298,7 +1158,7 @@ extern "C" int vsr_srfbn_forward_u8(vsr_srfbn_plan* pl, const float* x, float* y
   const int Mc = pl->chunk_maps;
   size_t ev = 0;
   for (int m0 = 0; m0 < c.num_maps; m0 += Mc) {        // one sweep over the layer list per chunk of maps
-    int rc = sweep_maps(pl, pl->layers, pl->conv_out_layer, pl->grouped, x, m0, Mc, st, &ev);
+    int rc = sweep_maps(pl, pl->layers, pl->conv_out_layer, x, m0, Mc, st, &ev);
     if (rc) return rc;
   }
   if (pl->profile && ev < pl->events.size()) cudaEventRecord(pl->events[ev++], st);
@@ -1319,8 +1179,8 @@ extern "C" int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* pl, const float* x, 
   if (!pl || !x || (!y && !y_u8)) return VSR_ERR_INVALID_ARG;
   if (!pl->bound || !pl->premix_valid || pl->refresh_first != first_map || first_map < 1) return VSR_ERR_STATE;
   cudaStream_t st = as_stream(stream);
-  int rc = sweep_maps(pl, pl->refresh_layers, pl->refresh_conv_out_layer, pl->refresh_grouped, x, first_map,
-                      pl->cfg.num_maps - first_map, st, nullptr);
+  int rc = sweep_maps(pl, pl->refresh_layers, pl->refresh_conv_out_layer, x, first_map, pl->cfg.num_maps - first_map,
+                      st, nullptr);
   if (rc) return rc;
   return fuse_maps(pl, y, y_u8, st);
 }
@@ -1328,7 +1188,7 @@ extern "C" int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* pl, const float* x, 
 extern "C" const char* vsr_srfbn_kernel_class_name(int k) {
   static const char* names[KC_COUNT] = {"im2col", "conv_in_gemm", "pointwise_lr", "pointwise_hr", "deconv8x8s4",
                                         "conv8x8s4", "conv_out3x3", "fc_fuse", "fused_downtran_conv8x8s4",
-                                        "finalize_lr", "group(deconv8x8s4+fused_downtran_conv8x8s4)"};
+                                        "finalize_lr"};
   return (k >= 0 && k < KC_COUNT) ? names[k] : "?";
 }
 
@@ -1381,17 +1241,6 @@ extern "C" int vsr_srfbn_profile_launches(vsr_srfbn_plan* pl, float* ms, int32_t
     kclass[i] = i == n - 1 ? KC_FC : (i % per == 0 ? KC_IM2COL : pl->layers[i % per - 1].kclass);
   }
   return (int)n;
-}
-
-extern "C" int vsr_srfbn_debug_group_error(const vsr_srfbn_plan* pl, vsr_stream_t stream) {
-  if (!pl) return -1;
-  if (!pl->bound) return -1;
-  if (!pl->grouped) return 0;
-  int32_t v[2] = {0, 0};
-  cudaStream_t st = as_stream(stream);
-  if (cudaMemcpyAsync(v, pl->ws + pl->o_flags, sizeof(v), cudaMemcpyDeviceToHost, st) != cudaSuccess) return -1;
-  if (cudaStreamSynchronize(st) != cudaSuccess) return -1;
-  return v[1];
 }
 
 #ifdef VSR_KNOCKOUT

@@ -208,12 +208,6 @@ class SRProjectionModule(nn.Module):
                                                      torch.cuda.current_stream().cuda_stream), "srfbn_debug_premix")
         return out
 
-    def group_error(self):
-        """Test hook: True if a co-scheduled group launch gave up waiting (see vsr_srfbn_debug_group_error)."""
-        L = _lib.lib()
-        return any(L.vsr_srfbn_debug_group_error(ent["plan"], torch.cuda.current_stream().cuda_stream) != 0
-                   for ent in self._plans.values())
-
     def profile(self, enable=True):
         """Bracket every kernel launch of subsequent forwards with CUDA events (bench.py)."""
         for ent in self._plans.values():
@@ -222,7 +216,7 @@ class SRProjectionModule(nn.Module):
     def profile_read(self):
         """{kernel class: dict(ms, launches, flops, bytes)} of the last forward of each plan, summed."""
         L = _lib.lib()
-        n = 11            # VSR_SRFBN_KERNEL_CLASSES
+        n = 10            # VSR_SRFBN_KERNEL_CLASSES
         out = {}
         for ent in self._plans.values():
             ms = (ctypes.c_double * n)()
