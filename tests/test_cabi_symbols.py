@@ -3,6 +3,7 @@
 import ctypes
 import os
 import re
+import subprocess
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -32,13 +33,25 @@ def test_python_binding_covers_header():
 
 
 def test_shipped_library_reads_no_variant_switches():
-    """The shipped library reads one environment variable, VSR_CORR_GENERIC (it chooses between two live correlation
-    kernels): no switch changes which conv-stack kernels a process runs.  The timing-experiment switches exist only in
-    the -DVSR_KNOCKOUT build."""
+    """The library is built one way only and reads one environment variable, VSR_CORR_GENERIC (it chooses between two
+    live correlation kernels): no switch changes which conv-stack kernels a process runs, no source carries a
+    compile-time experiment switch, and the library exports no entry point the header does not declare."""
     from video_super_resolution_b200 import build
-    with open(build.build(), "rb") as f:
+    path = build.build()
+    with open(path, "rb") as f:
         names = set(re.findall(rb"VSR_[A-Z0-9_]+", f.read()))
     assert names == {b"VSR_CORR_GENERIC"}, sorted(names)
+
+    nm = subprocess.run(["nm", "-D", "--defined-only", path], capture_output=True, text=True, check=True).stdout
+    exported = set(re.findall(r"\s[TW]\s+(vsr_[a-z0-9_]+)$", nm, flags=re.M))
+    assert exported, nm[:2000]
+    assert not exported - set(_declared()), sorted(exported - set(_declared()))
+
+    switched = []
+    for src in sorted(os.listdir(build.CSRC)):
+        text = open(os.path.join(build.CSRC, src)).read()
+        switched += [(src, m) for m in sorted(set(re.findall(r"\bVSR_(?:KNOCKOUT|DBG|TRACE)\b", text)))]
+    assert not switched, switched
 
 
 def test_host_side_entry_points_without_gpu():

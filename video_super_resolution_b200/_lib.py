@@ -6,8 +6,7 @@ import ctypes
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# VSR_B200_LIB: load another build of the same ABI (the knock-out build of timing experiments); never a fallback
-LIB_PATH = os.environ.get("VSR_B200_LIB") or os.path.join(_HERE, "libvsr_b200.so")
+LIB_PATH = os.path.join(_HERE, "libvsr_b200.so")
 
 c_void_p = ctypes.c_void_p
 c_int = ctypes.c_int

@@ -1,6 +1,6 @@
 """Builds libvsr_b200.so in-tree with nvcc for sm_100a (no JIT cache: the .so travels with the tree).
 
-    python -m video_super_resolution_b200.build [--force] [--verbose] [--knockout]
+    python -m video_super_resolution_b200.build [--force] [--verbose]
 """
 from __future__ import annotations
 
@@ -40,13 +40,7 @@ def _deps_mtime() -> float:
     return max(os.path.getmtime(f) for f in files)
 
 
-def build(force: bool = False, verbose: bool = False, knockout: bool = False) -> str:
-    """knockout=True compiles the timing-experiment switches in (-DVSR_KNOCKOUT: VSR_DECONV_DEBUG / VSR_FUSED_DEBUG
-    make results wrong on purpose); the shipped library never has them."""
-    # the knock-out build has its own objects and its own file name, so it can never be mistaken for the product
-    # (load it with VSR_B200_LIB=.../libvsr_b200_knockout.so)
-    LIB = globals()["LIB"] if not knockout else os.path.join(HERE, "libvsr_b200_knockout.so")
-    OBJ = globals()["OBJ"] if not knockout else os.path.join(HERE, "build_knockout")
+def build(force: bool = False, verbose: bool = False) -> str:
     if not force and os.path.exists(LIB) and os.path.getmtime(LIB) >= _deps_mtime():
         return LIB
     nvcc = _nvcc()
@@ -59,8 +53,7 @@ def build(force: bool = False, verbose: bool = False, knockout: bool = False) ->
         obj = os.path.join(OBJ, os.path.basename(src)[:-3] + ".o")
         if not force and os.path.exists(obj) and os.path.getmtime(obj) >= max(os.path.getmtime(src), hdr_mtime):
             return obj
-        cmd = [nvcc] + NVCC_FLAGS + (["-DVSR_KNOCKOUT"] if knockout else []) + \
-            (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
+        cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + ["-c", src, "-o", obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if verbose or r.returncode:
             sys.stderr.write(r.stdout + r.stderr)
@@ -79,4 +72,4 @@ def build(force: bool = False, verbose: bool = False, knockout: bool = False) ->
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv, knockout="--knockout" in sys.argv))
+    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv))

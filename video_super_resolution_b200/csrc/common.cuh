@@ -11,14 +11,6 @@
 #error "libvsr_b200 is written for sm_100a (Blackwell B200) only"
 #endif
 
-// Knock-out switches for timing experiments (they make results WRONG) exist only in builds with -DVSR_KNOCKOUT
-// (python -m video_super_resolution_b200.build --knockout); the shipped library compiles them out.
-#ifdef VSR_KNOCKOUT
-#define VSR_DBG(p) ((p).debug)
-#else
-#define VSR_DBG(p) 0
-#endif
-
 namespace vsr {
 
 extern std::atomic<uint64_t> g_launch_count;

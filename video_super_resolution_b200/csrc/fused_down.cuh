@@ -53,29 +53,18 @@ struct alignas(64) FusedDownParams {
   int32_t num_stages;
   int32_t tiles_x, tiles_y, batch;
   int32_t lr_h, lr_w;
-  int32_t debug;                      // timing experiments (results become wrong): bit0 skip phase-A MMAs, bit1 skip
-                                      // the TMEM reads + conversion of phase A, bit2 skip the final TMEM reads/stores,
-                                      // bit3 skip phase-B MMAs
   const float* tran_bias;             // [32] biases + [1] PReLU slope of the downtran
   const float* down_bias;             // [32] biases + [1] PReLU slope of the strided conv
   float* part;                        // (B, h, w, 4 slots, 32) fp32 partial sums of the BOUNDARY pixels (see final epilogue)
   void* lr_out;                       // (B, h, w, 32) bf16: finished interior pixels
-  long long* trace;                   // VSR_KNOCKOUT builds: clock64 stamps of CTA 0's roles, [tile][32]; nullptr = off
 };
 
-__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
                : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
                : "r"(taddr)
                : "memory");
 }
-
-#ifdef VSR_KNOCKOUT
-#define VSR_TRACE(slot) do { if (p.trace && cta == 0 && tile_n < 1024) p.trace[tile_n * 32 + (slot)] = clock64(); } while (0)
-#else
-#define VSR_TRACE(slot) do { } while (0)
-#endif
 
 template <bool HAS_TRAN>
 inline size_t fused_down_smem_bytes(int nsrc, int num_stages) {
@@ -166,12 +155,9 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
       __syncwarp();
       int s = 0;
       uint32_t phase = 0;
-      int tile_n = -1;
       for (int tile = cta; tile < total_tiles; tile += ncta) {
-        ++tile_n;
         int x0, y0, b;
         tile_coord(tile, x0, y0, b);
-        VSR_TRACE(0);
         for (int half = 0; half < 2; ++half) {
           if (HAS_TRAN) {
             // one box = 2 sub-positions x 128 blocks x 32 ch (16 KB): a [128 x 64] K-major tile whose K
@@ -187,7 +173,6 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
                 if (++s == p.num_stages) { s = 0; phase ^= 1; }
               }
             }
-            VSR_TRACE(1 + half);
           } else {
             for (int g = half * 2; g < half * 2 + 2; ++g) {
               mbar_wait(&empty_bar[s], phase ^ 1);
@@ -238,13 +223,11 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
           const uint64_t b0 = dWt + (uint64_t)((j * kWtChunkBytes) >> 4);
           const uint32_t d0 = tmem_base + (uint32_t)(buf * 128 + pair * 64);
           if (elect_one()) {
-            if (!(VSR_DBG(p) & 1)) {
-              const uint32_t acc = (uint32_t)(j != 0);
-              umma_bf16(d0, a0, b0, idesc_a, acc);
-              umma_bf16(d0, a0 + 2, b0 + 2, idesc_a, 1u);
-              umma_bf16(d0 + 32, a0 + 4, b0, idesc_a, acc);
-              umma_bf16(d0 + 32, a0 + 6, b0 + 2, idesc_a, 1u);
-            }
+            const uint32_t acc = (uint32_t)(j != 0);
+            umma_bf16(d0, a0, b0, idesc_a, acc);
+            umma_bf16(d0, a0 + 2, b0 + 2, idesc_a, 1u);
+            umma_bf16(d0 + 32, a0 + 4, b0, idesc_a, acc);
+            umma_bf16(d0 + 32, a0 + 6, b0 + 2, idesc_a, 1u);
             umma_commit(&empty_bar[s]);
             if (pair == 1 && j == p.nsrc - 1) umma_commit(&da_full[buf]);
           }
@@ -270,14 +253,12 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
       const uint32_t d = tmem_base + kDB + (uint32_t)(tb * 128);
       const uint64_t b0 = dWd + (uint64_t)((wslot * kWdGroupBytes) >> 4);
       if (elect_one()) {
-        if (!(VSR_DBG(p) & 8)) {
 #pragma unroll
-          for (int kc = 0; kc < 2; ++kc)
+        for (int kc = 0; kc < 2; ++kc)
 #pragma unroll
-            for (int k = 0; k < 4; ++k)
-              umma_bf16(d, a0 + (uint64_t)(kc * 1024 + k * 2), b0 + (uint64_t)(kc * 1024 + k * 2), idesc_b,
-                        (uint32_t)((g | kc | k) != 0));
-        }
+          for (int k = 0; k < 4; ++k)
+            umma_bf16(d, a0 + (uint64_t)(kc * 1024 + k * 2), b0 + (uint64_t)(kc * 1024 + k * 2), idesc_b,
+                      (uint32_t)((g | kc | k) != 0));
         umma_commit(&wd_empty[wslot]);
         if (HAS_TRAN) umma_commit(h_empty);
         else umma_commit(&empty_bar[s]);
@@ -293,14 +274,12 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
     // HAS_TRAN: this thread issues phase A only; phase B has its own issuing thread (warp kFusedBWarp), so
     // that waiting for the converted tile / the weights never holds up the consumption of TMA stages.
     // tcgen05.commit tracks the MMAs of the issuing thread, so each thread signals exactly its own work.
-    int tile_n = -1;
     for (int tile = cta; tile < total_tiles; tile += ncta) {
-      ++tile_n;
       if (HAS_TRAN) {
         if (warp == 1) {
-          for (int g = 0; g < 4; ++g) { issue_a(g); VSR_TRACE(4 + g); }          // phase-A MMAs of group g issued
+          for (int g = 0; g < 4; ++g) issue_a(g);
         } else {
-          for (int g = 0; g < 4; ++g) { issue_b(g); VSR_TRACE(8 + g); }          // phase-B MMAs of group g issued
+          for (int g = 0; g < 4; ++g) issue_b(g);
         }
       } else {
         for (int g = 0; g < 4; ++g) issue_b(g);
@@ -336,9 +315,7 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
     uint32_t m_a[2] = {0, 0}, m_b[2] = {0, 0}, m_h = 0;
     int tb = 0;
     const PreluCfg pc = make_prelu(HAS_TRAN ? s_bias[32] : 1.0f, 1);
-    int tile_n = -1;
     for (int tile = cta; tile < total_tiles; tile += ncta) {
-      ++tile_n;
       int x0, y0, b;
       tile_coord(tile, x0, y0, b);
       const int Yb = y0 + (row >> 4), Xb = x0 + (row & 15);
@@ -347,30 +324,21 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
 #pragma unroll 1
         for (int g = 0; g < 4; ++g) {
           const int buf = g & 1;
-          mbar_wait_sleep(&da_full[buf], m_a[buf] & 1, (uint32_t)(VSR_DBG(p) >> 8));
+          mbar_wait_poll(&da_full[buf], m_a[buf] & 1);
           tc_fence_after();
-          if (warp == 2 && lane == 0) VSR_TRACE(12 + g);                          // D_A of group g complete (seen by the epilogue)
           uint32_t o[16];
-          if (VSR_DBG(p) & 2) {
-            zero16(o);
-            tc_fence_before();
-            mbar_arrive_warp(&da_empty[buf]);
-          } else {
-            uint32_t v[32];
-            tmem_ld32(lane_base + (uint32_t)(buf * 128 + sub * 32), v);
-            tmem_ld_wait();
-            tc_fence_before();
-            mbar_arrive_warp(&da_empty[buf]);
-            const int s16 = g * 4 + sub, ry = s16 >> 2, rx = s16 & 3;
-            const bool ring = (Yb == 0 && ry < 2) || (Yb == p.lr_h && ry >= 2) || (Xb == 0 && rx < 2) ||
-                              (Xb == p.lr_w && rx >= 2);
-            convert32(v, s_bias, pc, o);
-            if (__builtin_expect(!(in_tensor && !ring), 0)) zero16(o);
-          }
+          uint32_t v[32];
+          tmem_ld32(lane_base + (uint32_t)(buf * 128 + sub * 32), v);
+          tmem_ld_wait();
+          tc_fence_before();
+          mbar_arrive_warp(&da_empty[buf]);
+          const int s16 = g * 4 + sub, ry = s16 >> 2, rx = s16 & 3;
+          const bool ring = (Yb == 0 && ry < 2) || (Yb == p.lr_h && ry >= 2) || (Xb == 0 && rx < 2) ||
+                            (Xb == p.lr_w && rx >= 2);
+          convert32(v, s_bias, pc, o);
+          if (__builtin_expect(!(in_tensor && !ring), 0)) zero16(o);
           ++m_a[buf];
-          if (warp == 2 && lane == 0) VSR_TRACE(16 + g);                          // converted, waiting for H to be free
           mbar_wait(h_empty, (m_h & 1) ^ 1);
-          if (warp == 2 && lane == 0) VSR_TRACE(20 + g);                          // H free
           // K index inside the group: k = sub*32 + c -> 64-element chunk kc = sub>>1, 16-byte piece (sub&1)*4 + j
           uint8_t* hrow = s_h + (sub >> 1) * 16384 + (row >> 3) * 1024 + (row & 7) * 128;
 #pragma unroll
@@ -379,7 +347,7 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
             *reinterpret_cast<uint4*>(hrow + ((piece ^ (row & 7)) << 4)) =
                 make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
           }
-          fence_proxy_async_smem();
+          fence_async_smem();
           mbar_arrive_warp(h_full);
           ++m_h;
         }
@@ -396,80 +364,72 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
       //    with exactly one writer each:  slot 2*dy   : tap (dy,0) + right neighbour's tap (dy,1)
       //                                   slot 2*dy+1 : tap (dy,1) arriving from the next tile
       //    finalize_lr_kernel sums them.  Same additions in the same order either way: deterministic.
-      if (warp == 2 && lane == 0) VSR_TRACE(24);                                  // H of the last group handed over
-      mbar_wait_sleep(&db_full[tb], m_b[tb] & 1, (uint32_t)(VSR_DBG(p) >> 8));
+      mbar_wait_poll(&db_full[tb], m_b[tb] & 1);
       tc_fence_after();
-      if (warp == 2 && lane == 0) VSR_TRACE(25);                                  // D_B complete
-      if (VSR_DBG(p) & 4) {
-        tc_fence_before();
-        mbar_arrive_warp(&db_empty[tb]);
-      } else {
-        uint32_t v[4][8];
+      uint32_t v[4][8];
 #pragma unroll
-        for (int t = 0; t < 4; ++t) tmem_ld8(lane_base + kDB + (uint32_t)(tb * 128 + t * 32 + sub * 8), v[t]);
-        tmem_ld_wait();
-        tc_fence_before();
-        mbar_arrive_warp(&db_empty[tb]);
-        const int xl = lane & 15, half = lane >> 4;
-        float comb[2][8];
+      for (int t = 0; t < 4; ++t) tmem_ld8(lane_base + kDB + (uint32_t)(tb * 128 + t * 32 + sub * 8), v[t]);
+      tmem_ld_wait();
+      tc_fence_before();
+      mbar_arrive_warp(&db_empty[tb]);
+      const int xl = lane & 15, half = lane >> 4;
+      float comb[2][8];
 #pragma unroll
-        for (int dy = 0; dy < 2; ++dy)
+      for (int dy = 0; dy < 2; ++dy)
 #pragma unroll
-          for (int k = 0; k < 8; ++k) {
-            const float right = __uint_as_float(v[dy * 2 + 1][k]);
-            const float from_right = __shfl_down_sync(0xffffffffu, right, 1);
-            comb[dy][k] = __uint_as_float(v[dy * 2][k]) + (xl < 15 ? from_right : 0.0f);
+        for (int k = 0; k < 8; ++k) {
+          const float right = __uint_as_float(v[dy * 2 + 1][k]);
+          const float from_right = __shfl_down_sync(0xffffffffu, right, 1);
+          comb[dy][k] = __uint_as_float(v[dy * 2][k]) + (xl < 15 ? from_right : 0.0f);
+        }
+      // second row partial of this lane's pixel (Yb, Xb): block row Yb+1's comb[1].  Even tile rows: lane + 16 of
+      // this warp.  Odd tile rows 1, 3, 5: lanes 0-15 of the next lane quarter, through shared memory.
+      float below[8];
+#pragma unroll
+      for (int k = 0; k < 8; ++k) below[k] = __shfl_down_sync(0xffffffffu, comb[1][k], 16);
+      if (half == 0 && q > 0) {
+        float4* x = s_x + (((q - 1) * 4 + sub) * 16 + xl) * 2;
+        x[0] = make_float4(comb[1][0], comb[1][1], comb[1][2], comb[1][3]);
+        x[1] = make_float4(comb[1][4], comb[1][5], comb[1][6], comb[1][7]);
+      }
+      asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");     // the 16 epilogue warps only
+      if (half == 1 && q < 3) {
+        const float4* x = s_x + ((q * 4 + sub) * 16 + xl) * 2;
+        const float4 x0v = x[0], x1v = x[1];
+        below[0] = x0v.x; below[1] = x0v.y; below[2] = x0v.z; below[3] = x0v.w;
+        below[4] = x1v.x; below[5] = x1v.y; below[6] = x1v.z; below[7] = x1v.w;
+      }
+      asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");     // reads done before the next tile's writes
+      const int rr = 2 * q + half;                                               // block row inside the tile
+      if (rr < 7 && xl < 15 && in_tensor && Yb < p.lr_h && Xb < p.lr_w) {   // interior pixel (Yb, Xb)
+        const float slope = s_down[32];
+        float r[8];
+#pragma unroll
+        for (int k = 0; k < 8; ++k) r[k] = prelu(comb[0][k] + below[k] + s_down[sub * 8 + k], slope, 1);
+        uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(p.lr_out) +
+                                               ((((int64_t)b * p.lr_h + Yb) * p.lr_w + Xb) * 64 + sub * 16));
+        *dst = make_uint4(pack_bf16(r[0], r[1]), pack_bf16(r[2], r[3]), pack_bf16(r[4], r[5]), pack_bf16(r[6], r[7]));
+      }
+#pragma unroll
+      for (int dy = 0; dy < 2; ++dy) {
+        const int Y = Yb - dy;
+        if (in_tensor && Y >= 0 && Y < p.lr_h) {
+          // row 7 of a tile, or the tile's last column
+          const bool boundary = (((rr - dy) & 7) == 7) || (xl == 15);
+          if (Xb < p.lr_w && boundary) {
+            float4* dst = reinterpret_cast<float4*>(p.part + ((((int64_t)b * p.lr_h + Y) * p.lr_w + Xb) * 4 + 2 * dy) * 32 + sub * 8);
+            dst[0] = make_float4(comb[dy][0], comb[dy][1], comb[dy][2], comb[dy][3]);
+            dst[1] = make_float4(comb[dy][4], comb[dy][5], comb[dy][6], comb[dy][7]);
           }
-        // second row partial of this lane's pixel (Yb, Xb): block row Yb+1's comb[1].  Even tile rows: lane + 16 of
-        // this warp.  Odd tile rows 1, 3, 5: lanes 0-15 of the next lane quarter, through shared memory.
-        float below[8];
-#pragma unroll
-        for (int k = 0; k < 8; ++k) below[k] = __shfl_down_sync(0xffffffffu, comb[1][k], 16);
-        if (half == 0 && q > 0) {
-          float4* x = s_x + (((q - 1) * 4 + sub) * 16 + xl) * 2;
-          x[0] = make_float4(comb[1][0], comb[1][1], comb[1][2], comb[1][3]);
-          x[1] = make_float4(comb[1][4], comb[1][5], comb[1][6], comb[1][7]);
-        }
-        asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");     // the 16 epilogue warps only
-        if (half == 1 && q < 3) {
-          const float4* x = s_x + ((q * 4 + sub) * 16 + xl) * 2;
-          const float4 x0v = x[0], x1v = x[1];
-          below[0] = x0v.x; below[1] = x0v.y; below[2] = x0v.z; below[3] = x0v.w;
-          below[4] = x1v.x; below[5] = x1v.y; below[6] = x1v.z; below[7] = x1v.w;
-        }
-        asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");     // reads done before the next tile's writes
-        const int rr = 2 * q + half;                                               // block row inside the tile
-        if (rr < 7 && xl < 15 && in_tensor && Yb < p.lr_h && Xb < p.lr_w) {   // interior pixel (Yb, Xb)
-          const float slope = s_down[32];
-          float r[8];
-#pragma unroll
-          for (int k = 0; k < 8; ++k) r[k] = prelu(comb[0][k] + below[k] + s_down[sub * 8 + k], slope, 1);
-          uint4* dst = reinterpret_cast<uint4*>(reinterpret_cast<uint8_t*>(p.lr_out) +
-                                                 ((((int64_t)b * p.lr_h + Yb) * p.lr_w + Xb) * 64 + sub * 16));
-          *dst = make_uint4(pack_bf16(r[0], r[1]), pack_bf16(r[2], r[3]), pack_bf16(r[4], r[5]), pack_bf16(r[6], r[7]));
-        }
-#pragma unroll
-        for (int dy = 0; dy < 2; ++dy) {
-          const int Y = Yb - dy;
-          if (in_tensor && Y >= 0 && Y < p.lr_h) {
-            // row 7 of a tile, or the tile's last column
-            const bool boundary = (((rr - dy) & 7) == 7) || (xl == 15);
-            if (Xb < p.lr_w && boundary) {
-              float4* dst = reinterpret_cast<float4*>(p.part + ((((int64_t)b * p.lr_h + Y) * p.lr_w + Xb) * 4 + 2 * dy) * 32 + sub * 8);
-              dst[0] = make_float4(comb[dy][0], comb[dy][1], comb[dy][2], comb[dy][3]);
-              dst[1] = make_float4(comb[dy][4], comb[dy][5], comb[dy][6], comb[dy][7]);
-            }
-            if (xl == 0 && Xb > 0) {
-              float4* dst = reinterpret_cast<float4*>(p.part + ((((int64_t)b * p.lr_h + Y) * p.lr_w + Xb - 1) * 4 + 2 * dy + 1) * 32 + sub * 8);
-              dst[0] = make_float4(__uint_as_float(v[dy * 2 + 1][0]), __uint_as_float(v[dy * 2 + 1][1]),
-                                   __uint_as_float(v[dy * 2 + 1][2]), __uint_as_float(v[dy * 2 + 1][3]));
-              dst[1] = make_float4(__uint_as_float(v[dy * 2 + 1][4]), __uint_as_float(v[dy * 2 + 1][5]),
-                                   __uint_as_float(v[dy * 2 + 1][6]), __uint_as_float(v[dy * 2 + 1][7]));
-            }
+          if (xl == 0 && Xb > 0) {
+            float4* dst = reinterpret_cast<float4*>(p.part + ((((int64_t)b * p.lr_h + Y) * p.lr_w + Xb - 1) * 4 + 2 * dy + 1) * 32 + sub * 8);
+            dst[0] = make_float4(__uint_as_float(v[dy * 2 + 1][0]), __uint_as_float(v[dy * 2 + 1][1]),
+                                 __uint_as_float(v[dy * 2 + 1][2]), __uint_as_float(v[dy * 2 + 1][3]));
+            dst[1] = make_float4(__uint_as_float(v[dy * 2 + 1][4]), __uint_as_float(v[dy * 2 + 1][5]),
+                                 __uint_as_float(v[dy * 2 + 1][6]), __uint_as_float(v[dy * 2 + 1][7]));
           }
         }
       }
-      if (warp == 2 && lane == 0) VSR_TRACE(26);                                  // final epilogue of the tile done
       ++m_b[tb];
       tb ^= 1;
     }

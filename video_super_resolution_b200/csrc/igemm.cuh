@@ -86,7 +86,6 @@ struct alignas(64) IgemmParams {
   int32_t lr_h, lr_w;          // LR size (block-layout masks, deconv geometry)
   int32_t hrb_mask;            // EPI_ROWS flat over the HR block layout: zero the padding ring
   int32_t deconv_nhwc;         // EPI_DECONV: 1 = write plain NHWC HR instead of the block layout
-  int32_t debug;               // timing experiments (wrong results): bit0 no TMA stores, bit1 no TMEM reads/convert, bit2 no MMAs, bit3 all stores to one place
   // EPI_CONV_OUT extras
   const float* skip_src;       // network input x (M,3,h,w) fp32
   float inv_scale;             // 1 / upscale factor of the bilinear skip (0.25 or 0.5)
@@ -127,38 +126,22 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
       "r"(parity)
       : "memory");
 }
-// wait with back-off: the many epilogue warps of a memory-bound kernel spend most of their life here;
-// sleeping between probes takes their polling off the issue ports (and off the power budget)
-__device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity, uint32_t ns) {
-  uint32_t addr = smem_u32(bar);
-  uint32_t done = 0;
-  const uint32_t hint = (ns >> 16) * 256u;   // knob: bits 16+ = suspend-time hint of try_wait in units of 256 ns, low 16 bits = nanosleep
-  ns &= 0xffffu;
-  while (true) {
-    if (hint) {
-      asm volatile(
-          "{\n"
-          ".reg .pred P1;\n"
-          "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2, %3;\n"
-          "selp.u32 %0, 1, 0, P1;\n"
-          "}\n"
-          : "=r"(done)
-          : "r"(addr), "r"(parity), "r"(hint)
-          : "memory");
-    } else {
-      asm volatile(
-          "{\n"
-          ".reg .pred P1;\n"
-          "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n"
-          "selp.u32 %0, 1, 0, P1;\n"
-          "}\n"
-          : "=r"(done)
-          : "r"(addr), "r"(parity)
-          : "memory");
-    }
-    if (done) break;
-    if (ns) __nanosleep(ns);
-  }
+// the same wait with the retry loop in C++ instead of inside the asm: the fused kernel's epilogue waits were
+// tuned in this form, and mbar_wait there compiles to different code (one more register, ~90 more instructions)
+__device__ __forceinline__ void mbar_wait_poll(uint64_t* bar, uint32_t parity) {
+  const uint32_t addr = smem_u32(bar);
+  uint32_t done;
+  do {
+    asm volatile(
+        "{\n"
+        ".reg .pred P1;\n"
+        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n"
+        "selp.u32 %0, 1, 0, P1;\n"
+        "}\n"
+        : "=r"(done)
+        : "r"(addr), "r"(parity)
+        : "memory");
+  } while (!done);
 }
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 
@@ -580,7 +563,6 @@ igemm_kernel(const __grid_constant__ IgemmParams p) {
               const int kc = kc0 + j;
               const uint64_t a0 = dA + (uint64_t)((s * p.stage_bytes + p.chunks[kc].a_off) >> 4);
               const uint64_t b0 = dB + (uint64_t)((kc * kBBytes) >> 4);
-              if (!(VSR_DBG(p) & 4))
 #pragma unroll
               for (int k = 0; k < CK / 16; ++k) umma_bf16(d_tmem, a0 + 2 * k, b0 + 2 * k, idesc, (uint32_t)((kc | k) != 0));
             }
@@ -695,15 +677,12 @@ igemm_kernel(const __grid_constant__ IgemmParams p) {
           for (int c2 = 0; c2 < 2; ++c2) {
             const int cg = sub * 2 + c2;
             uint32_t v[32];
-            if (!(VSR_DBG(p) & 2)) {       // (the knock-out leaves v undefined; zeroing it here cost 32 CS2R per read even
-              tmem_ld32(taddr + cg * 32, v);   //  in production, ncu: 10 % of the kernel's instructions)
-              tmem_ld_wait();
-            }
+            tmem_ld32(taddr + cg * 32, v);
+            tmem_ld_wait();
             if (c2 == 1) {
               tc_fence_before();
               mbar_arrive_warp(&tmem_empty[as]);
             }
-            if (VSR_DBG(p) & 2) continue;
             const int s16 = t.n_tile * 8 + cg;
             const int ry = s16 >> 2, rx = s16 & 3;
             const int Yt = 4 * Y + ry - 2, Xt = 4 * X + rx - 2;
@@ -727,9 +706,7 @@ igemm_kernel(const __grid_constant__ IgemmParams p) {
           if (elect_one()) {   // (the same lane every time: bulk groups are per thread)
             // one box = this warp's 2 block rows x 16 blocks of one sub-position-pair plane; rows or
             // columns beyond the tensor edge are clipped by the TMA unit
-            if (VSR_DBG(p) & 8)   // timing experiment: every tile stores to the first tile's place (L2-resident, no DRAM)
-              tma_store_4d(&p.out_map, stg, 0, 0, 2 * q, t.n_tile * 4 + sub);
-            else if (t.y0 + 2 * q <= p.lr_h && !(VSR_DBG(p) & 1))
+            if (t.y0 + 2 * q <= p.lr_h)
               tma_store_4d(&p.out_map, stg, 0, t.x0, t.y0 + 2 * q, t.b * 8 + t.n_tile * 4 + sub);
             tma_store_commit();
           }

@@ -27,7 +27,6 @@
 // keeps `outs[-1:]` (SRProjectionModule.py:145), the earlier steps' images are dead values.
 #include "fused_down.cuh"
 
-#include <stdlib.h>
 #include <string.h>
 
 #include <new>
@@ -111,10 +110,6 @@ struct Layer {
   double flops;   // 2*MAC of the layer as specified (padding / ring rows not counted)
   double bytes;   // compulsory HBM bytes of this launch: its inputs + outputs, each once
 };
-
-#ifdef VSR_KNOCKOUT
-long long* g_trace_buf = nullptr;
-#endif
 
 template <int MODE, int CK, int BN>
 int launch_variant(const Layer& L, cudaStream_t st) {
@@ -296,12 +291,6 @@ int build_deconv(Layer& L, const void* x, int B, int h, int w, const void* w_dev
   p.lr_h = h;
   p.lr_w = w;
   p.deconv_nhwc = nhwc;
-#ifdef VSR_KNOCKOUT
-  {
-    const char* e = getenv("VSR_DECONV_DEBUG");
-    p.debug = e ? atoi(e) : 0;
-  }
-#endif
   if (!nhwc) {
     EncodeTiledFn enc = encode_fn();
     if (!enc) return VSR_ERR_STATE;
@@ -481,20 +470,6 @@ int build_fused_down(Layer& L, const void* const* hr, int nsrc, int B, int h, in
   f.batch = B;
   f.lr_h = h;
   f.lr_w = w;
-#ifdef VSR_KNOCKOUT
-  {
-    const char* e = getenv("VSR_FUSED_DEBUG");
-    f.debug = e ? atoi(e) : 0;
-    // timeline of CTA 0 of the launch with VSR_FUSED_TRACE=<nsrc>: clock64 stamps into a debug buffer
-    e = getenv("VSR_FUSED_TRACE");
-    if (e && atoi(e) == nsrc) {
-      static long long* buf = nullptr;
-      if (!buf && cudaMalloc(&buf, 1024 * 32 * sizeof(long long)) == cudaSuccess) cudaMemset(buf, 0, 1024 * 32 * sizeof(long long));
-      f.trace = buf;
-      g_trace_buf = buf;
-    }
-  }
-#endif
   f.tran_bias = tran_bias_dev;
   f.down_bias = down_bias_dev;
   f.part = part;
@@ -1242,13 +1217,6 @@ extern "C" int vsr_srfbn_profile_launches(vsr_srfbn_plan* pl, float* ms, int32_t
   }
   return (int)n;
 }
-
-#ifdef VSR_KNOCKOUT
-extern "C" int vsr_debug_fused_trace(long long* host_out) {      // knock-out build only: 1024 tiles x 32 stamps
-  if (!g_trace_buf || !host_out) return -1;
-  return cuda_status(cudaMemcpy(host_out, g_trace_buf, 1024 * 32 * sizeof(long long), cudaMemcpyDeviceToHost));
-}
-#endif
 
 extern "C" int vsr_srfbn_debug_premix(const vsr_srfbn_plan* pl, float* out_maps, vsr_stream_t stream) {
   if (!pl || !out_maps) return VSR_ERR_INVALID_ARG;
