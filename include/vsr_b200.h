@@ -118,6 +118,19 @@ int vsr_resample2d_backward(const float* input1, const float* flow, const float*
                             int B, int C, int H, int W, int kernel_size, int bilinear, vsr_stream_t stream);
 int vsr_channelnorm_backward(const float* input, const float* output, const float* grad_output,
                              float* grad_input, int B, int C, int H, int W, int norm_deg, vsr_stream_t stream);
+/* Deterministic variant of vsr_resample2d_backward: grad_input1 is bit-identical to oracle/oracle.c
+ * or_resample2d_backward (fp32 sums of w*g in row-major source order, taps TL, TR, BL, BR), so it is the same on
+ * every run; grad_input2 comes from the same kernel as above.  Every element of grad_input1 is written (any contents on
+ * entry).  workspace: vsr_resample2d_backward_deterministic_workspace_bytes(B,H,W) bytes of device memory (any
+ * contents, 16-byte aligned).  kernel_size must be 1 (VSR_ERR_UNSUPPORTED otherwise, and for B*H*W >= 2^32).  The
+ * scatter is turned into a gather (stable radix sort of the sources by their top-left tap, then one thread per
+ * target): a target that many sources reach -- every out-of-image sample is clamped to a border pixel -- sums them
+ * in sequence on one thread. */
+size_t vsr_resample2d_backward_deterministic_workspace_bytes(int B, int H, int W);
+int vsr_resample2d_backward_deterministic(const float* input1, const float* flow, const float* grad_output,
+                                          float* grad_input1, float* grad_input2, int B, int C, int H, int W,
+                                          int kernel_size, int bilinear, void* workspace, size_t workspace_bytes,
+                                          vsr_stream_t stream);
 
 /* FlowNetC cost volume (SURVEY.md 8f rank 1; outside the warp-and-fuse hot path).
  * ref: correlation_cuda.cc:10-86 `correlation_forward_cuda(input1, input2, rInput1, rInput2, output,
@@ -174,6 +187,17 @@ int vsr_flow_projection_forward_bounded(const float* flow, const float* inv_dept
                                         float* proj, float* wsum, int32_t* count, uint8_t* hole,
                                         void* workspace, size_t workspace_bytes,
                                         int B, int h, int w, float max_disp, vsr_stream_t stream);
+/* Deterministic projection: proj, wsum, count and hole are bit-identical to oracle/oracle.c or_flow_projection --
+ * for every target the fp32 contributions of its sources are added in fp64 in row-major source order, then rounded
+ * and divided in fp32 -- so they are the same on every run, whatever the flow.  Same arguments as
+ * vsr_flow_projection_forward; workspace: vsr_flow_projection_deterministic_workspace_bytes(B,h,w) bytes (any contents,
+ * 16-byte aligned; the images are processed one after another and share it).  Slower than the default paths: a stable
+ * radix sort of the sources by cell, then one thread per target merging its four cells' lists. */
+size_t vsr_flow_projection_deterministic_workspace_bytes(int B, int h, int w);
+int vsr_flow_projection_forward_deterministic(const float* flow, const float* inv_depth,
+                                              float* proj, float* wsum, int32_t* count, uint8_t* hole,
+                                              void* workspace, size_t workspace_bytes,
+                                              int B, int h, int w, vsr_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * a5: VOS mask arithmetic.  ref: VOSProjectionModule.py:22-25 (sigmoid(a)+sigmoid(b) > 0.7),

@@ -61,12 +61,16 @@ SIGNATURES = {
     "vsr_channelnorm_backward_typed": (c_int, [c_void_p] * 4 + [c_int] * 6 + [c_void_p]),
     "vsr_resample2d_backward": (c_int, [c_void_p] * 5 + [c_int] * 6 + [c_void_p]),
     "vsr_channelnorm_backward": (c_int, [c_void_p] * 4 + [c_int] * 5 + [c_void_p]),
+    "vsr_resample2d_backward_deterministic_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "vsr_resample2d_backward_deterministic": (c_int, [c_void_p] * 5 + [c_int] * 6 + [c_void_p, c_size_t, c_void_p]),
     "vsr_correlation_output_shape": (c_int, [c_int] * 8 + [ctypes.POINTER(c_int)] * 3),
     "vsr_correlation_forward": (c_int, [c_void_p] * 3 + [c_int] * 10 + [c_void_p]),
     "vsr_correlation_backward": (c_int, [c_void_p] * 5 + [c_int] * 10 + [c_void_p]),
     "vsr_flow_projection_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "vsr_flow_projection_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_void_p]),
     "vsr_flow_projection_forward_bounded": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_float, c_void_p]),
+    "vsr_flow_projection_deterministic_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "vsr_flow_projection_forward_deterministic": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_void_p]),
     "vsr_vos_threshold": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "vsr_flow_to_image": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "vsr_mask_fill": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),

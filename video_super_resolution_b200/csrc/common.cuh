@@ -108,4 +108,12 @@ __device__ __forceinline__ void stg_stream_f4(float4* p, float4 v) {
                : "memory");
 }
 
+// Stages shared with the deterministic paths (deterministic.cu), launched from the translation unit that owns them.
+// The projection's 4-direction hole fill over a list of row words with holes (projection.cu's general path).
+int launch_projection_fill(const uint32_t* rowmask, const uint32_t* colmask, const int* n_holewords,
+                           const uint32_t* holelist, float* proj, int h, int w, cudaStream_t st);
+// Resample2d's gradient w.r.t. the flow (warp.cu), bit-identical to the reference binary.
+int launch_resample2d_backward_input2(const float* input1, const float* flow, const float* grad_output,
+                                      float* grad_input2, int B, int C, int H, int W, cudaStream_t st);
+
 }  // namespace vsr

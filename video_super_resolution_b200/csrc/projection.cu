@@ -1001,6 +1001,14 @@ int run_general(const ProjArgs& a, cudaStream_t st) {
 }
 
 }  // namespace
+
+int launch_projection_fill(const uint32_t* rowmask, const uint32_t* colmask, const int* n_holewords,
+                           const uint32_t* holelist, float* proj, int h, int w, cudaStream_t st) {
+  const int fill_blocks = min(ceil_div(h * ceil_div(w, 32), kThreads / 32), kNumSMs * 16);
+  stage_fill_kernel<<<fill_blocks, kThreads, 0, st>>>(rowmask, colmask, n_holewords, holelist, proj, nullptr, h, w);
+  return after_launch();
+}
+
 }  // namespace vsr
 
 using namespace vsr;

@@ -705,6 +705,15 @@ channelnorm_backward_kernel(const float* __restrict__ in, const float* __restric
 }
 
 }  // namespace
+
+int launch_resample2d_backward_input2(const float* input1, const float* flow, const float* grad_output,
+                                      float* grad_input2, int B, int C, int H, int W, cudaStream_t st) {
+  const int64_t n = (int64_t)B * H * W;
+  resample2d_backward_input2_kernel<<<grid_for(n, kThreads), kThreads, 0, st>>>(input1, flow, grad_output, grad_input2, B, C,
+                                                                               H, W, make_pixdecode(H, W));
+  return after_launch();
+}
+
 }  // namespace vsr
 
 extern "C" int vsr_resample2d_backward(const float* input1, const float* flow, const float* grad_output,
@@ -721,9 +730,7 @@ extern "C" int vsr_resample2d_backward(const float* input1, const float* flow, c
   resample2d_backward_input1_kernel<<<grid_for(n, kThreads), kThreads, 0, st>>>(flow, grad_output, grad_input1, B, C, H, W, pd);
   int rc = after_launch();
   if (rc) return rc;
-  resample2d_backward_input2_kernel<<<grid_for(n, kThreads), kThreads, 0, st>>>(input1, flow, grad_output, grad_input2, B, C, H,
-                                                                               W, pd);
-  return after_launch();
+  return launch_resample2d_backward_input2(input1, flow, grad_output, grad_input2, B, C, H, W, st);
 }
 
 extern "C" int vsr_channelnorm_forward_typed(const void* input, void* output, int B, int C, int H, int W, int norm_deg,

@@ -56,9 +56,36 @@ def resample2d(input1: torch.Tensor, flow: torch.Tensor, kernel_size: int = 1, b
     return out
 
 
+def _deterministic(flag: bool | None) -> bool:
+    """None follows torch.use_deterministic_algorithms; True / False force the choice."""
+    return torch.are_deterministic_algorithms_enabled() if flag is None else bool(flag)
+
+
+def _resample2d_backward_into(input1: torch.Tensor, flow: torch.Tensor, grad_output: torch.Tensor,
+                             grad_input1: torch.Tensor, grad_input2: torch.Tensor, kernel_size: int = 1,
+                             bilinear: bool = True, deterministic: bool | None = None) -> None:
+    """Resample2d's backward into caller-allocated gradients (grad_input1 zero-filled, as the reference's caller
+    passes it).  deterministic: grad_input1 bit-identical to the CPU restatement instead of fp32 atomics in arrival
+    order; None follows torch.are_deterministic_algorithms_enabled()."""
+    B, C, H, W = grad_output.shape
+    L = _lib.lib()
+    with torch.cuda.device(grad_output.device):
+        if _deterministic(deterministic):
+            ws = _workspace(int(L.vsr_resample2d_backward_deterministic_workspace_bytes(B, H, W)), grad_output.device)
+            _lib.check(L.vsr_resample2d_backward_deterministic(
+                input1.data_ptr(), flow.data_ptr(), grad_output.data_ptr(), grad_input1.data_ptr(),
+                grad_input2.data_ptr(), B, C, H, W, int(kernel_size), int(bool(bilinear)), ws.data_ptr(), ws.numel(),
+                _stream()), "resample2d_backward")
+        else:
+            _lib.check(L.vsr_resample2d_backward(input1.data_ptr(), flow.data_ptr(), grad_output.data_ptr(),
+                                                 grad_input1.data_ptr(), grad_input2.data_ptr(), B, C, H, W,
+                                                 int(kernel_size), int(bool(bilinear)), _stream()), "resample2d_backward")
+
+
 def resample2d_backward(input1: torch.Tensor, flow: torch.Tensor, grad_output: torch.Tensor, kernel_size: int = 1,
-                        bilinear: bool = True):
-    """(grad_input1, grad_input2) of Resample2d.  ref: Resample2dFunction.backward (resample2d.py:25-39)."""
+                        bilinear: bool = True, deterministic: bool | None = None):
+    """(grad_input1, grad_input2) of Resample2d.  ref: Resample2dFunction.backward (resample2d.py:25-39).
+    deterministic: see _resample2d_backward_into."""
     for t, n in ((input1, "input1"), (flow, "input2"), (grad_output, "grad_output")):
         _req(t, torch.float32, n)
     B, C, H, W = grad_output.shape
@@ -66,10 +93,7 @@ def resample2d_backward(input1: torch.Tensor, flow: torch.Tensor, grad_output: t
         raise ValueError("resample2d_backward: input1/grad_output (B,C,H,W) and flow (B,2,H,W) must agree")
     g1 = torch.zeros_like(input1)                     # the scatter accumulates into it (resample2d.py:32)
     g2 = torch.empty_like(flow)
-    with torch.cuda.device(input1.device):
-        _lib.check(_lib.lib().vsr_resample2d_backward(input1.data_ptr(), flow.data_ptr(), grad_output.data_ptr(),
-                                                      g1.data_ptr(), g2.data_ptr(), B, C, H, W, int(kernel_size),
-                                                      int(bool(bilinear)), _stream()), "resample2d_backward")
+    _resample2d_backward_into(input1, flow, grad_output, g1, g2, kernel_size, bilinear, deterministic)
     return g1, g2
 
 
@@ -225,11 +249,14 @@ def channelnorm(x: torch.Tensor, norm_deg: int = 2) -> torch.Tensor:
     return out
 
 
-def project_flow(flow: torch.Tensor, inv_depth: torch.Tensor | None = None, max_disp: float | None = None):
+def project_flow(flow: torch.Tensor, inv_depth: torch.Tensor | None = None, max_disp: float | None = None,
+                 deterministic: bool | None = None):
     """Forward flow projection (SURVEY.md Appendix B).  flow (B,h,w,2); inv_depth (B,h,w) or None.
     Returns proj (B,h,w,2) f32, wsum (B,h,w) f32, count (B,h,w) i32, hole (B,h,w) u8.
     max_disp: a promised bound on |fx|, |fy| (<= 8 px) selects the shared-memory tile path; a broken promise is
-    detected on the device and costs time, never correctness.  None: no assumption (atomic scatter path)."""
+    detected on the device and costs time, never correctness.  None: no assumption (atomic scatter path).
+    deterministic: the sort-and-gather path, bit-identical to the CPU restatement (oracle.or_flow_projection) on every
+    run; max_disp is then ignored.  None follows torch.are_deterministic_algorithms_enabled()."""
     _req(flow, torch.float32, "flow")
     B, h, w, two = flow.shape
     if two != 2:
@@ -245,6 +272,13 @@ def project_flow(flow: torch.Tensor, inv_depth: torch.Tensor | None = None, max_
     hole = torch.empty((B, h, w), dtype=torch.uint8, device=dev)
     L = _lib.lib()
     with torch.cuda.device(dev):
+        if _deterministic(deterministic):
+            ws = _workspace(int(L.vsr_flow_projection_deterministic_workspace_bytes(B, h, w)), dev)
+            _lib.check(L.vsr_flow_projection_forward_deterministic(
+                flow.data_ptr(), inv_depth.data_ptr() if inv_depth is not None else None, proj.data_ptr(),
+                wsum.data_ptr(), count.data_ptr(), hole.data_ptr(), ws.data_ptr(), ws.numel(), B, h, w, _stream()),
+                "project_flow")
+            return proj, wsum, count, hole
         nbytes = int(L.vsr_flow_projection_workspace_bytes(B, h, w))
         ws = _workspace(nbytes, dev)
         _lib.check(L.vsr_flow_projection_forward_bounded(
@@ -254,11 +288,12 @@ def project_flow(flow: torch.Tensor, inv_depth: torch.Tensor | None = None, max_
     return proj, wsum, count, hole
 
 
-def project_depth_flow(flow: torch.Tensor, inv_depth: torch.Tensor, max_disp: float | None = None):
+def project_depth_flow(flow: torch.Tensor, inv_depth: torch.Tensor, max_disp: float | None = None,
+                       deterministic: bool | None = None):
     """Inverse-depth-weighted projection (nearer surfaces dominate contested targets)."""
     if inv_depth is None:
         raise ValueError("project_depth_flow: inv_depth is required")
-    return project_flow(flow, inv_depth, max_disp)
+    return project_flow(flow, inv_depth, max_disp, deterministic)
 
 
 def flow_to_image(flow: torch.Tensor, out_size=None, want_u8: bool = True):

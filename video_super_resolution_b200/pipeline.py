@@ -152,7 +152,9 @@ class GraphedStep:
     Inputs live in static device buffers (`inputs`: copy -- or H2D-copy -- each window into them, then `replay()`);
     outputs are the static `frame_u8` (s*h, s*w, 3) and, with want_f32, `frame` (1,3,s*h,s*w).
     The step is GPU-bound (100 ms of kernels against ~1 ms of launch calls), so this buys little at C2; it matters for
-    small frames, where the front's 40 launches of 5-10 us each are launch-latency bound."""
+    small frames, where the front's 40 launches of 5-10 us each are launch-latency bound.
+    The graph holds whichever projection path torch.are_deterministic_algorithms_enabled() selected at capture time
+    (ops.project_flow): changing the flag afterwards does not change what replay() runs."""
 
     def __init__(self, pipe: "WarpFusePipeline", want_f32: bool = False, warmup: int = 2):
         T, h, w, s, dev = pipe.T, pipe.h, pipe.w, pipe.scale, pipe.device
