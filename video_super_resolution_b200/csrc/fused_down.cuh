@@ -43,6 +43,9 @@ constexpr int kWdRingBytes = 2 * kWdGroupBytes;  // streamed per group from L2 t
 constexpr int kWtChunkBytes = 32 * 32 * 2;   // one 32x32 downtran slice (64-byte rows, 64B swizzle)
 constexpr int kHBytes = 128 * 128 * 2;       // phase-B A operand of one sub-position group
 constexpr int kXchgBytes = 3 * 4 * 16 * 8 * 4;   // row partials handed from lane quarter q+1 to q: [3][4 subs][16 px][8 ch] fp32
+constexpr int kLRBox = 16 * 9 * 64;         // fused_updown_kernel: one LR box [32 ch, 16, 9 rows] (64B swizzle)
+constexpr int kLRBytes = 2 * kLRBox;         // the dx = -1 and dx = 0 boxes of a tile
+constexpr int kWuTapBytes = 128 * 32 * 2;    // transposed-conv weights of one LR tap for 4 sub-positions: [128 n][32 k]
 
 struct alignas(64) FusedDownParams {
   CUtensorMap hr_maps[kMaxSources];   // HAS_TRAN: 4-D (64, w+1, h+1, 8*B) pair planes, box (64,16,8,1) = 2 sub-positions, 128B swizzle
@@ -57,6 +60,11 @@ struct alignas(64) FusedDownParams {
   const float* down_bias;             // [32] biases + [1] PReLU slope of the strided conv
   float* part;                        // (B, h, w, 4 slots, 32) fp32 partial sums of the BOUNDARY pixels (see final epilogue)
   void* lr_out;                       // (B, h, w, 32) bf16: finished interior pixels
+  // fused_updown_kernel only (hr_maps[nsrc-1] is then the store view of hr[nsrc-1])
+  CUtensorMap up_map;                 // the transposed conv's input (B, h, w, 32), box (32,16,9,1), 64B swizzle
+  CUtensorMap wu_map;                 // its weights 2-D (128, 512), box (32,128), 64B swizzle
+  const float* up_bias;               // [32] biases + [1] PReLU slope of the transposed conv
+  int32_t hr_store;                   // 1: store U into hr[nsrc-1] (a later group reads it)
 };
 
 __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
@@ -73,12 +81,20 @@ inline size_t fused_down_smem_bytes(int nsrc, int num_stages) {
   return 1024 + kWdRingBytes + wt + (HAS_TRAN ? kHBytes : 0) + (size_t)num_stages * stage + 1024 + kXchgBytes;
 }
 
-template <bool HAS_TRAN>
-__global__ void __launch_bounds__(kFusedThreads, 1)
-fused_down_kernel(const __grid_constant__ FusedDownParams p) {
+inline size_t fused_updown_smem_bytes(int nsrc, int num_stages) {
+  return fused_down_smem_bytes<true>(nsrc, num_stages) + kLRBytes;
+}
+
+// MERGED (HAS_TRAN only): the kernel also computes the newest source hr[nsrc-1] itself (see fused_updown_kernel)
+template <bool HAS_TRAN, bool MERGED>
+__device__ __forceinline__ void fused_down_body(const FusedDownParams& p) {
+  static_assert(HAS_TRAN || !MERGED, "the merged kernel needs phase A");
   constexpr int kStageBytes = HAS_TRAN ? 16384 : 2 * 16384;
   constexpr int kTmemCols = HAS_TRAN ? 512 : 256;
-  constexpr uint32_t kDB = HAS_TRAN ? 256 : 0;       // first column of the two D_B accumulators
+  // TMEM columns: D_A [0, 256) (two buffers, HAS_TRAN), D_B [kDB, kDB + 128 * kDBufs); MERGED: T_U [kTU, kTU + 128)
+  constexpr uint32_t kDB = MERGED ? 384 : HAS_TRAN ? 256 : 0;
+  constexpr int kDBToggle = MERGED ? 0 : 1;          // MERGED: one D_B buffer (tb stays 0)
+  constexpr uint32_t kTU = 256;
 
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -86,7 +102,8 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
   uint8_t* s_wt = s_wd + kWdRingBytes;
   const int wt_region = HAS_TRAN ? ((p.nsrc * kWtChunkBytes + 1023) / 1024 * 1024) : 0;
   uint8_t* s_h = s_wt + wt_region;
-  uint8_t* s_a = s_h + (HAS_TRAN ? kHBytes : 0);
+  uint8_t* s_lr = s_h + (HAS_TRAN ? kHBytes : 0);                // MERGED: the tile's two LR boxes
+  uint8_t* s_a = s_lr + (MERGED ? kLRBytes : 0);
   uint8_t* tail = s_a + p.num_stages * kStageBytes;
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(tail);      // [kFusedMaxStages]
   uint64_t* empty_bar = full_bar + kFusedMaxStages;            // [kFusedMaxStages]
@@ -100,8 +117,14 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
   uint64_t* db_full = h_empty + 1;                             // [2]
   uint64_t* db_empty = db_full + 2;                            // [2]
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(db_empty + 2);
+  uint64_t* tu_full = db_empty + 3;                            // MERGED: [1] T_U accumulated
+  uint64_t* tu_empty = tu_full + 1;                            // [1] T_U read by the epilogue
+  uint64_t* u_full = tu_empty + 1;                             // [1] U_g written into s_h
+  uint64_t* lr_full = u_full + 1;                              // [1] LR boxes of the tile loaded
+  uint64_t* lr_empty = lr_full + 1;                            // [1] LR boxes consumed (last T_U MMA of the tile)
   float* s_bias = reinterpret_cast<float*>(tail + 512);        // 33 floats: downtran bias + slope
   float* s_down = s_bias + 36;                                 // 33 floats: strided-conv bias + slope
+  float* s_ubias = s_down + 36;                                // MERGED: 33 floats: transposed-conv bias + slope
   float4* s_x = reinterpret_cast<float4*>(tail + 1024);        // kXchgBytes: final-epilogue row exchange
 
   const int cta = blockIdx.x, ncta = gridDim.x;   // persistent CTAs: tiles cta, cta + ncta, ...
@@ -125,11 +148,20 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
     }
     mbar_init(h_full, kFusedEpiWarps);
     mbar_init(h_empty, 1);
+    if (MERGED) {
+      mbar_init(tu_full, 1);
+      mbar_init(tu_empty, kFusedEpiWarps);
+      mbar_init(u_full, 1);
+      mbar_init(lr_full, 1);
+      mbar_init(lr_empty, 1);
+    }
     fence_barrier_init();
   }
   if (warp == 1) tmem_alloc<kTmemCols>(tmem_ptr);
   if (HAS_TRAN)
     for (int i = threadIdx.x; i < 33; i += kFusedThreads) s_bias[i] = p.tran_bias[i];
+  if (MERGED)
+    for (int i = threadIdx.x; i < 33; i += kFusedThreads) s_ubias[i] = p.up_bias[i];
   for (int i = threadIdx.x; i < 33; i += kFusedThreads) s_down[i] = p.down_bias[i];
   tc_fence_before();
   __syncthreads();
@@ -163,7 +195,7 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
             // one box = 2 sub-positions x 128 blocks x 32 ch (16 KB): a [128 x 64] K-major tile whose K
             // halves are the two sub-positions (box count, not bytes, limits a single-thread producer)
             for (int sp = half * 8; sp < half * 8 + 8; sp += 2) {
-              for (int j = 0; j < p.nsrc; ++j) {
+              for (int j = 0; j < p.nsrc - (MERGED ? 1 : 0); ++j) {   // MERGED: the newest source is made on chip
                 mbar_wait(&empty_bar[s], phase ^ 1);
                 if (elect_one()) {
                   mbar_expect_tx(&full_bar[s], kStageBytes);
@@ -209,6 +241,34 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
     const uint64_t dWt = make_smem_desc<64>(smem_u32(s_wt));
     const uint64_t dH = make_smem_desc<128>(smem_u32(s_h));
     const uint64_t dWd = make_smem_desc<128>(smem_u32(s_wd));
+    uint32_t n_tu = 0, n_lr = 0, n_u = 0;
+
+    // MERGED, transposed conv of group g: T_U[128 blocks, 4 sub-positions x 32] = LR taps * Wu_g^T, K = 4 taps x 32
+    // channels in igemm_kernel<EPI_DECONV>'s order (tap, then 16-wide K steps): every accumulator column gets the
+    // same additions in the same order as there, N = 128 instead of 256 changes no column's sum
+    auto issue_u = [&](int g) {
+      constexpr uint32_t idesc_u = make_idesc(128);
+      const uint64_t dLR = make_smem_desc<64>(smem_u32(s_lr));
+      const uint64_t dWu = make_smem_desc<64>(smem_u32(s_wd));
+      if (g == 0) mbar_wait(lr_full, n_lr & 1);
+      mbar_wait(tu_empty, (n_tu & 1) ^ 1);
+      mbar_wait(&wd_full[0], n_tu & 1);
+      tc_fence_after();
+      if (elect_one()) {
+#pragma unroll
+        for (int t = 0; t < 4; ++t)
+#pragma unroll
+          for (int k = 0; k < 2; ++k)
+            umma_bf16(tmem_base + kTU, dLR + (uint64_t)(((t & 1) * kLRBox + (t >> 1) * 1024) >> 4) + 2 * k,
+                      dWu + (uint64_t)((t * kWuTapBytes) >> 4) + 2 * k, idesc_u, (uint32_t)((t | k) != 0));
+        umma_commit(&wd_empty[0]);
+        umma_commit(tu_full);
+        if (g == 3) umma_commit(lr_empty);
+      }
+      __syncwarp();
+      ++n_tu;
+      if (g == 3) ++n_lr;
+    };
 
     // phase A of sub-position group g: D_A[g&1] = sum_j A(s, j) * Wt_j^T for the 4 sub-positions
     auto issue_a = [&](int g) {
@@ -216,7 +276,7 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
       mbar_wait(&da_empty[buf], (n_a[buf] & 1) ^ 1);
       tc_fence_after();
       for (int pair = 0; pair < 2; ++pair)
-        for (int j = 0; j < p.nsrc; ++j) {
+        for (int j = 0; j < p.nsrc - (MERGED ? 1 : 0); ++j) {
           mbar_wait(&full_bar[s], phase);
           tc_fence_after();
           const uint64_t a0 = dA + (uint64_t)((s * kStageBytes) >> 4);
@@ -229,11 +289,31 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
             umma_bf16(d0 + 32, a0 + 4, b0, idesc_a, acc);
             umma_bf16(d0 + 32, a0 + 6, b0 + 2, idesc_a, 1u);
             umma_commit(&empty_bar[s]);
-            if (pair == 1 && j == p.nsrc - 1) umma_commit(&da_full[buf]);
+            if (!MERGED && pair == 1 && j == p.nsrc - 1) umma_commit(&da_full[buf]);
           }
           __syncwarp();
           if (++s == p.num_stages) { s = 0; phase ^= 1; }
         }
+      if (MERGED) {
+        // the last source, j = nsrc - 1, is U_g in s_h (the epilogue's conversion of T_U): the same operand bytes a TMA
+        // box of hr[nsrc-1] would bring, added last into each column as before
+        mbar_wait(u_full, n_u & 1);
+        tc_fence_after();
+        const uint64_t b0 = dWt + (uint64_t)(((p.nsrc - 1) * kWtChunkBytes) >> 4);
+        if (elect_one()) {
+          for (int pair = 0; pair < 2; ++pair) {
+            const uint64_t a0 = dH + (uint64_t)((pair * 16384) >> 4);
+            const uint32_t d0 = tmem_base + (uint32_t)(buf * 128 + pair * 64);
+            umma_bf16(d0, a0, b0, idesc_a, 1u);
+            umma_bf16(d0, a0 + 2, b0 + 2, idesc_a, 1u);
+            umma_bf16(d0 + 32, a0 + 4, b0, idesc_a, 1u);
+            umma_bf16(d0 + 32, a0 + 6, b0 + 2, idesc_a, 1u);
+          }
+          umma_commit(&da_full[buf]);
+        }
+        __syncwarp();
+        ++n_u;
+      }
       ++n_a[buf];
     };
     // phase B of group g: D_B[tb] += H_g * Wd_g^T
@@ -247,8 +327,9 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
         a0 = dA + (uint64_t)((s * kStageBytes) >> 4);
       }
       if (g == 0) mbar_wait(&db_empty[tb], (n_b[tb] & 1) ^ 1);
-      const int wslot = (int)(n_wd & 1);
-      mbar_wait(&wd_full[wslot], (n_wd >> 1) & 1);
+      // MERGED: slot 0 of the weight ring holds the transposed-conv weights, slot 1 the conv weights
+      const int wslot = MERGED ? 1 : (int)(n_wd & 1);
+      mbar_wait(&wd_full[wslot], MERGED ? (n_wd & 1) : ((n_wd >> 1) & 1));
       tc_fence_after();
       const uint32_t d = tmem_base + kDB + (uint32_t)(tb * 128);
       const uint64_t b0 = dWd + (uint64_t)((wslot * kWdGroupBytes) >> 4);
@@ -268,7 +349,7 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
       ++n_wd;
       if (HAS_TRAN) ++n_h;
       else if (++s == p.num_stages) { s = 0; phase ^= 1; }
-      if (g == 3) { ++n_b[tb]; tb ^= 1; }
+      if (g == 3) { ++n_b[tb]; tb ^= kDBToggle; }
     };
 
     // HAS_TRAN: this thread issues phase A only; phase B has its own issuing thread (warp kFusedBWarp), so
@@ -277,7 +358,10 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
     for (int tile = cta; tile < total_tiles; tile += ncta) {
       if (HAS_TRAN) {
         if (warp == 1) {
-          for (int g = 0; g < 4; ++g) issue_a(g);
+          for (int g = 0; g < 4; ++g) {
+            if (MERGED) issue_u(g);
+            issue_a(g);
+          }
         } else {
           for (int g = 0; g < 4; ++g) issue_b(g);
         }
@@ -286,6 +370,49 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
       }
     }
     }
+  } else if (MERGED && warp == kFusedWdWarp) {
+    // ===================== LR-box + weight streamer (MERGED) =====================
+    // slot 0 of the weight ring: the transposed-conv weights Wu_g (4 taps x [128 n][32 k], 64B swizzle), slot 1: the
+    // conv weights Wd_g.  Wu of the next group is requested before Wd of this one: Wu_{g+1} only waits for the T_U
+    // MMAs of group g, Wd_g for phase B of group g-1.  The LR boxes of a tile go with its Wu_0 (both wait for the last
+    // T_U MMAs of the previous tile).
+    uint32_t n_wu = 0, n_wdm = 0, n_lrl = 0;
+    auto load_u = [&](int tile, int g) {
+      if (g == 0) {
+        int x0, y0, b;
+        tile_coord(tile, x0, y0, b);
+        mbar_wait(lr_empty, (n_lrl & 1) ^ 1);
+        if (elect_one()) {
+          // dx = -1 and dx = 0 boxes of 16 x 9 LR pixels; the dy = -1 / 0 taps are rows 0 and 1 of them
+          mbar_expect_tx(lr_full, (uint32_t)kLRBytes);
+          tma_load_4d(s_lr, &p.up_map, lr_full, 0, x0 - 1, y0 - 1, b);
+          tma_load_4d(s_lr + kLRBox, &p.up_map, lr_full, 0, x0, y0 - 1, b);
+        }
+        __syncwarp();
+        ++n_lrl;
+      }
+      mbar_wait(&wd_empty[0], (n_wu & 1) ^ 1);
+      if (elect_one()) {
+        mbar_expect_tx(&wd_full[0], kWdGroupBytes);
+        for (int t = 0; t < 4; ++t) tma_load_2d(s_wd + t * kWuTapBytes, &p.wu_map, &wd_full[0], t * 32, g * 128);
+      }
+      __syncwarp();
+      ++n_wu;
+    };
+    if (cta < total_tiles) load_u(cta, 0);
+    for (int tile = cta; tile < total_tiles; tile += ncta)
+      for (int g = 0; g < 4; ++g) {
+        if (g < 3) load_u(tile, g + 1);
+        else if (tile + ncta < total_tiles) load_u(tile + ncta, 0);
+        mbar_wait(&wd_empty[1], (n_wdm & 1) ^ 1);
+        if (elect_one()) {
+          mbar_expect_tx(&wd_full[1], kWdGroupBytes);
+          tma_load_2d(s_wd + kWdGroupBytes, &p.wd_map, &wd_full[1], (2 * g) * 64, 0);
+          tma_load_2d(s_wd + kWdGroupBytes + 16384, &p.wd_map, &wd_full[1], (2 * g + 1) * 64, 0);
+        }
+        __syncwarp();
+        ++n_wdm;
+      }
   } else if (warp == kFusedWdWarp) {
     // ===================== conv-weight streamer =====================
     // every tile needs the 128 KB of 8x8-s4 weights once, 32 KB per sub-position group; all SMs
@@ -315,6 +442,7 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
     uint32_t m_a[2] = {0, 0}, m_b[2] = {0, 0}, m_h = 0;
     int tb = 0;
     const PreluCfg pc = make_prelu(HAS_TRAN ? s_bias[32] : 1.0f, 1);
+    uint32_t m_u = 0;
     for (int tile = cta; tile < total_tiles; tile += ncta) {
       int x0, y0, b;
       tile_coord(tile, x0, y0, b);
@@ -324,6 +452,44 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
 #pragma unroll 1
         for (int g = 0; g < 4; ++g) {
           const int buf = g & 1;
+          if (MERGED) {
+            // U_g = PReLU(T_U + b): sub-position s16 of this warp, zero ring as in igemm_kernel<EPI_DECONV>, written
+            // into s_h in the layout of the two pair-plane TMA boxes -- phase A's operand for source nsrc-1 and, for
+            // the groups whose hr map a later group reads, the source of two TMA stores into it
+            mbar_wait_poll(tu_full, m_u & 1);
+            tc_fence_after();
+            uint32_t v[32];
+            tmem_ld32(lane_base + kTU + (uint32_t)(sub * 32), v);
+            tmem_ld_wait();
+            tc_fence_before();
+            mbar_arrive_warp(tu_empty);
+            ++m_u;
+            const int s16 = g * 4 + sub, ry = s16 >> 2, rx = s16 & 3;
+            const int Yt = 4 * Yb + ry - 2, Xt = 4 * Xb + rx - 2;
+            const bool inside = (Yt >= 0) && (Yt < 4 * p.lr_h) && (Xt >= 0) && (Xt < 4 * p.lr_w);
+            uint32_t o[16];
+            const PreluCfg pcu = make_prelu(s_ubias[32], 1);
+            convert32(v, s_ubias, pcu, o);
+            if (__builtin_expect(!inside, 0)) zero16(o);
+            mbar_wait(h_empty, (m_h & 1) ^ 1);     // phase B of the previous group has read H from s_h
+            uint8_t* urow = s_h + (sub >> 1) * 16384 + row * 128;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              const int piece = (sub & 1) * 4 + j;
+              *reinterpret_cast<uint4*>(urow + ((piece ^ (row & 7)) << 4)) =
+                  make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
+            }
+            fence_async_smem();
+            asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");   // all of U_g is written
+            if (threadIdx.x == 64) {   // one thread issues and later waits for the stores (bulk groups are per thread)
+              if (p.hr_store) {
+                tma_store_4d(&p.hr_maps[p.nsrc - 1], s_h, 0, x0, y0, b * 8 + 2 * g);
+                tma_store_4d(&p.hr_maps[p.nsrc - 1], s_h + 16384, 0, x0, y0, b * 8 + 2 * g + 1);
+                tma_store_commit();
+              }
+              mbar_arrive(u_full);
+            }
+          }
           mbar_wait_poll(&da_full[buf], m_a[buf] & 1);
           tc_fence_after();
           uint32_t o[16];
@@ -338,7 +504,15 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
           convert32(v, s_bias, pc, o);
           if (__builtin_expect(!(in_tensor && !ring), 0)) zero16(o);
           ++m_a[buf];
-          mbar_wait(h_empty, (m_h & 1) ^ 1);
+          if (MERGED) {
+            // D_A is complete, so phase A has read U_g; the stores must have read it too before H overwrites it
+            if (p.hr_store) {
+              if (threadIdx.x == 64) tma_store_wait_read();
+              asm volatile("bar.sync 1, %0;" ::"n"(32 * kFusedEpiWarps) : "memory");
+            }
+          } else {
+            mbar_wait(h_empty, (m_h & 1) ^ 1);
+          }
           // K index inside the group: k = sub*32 + c -> 64-element chunk kc = sub>>1, 16-byte piece (sub&1)*4 + j
           uint8_t* hrow = s_h + (sub >> 1) * 16384 + (row >> 3) * 1024 + (row & 7) * 128;
 #pragma unroll
@@ -431,8 +605,9 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
         }
       }
       ++m_b[tb];
-      tb ^= 1;
+      tb ^= kDBToggle;
     }
+    if (MERGED && threadIdx.x == 64) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // the last stores
   }
 
   tc_fence_before();
@@ -441,6 +616,39 @@ fused_down_kernel(const __grid_constant__ FusedDownParams p) {
     tc_fence_after();
     tmem_dealloc<kTmemCols>(tmem_base);
   }
+}
+
+template <bool HAS_TRAN>
+__global__ void __launch_bounds__(kFusedThreads, 1)
+fused_down_kernel(const __grid_constant__ FusedDownParams p) {
+  fused_down_body<HAS_TRAN, false>(p);
+}
+
+// One feedback group i >= 1 of the x4 stack with its transposed conv inside:
+//
+//     lr[i+1] = PReLU( Conv8x8s4( PReLU( Conv1x1( cat(hr[0..i-1], U_i) ) ) ) ),   U_i = PReLU( Deconv8x8s4(up_in) + b )
+//
+// U_i is made on chip one sub-position group g at a time, in the order phase A walks: the transposed conv's MMAs
+// (T_U = LR taps * Wu_g^T, the 2 LR boxes of igemm_kernel<EPI_DECONV> loaded once per tile), the epilogue's conversion
+// into s_h in the 128B-swizzled layout of the two pair-plane boxes phase A would load, two TMA stores of that buffer
+// into hr[i] (only when a later group reads hr[i]: hr_store), and phase A's MMAs for source i from it.  Against the
+// layered pair this removes the read of hr[i] (and for the last group its write) and the transposed conv's launch;
+// the sums are the same additions in the same order, so the results are bit-identical.
+//
+// Resources (-Xptxas -v: 1 CTA per SM, no spills):
+//  * TMEM, 512 columns: D_A double-buffered [0, 256), T_U [256, 384), D_B single [384, 512).  The epilogue is one
+//    in-order sequence (U_g, H_g for g = 0..3, then the tile's D_B), so it always reads D_B before it produces the
+//    next tile's first H and a second D_B buffer could never be used; a second D_A buffer lets phase A of group g+1
+//    consume ring stages while the epilogue still reads D_A of group g.
+//  * Weights: the 2 x 32 KB ring of the conv weights; slot 0 carries Wu_g (transposed conv, 32 KB per g), slot 1
+//    Wd_g.  Both are L2 hits (every SM streams the same bytes).
+//  * Shared memory: U_g and H_g share the 32 KB s_h (U_g is dead once D_A of g is complete and its stores have read
+//    it; U_{g+1} waits for phase B of g); the LR boxes take 18 KB.  Activation ring: the deepest that fits, 6 x 16 KB
+//    stages for nsrc 4, 5 for nsrc 5-6 (the layered kernel: 7 / 6); a ring one stage deeper does not fit, so the
+//    comparison against one stage more is not measured.
+__global__ void __launch_bounds__(kFusedThreads, 1)
+fused_updown_kernel(const __grid_constant__ FusedDownParams p) {
+  fused_down_body<true, true>(p);
 }
 
 // Boundary pixels (rows Y % 8 == 7 and columns X % 16 == 15; see the fused kernel's final epilogue):

@@ -89,7 +89,7 @@ int make_w_map(CUtensorMap* m, const void* base, int64_t K, int64_t N, int ck, i
 // ------------------------------------------------------------------------------------------------
 // kernel variants
 // ------------------------------------------------------------------------------------------------
-enum Variant : int { V_PW32 = 0, V_PW128, V_DECONV, V_CONVOUT, V_FUSED_TRAN, V_FUSED_PLAIN, V_FINALIZE, V_DECONV2, V_DOWN2, V_COUNT };
+enum Variant : int { V_PW32 = 0, V_PW128, V_DECONV, V_CONVOUT, V_FUSED_TRAN, V_FUSED_PLAIN, V_FINALIZE, V_DECONV2, V_DOWN2, V_FUSED_UPDOWN, V_COUNT };
 
 // kernel classes for the per-launch accounting bench.py reads (vsr_srfbn_profile_*)
 static_assert(VSR_SRFBN_KERNEL_CLASSES == 10, "header constant");
@@ -139,8 +139,21 @@ int launch_fused(const Layer& L, cudaStream_t st) {
   return after_launch();
 }
 
+int launch_fused_updown(const Layer& L, cudaStream_t st) {
+  static PerDeviceOnce once;
+  int dev;
+  if (once.needed(&dev)) {
+    cudaError_t e = cudaFuncSetAttribute(fused_updown_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (e != cudaSuccess) return cuda_status(e);
+    once.mark(dev);
+  }
+  fused_updown_kernel<<<L.grid, kFusedThreads, L.smem, st>>>(L.f);
+  return after_launch();
+}
+
 int launch_layer(const Layer& L, cudaStream_t st) {
   switch (L.variant) {
+    case V_FUSED_UPDOWN: return launch_fused_updown(L, st);
     case V_FUSED_TRAN: return launch_fused<true>(L, st);
     case V_FUSED_PLAIN: return launch_fused<false>(L, st);
     case V_FINALIZE: {
@@ -488,6 +501,62 @@ int build_fused_down(Layer& L, const void* const* hr, int nsrc, int B, int h, in
   return VSR_OK;
 }
 
+// Feedback groups whose transposed conv runs inside the down kernel (fused_updown_kernel) instead of as its own launch
+// in front of it.  The merged kernel does not go below ~2.0 ms per C2 launch (its per-group chain T_U -> U_g -> phase A
+// -> H_g -> phase B bounds it, not HBM).  Measured on a B200 at 1000 W against transposed conv + fused down kernel, us
+// per launch, nsrc 2..6: 1969 / 1992 / 2002 / 2289 / 2410 against 1762 / 1949 / 2256 / 2657 / 3121 (profiles/
+// updown_ab.log).  So groups 3-5 run merged; groups 1-2 and group 0 (no phase A) keep the layered pair.
+inline bool updown_merged(int nsrc) { return nsrc >= 4; }
+
+// ConvTranspose2d(32,32,8,4,2) of up_in into hr[nsrc-1] (kept only if `store`) + downtran over hr[0..nsrc-1] + PReLU +
+// Conv2d(32,32,8,4,2) pre-activation sums, one launch (fused_updown_kernel); nsrc >= 2.  hr[nsrc-1] may be null when
+// !store.
+int build_fused_updown(Layer& L, const void* up_in, const void* const* hr, int nsrc, int store, int B, int h, int w,
+                       const void* wu_dev, const float* up_bias_dev, const void* wt_dev, const float* tran_bias_dev,
+                       const void* wd_dev, const float* down_bias_dev, float* part, void* lr_out) {
+  memset(&L, 0, sizeof(L));
+  L.variant = V_FUSED_UPDOWN;
+  FusedDownParams& f = L.f;
+  if (nsrc < 2 || nsrc > kMaxSources || (store && !hr[nsrc - 1])) return VSR_ERR_UNSUPPORTED;
+  int rc;
+  // hr[0..nsrc-2]: phase-A loads; hr[nsrc-1]: the store view (the same pair-plane boxes)
+  for (int j = 0; j < nsrc - (store ? 0 : 1); ++j) {
+    rc = make_act_map(&f.hr_maps[j], hr[j], 64, w + 1, h + 1, 8 * B, 64, 16, 8);
+    if (rc) return rc;
+  }
+  rc = make_w_map(&f.wt_map, wt_dev, 32 * nsrc, 32, 32, 32);
+  if (rc) return rc;
+  rc = make_w_map(&f.wd_map, wd_dev, 512, 128, 64, 128);
+  if (rc) return rc;
+  rc = make_act_map(&f.up_map, up_in, kNF, w, h, B, 32, kTW, kTH + 1);   // igemm_kernel<EPI_DECONV>'s LR box
+  if (rc) return rc;
+  rc = make_w_map(&f.wu_map, wu_dev, 4 * kNF, 512, 32, 128);
+  if (rc) return rc;
+  f.nsrc = nsrc;
+  f.tiles_x = ceil_div(w + 1, 16);
+  f.tiles_y = ceil_div(h + 1, 8);
+  f.batch = B;
+  f.lr_h = h;
+  f.lr_w = w;
+  f.tran_bias = tran_bias_dev;
+  f.down_bias = down_bias_dev;
+  f.up_bias = up_bias_dev;
+  f.part = part;
+  f.lr_out = lr_out;
+  f.hr_store = store;
+  const int64_t total = (int64_t)f.tiles_x * f.tiles_y * B;
+  L.grid = (int)(total < kNumSMs ? total : kNumSMs);
+  f.num_stages = 7;
+  while (f.num_stages > 2 && fused_updown_smem_bytes(nsrc, f.num_stages) > 227 * 1024) --f.num_stages;
+  L.smem = fused_updown_smem_bytes(nsrc, f.num_stages);
+  const double lrpx = (double)B * h * w;
+  L.kclass = KC_FUSED_DOWN;
+  L.flops = lrpx * 131072.0 * 2.0 + lrpx * 16.0 * 2.0 * 32.0 * nsrc * 32.0;   // transposed conv + downtran + conv
+  // LR map in, nsrc - 1 HR maps in, hr[nsrc-1] out if stored, one BF16 LR map out
+  L.bytes = lrpx * 64.0 + lrpx * 64.0 * 16.0 * (nsrc - 1 + (store ? 1 : 0)) + lrpx * 64.0;
+  return VSR_OK;
+}
+
 int build_finalize(Layer& L, float* acc, const float* bias_dev, void* out, int64_t pixels, int h, int w) {
   memset(&L, 0, sizeof(L));
   L.variant = V_FINALIZE;
@@ -832,7 +901,8 @@ static void layout_workspace(vsr_srfbn_plan* pl) {
   pl->o_u = put(P * 64);
   const size_t s2 = (size_t)c.upscale * c.upscale;
   const bool x2 = c.upscale == 2;
-  for (int i = 0; i < 6; ++i) pl->o_hr[i] = put(x2 ? P * s2 * 64 : Rb * 64);   // x2: plain NHWC
+  // x2: plain NHWC.  x4: hr[5] exists only when its group runs layered (the merged kernel keeps it on chip)
+  for (int i = 0; i < 6; ++i) pl->o_hr[i] = put(x2 ? P * s2 * 64 : (i == 5 && updown_merged(6)) ? 0 : Rb * 64);
   pl->o_hb = put(P * s2 * 64);   // plain-NHWC result of the `out` deconv
   pl->o_ht = put(x2 ? P * s2 * 64 : 0);   // x2: downtran result (the x4 path keeps it on chip)
   pl->o_acc = put(x2 ? 0 : P * 512);   // fp32 partial slots of the fused down kernel
@@ -1034,7 +1104,16 @@ static int build_layer_list(vsr_srfbn_plan* pl, int M, std::vector<Layer>& layer
         PUSH(build_downconv2(L, down_in, M, h, w, Wp(W_DOWN0 + i), Bp(W_DOWN0 + i), ws + pl->o_lr[i + 1]));
         continue;
       }
-      {  // upBlocks[i], then downtran(cat(hr[0..i])) + downBlocks[i] fused; sums land in the fp32 LR accumulator
+      if (updown_merged(i + 1)) {   // upBlocks[i] + downtran(cat(hr[0..i])) + downBlocks[i] in one launch
+        const void* hrs[6];
+        for (int j = 0; j <= i; ++j) hrs[j] = ws + pl->o_hr[j];
+        const int store = i + 1 < kGroups;     // hr[5] is read by no later group
+        if (!store) hrs[i] = nullptr;
+        PUSH(build_fused_updown(L, up_in, hrs, i + 1, store, M, h, w, Wp(W_UP0 + i), Bp(W_UP0 + i),
+                                Wp(W_DOWNTRAN0 + i - 1), Bp(W_DOWNTRAN0 + i - 1), Wp(W_DOWN0 + i), Bp(W_DOWN0 + i),
+                                reinterpret_cast<float*>(ws + pl->o_acc), ws + pl->o_lr[i + 1]));
+        PUSH(build_finalize(L, reinterpret_cast<float*>(ws + pl->o_acc), Bp(W_DOWN0 + i), ws + pl->o_lr[i + 1], P, h, w));
+      } else {  // upBlocks[i], then downtran(cat(hr[0..i])) + downBlocks[i] fused; sums land in the fp32 LR accumulator
         Layer D, F;
         rc = build_deconv(D, up_in, M, h, w, Wp(W_UP0 + i), Bp(W_UP0 + i), ws + pl->o_hr[i], 0);
         if (rc) return rc;
