@@ -386,6 +386,18 @@ int vsr_test_fused_down(const void* hr_bf16, int nsrc, int B, int h, int w, cons
                         const float* bt_host, float slope_t, const float* wd_host, const float* bd_host,
                         float slope_d, void* y_bf16, void* workspace, size_t workspace_bytes,
                         vsr_stream_t stream);
+/*   fused_updown: the kernel the plan uses for feedback groups 3-5 of the x4 stack, with the group's
+ *              transposed conv inside: U = PReLU(ConvTranspose2d(32,32,8,4,2)(lr)) is source nsrc-1
+ *              of the fused_down computation above.  lr (B,h,w,32) bf16;
+ *              hr: (nsrc,B,8,h+1,w+1,64) bf16 block layout, slots 0..nsrc-2 read, slot nsrc-1 receives U
+ *              (zero ring included) iff store, untouched otherwise; nsrc 2..6.  wu (32 in,32 out,8,8),
+ *              wt (32,32*nsrc), wd (32,32,8,8) fp32 host.  y (B,h,w,32) bf16.
+ *              workspace: vsr_test_workspace_bytes + B*h*w*512 bytes, any contents. */
+int vsr_test_fused_updown(const void* lr_bf16, void* hr_bf16, int nsrc, int store, int B, int h, int w,
+                          const float* wu_host, const float* bu_host, float slope_u, const float* wt_host,
+                          const float* bt_host, float slope_t, const float* wd_host, const float* bd_host,
+                          float slope_d, void* y_bf16, void* workspace, size_t workspace_bytes,
+                          vsr_stream_t stream);
 
 #ifdef __cplusplus
 }

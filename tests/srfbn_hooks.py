@@ -92,7 +92,7 @@ def fused_down(hr_bf16, wt, bt, slope_t, wd, bd, slope_d):
     dev = hr_bf16.device
     y = torch.full((B, h, wd_, 32), float("nan"), dtype=torch.bfloat16, device=dev)
     n = int(_lib.lib().vsr_test_workspace_bytes(B, h, wd_)) + B * h * wd_ * 512
-    ws = torch.empty(n, dtype=torch.uint8, device=dev)
+    ws = torch.full((n,), 0xFF, dtype=torch.uint8, device=dev)   # the fp32 partial slots start as NaN
     wd = wd.contiguous().float()
     bd = bd.contiguous().float()
     if nsrc > 1:
@@ -104,3 +104,57 @@ def fused_down(hr_bf16, wt, bt, slope_t, wd, bd, slope_d):
                                               ws.data_ptr(), ws.numel(), torch.cuda.current_stream().cuda_stream),
                "test_fused_down")
     return y
+
+
+GUARD_BITS = 0x1234          # bf16 bit pattern of the guard bands
+SENTINEL_BITS = 0x5A5A       # bf16 bit pattern of an hr slot the kernel must not write
+
+
+def _guarded(shape, dev):
+    """A bf16 tensor of `shape` between two guard bands of GUARD_BITS; returns (whole buffer, tensor, guard size)."""
+    n = 1
+    for s in shape:
+        n *= s
+    G = 1 << 16                                   # guard elements on each side (128 KB: more than a tile row)
+    buf = torch.empty((n + 2 * G,), dtype=torch.bfloat16, device=dev)
+    buf.view(torch.int16).fill_(GUARD_BITS)
+    return buf, buf[G:G + n].view(shape), G
+
+
+def _guards_intact(buf, G):
+    bits = buf.view(torch.int16)
+    return bool((bits[:G] == GUARD_BITS).all()) and bool((bits[-G:] == GUARD_BITS).all())
+
+
+def fused_updown(lr_bf16, hr_bf16, store, wu, bu, slope_u, wt, bt, slope_t, wd, bd, slope_d):
+    """One feedback group through the merged kernel (vsr_test_fused_updown).  lr (B,h,w,32) bf16: the transposed conv's
+    input; hr (nsrc,B,8,h+1,w+1,64) bf16 block layout: slots 0..nsrc-2 are the earlier sources (slot nsrc-1 is not
+    read from the caller's tensor); wu (32 in,32 out,8,8); wt (32,32*nsrc); wd (32,32,8,8).
+    Returns (y (B,h,w,32), the hr array after the call).  y and the hr array sit between guard bands that must come back
+    untouched; y starts as NaN, slot nsrc-1 as NaN (store) or SENTINEL_BITS (not store), the workspace (weights and fp32
+    partial slots) as 0xFF bytes; slots 0..nsrc-2 must come back unchanged."""
+    nsrc, B, _, hb, wb = hr_bf16.shape[:5]
+    h, w_ = hb - 1, wb - 1
+    dev = lr_bf16.device
+    assert tuple(lr_bf16.shape) == (B, h, w_, 32)
+    hbuf, hr, Gh = _guarded(tuple(hr_bf16.shape), dev)
+    hr[:nsrc - 1].copy_(hr_bf16[:nsrc - 1])
+    if store:
+        hr[nsrc - 1].fill_(float("nan"))
+    else:
+        hr[nsrc - 1].view(torch.int16).fill_(SENTINEL_BITS)
+    ybuf, y, Gy = _guarded((B, h, w_, 32), dev)
+    y.fill_(float("nan"))
+    n = int(_lib.lib().vsr_test_workspace_bytes(B, h, w_)) + B * h * w_ * 512
+    ws = torch.full((n,), 0xFF, dtype=torch.uint8, device=dev)
+    wu, bu, wt, bt, wd, bd = (t.contiguous().float() for t in (wu, bu, wt, bt, wd, bd))
+    _lib.check(_lib.lib().vsr_test_fused_updown(lr_bf16.data_ptr(), hr.data_ptr(), nsrc, int(store), B, h, w_,
+                                                _fp(wu), _fp(bu), float(slope_u), _fp(wt), _fp(bt), float(slope_t),
+                                                _fp(wd), _fp(bd), float(slope_d), y.data_ptr(), ws.data_ptr(),
+                                                ws.numel(), torch.cuda.current_stream().cuda_stream),
+               "test_fused_updown")
+    assert _guards_intact(ybuf, Gy), "fused_updown wrote outside y"
+    assert _guards_intact(hbuf, Gh), "fused_updown wrote outside the hr array"
+    assert torch.equal(hr[:nsrc - 1].view(torch.int16), hr_bf16[:nsrc - 1].view(torch.int16)), \
+        "fused_updown wrote into a source slot it only reads"
+    return y.clone(), hr.clone()

@@ -66,6 +66,21 @@ def test_host_side_entry_points_without_gpu():
     assert L.vsr_resample2d_forward(None, None, None, 1, 3, 4, 4, 1, 1, None) == 1
     assert L.vsr_resample2d_forward(1, 1, 1, 1, 3, 4, 4, 17, 1, None) == 2  # kernel_size outside 1..16
 
+    # vsr_test_fused_updown: device pointers stand in as 1 (never dereferenced), weights are real host arrays
+    w8 = (ctypes.c_float * (32 * 32 * 64))()
+    wt = (ctypes.c_float * (32 * 32 * 6))()
+    b = (ctypes.c_float * 32)()
+    B, h, w = 2, 5, 7
+    need = L.vsr_test_workspace_bytes(B, h, w) + B * h * w * 512
+
+    def updown(nsrc, wu=w8, wd=w8, ws_bytes=need, y=1):
+        return L.vsr_test_fused_updown(1, 1, nsrc, 1, B, h, w, wu, b, 0.25, wt, b, 0.3, wd, b, 0.15, y, 1, ws_bytes,
+                                       None)
+    assert updown(1) == 1 and updown(7) == 1              # nsrc outside 2..6
+    assert updown(4, wu=None) == 1 and updown(4, wd=None) == 1 and updown(4, y=None) == 1
+    assert updown(2, ws_bytes=need - 1) == 3              # VSR_ERR_WORKSPACE: one byte short of the partial slots
+    assert updown(6, ws_bytes=0) == 3
+
 
 def test_ops_refuse_cpu_tensors():
     import pytest

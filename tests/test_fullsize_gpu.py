@@ -62,7 +62,7 @@ def test_c2_conv_stack_full_size_is_deterministic_and_tiling_consistent():
     """C2 (M=20, 270x480 -> 1080x1920): (1) two runs give identical bits (no atomics in the stack);
     (2) the output over an interior window equals the output of the same network run on a crop of the
     input that contains the window's receptive field -- a check of every tile / ring / edge rule at
-    full size that needs no CPU oracle."""
+    full size that needs no CPU oracle; (3) chunked plans under workspace caps give the same bits."""
     M, h, w = 20, 270, 480
     torch.manual_seed(0)
     sr = SRProjectionModule(num_maps=M)
@@ -82,6 +82,24 @@ def test_c2_conv_stack_full_size_is_deterministic_and_tiling_consistent():
     b = yc[:, :, 4 * m:4 * (ch - m), 4 * m:4 * (cw - m)]
     assert a.shape == b.shape and a.numel() > 0
     assert (a - b).abs().max().item() <= 1e-2 * (a.abs().mean().item() + 1.0)
+    # (3) the same frame under workspace caps: 10, 5 and 4 maps per sweep over the layer list instead of 20, bit for
+    # bit (every chunk runs the merged up-down kernel of groups 3-5 on its own slice of the maps)
+    import gc
+    full = sr._plans[(M, h, w, 0)]["workspace"].numel()
+    sd = {k: v.detach().clone() for k, v in sr.state_dict().items()}
+    del sr, y2, yc, a, b
+    gc.collect()
+    torch.cuda.empty_cache()
+    for frac, chunk in ((0.55, 10), (0.3, 5), (0.23, 4)):
+        cap = SRProjectionModule(num_maps=M, workspace_cap_bytes=int(full * frac))
+        cap.load_state_dict(sd)
+        y3 = cap(x)
+        ent = next(iter(cap._plans.values()))
+        assert ent["chunk_maps"] == chunk and ent["workspace"].numel() <= full * frac, (frac, ent["chunk_maps"])
+        assert torch.equal(y3, y1), frac
+        del cap, y3, ent
+        gc.collect()
+        torch.cuda.empty_cache()
 
 
 def _oracle_maps_on_gpu(x, sd, steps, scale):

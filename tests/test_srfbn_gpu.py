@@ -88,13 +88,103 @@ def test_fused_downtran_downconv(nsrc, B, h, w):
     bt = torch.randn(32, generator=g) * 0.1
     hrb = torch.stack([hk.to_block(hr[j]) for j in range(nsrc)])
     got = hk.fused_down(hrb.to(DEV), wt, bt, 0.3, wd, bd, 0.15)
-    x = hr.float().permute(1, 4, 0, 2, 3)                                  # (B, c, nsrc, H, W)
-    x = x.permute(0, 2, 1, 3, 4).reshape(B, nsrc * 32, 4 * h, 4 * w)       # cat over sources along channels
-    if nsrc > 1:
-        x = F.prelu(F.conv2d(x, wt.view(32, 32 * nsrc, 1, 1), bt), torch.tensor([0.3]))
-        x = _bf(x).float()                                                 # the kernel rounds H to BF16 on chip
-    want = F.prelu(F.conv2d(x, wd, bd, stride=4, padding=2), torch.tensor([0.15])).permute(0, 2, 3, 1)
+    want = _down_reference([hr[j].float() for j in range(nsrc)], wt, bt, 0.3, wd, bd, 0.15)
     _close(got, want, f"fused_down nsrc={nsrc} B={B} {h}x{w}")
+
+
+def _down_reference(srcs, wt, bt, slope_t, wd, bd, slope_d):
+    """fp32 HR half of a feedback group: srcs = nsrc maps (B,4h,4w,32) -> cat along channels -> 1x1 (nsrc > 1) ->
+    PReLU -> BF16 (the kernel rounds H to BF16 on chip) -> Conv2d(32,32,8,4,2) -> PReLU -> (B,h,w,32)."""
+    x = torch.cat([s.permute(0, 3, 1, 2) for s in srcs], dim=1)
+    if len(srcs) > 1:
+        x = F.prelu(F.conv2d(x, wt.view(32, 32 * len(srcs), 1, 1), bt), torch.tensor([slope_t]))
+        x = _bf(x).float()
+    return F.prelu(F.conv2d(x, wd, bd, stride=4, padding=2), torch.tensor([slope_d])).permute(0, 2, 3, 1)
+
+
+def _bits_equal(got, want, what, dims="b,y,x,c"):
+    """Raw-bit equality of two BF16 tensors (-0 and +0 differ); on failure names the first differing elements."""
+    a, b = got.view(torch.int16), want.view(torch.int16)
+    if torch.equal(a, b):
+        return
+    idx = (a != b).nonzero().cpu()
+    first = [tuple(i.tolist()) for i in idx[:8]]
+    pairs = [(got[i].item(), want[i].item()) for i in first]
+    raise AssertionError(f"{what}: {idx.shape[0]}/{a.numel()} elements differ; first ({dims}) got/want: "
+                         + ", ".join(f"{i}: {g}/{w}" for i, (g, w) in zip(first, pairs)))
+
+
+def _group_operands(nsrc, B, h, w, seed):
+    """Seeded, signed, O(1) operands of one feedback group: the transposed conv's LR input, the earlier HR sources
+    (plain NHWC), and the three layers' weights (rounded to BF16, as the kernels see them) and biases."""
+    g = torch.Generator().manual_seed(seed)
+    lr = _bf(torch.randn((B, h, w, 32), generator=g))
+    prev = _bf(torch.randn((nsrc - 1, B, 4 * h, 4 * w, 32), generator=g))
+    wu = _bf(torch.randn((32, 32, 8, 8), generator=g) / 16).float()
+    bu = torch.randn(32, generator=g) * 0.1
+    wt = _bf(torch.randn((32, 32 * nsrc), generator=g) / math.sqrt(32 * nsrc)).float()
+    bt = torch.randn(32, generator=g) * 0.1
+    wd = _bf(torch.randn((32, 32, 8, 8), generator=g) / 45).float()
+    bd = torch.randn(32, generator=g) * 0.1
+    return lr, prev, (wu, bu), (wt, bt), (wd, bd)
+
+
+def _check_fused_updown(nsrc, store, B, h, w, slope_u, seed):
+    """The merged kernel (transposed conv inside the down kernel) against the layered pair it replaces -- the
+    standalone transposed conv into slot nsrc-1, then the fused down kernel over all nsrc slots -- bit for bit, and the
+    whole group against an fp32 reference."""
+    slope_t, slope_d = 0.3, 0.15
+    lr, prev, (wu, bu), (wt, bt), (wd, bd) = _group_operands(nsrc, B, h, w, seed)
+    lr_d = lr.to(DEV)
+    u_blk = hk.deconv(lr_d, wu, bu, slope_u, block_layout=True)                       # (B,8,h+1,w+1,64)
+    hr = torch.stack([hk.to_block(prev[j]).to(DEV) for j in range(nsrc - 1)] + [u_blk])
+    want_y = hk.fused_down(hr, wt, bt, slope_t, wd, bd, slope_d)
+    where = f"nsrc={nsrc} store={store} B={B} {h}x{w} slope_u={slope_u}"
+    assert torch.isfinite(u_blk.float()).all() and torch.isfinite(want_y.float()).all(), where
+
+    y, hr_after = hk.fused_updown(lr_d, hr, store, wu, bu, slope_u, wt, bt, slope_t, wd, bd, slope_d)
+    # y of the merged kernel is the layered pair's, bit for bit (LR tile: 16 x 8 blocks -> tile (x // 16, y // 8))
+    _bits_equal(y, want_y, f"fused_updown y vs layered pair, {where}")
+    if store:   # the stored hr map is the standalone transposed conv's, zero ring included
+        _bits_equal(hr_after[nsrc - 1], u_blk, f"fused_updown hr[{nsrc - 1}] vs transposed conv, {where}",
+                    dims="b,pair,Yb,Xb,el")
+    else:       # the merged kernel keeps U on chip and leaves the slot alone
+        assert bool((hr_after[nsrc - 1].view(torch.int16) == hk.SENTINEL_BITS).all()), \
+            f"fused_updown wrote hr[{nsrc - 1}] with store=0, {where}"
+    # the two paths share packing and conventions: the whole group against fp32 as well
+    u = F.prelu(F.conv_transpose2d(lr.float().permute(0, 3, 1, 2), wu, bu, stride=4, padding=2),
+                torch.tensor([slope_u]))
+    u = _bf(u).float().permute(0, 2, 3, 1)                   # the kernel rounds U to BF16 (it is an HR map)
+    want = _down_reference([prev[j].float() for j in range(nsrc - 1)] + [u], wt, bt, slope_t, wd, bd, slope_d)
+    _close(y, want, f"fused_updown vs fp32, {where}")
+
+
+# (1,7,15): exactly one 16 x 8-block tile; (1,8,16): ring blocks alone in a second tile row and column; (1,7,2370):
+# 149 tiles on 148 CTAs, so one CTA walks two; (4,70,150) / (2,135,240): 360 / 544 tiles, several per CTA (the next
+# tile's LR boxes are loaded while the current one runs, one D_B buffer, mbarrier parity over many tiles)
+_UPDOWN_SHAPES = [(1, 1, 1), (1, 7, 15), (1, 8, 16), (2, 5, 7), (1, 19, 33), (3, 40, 61), (1, 7, 2370), (4, 70, 150),
+                  (2, 135, 240)]
+_UPDOWN_CASES = (
+    [(n, 1) + s for n in (4, 6) for s in _UPDOWN_SHAPES]                               # the plan's nsrc: every shape
+    + [(n, 1) + s for n in (2, 3, 5) for s in [(1, 8, 16), (2, 5, 7), (1, 19, 33), (3, 40, 61)]]
+    + [(5, 1, 4, 70, 150), (2, 1, 1, 7, 2370), (3, 1, 1, 1, 1)]
+    # store = 0: the plan's last group (hr[5] is read by no one); no TMA stores, no wait for them to read U
+    + [(6, 0) + s for s in [(1, 1, 1), (1, 7, 15), (1, 19, 33), (1, 7, 2370), (4, 70, 150)]]
+    + [(3, 0) + s for s in [(2, 5, 7), (3, 40, 61)]])
+
+
+@pytest.mark.parametrize("nsrc,store,B,h,w", _UPDOWN_CASES)
+def test_fused_updown_against_layered_pair(nsrc, store, B, h, w):
+    """fused_updown_kernel (feedback groups 3-5 of the x4 stack; it accepts nsrc 2..6) at tile, ring and multi-tile
+    edges: y and the stored hr map bit-identical to the layered pair, y within BF16 tolerance of fp32, guard bands
+    around y and the hr array untouched, the workspace poisoned with NaN bytes."""
+    _check_fused_updown(nsrc, store, B, h, w, 0.25, seed=nsrc * 7919 + B * 1000 + h * 37 + w)
+
+
+@pytest.mark.parametrize("slope_u", [0.0, 1.0, -0.3, 1.7])
+def test_fused_updown_prelu_slope_forms(slope_u):
+    """The merged kernel's conversion of the transposed conv picks the packed-BF16 PReLU form by the slope."""
+    _check_fused_updown(5, 1, 2, 19, 33, slope_u, seed=77)
 
 
 @pytest.mark.parametrize("B,h,w", [(1, 8, 16), (2, 5, 7), (1, 19, 33), (1, 9, 14), (1, 17, 29), (3, 40, 61)])
@@ -192,6 +282,40 @@ def test_workspace_cap_chunks_the_maps_bit_identically(scale):
         assert prof["im2col"]["launches"] == M // chunk and prof["fc_fuse"]["launches"] == 1
     with pytest.raises(Exception, match="workspace"):
         SRProjectionModule(num_maps=M, upscale_factor=scale, workspace_cap_bytes=1 << 16)(x)
+
+
+@pytest.mark.parametrize("scale", [4, 2])
+def test_plan_reads_only_workspace_bytes_written_in_the_same_forward(scale):
+    """The plan's workspace may hold anything when a forward starts: the hr rings, the fp32 partial slots of the fused
+    down kernels and the x4 plan's omission of hr[5] all rely on every byte a forward reads having been written by that
+    forward.  A workspace filled with 0xFF bytes (NaN in BF16 and fp32) before the forward -- unchunked and chunked,
+    before the first forward and again between two -- gives the frame and the per-map images of a zero-filled one,
+    bit for bit."""
+    M, h, w = 6, 17, 26
+    sd = so.init_state_dict(num_maps=M, seed=8, gain=2.3, upscale=scale)
+    x = (torch.rand((M, 3, h, w), generator=torch.Generator().manual_seed(9)) * 255).to(DEV)
+
+    def module(poison, cap=None):
+        mod = SRProjectionModule(num_maps=M, upscale_factor=scale, workspace_cap_bytes=cap)
+        mod.load_state_dict(sd)
+        ent = mod._plan_for(M, h, w, x.device)
+        ent["workspace"].fill_(0xFF if poison else 0)
+        return mod, ent
+
+    clean, ent = module(False)
+    want, want_maps = clean(x), clean.premix(x)
+    assert torch.isfinite(want).all() and torch.isfinite(want_maps).all()
+    full = ent["workspace"].numel()
+    for cap in (None, int(full * 0.45)):
+        mod, ent = module(True, cap)
+        assert ent["chunk_maps"] == (M if cap is None else 2)
+        assert torch.equal(mod(x).view(torch.int32), want.view(torch.int32)), cap
+        ent["workspace"].fill_(0xFF)                     # poisoned again between two full forwards
+        got_maps = mod.premix(x)
+        assert torch.equal(got_maps.view(torch.int32), want_maps.view(torch.int32)), cap
+        ent["workspace"].fill_(0xFF)
+        assert torch.equal(mod(x).view(torch.int32), want.view(torch.int32)), cap
+        del mod
 
 
 @pytest.mark.parametrize("scale", [4, 2])

@@ -97,6 +97,9 @@ SIGNATURES = {
     "vsr_test_deconv": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "vsr_test_fused_down": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
                                     c_float, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "vsr_test_fused_updown": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float,
+                                      c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_float, c_void_p, c_void_p,
+                                      c_size_t, c_void_p]),
     "vsr_test_x2_layer": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_size_t, c_void_p]),
     "vsr_test_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
 }

@@ -1450,3 +1450,61 @@ extern "C" int vsr_test_fused_down(const void* hr_bf16, int nsrc, int B, int h, 
   if (rc) return rc;
   return cuda_status(cudaStreamSynchronize(st));
 }
+
+// One feedback group with its transposed conv inside (fused_updown_kernel + finalize_lr_kernel, the plan's two launches
+// for groups 3-5): ConvTranspose2d(32,32,8,4,2) (wu (32 in,32 out,8,8), bu, slope_u) + PReLU of lr (B,h,w,32) is source
+// nsrc-1; downtran over hr[0..nsrc-1] (wt (32,32*nsrc), bt, slope_t) + PReLU + Conv2d(32,32,8,4,2) (wd, bd, slope_d) +
+// PReLU -> y (B,h,w,32).  hr: nsrc slots (nsrc,B,8,h+1,w+1,64) in block layout; slots 0..nsrc-2 are read, slot nsrc-1
+// receives the transposed conv's output iff store.  Packed operands in the first 512 KB of the workspace: wd [0, 128K),
+// wt at 160K, biases at 256K / 257K / 258K (down, downtran, up), wu [384K, 512K); then the fp32 partial-sum slots.
+extern "C" int vsr_test_fused_updown(const void* lr_bf16, void* hr_bf16, int nsrc, int store, int B, int h, int w,
+                                     const float* wu_host, const float* bu_host, float slope_u, const float* wt_host,
+                                     const float* bt_host, float slope_t, const float* wd_host, const float* bd_host,
+                                     float slope_d, void* y_bf16, void* workspace, size_t workspace_bytes,
+                                     vsr_stream_t stream) {
+  if (!lr_bf16 || !hr_bf16 || !wu_host || !bu_host || !wt_host || !bt_host || !wd_host || !bd_host || !y_bf16 ||
+      !workspace || B <= 0 || h <= 0 || w <= 0 || nsrc < 2 || nsrc > 6)
+    return VSR_ERR_INVALID_ARG;
+  const size_t base_bytes = vsr_test_workspace_bytes(B, h, w);
+  const size_t acc_bytes = (size_t)B * h * w * 512;
+  if (workspace_bytes < base_bytes + acc_bytes) return VSR_ERR_WORKSPACE;
+  cudaStream_t st = as_stream(stream);
+  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
+  std::vector<uint16_t> wd((size_t)128 * 512), wu((size_t)512 * 128), wt((size_t)32 * 32 * nsrc);
+  pack_downconv_fused(wd_host, wd.data());
+  pack_deconv(wu_host, wu.data());
+  pack_pointwise(wt_host, 32, 32 * nsrc, wt.data());
+  float bd[33], bt[33], bu[33];
+  memcpy(bd, bd_host, 32 * 4);
+  bd[32] = slope_d;
+  memcpy(bt, bt_host, 32 * 4);
+  bt[32] = slope_t;
+  memcpy(bu, bu_host, 32 * 4);
+  bu[32] = slope_u;
+  int rc = upload(ws, wd.data(), wd.size() * 2, st);
+  if (!rc) rc = upload(ws + 160 * 1024, wt.data(), wt.size() * 2, st);
+  if (!rc) rc = upload(ws + 384 * 1024, wu.data(), wu.size() * 2, st);
+  if (!rc) rc = upload(ws + 256 * 1024, bd, sizeof(bd), st);
+  if (!rc) rc = upload(ws + 257 * 1024, bt, sizeof(bt), st);
+  if (!rc) rc = upload(ws + 258 * 1024, bu, sizeof(bu), st);
+  if (rc) return rc;
+  float* acc = reinterpret_cast<float*>(ws + base_bytes);
+  const void* hrs[6];
+  const size_t plane = (size_t)B * (h + 1) * (w + 1) * 16 * 64;
+  for (int j = 0; j < nsrc; ++j) hrs[j] = reinterpret_cast<const uint8_t*>(hr_bf16) + j * plane;
+  if (!store) hrs[nsrc - 1] = nullptr;   // as in the plan: the kernel must not touch the slot
+  const float* bd_dev = reinterpret_cast<const float*>(ws + 256 * 1024);
+  const float* bt_dev = reinterpret_cast<const float*>(ws + 257 * 1024);
+  const float* bu_dev = reinterpret_cast<const float*>(ws + 258 * 1024);
+  Layer L;
+  rc = build_fused_updown(L, lr_bf16, hrs, nsrc, store, B, h, w, ws + 384 * 1024, bu_dev, ws + 160 * 1024, bt_dev, ws,
+                          bd_dev, acc, y_bf16);
+  if (rc) return rc;
+  rc = launch_layer(L, st);
+  if (rc) return rc;
+  rc = build_finalize(L, acc, bd_dev, y_bf16, (int64_t)B * h * w, h, w);
+  if (rc) return rc;
+  rc = launch_layer(L, st);
+  if (rc) return rc;
+  return cuda_status(cudaStreamSynchronize(st));
+}
