@@ -75,18 +75,32 @@ int vsr_warp_nhwc_f32(const float* src, const float* flow, float* dst,
  * `bilinear` modes as vsr_warp_nhwc_f32. */
 int vsr_warp_window_nhwc3(const float* frames, const float* flows, float* warped, float* resid,
                           int T, int centre, int H, int W, int bilinear, vsr_stream_t stream);
+/* The same for `windows` independent frame windows in one launch (1..65535): frames (windows,T,H,W,3), flows
+ * (windows,T-1,H,W,2), warped (windows,T-1,H,W,3), resid (windows,T-1,H,W) or NULL; window b is warped to its own
+ * centre frame, bit-identical to a one-window call on it.  vsr_warp_window_nhwc3 is this with windows = 1. */
+int vsr_warp_windows_nhwc3(const float* frames, const float* flows, float* warped, float* resid, int windows,
+                           int T, int centre, int H, int W, int bilinear, vsr_stream_t stream);
 
 /* Flow composition out(p) = g(p) + f(p + g(p)) with f sampled bilinearly (the warp's taps and border rule,
  * fp32 blend): if g maps image A to B and f maps B to C, out maps A to C.  g, f, out (B,H,W,2) f32.  Used to chain
  * adjacent-pair flows into centre -> neighbour flows for windows longer than 3 frames.  g == NULL is the identity
  * field: out = f (the first link of a chain, placed into the caller's contiguous (T-1,H,W,2) array). */
 int vsr_compose_flow(const float* g, const float* f, float* out, int B, int H, int W, vsr_stream_t stream);
+/* One link of the chains of `windows` frame windows in one launch (1..65535): window b composes the (H,W,2) fields at
+ * g + b*stride and f + b*stride into out + b*stride (stride in floats, even).  The centre -> neighbour fields of a
+ * (windows,T-1,H,W,2) array are (T-1)*H*W*2 floats apart. */
+int vsr_compose_flow_windows(const float* g, const float* f, float* out, int windows, int64_t stride, int H, int W,
+                             vsr_stream_t stream);
 
 /* Nearest-neighbour label/mask warp on u8 (north star "VOSProjection: mask/label warping"),
  * ref arithmetic: resample2d_kernel.cu:65-70 (floor(xf + 0.5) in double, border clamp).
  * labels/dst (B,H,W) u8, flow (B,H,W,2) f32.  Bit-exact. */
 int vsr_warp_labels_u8(const uint8_t* labels, const float* flow, uint8_t* dst,
                        int B, int H, int W, vsr_stream_t stream);
+/* `windows` label images (windows,H,W) -> dst (windows,H,W) in one launch (1..65535); window b is warped along the
+ * (H,W,2) field at flow + b*flow_stride (floats, even). */
+int vsr_warp_labels_u8_windows(const uint8_t* labels, const float* flow, uint8_t* dst, int windows,
+                               int64_t flow_stride, int H, int W, vsr_stream_t stream);
 
 /* ref: channelnorm_cuda.cc `channelnorm_cuda_forward(input1, output, norm_deg)` ->
  * channelnorm_kernel.cu:19-60.  input (B,C,H,W) f32 NCHW, output (B,1,H,W).  norm_deg is accepted
@@ -208,6 +222,10 @@ int vsr_flow_projection_forward_deterministic(const float* flow, const float* in
  * ---------------------------------------------------------------------------------------- */
 int vsr_vos_threshold(const float* logits_a, const float* logits_b, uint8_t* mask,
                       int h, int w, vsr_stream_t stream);
+/* `windows` logit pairs in one launch: logits_a/logits_b (windows,h,w) -> mask (windows,h,w).
+ * vsr_vos_threshold is this with windows = 1. */
+int vsr_vos_threshold_windows(const float* logits_a, const float* logits_b, uint8_t* mask,
+                              int windows, int h, int w, vsr_stream_t stream);
 int vsr_mask_fill(const float* image, const uint8_t* mask, float* masked,
                   int C, int h, int w, vsr_stream_t stream);
 
@@ -229,6 +247,20 @@ int vsr_assemble_stack(const float* warped, const float* centre, const float* pr
                        int T, int centre_idx, int h, int w, vsr_stream_t stream);
 int vsr_estimate_slot(const float* hr, const uint8_t* mask, float* slot, int h, int w, int scale,
                       vsr_stream_t stream);
+/* `windows` frame windows in one launch each (1..65535), window b bit-identical to a one-window call on it:
+ * vsr_assemble_stack_windows: warped (windows,T-1,h,w,3), proj (windows,T-1,h,w,2), resid / depth (windows,T-1,h,w),
+ * estimate (windows,3,h,w) or NULL, stack (windows,M,3,h,w); the centre frame and the fallback frame of window b are
+ * the (h,w,3) images at centre + b*frame_stride and fallback + b*frame_stride (floats; for frames (windows,T,h,w,3)
+ * frame_stride = T*h*w*3 and centre / fallback point at frame centre_idx / 0 of window 0).
+ * vsr_estimate_slot_windows: hr (windows,3,h*scale,w*scale), mask (windows,h,w) or NULL; the slot of window b is the
+ * (3,h,w) image at slot + b*slot_stride (floats; the estimate slots of a (windows,M,3,h,w) stack: slot = map M-1 of
+ * window 0, slot_stride = M*3*h*w).  The one-window entry points above are these with windows = 1. */
+int vsr_assemble_stack_windows(const float* warped, const float* centre, const float* proj, const float* resid,
+                               const float* depth, const float* estimate, const float* fallback, float* stack,
+                               int windows, int64_t frame_stride, int T, int centre_idx, int h, int w,
+                               vsr_stream_t stream);
+int vsr_estimate_slot_windows(const float* hr, const uint8_t* mask, float* slot, int windows, int64_t slot_stride,
+                              int h, int w, int scale, vsr_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * SURVEY.md 8f rank 3: flow colour coding + resize glue on the device.
@@ -314,6 +346,14 @@ void vsr_srfbn_plan_destroy(vsr_srfbn_plan* plan);
  * VSR_ERR_WORKSPACE if not even one map at a time fits; VSR_ERR_STATE after bind.  (Config C4 unchunked: 89 GB.) */
 int vsr_srfbn_plan_set_workspace_cap(vsr_srfbn_plan* plan, size_t cap_bytes);
 int vsr_srfbn_chunk_maps(const vsr_srfbn_plan* plan);
+/* Optional, before vsr_srfbn_bind: the number of frame windows W (1..65535, default 1) one forward fuses.  x is then
+ * (W*M,3,h,w), window-major; y (W,3,s*h,s*w), y_u8 (W,s*h,s*w,3), vsr_srfbn_debug_premix (W*M,3,s*h,s*w).  The layers
+ * sweep all W*M maps (chunk_maps is a divisor of W*M under a workspace cap, W*M without one) and the fc fuse writes
+ * frame b from the maps [b*M, (b+1)*M), bit-identical to a one-window forward of window b.  M (num_maps) stays the fc
+ * in-features.  The refresh entry points refresh the maps [first_map, M) of every window, one sweep per window.
+ * Workspace and profile counts scale with W.  VSR_ERR_INVALID_ARG for W outside 1..65535; VSR_ERR_STATE after bind;
+ * VSR_ERR_WORKSPACE if a workspace cap is set and not even one map fits (the plan is then unchanged). */
+int vsr_srfbn_plan_set_windows(vsr_srfbn_plan* plan, int windows);
 /* bytes of device memory the caller must provide */
 size_t vsr_srfbn_weight_bytes(const vsr_srfbn_plan* plan);
 size_t vsr_srfbn_workspace_bytes(const vsr_srfbn_plan* plan);
@@ -323,7 +363,8 @@ int vsr_srfbn_pack_weights(const vsr_srfbn_plan* plan, const vsr_srfbn_weights* 
 /* Binds device buffers (packed weights + workspace) and builds the TMA descriptors. */
 int vsr_srfbn_bind(vsr_srfbn_plan* plan, const void* dev_weights, void* dev_workspace,
                    size_t workspace_bytes);
-/* x: (M,3,h,w) f32 NCHW, 0..255 (video_super_resolution.py:40,62); y: (1,3,s*h,s*w) f32. */
+/* x: (M,3,h,w) f32 NCHW, 0..255 (video_super_resolution.py:40,62); y: (1,3,s*h,s*w) f32.
+ * With vsr_srfbn_plan_set_windows(W): x (W*M,3,h,w), y (W,3,s*h,s*w), y_u8 (W,s*h,s*w,3). */
 int vsr_srfbn_forward(vsr_srfbn_plan* plan, const float* x, float* y, vsr_stream_t stream);
 /* Same, with the fused frame also (or only) as u8 pixels: y_u8 (s*h,s*w,3) NHWC = clamp(y,0,255) rounded half to
  * even, the format the reference's loader holds frames in (utils/video_utils.py:23) -- what a frame writer or the

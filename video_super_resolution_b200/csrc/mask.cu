@@ -44,12 +44,18 @@ inline int grid_for(int64_t n) {
 
 using namespace vsr;
 
-extern "C" int vsr_vos_threshold(const float* logits_a, const float* logits_b, uint8_t* mask, int h, int w,
-                                 vsr_stream_t stream) {
-  if (!logits_a || !logits_b || !mask || h <= 0 || w <= 0) return VSR_ERR_INVALID_ARG;
-  int64_t n = (int64_t)h * w;
+// windows (h,w) logit pairs in sequence: the threshold is elementwise, so the windows are one flat launch
+extern "C" int vsr_vos_threshold_windows(const float* logits_a, const float* logits_b, uint8_t* mask, int windows, int h,
+                                         int w, vsr_stream_t stream) {
+  if (!logits_a || !logits_b || !mask || windows < 1 || h <= 0 || w <= 0) return VSR_ERR_INVALID_ARG;
+  int64_t n = (int64_t)windows * h * w;
   vos_threshold_kernel<<<grid_for(n), kThreads, 0, as_stream(stream)>>>(logits_a, logits_b, mask, n);
   return after_launch();
+}
+
+extern "C" int vsr_vos_threshold(const float* logits_a, const float* logits_b, uint8_t* mask, int h, int w,
+                                 vsr_stream_t stream) {
+  return vsr_vos_threshold_windows(logits_a, logits_b, mask, 1, h, w, stream);
 }
 
 extern "C" int vsr_mask_fill(const float* image, const uint8_t* mask, float* masked, int C, int h, int w,

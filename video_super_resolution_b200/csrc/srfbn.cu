@@ -726,11 +726,15 @@ im2col_kernel(const float* __restrict__ x, const float* __restrict__ sub_bias, u
 }
 
 // fc over the map axis per (channel, HR pixel): Linear(M,32)-ReLU-Linear(32,1)-ReLU
-// (SRProjectionModule.py:126-131,146).  maps (M,3,H,W) f32 -> y (1,3,H,W) f32.
+// (SRProjectionModule.py:126-131,146).  maps (W*M,3,H,W) f32 -> y (W,3,H,W) f32: window b = blockIdx.y fuses the
+// maps [b*M, (b+1)*M) into frame b with the same per-pixel arithmetic as a one-window launch.
 // fcw: [32*M fc0_w][32 fc0_b][32 fc2_w][1 fc2_b]
 __global__ void __launch_bounds__(256)
 fc_fuse_kernel(const float* __restrict__ maps, const float* __restrict__ fcw, float* __restrict__ y,
                uint8_t* __restrict__ y_u8, int M, int64_t n) {
+  maps += (int64_t)blockIdx.y * M * n;
+  if (y) y += (int64_t)blockIdx.y * n;
+  if (y_u8) y_u8 += (int64_t)blockIdx.y * n;      // the u8 frame (H,W,3) has n bytes
   // y (3,H,W) f32 planar and / or y_u8 (H,W,3): the frame quantised the way the reference's loader stores frames
   // (utils/video_utils.py:23): clamp to 0..255, round half to even -- what a u8 frame writer or gather needs,
   // a quarter of the fp32 bytes.
@@ -839,6 +843,7 @@ struct vsr_srfbn_plan {
   size_t o_a0, o_c128, o_xfeat, o_hidden, o_lr[7], o_u, o_hr[6], o_hb, o_ht, o_acc, o_premix, ws_bytes;
   int chunk_maps;         // maps processed per sweep over the layer list (a divisor of num_maps; == num_maps: no chunking)
   size_t ws_cap;          // caller's workspace cap in bytes (0 = none)
+  int windows;            // frame windows per forward: the sweeps run over windows * num_maps maps
   bool bound;
   const uint8_t* dev_w;
   uint8_t* ws;
@@ -882,7 +887,7 @@ static void layout_weights(vsr_srfbn_plan* pl) {
 }
 
 // Activations are laid out for `chunk_maps` maps at a time (the maps are independent until the fc fuse, so the layer
-// list is swept once per chunk); only the per-map SR images in front of the fc fuse exist for all num_maps.
+// list is swept once per chunk); only the per-map SR images in front of the fc fuse exist for all windows * num_maps.
 static void layout_workspace(vsr_srfbn_plan* pl) {
   const vsr_srfbn_config& c = pl->cfg;
   const size_t P = (size_t)pl->chunk_maps * c.h * c.w;
@@ -906,7 +911,7 @@ static void layout_workspace(vsr_srfbn_plan* pl) {
   pl->o_hb = put(P * s2 * 64);   // plain-NHWC result of the `out` deconv
   pl->o_ht = put(x2 ? P * s2 * 64 : 0);   // x2: downtran result (the x4 path keeps it on chip)
   pl->o_acc = put(x2 ? 0 : P * 512);   // fp32 partial slots of the fused down kernel
-  pl->o_premix = put((size_t)c.num_maps * c.h * c.w * s2 * 3 * 4);
+  pl->o_premix = put((size_t)pl->windows * c.num_maps * c.h * c.w * s2 * 3 * 4);
   pl->ws_bytes = off;
 }
 
@@ -932,18 +937,16 @@ extern "C" int vsr_srfbn_plan_create(const vsr_srfbn_config* cfg, vsr_srfbn_plan
   pl->profile = false;
   pl->chunk_maps = cfg->num_maps;
   pl->ws_cap = 0;
+  pl->windows = 1;
   layout_weights(pl);
   layout_workspace(pl);
   *out_plan = pl;
   return VSR_OK;
 }
 
-extern "C" int vsr_srfbn_plan_set_workspace_cap(vsr_srfbn_plan* pl, size_t cap_bytes) {
-  if (!pl) return VSR_ERR_INVALID_ARG;
-  if (pl->bound) return VSR_ERR_STATE;                // the layer list is built for a chunk size: set the cap before bind
-  pl->ws_cap = cap_bytes;
-  // the largest divisor of num_maps whose workspace fits under the cap (no ragged tail chunk: one layer list)
-  const int M = pl->cfg.num_maps;
+// the largest divisor of windows * num_maps whose workspace fits under the cap (no ragged tail chunk: one layer list)
+static int choose_chunk(vsr_srfbn_plan* pl, size_t cap_bytes) {
+  const int M = pl->windows * pl->cfg.num_maps;
   for (int mc = M; mc >= 1; --mc) {
     if (M % mc) continue;
     pl->chunk_maps = mc;
@@ -951,6 +954,26 @@ extern "C" int vsr_srfbn_plan_set_workspace_cap(vsr_srfbn_plan* pl, size_t cap_b
     if (cap_bytes == 0 || pl->ws_bytes <= cap_bytes) return VSR_OK;
   }
   return VSR_ERR_WORKSPACE;                            // not even one map at a time fits
+}
+
+extern "C" int vsr_srfbn_plan_set_workspace_cap(vsr_srfbn_plan* pl, size_t cap_bytes) {
+  if (!pl) return VSR_ERR_INVALID_ARG;
+  if (pl->bound) return VSR_ERR_STATE;                // the layer list is built for a chunk size: set the cap before bind
+  pl->ws_cap = cap_bytes;
+  return choose_chunk(pl, cap_bytes);
+}
+
+extern "C" int vsr_srfbn_plan_set_windows(vsr_srfbn_plan* pl, int windows) {
+  if (!pl || windows < 1 || windows > 65535) return VSR_ERR_INVALID_ARG;   // fc_fuse_kernel: one grid row per window
+  if (pl->bound) return VSR_ERR_STATE;                // buffers and layer list are sized for the window count
+  const int old = pl->windows;
+  pl->windows = windows;
+  const int rc = choose_chunk(pl, pl->ws_cap);
+  if (rc) {                                            // leave the plan as it was
+    pl->windows = old;
+    choose_chunk(pl, pl->ws_cap);
+  }
+  return rc;
 }
 
 extern "C" int vsr_srfbn_chunk_maps(const vsr_srfbn_plan* pl) { return pl ? pl->chunk_maps : 0; }
@@ -1149,7 +1172,7 @@ extern "C" int vsr_srfbn_prepare_refresh(vsr_srfbn_plan* pl, int first_map) {
   if (!pl) return VSR_ERR_INVALID_ARG;
   if (!pl->bound) return VSR_ERR_STATE;
   if (first_map < 1 || first_map >= pl->cfg.num_maps) return VSR_ERR_INVALID_ARG;
-  if (pl->chunk_maps != pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;     // not with a workspace cap (chunked sweeps)
+  if (pl->chunk_maps != pl->windows * pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;   // not with chunked sweeps
   if (pl->refresh_first == first_map) return VSR_OK;
   pl->refresh_first = -1;
   const int rc = build_layer_list(pl, pl->cfg.num_maps - first_map, pl->refresh_layers, pl->refresh_conv_out_layer);
@@ -1193,13 +1216,13 @@ static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_o
   return VSR_OK;
 }
 
-// the per-pixel fc across the num_maps per-map images (SRProjectionModule.py:146)
+// the per-pixel fc across the num_maps per-map images of each window (SRProjectionModule.py:146), one window per grid row
 static int fuse_maps(vsr_srfbn_plan* pl, float* y, uint8_t* y_u8, cudaStream_t st) {
   const vsr_srfbn_config& c = pl->cfg;
   const int64_t n = (int64_t)3 * c.upscale * c.upscale * c.h * c.w;
   int64_t blocks = ceil_div64(ceil_div64(n, 4), 256);
   if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
-  fc_fuse_kernel<<<(int)blocks, 256, 0, st>>>(reinterpret_cast<const float*>(pl->ws + pl->o_premix),
+  fc_fuse_kernel<<<dim3((unsigned)blocks, (unsigned)pl->windows), 256, 0, st>>>(reinterpret_cast<const float*>(pl->ws + pl->o_premix),
                                               reinterpret_cast<const float*>(pl->dev_w + pl->fc_off), y, y_u8, c.num_maps, n);
   return after_launch();
 }
@@ -1211,7 +1234,7 @@ extern "C" int vsr_srfbn_forward_u8(vsr_srfbn_plan* pl, const float* x, float* y
   const vsr_srfbn_config& c = pl->cfg;
   const int Mc = pl->chunk_maps;
   size_t ev = 0;
-  for (int m0 = 0; m0 < c.num_maps; m0 += Mc) {        // one sweep over the layer list per chunk of maps
+  for (int m0 = 0; m0 < pl->windows * c.num_maps; m0 += Mc) {   // one sweep over the layer list per chunk of maps
     int rc = sweep_maps(pl, pl->layers, pl->conv_out_layer, x, m0, Mc, st, &ev);
     if (rc) return rc;
   }
@@ -1228,14 +1251,20 @@ extern "C" int vsr_srfbn_forward_u8(vsr_srfbn_plan* pl, const float* x, float* y
 // independent until the per-pixel fc, so the per-map images of the unchanged maps are still in the workspace and only
 // the changed ones are swept again -- bit-identical to a full forward on the same stack.  Needs
 // vsr_srfbn_prepare_refresh(plan, first_map) and a preceding vsr_srfbn_forward[_u8] on the same stream.
+// With several windows the changed maps of window b are [b*M + first_map, (b+1)*M): one sweep of the refresh layer list
+// per window.  The stack keeps the caller's window-major layout, so no map is copied or reordered to make the changed
+// maps contiguous; the price is windows sweeps instead of one, which only matters where launches dominate.
 extern "C" int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* pl, const float* x, float* y, uint8_t* y_u8, int first_map,
                                             vsr_stream_t stream) {
   if (!pl || !x || (!y && !y_u8)) return VSR_ERR_INVALID_ARG;
   if (!pl->bound || !pl->premix_valid || pl->refresh_first != first_map || first_map < 1) return VSR_ERR_STATE;
   cudaStream_t st = as_stream(stream);
-  int rc = sweep_maps(pl, pl->refresh_layers, pl->refresh_conv_out_layer, x, first_map, pl->cfg.num_maps - first_map,
-                      st, nullptr);
-  if (rc) return rc;
+  const int M = pl->cfg.num_maps;
+  for (int b = 0; b < pl->windows; ++b) {
+    int rc = sweep_maps(pl, pl->refresh_layers, pl->refresh_conv_out_layer, x, b * M + first_map, M - first_map, st,
+                        nullptr);
+    if (rc) return rc;
+  }
   return fuse_maps(pl, y, y_u8, st);
 }
 
@@ -1251,7 +1280,7 @@ extern "C" int vsr_srfbn_profile_enable(vsr_srfbn_plan* pl, int enable) {
   if (!pl->bound) return VSR_ERR_STATE;
   pl->profile = enable != 0;
   if (pl->profile && pl->events.empty()) {
-    pl->events.resize((pl->layers.size() + 1) * (size_t)(pl->cfg.num_maps / pl->chunk_maps) + 2);
+    pl->events.resize((pl->layers.size() + 1) * (size_t)(pl->windows * pl->cfg.num_maps / pl->chunk_maps) + 2);
     for (cudaEvent_t& e : pl->events) {
       cudaError_t r = cudaEventCreate(&e);
       if (r != cudaSuccess) return cuda_status(r);
@@ -1267,7 +1296,7 @@ extern "C" int vsr_srfbn_profile_read(vsr_srfbn_plan* pl, double* ms, int32_t* l
   cudaError_t r = cudaEventSynchronize(pl->events.back());
   if (r != cudaSuccess) return cuda_status(r);
   const vsr_srfbn_config& c = pl->cfg;
-  const double Pc = (double)pl->chunk_maps * c.h * c.w, Pall = (double)c.num_maps * c.h * c.w;
+  const double Pc = (double)pl->chunk_maps * c.h * c.w, Pall = (double)pl->windows * c.num_maps * c.h * c.w;
   const size_t per = pl->layers.size() + 1, n = pl->events.size() - 1;     // launches per chunk sweep; intervals
   for (size_t i = 0; i < n; ++i) {
     float t = 0;
@@ -1301,7 +1330,7 @@ extern "C" int vsr_srfbn_debug_premix(const vsr_srfbn_plan* pl, float* out_maps,
   if (!pl || !out_maps) return VSR_ERR_INVALID_ARG;
   if (!pl->bound) return VSR_ERR_STATE;
   const vsr_srfbn_config& c = pl->cfg;
-  size_t bytes = (size_t)c.num_maps * 3 * c.upscale * c.upscale * c.h * c.w * 4;
+  size_t bytes = (size_t)pl->windows * c.num_maps * 3 * c.upscale * c.upscale * c.h * c.w * 4;
   return cuda_status(cudaMemcpyAsync(out_maps, pl->ws + pl->o_premix, bytes, cudaMemcpyDeviceToDevice, as_stream(stream)));
 }
 

@@ -27,7 +27,20 @@ assemble_stack_kernel(const float* __restrict__ warped,   // (T-1,h,w,3) NHWC
                       const float* __restrict__ estimate, // (3,h,w) NCHW or nullptr (-> fallback frame)
                       const float* __restrict__ fallback, // (h,w,3) NHWC: LR frame 0 of the window
                                                           // (video_super_resolution.py:37-38 `data_clone[0:1]`)
-                      float* __restrict__ stack, int T, int centre_idx, int64_t hw) {
+                      float* __restrict__ stack, int T, int centre_idx, int64_t hw, int64_t frame_stride) {
+  // blockIdx.y: the frame window.  Per window: warped / proj / resid / depth advance by their (T-1) images, the stack by
+  // its M = 3T-1 maps, the estimate by one (3,h,w) image, centre and fallback by frame_stride floats.
+  if (blockIdx.y) {
+    const int64_t wb = blockIdx.y;
+    warped += wb * (T - 1) * hw * 3;
+    proj += wb * (T - 1) * hw * 2;
+    resid += wb * (T - 1) * hw;
+    depth += wb * (T - 1) * hw;
+    stack += wb * (3 * T - 1) * 3 * hw;
+    centre += wb * frame_stride;
+    if (estimate) estimate += wb * 3 * hw;
+    else fallback += wb * frame_stride;
+  }
   for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < hw; p += (int64_t)gridDim.x * blockDim.x) {
     const float c0 = __ldg(centre + p * 3), c1 = __ldg(centre + p * 3 + 1), c2 = __ldg(centre + p * 3 + 2);
     for (int t = 0, n = 0; t < T; ++t) {
@@ -58,8 +71,14 @@ assemble_stack_kernel(const float* __restrict__ warped,   // (T-1,h,w,3) NHWC
 // floor(dst * in/out) = dst*s (video_super_resolution.py:44), then MaskedArray(...).filled(0) (:58-60).
 __global__ void __launch_bounds__(kThreads)
 estimate_slot_kernel(const float* __restrict__ hr, const uint8_t* __restrict__ mask, float* __restrict__ slot, int h,
-                     int w, int s) {
+                     int w, int s, int64_t slot_stride) {
   const int64_t hw = (int64_t)h * w, HW = hw * s * s;
+  if (blockIdx.y) {     // window blockIdx.y: hr (3,H,W) and mask (h,w) images in sequence, slots slot_stride floats apart
+    const int64_t wb = blockIdx.y;
+    hr += wb * 3 * HW;
+    if (mask) mask += wb * hw;
+    slot += wb * slot_stride;
+  }
   for (int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; p < hw; p += (int64_t)gridDim.x * blockDim.x) {
     const int y = (int)(p / w), x = (int)(p - (int64_t)y * w);
     const bool m = mask != nullptr && __ldg(mask + p) != 0;
@@ -79,22 +98,37 @@ inline int grid_for(int64_t n) {
 
 using namespace vsr;
 
-extern "C" int vsr_assemble_stack(const float* warped, const float* centre, const float* proj, const float* resid,
-                                  const float* depth, const float* estimate, const float* fallback, float* stack, int T,
-                                  int centre_idx, int h, int w, vsr_stream_t stream) {
-  if (!warped || !centre || !proj || !resid || !depth || !stack || T < 2 || centre_idx < 0 || centre_idx >= T ||
-      h <= 0 || w <= 0 || (!estimate && !fallback))
+extern "C" int vsr_assemble_stack_windows(const float* warped, const float* centre, const float* proj,
+                                          const float* resid, const float* depth, const float* estimate,
+                                          const float* fallback, float* stack, int windows, int64_t frame_stride, int T,
+                                          int centre_idx, int h, int w, vsr_stream_t stream) {
+  if (!warped || !centre || !proj || !resid || !depth || !stack || windows < 1 || windows > 65535 || frame_stride < 0 ||
+      T < 2 || centre_idx < 0 || centre_idx >= T || h <= 0 || w <= 0 || (!estimate && !fallback))
     return VSR_ERR_INVALID_ARG;
   if (reinterpret_cast<uintptr_t>(proj) % 8) return VSR_ERR_INVALID_ARG;
   const int64_t hw = (int64_t)h * w;
-  assemble_stack_kernel<<<grid_for(hw), kThreads, 0, as_stream(stream)>>>(warped, centre, proj, resid, depth, estimate,
-                                                                         fallback, stack, T, centre_idx, hw);
+  assemble_stack_kernel<<<dim3(grid_for(hw), windows), kThreads, 0, as_stream(stream)>>>(
+      warped, centre, proj, resid, depth, estimate, fallback, stack, T, centre_idx, hw, frame_stride);
+  return after_launch();
+}
+
+extern "C" int vsr_assemble_stack(const float* warped, const float* centre, const float* proj, const float* resid,
+                                  const float* depth, const float* estimate, const float* fallback, float* stack, int T,
+                                  int centre_idx, int h, int w, vsr_stream_t stream) {
+  return vsr_assemble_stack_windows(warped, centre, proj, resid, depth, estimate, fallback, stack, 1, 0, T, centre_idx, h,
+                                    w, stream);
+}
+
+extern "C" int vsr_estimate_slot_windows(const float* hr, const uint8_t* mask, float* slot, int windows,
+                                         int64_t slot_stride, int h, int w, int scale, vsr_stream_t stream) {
+  if (!hr || !slot || windows < 1 || windows > 65535 || slot_stride < 0 || h <= 0 || w <= 0 || scale < 1)
+    return VSR_ERR_INVALID_ARG;
+  estimate_slot_kernel<<<dim3(grid_for((int64_t)h * w), windows), kThreads, 0, as_stream(stream)>>>(hr, mask, slot, h, w,
+                                                                                                   scale, slot_stride);
   return after_launch();
 }
 
 extern "C" int vsr_estimate_slot(const float* hr, const uint8_t* mask, float* slot, int h, int w, int scale,
                                  vsr_stream_t stream) {
-  if (!hr || !slot || h <= 0 || w <= 0 || scale < 1) return VSR_ERR_INVALID_ARG;
-  estimate_slot_kernel<<<grid_for((int64_t)h * w), kThreads, 0, as_stream(stream)>>>(hr, mask, slot, h, w, scale);
-  return after_launch();
+  return vsr_estimate_slot_windows(hr, mask, slot, 1, 0, h, w, scale, stream);
 }

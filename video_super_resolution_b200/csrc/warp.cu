@@ -188,10 +188,20 @@ __global__ void __launch_bounds__(kThreads)      // (kThreads, 8) = 32 registers
 warp_nhwc3_kernel(const float* __restrict__ src, const float* __restrict__ flow, float* __restrict__ dst,
                   const float* __restrict__ ref, float* __restrict__ norm_out,
                   int64_t n_pix, int H, int W, int bilinear, int vec_store, const PixDecode pd,
-                  int skip, int ref_shared) {
+                  int skip, int ref_shared, int64_t win_src) {
   // skip >= 0 (window mode): batch item b samples image b of `src` when b < skip, else image b+1 -- the
   // neighbours of a frame window with the centre frame left out, no gathered copy of the frames needed;
   // ref_shared: every batch item is compared with the SAME reference image (the centre frame).
+  // blockIdx.y: the frame window (src and ref advance by win_src floats per window, flow / dst / norm_out by the
+  // window's n_pix pixels); a single-window launch has gridDim.y == 1.
+  if (blockIdx.y) {
+    const int64_t wb = blockIdx.y;
+    src += wb * win_src;
+    flow += wb * n_pix * 2;
+    dst += wb * n_pix * 3;
+    if (ref) ref += wb * win_src;
+    if (norm_out) norm_out += wb * n_pix;
+  }
   // two staging buffers, used alternately: one barrier per iteration (the barrier of iteration k+1 separates the
   // reads of buffer k & 1 from its next writes in iteration k+2)
   __shared__ __align__(16) float stage2[2][kThreads * 3];
@@ -356,8 +366,14 @@ warp_nhwc_generic_kernel(const float* __restrict__ src, const float* __restrict_
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kThreads)
 warp_labels_kernel(const uint8_t* __restrict__ labels, const float* __restrict__ flow, uint8_t* __restrict__ dst,
-                   int64_t n_pix, int H, int W, int vec, const PixDecode pd) {
+                   int64_t n_pix, int H, int W, int vec, const PixDecode pd, int64_t flow_stride) {
   const int64_t HW = (int64_t)H * W;
+  if (blockIdx.y) {     // window blockIdx.y: labels / dst advance by its n_pix pixels, flow by flow_stride floats
+    const int64_t wb = blockIdx.y;
+    labels += wb * n_pix;
+    dst += wb * n_pix;
+    flow += wb * flow_stride;
+  }
   const int64_t n8 = vec ? n_pix / 8 : 0;
   for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n8; q += (int64_t)gridDim.x * blockDim.x) {
     float4 f[4];
@@ -467,8 +483,14 @@ channelnorm_nchw_kernel(const float* __restrict__ in, float* __restrict__ out, i
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kThreads)
 compose_flow_kernel(const float2* __restrict__ g, const float2* __restrict__ f, float2* __restrict__ out,
-                    int64_t n_pix, int H, int W, const PixDecode pd) {
+                    int64_t n_pix, int H, int W, const PixDecode pd, int64_t win_stride) {
   const int64_t HW = (int64_t)H * W;
+  if (blockIdx.y) {     // window blockIdx.y: g, f and out advance by win_stride flow vectors
+    const int64_t o = blockIdx.y * win_stride;
+    if (g) g += o;
+    f += o;
+    out += o;
+  }
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_pix; i += (int64_t)gridDim.x * blockDim.x) {
     int x, y, bi;
     decode_pix((uint32_t)i, pd, bi, y, x);
@@ -527,10 +549,10 @@ extern "C" int vsr_warp_nhwc_f32(const float* src, const float* flow, float* dst
     int vec = aligned(dst, 16) ? 1 : 0;
     if (bilinear == kModeFast)
       warp_nhwc3_kernel<true><<<grid_for(n_pix, kThreads), kThreads, 0, st>>>(src, flow, dst, ref, norm_out, n_pix, H, W,
-                                                                              1, vec, pd, -1, 0);
+                                                                              1, vec, pd, -1, 0, 0);
     else
       warp_nhwc3_kernel<false><<<grid_for(n_pix, kThreads), kThreads, 0, st>>>(src, flow, dst, ref, norm_out, n_pix, H,
-                                                                               W, bilinear, vec, pd, -1, 0);
+                                                                               W, bilinear, vec, pd, -1, 0, 0);
   } else if ((C % 4) == 0 && norm_out == nullptr && aligned(src, 16) && aligned(dst, 16)) {
     if (bilinear == kModeFast)
       warp_nhwc_vec4_kernel<true><<<grid_for(n_pix * (C / 4), kThreads), kThreads, 0, st>>>(src, flow, dst, n_pix, H, W,
@@ -545,23 +567,33 @@ extern "C" int vsr_warp_nhwc_f32(const float* src, const float* flow, float* dst
   return after_launch();
 }
 
-extern "C" int vsr_warp_window_nhwc3(const float* frames, const float* flows, float* warped, float* resid, int T,
-                                     int centre, int H, int W, int bilinear, vsr_stream_t stream) {
-  if (!frames || !flows || !warped || T < 2 || centre < 0 || centre >= T || H <= 0 || W <= 0) return VSR_ERR_INVALID_ARG;
+extern "C" int vsr_warp_windows_nhwc3(const float* frames, const float* flows, float* warped, float* resid, int windows,
+                                      int T, int centre, int H, int W, int bilinear, vsr_stream_t stream) {
+  if (!frames || !flows || !warped || windows < 1 || windows > 65535 || T < 2 || centre < 0 || centre >= T || H <= 0 ||
+      W <= 0)
+    return VSR_ERR_INVALID_ARG;
   if (bilinear < 0 || bilinear > kModeFast || !aligned(flows, 8)) return VSR_ERR_INVALID_ARG;
-  const int64_t n_pix = (int64_t)(T - 1) * H * W;
+  const int64_t n_pix = (int64_t)(T - 1) * H * W;     // per window
   if (n_pix >= ((int64_t)1 << 32)) return VSR_ERR_UNSUPPORTED;
   const PixDecode pd = make_pixdecode(H, W);
   const float* ref = resid ? frames + (int64_t)centre * H * W * 3 : nullptr;
-  const int vec = aligned(warped, 16) ? 1 : 0;
+  // 16-byte stores need every window's output to start 16-byte aligned
+  const int vec = aligned(warped, 16) && (windows == 1 || (n_pix * 3) % 4 == 0) ? 1 : 0;
+  const int64_t win_src = (int64_t)T * H * W * 3;
+  const dim3 grid(grid_for(n_pix, kThreads), windows);
   cudaStream_t st = as_stream(stream);
   if (bilinear == kModeFast)
-    warp_nhwc3_kernel<true><<<grid_for(n_pix, kThreads), kThreads, 0, st>>>(frames, flows, warped, ref, resid, n_pix, H, W,
-                                                                            1, vec, pd, centre, 1);
+    warp_nhwc3_kernel<true><<<grid, kThreads, 0, st>>>(frames, flows, warped, ref, resid, n_pix, H, W, 1, vec, pd, centre,
+                                                       1, win_src);
   else
-    warp_nhwc3_kernel<false><<<grid_for(n_pix, kThreads), kThreads, 0, st>>>(frames, flows, warped, ref, resid, n_pix, H,
-                                                                             W, bilinear, vec, pd, centre, 1);
+    warp_nhwc3_kernel<false><<<grid, kThreads, 0, st>>>(frames, flows, warped, ref, resid, n_pix, H, W, bilinear, vec, pd,
+                                                        centre, 1, win_src);
   return after_launch();
+}
+
+extern "C" int vsr_warp_window_nhwc3(const float* frames, const float* flows, float* warped, float* resid, int T,
+                                     int centre, int H, int W, int bilinear, vsr_stream_t stream) {
+  return vsr_warp_windows_nhwc3(frames, flows, warped, resid, 1, T, centre, H, W, bilinear, stream);
 }
 
 extern "C" int vsr_compose_flow(const float* g, const float* f, float* out, int B, int H, int W, vsr_stream_t stream) {
@@ -571,7 +603,20 @@ extern "C" int vsr_compose_flow(const float* g, const float* f, float* out, int 
   if (n_pix >= ((int64_t)1 << 32)) return VSR_ERR_UNSUPPORTED;
   compose_flow_kernel<<<grid_for(n_pix, kThreads), kThreads, 0, as_stream(stream)>>>(
       reinterpret_cast<const float2*>(g), reinterpret_cast<const float2*>(f), reinterpret_cast<float2*>(out), n_pix, H, W,
-      make_pixdecode(H, W));
+      make_pixdecode(H, W), 0);
+  return after_launch();
+}
+
+extern "C" int vsr_compose_flow_windows(const float* g, const float* f, float* out, int windows, int64_t stride, int H,
+                                        int W, vsr_stream_t stream) {
+  if (!f || !out || windows < 1 || windows > 65535 || stride < 0 || (stride & 1) || H <= 0 || W <= 0)
+    return VSR_ERR_INVALID_ARG;
+  if (!aligned(g, 8) || !aligned(f, 8) || !aligned(out, 8)) return VSR_ERR_INVALID_ARG;
+  const int64_t n_pix = (int64_t)H * W;
+  if (n_pix >= ((int64_t)1 << 32)) return VSR_ERR_UNSUPPORTED;
+  compose_flow_kernel<<<dim3(grid_for(n_pix, kThreads), windows), kThreads, 0, as_stream(stream)>>>(
+      reinterpret_cast<const float2*>(g), reinterpret_cast<const float2*>(f), reinterpret_cast<float2*>(out), n_pix, H, W,
+      make_pixdecode(H, W), stride / 2);
   return after_launch();
 }
 
@@ -583,7 +628,22 @@ extern "C" int vsr_warp_labels_u8(const uint8_t* labels, const float* flow, uint
   if (n_pix >= ((int64_t)1 << 32)) return VSR_ERR_UNSUPPORTED;   // 32-bit index decode
   int vec = (aligned(flow, 16) && aligned(dst, 8)) ? 1 : 0;
   warp_labels_kernel<<<grid_for(ceil_div64(n_pix, 8), kThreads), kThreads, 0, as_stream(stream)>>>(labels, flow, dst,
-                                                                                                  n_pix, H, W, vec, make_pixdecode(H, W));
+                                                                                                  n_pix, H, W, vec, make_pixdecode(H, W), 0);
+  return after_launch();
+}
+
+extern "C" int vsr_warp_labels_u8_windows(const uint8_t* labels, const float* flow, uint8_t* dst, int windows,
+                                          int64_t flow_stride, int H, int W, vsr_stream_t stream) {
+  if (!labels || !flow || !dst || windows < 1 || windows > 65535 || flow_stride < 0 || H <= 0 || W <= 0)
+    return VSR_ERR_INVALID_ARG;
+  if (!aligned(flow, 8) || (flow_stride & 1)) return VSR_ERR_INVALID_ARG;
+  const int64_t n_pix = (int64_t)H * W;     // per window
+  if (n_pix >= ((int64_t)1 << 32)) return VSR_ERR_UNSUPPORTED;
+  // the vector path needs every window's flow 16-byte and output 8-byte aligned
+  const int vec = (aligned(flow, 16) && aligned(dst, 8) && (windows == 1 || (flow_stride % 4 == 0 && n_pix % 8 == 0)))
+                      ? 1 : 0;
+  warp_labels_kernel<<<dim3(grid_for(ceil_div64(n_pix, 8), kThreads), windows), kThreads, 0, as_stream(stream)>>>(
+      labels, flow, dst, n_pix, H, W, vec, make_pixdecode(H, W), flow_stride);
   return after_launch();
 }
 

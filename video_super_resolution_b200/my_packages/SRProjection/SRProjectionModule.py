@@ -5,6 +5,8 @@ maps) with the reference's surface:
                        num_steps=3, num_groups=6, act_type='prelu', norm_type=None)
     .forward(x (M,3,h,w) fp32 0..255) -> (1,3,s*h,s*w) fp32
     ref: my_packages/SRProjection/SRProjectionModule.py:96-150
+    .forward(x (W*M,3,h,w) or (W,M,3,h,w)) -> (W,3,s*h,s*w): W frame windows in one pass of the plan, frame b
+    bit-identical to a forward of window b alone
 
 Parameters carry the reference's state-dict names and shapes (SURVEY.md Appendix C), so a
 checkpoint written by the reference's main.py:233-237 loads with load_state_dict unchanged; the only
@@ -84,7 +86,7 @@ class SRProjectionModule(nn.Module):
         self.conv_out = _block(nn.Conv2d(nf, out_channels, 3, padding=1), act=False)
         self.add_mean = _MeanShift(RGB_MEAN, 1)
         self.fc = nn.Sequential(nn.Linear(num_maps, 32), nn.ReLU(), nn.Linear(32, 1), nn.ReLU())
-        self._plans = {}          # (h, w, device) -> dict(plan, weights, workspace, version)
+        self._plans = {}          # (M, h, w, device[, W if W > 1]) -> dict(plan, weights, workspace, version)
         self._keep = []
 
     # -- C ABI plumbing ---------------------------------------------------------------------------
@@ -127,8 +129,9 @@ class SRProjectionModule(nn.Module):
     def _version(self):
         return tuple((p.data_ptr(), p._version) for p in self.parameters())
 
-    def _plan_for(self, M, h, w, device):
-        key = (M, h, w, device.index)
+    def _plan_for(self, M, h, w, device, windows=1):
+        # one plan per window count; a one-window plan keeps the key it has always had
+        key = (M, h, w, device.index) + ((windows,) if windows > 1 else ())
         ent = self._plans.get(key)
         ver = self._version()
         L = _lib.lib()
@@ -136,6 +139,11 @@ class SRProjectionModule(nn.Module):
             cfg = _lib.SrfbnConfig(M, h, w, self.num_steps, 6, self.num_features, self.upscale_factor)
             plan = ctypes.c_void_p()
             _lib.check(L.vsr_srfbn_plan_create(ctypes.byref(cfg), ctypes.byref(plan)), "srfbn_plan_create")
+            if windows > 1:
+                rc = L.vsr_srfbn_plan_set_windows(plan, int(windows))
+                if rc:
+                    L.vsr_srfbn_plan_destroy(plan)
+                    _lib.check(rc, "srfbn_plan_set_windows")
             if self.workspace_cap_bytes:
                 _lib.check(L.vsr_srfbn_plan_set_workspace_cap(plan, int(self.workspace_cap_bytes)), "srfbn_plan_set_workspace_cap")
             ent = {"plan": plan, "version": None, "chunk_maps": int(L.vsr_srfbn_chunk_maps(plan)),
@@ -156,29 +164,41 @@ class SRProjectionModule(nn.Module):
             ent["refresh_first"] = None
         return ent
 
+    def _windows_of(self, x):
+        """(W*M,3,h,w) or (W,M,3,h,w) -> W; ValueError for any other shape."""
+        M = self.num_maps
+        if x.dim() == 5 and x.shape[0] >= 1 and tuple(x.shape[1:3]) == (M, 3):
+            return x.shape[0]
+        if x.dim() == 4 and x.shape[1] == 3 and x.shape[0] >= M and x.shape[0] % M == 0:
+            return x.shape[0] // M
+        raise ValueError(f"SRProjectionModule: expected ({M},3,h,w), (W*{M},3,h,w) or (W,{M},3,h,w), "
+                         f"got {tuple(x.shape)}")
+
     def forward(self, x, out_u8=None, want_f32=True, changed_from=None):
-        """out_u8: optional (s*h, s*w, 3) u8 CUDA tensor that additionally receives the frame as clamp(y,0,255) rounded
-        half to even (the loader's pixel format, utils/video_utils.py:23), written by the fc-fuse kernel itself;
-        want_f32=False skips the fp32 frame (then the u8 frame is the only output and is what is returned).
+        """x: (M,3,h,w), or W frame windows as (W*M,3,h,w) / (W,M,3,h,w) -> (W,3,s*h,s*w) (W = 1: (1,3,s*h,s*w)).
+        out_u8: optional (W,s*h,s*w,3) (W = 1: also (s*h,s*w,3)) u8 CUDA tensor that additionally receives the frames as
+        clamp(y,0,255) rounded half to even (the loader's pixel format, utils/video_utils.py:23), written by the fc-fuse
+        kernel itself; want_f32=False skips the fp32 frames (then the u8 frames are the only output and are returned).
         changed_from=k: the caller states that, since the previous forward of this module on a stack of this shape, only
-        the maps x[k:] changed (the fuse pass, network/video_super_resolution.py:62, feeds the frames unchanged): the
-        maps are independent until the per-pixel fc, so only x[k:] go through the conv stack again and the per-map images
-        of x[:k] are reused -- bit-identical to a full forward."""
+        the maps [k, M) of each window changed (the fuse pass, network/video_super_resolution.py:62, feeds the frames
+        unchanged): the maps are independent until the per-pixel fc, so only those go through the conv stack again and
+        the per-map images of the others are reused -- bit-identical to a full forward."""
         if not x.is_cuda:
             raise RuntimeError("SRProjectionModule: CUDA tensors only (no CPU fallback)")
-        if x.dim() != 4 or x.shape[1] != 3 or x.shape[0] != self.num_maps:
-            raise ValueError(f"SRProjectionModule: expected ({self.num_maps},3,h,w), got {tuple(x.shape)}")
+        nw = self._windows_of(x)
+        x = x.reshape(nw * self.num_maps, *x.shape[-3:])
         if x.dtype != torch.float32 or not x.is_contiguous():
             x = x.to(torch.float32).contiguous()
-        M, _, h, w = x.shape
-        ent = self._plan_for(M, h, w, x.device)
+        M, h, w = self.num_maps, x.shape[2], x.shape[3]
         s = self.upscale_factor
+        shapes = [(nw, s * h, s * w, 3)] + ([(s * h, s * w, 3)] if nw == 1 else [])
         if out_u8 is not None and (not out_u8.is_cuda or out_u8.dtype != torch.uint8 or not out_u8.is_contiguous()
-                                   or tuple(out_u8.shape) != (s * h, s * w, 3)):
-            raise ValueError(f"SRProjectionModule: out_u8 must be a contiguous CUDA u8 tensor of shape {(s * h, s * w, 3)}")
+                                   or tuple(out_u8.shape) not in shapes):
+            raise ValueError(f"SRProjectionModule: out_u8 must be a contiguous CUDA u8 tensor of shape {shapes[-1]}")
         if out_u8 is None and not want_f32:
             raise ValueError("SRProjectionModule: nothing to compute")
-        y = torch.empty((1, 3, s * h, s * w), dtype=torch.float32, device=x.device) if want_f32 else None
+        ent = self._plan_for(M, h, w, x.device, nw)
+        y = torch.empty((nw, 3, s * h, s * w), dtype=torch.float32, device=x.device) if want_f32 else None
         L = _lib.lib()
         with torch.cuda.device(x.device):
             yp = y.data_ptr() if y is not None else None
@@ -198,12 +218,13 @@ class SRProjectionModule(nn.Module):
         return y if want_f32 else out_u8
 
     def premix(self, x):
-        """Test hook: per-map outputs before the fc fuse, (M,3,4h,4w) (SRProjectionModule.py:143)."""
+        """Test hook: per-map outputs before the fc fuse, (W*M,3,s*h,s*w) (SRProjectionModule.py:143)."""
         self.forward(x)
-        M, _, h, w = x.shape
-        ent = self._plans[(M, h, w, x.device.index)]
+        nw = self._windows_of(x)
+        M, h, w = self.num_maps, x.shape[-2], x.shape[-1]
+        ent = self._plan_for(M, h, w, x.device, nw)
         s = self.upscale_factor
-        out = torch.empty((M, 3, s * h, s * w), dtype=torch.float32, device=x.device)
+        out = torch.empty((nw * M, 3, s * h, s * w), dtype=torch.float32, device=x.device)
         _lib.check(_lib.lib().vsr_srfbn_debug_premix(ent["plan"], out.data_ptr(),
                                                      torch.cuda.current_stream().cuda_stream), "srfbn_debug_premix")
         return out

@@ -34,10 +34,11 @@ class VSR(torch.nn.Module):
         self.VOSModule = VOSProjectionModule(estimator=vos_estimator).eval()
         self._pipes = {}
 
-    def _pipe(self, h, w, device):
-        key = (h, w, device.index)
+    def _pipe(self, h, w, device, windows=1):
+        key = (h, w, device.index) + ((windows,) if windows > 1 else ())
         if key not in self._pipes:
-            self._pipes[key] = WarpFusePipeline(self.window, h, w, self.model, self.model.upscale_factor, device=device)
+            self._pipes[key] = WarpFusePipeline(self.window, h, w, self.model, self.model.upscale_factor, device=device,
+                                                windows=windows)
         return self._pipes[key]
 
     def forward_geometry(self, data, flows, inv_depth, logits_a, logits_b, estimated_image=None):

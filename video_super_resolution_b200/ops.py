@@ -398,3 +398,129 @@ def estimate_slot(hr: torch.Tensor, mask: torch.Tensor | None, slot: torch.Tenso
         _lib.check(_lib.lib().vsr_estimate_slot(hr.data_ptr(), mask.data_ptr() if mask is not None else None,
                                                 slot.data_ptr(), h, w, int(scale), _stream()), "estimate_slot")
     return slot
+
+
+# -- several frame windows per launch ------------------------------------------------------------------------------
+# The per-window stages above with a leading window dimension W: one launch per stage for all W windows, window b
+# bit-identical to the one-window call on it (the one-window entry points are the same kernels with W = 1).
+
+def warp_windows(frames: torch.Tensor, flows: torch.Tensor, centre: int, bilinear: bool | int = 2,
+                 want_resid: bool = True):
+    """warp_window over W windows: frames (W,T,H,W,3), flows (W,T-1,H,W,2) -> warped (W,T-1,H,W,3) and, with
+    want_resid, resid (W,T-1,H,W)."""
+    _req(frames, torch.float32, "frames")
+    _req(flows, torch.float32, "flows")
+    if frames.dim() != 5:
+        raise ValueError("warp_windows: frames (W,T,H,W,3) expected")
+    nw, T, H, W, C = frames.shape
+    if nw < 1 or C != 3 or tuple(flows.shape) != (nw, T - 1, H, W, 2) or not 0 <= centre < T:
+        raise ValueError("warp_windows: frames (W,T,H,W,3), flows (W,T-1,H,W,2), 0 <= centre < T expected")
+    warped = torch.empty((nw, T - 1, H, W, 3), dtype=torch.float32, device=frames.device)
+    resid = torch.empty((nw, T - 1, H, W), dtype=torch.float32, device=frames.device) if want_resid else None
+    with torch.cuda.device(frames.device):
+        _lib.check(_lib.lib().vsr_warp_windows_nhwc3(frames.data_ptr(), flows.data_ptr(), warped.data_ptr(),
+                                                     resid.data_ptr() if resid is not None else None, nw, T,
+                                                     int(centre), H, W, int(bilinear), _stream()), "warp_windows")
+    return warped, resid
+
+
+def vos_threshold_windows(logits_a: torch.Tensor, logits_b: torch.Tensor) -> torch.Tensor:
+    """vos_threshold over W windows: logits (W,h,w) x2 -> mask (W,h,w) u8."""
+    _req(logits_a, torch.float32, "logits_a")
+    _req(logits_b, torch.float32, "logits_b")
+    if logits_a.shape != logits_b.shape or logits_a.dim() != 3 or logits_a.shape[0] < 1:
+        raise ValueError("vos_threshold_windows: two (W,h,w) tensors expected")
+    nw, h, w = logits_a.shape
+    mask = torch.empty((nw, h, w), dtype=torch.uint8, device=logits_a.device)
+    with torch.cuda.device(logits_a.device):
+        _lib.check(_lib.lib().vsr_vos_threshold_windows(logits_a.data_ptr(), logits_b.data_ptr(), mask.data_ptr(), nw,
+                                                        h, w, _stream()), "vos_threshold_windows")
+    return mask
+
+
+def assemble_stacks(warped: torch.Tensor, frames: torch.Tensor, proj: torch.Tensor, resid: torch.Tensor,
+                    depth: torch.Tensor, estimate: torch.Tensor | None, centre_idx: int,
+                    out: torch.Tensor | None = None) -> torch.Tensor:
+    """assemble_stack over W windows -> (W,3T-1,3,h,w).  warped (W,T-1,h,w,3), frames (W,T,h,w,3) (the centre frame
+    and, without an estimate, the fallback LR frame 0 of each window are read from it in place), proj (W,T-1,h,w,2),
+    resid / depth (W,T-1,h,w), estimate (W,3,h,w) | None."""
+    for t, n in ((warped, "warped"), (frames, "frames"), (proj, "proj"), (resid, "resid"), (depth, "depth")):
+        _req(t, torch.float32, n)
+    if frames.dim() != 5:
+        raise ValueError("assemble_stacks: frames (W,T,h,w,3) expected")
+    nw, T, h, w, _ = frames.shape
+    if nw < 1 or frames.shape[4] != 3 or tuple(warped.shape) != (nw, T - 1, h, w, 3) or \
+            tuple(proj.shape) != (nw, T - 1, h, w, 2) or tuple(resid.shape) != (nw, T - 1, h, w) or \
+            tuple(depth.shape) != (nw, T - 1, h, w) or not 0 <= centre_idx < T:
+        raise ValueError("assemble_stacks: inconsistent shapes")
+    if estimate is not None:
+        _req(estimate, torch.float32, "estimate")
+        if tuple(estimate.shape) != (nw, 3, h, w):
+            raise ValueError("assemble_stacks: estimate must be (W,3,h,w)")
+    if out is None:
+        out = torch.empty((nw, 3 * T - 1, 3, h, w), dtype=torch.float32, device=warped.device)
+    else:
+        _req(out, torch.float32, "out")
+        if tuple(out.shape) != (nw, 3 * T - 1, 3, h, w):
+            raise ValueError("assemble_stacks: out must be (W,3T-1,3,h,w)")
+    with torch.cuda.device(warped.device):
+        _lib.check(_lib.lib().vsr_assemble_stack_windows(
+            warped.data_ptr(), frames[0, centre_idx].data_ptr(), proj.data_ptr(), resid.data_ptr(), depth.data_ptr(),
+            estimate.data_ptr() if estimate is not None else None, frames.data_ptr(), out.data_ptr(), nw,
+            T * h * w * 3, T, int(centre_idx), h, w, _stream()), "assemble_stacks")
+    return out
+
+
+def estimate_slots(hr: torch.Tensor, mask: torch.Tensor | None, stack: torch.Tensor, scale: int = 4) -> torch.Tensor:
+    """estimate_slot over W windows: the last map of each window of stack (W,M,3,h,w) <- nearest-downsized hr
+    (W,3,h*scale,w*scale) with the pixels of mask (W,h,w) zeroed.  Written in place; returns stack."""
+    _req(hr, torch.float32, "hr")
+    _req(stack, torch.float32, "stack")
+    if stack.dim() != 5 or stack.shape[2] != 3:
+        raise ValueError("estimate_slots: stack must be (W,M,3,h,w)")
+    nw, M, _, h, w = stack.shape
+    if nw < 1 or tuple(hr.shape) != (nw, 3, h * scale, w * scale):
+        raise ValueError("estimate_slots: hr must be (W,3,h*scale,w*scale)")
+    if mask is not None:
+        _req(mask, torch.uint8, "mask")
+        if tuple(mask.shape) != (nw, h, w):
+            raise ValueError("estimate_slots: mask must be (W,h,w)")
+    with torch.cuda.device(hr.device):
+        _lib.check(_lib.lib().vsr_estimate_slot_windows(hr.data_ptr(), mask.data_ptr() if mask is not None else None,
+                                                        stack[0, M - 1].data_ptr(), nw, M * 3 * h * w, h, w,
+                                                        int(scale), _stream()), "estimate_slots")
+    return stack
+
+
+def compose_flow_windows(g: torch.Tensor | None, f: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+    """compose_flow over W windows on strided views: g, f, out (W,H,W,2) with the same stride between windows (e.g.
+    neighbour n of a (W,T-1,H,W,2) array, x[:, n]), each window's field contiguous.  g=None: out = f."""
+    _req(f.select(0, 0), torch.float32, "f")
+    for t, n in ((g, "g"), (out, "out")):
+        if t is not None:
+            _req(t.select(0, 0), torch.float32, n)
+            if t.shape != f.shape or t.stride(0) != f.stride(0):
+                raise ValueError(f"compose_flow_windows: {n} must have the shape and window stride of f")
+    if f.dim() != 4 or f.shape[3] != 2 or f.shape[0] < 1:
+        raise ValueError("compose_flow_windows: (W,H,W,2) fields expected")
+    nw, H, W, _ = f.shape
+    with torch.cuda.device(f.device):
+        _lib.check(_lib.lib().vsr_compose_flow_windows(g.data_ptr() if g is not None else None, f.data_ptr(),
+                                                       out.data_ptr(), nw, f.stride(0), H, W, _stream()),
+                   "compose_flow_windows")
+    return out
+
+
+def warp_labels_windows(labels: torch.Tensor, flow: torch.Tensor) -> torch.Tensor:
+    """warp_labels over W windows: labels (W,H,W) u8, flow (W,H,W,2) with each window's field contiguous (a view such
+    as x[:, n] of a (W,T-1,H,W,2) array is fine) -> (W,H,W) u8."""
+    _req(labels, torch.uint8, "labels")
+    _req(flow.select(0, 0), torch.float32, "flow")
+    nw, H, W = labels.shape
+    if tuple(flow.shape) != (nw, H, W, 2):
+        raise ValueError("warp_labels_windows: flow must be (W,H,W,2)")
+    dst = torch.empty_like(labels)
+    with torch.cuda.device(labels.device):
+        _lib.check(_lib.lib().vsr_warp_labels_u8_windows(labels.data_ptr(), flow.data_ptr(), dst.data_ptr(), nw,
+                                                         flow.stride(0), H, W, _stream()), "warp_labels_windows")
+    return dst

@@ -16,6 +16,8 @@ out of scope), generalised from the reference's 3-frame window to T frames (M = 
 
 Sharding (SURVEY.md 8e): windows are independent once the recurrence is reset at chunk starts
 (main.py:196), so rank r takes a contiguous chunk of windows; no collective on the hot path.
+Window batching: `WarpFusePipeline(..., windows=W)` runs W independent windows per step with one launch per stage,
+and `run_sequence(..., windows=W)` uses it to advance W of a rank's chunks in lockstep.
 `gather_frames` is the one collective: an all-gather of the u8-quantised output frames.
 """
 from __future__ import annotations
@@ -81,16 +83,25 @@ class WarpFusePipeline:
         "frames"     the T frame maps, which network/video_super_resolution.py:62 feeds unchanged (`data`), are reused;
                      the 2(T-1) flow / depth maps, which the reference re-estimates for pass 2, and the estimate are not
         "unchanged"  every map this pipeline leaves unchanged: all but the estimate slot (flow and depth are inputs
-                     here, not re-estimated)."""
+                     here, not re-estimated).
+    windows: W independent frame windows per step (default 1).  Every stage is one launch for all W windows and window
+    b's results are bit-identical to a one-window step on it.  With W > 1 the inputs and outputs carry a leading window
+    dimension: frames (W,T,h,w,3), flows (W,T-1,h,w,2), inv_depth (W,T-1,h,w), logits (W,h,w), estimate (W,3,h,w),
+    estimate_hr (W,3,s*h,s*w); the stack is (W,M,3,h,w) and the SR frames (W,3,s*h,s*w).  With W = 1 the one-window
+    shapes are taken as before (and the batched ones with a leading 1)."""
 
     def __init__(self, T: int, h: int, w: int, sr: SRProjectionModule | None = None, scale: int = 4,
-                 device="cuda:0", run_fusion: bool = True, max_disp: float | None = None, reuse: str | None = None):
+                 device="cuda:0", run_fusion: bool = True, max_disp: float | None = None, reuse: str | None = None,
+                 windows: int = 1):
         if T < 2:
             raise ValueError("window must hold at least 2 frames")
         if reuse not in (None, "frames", "unchanged"):
             raise ValueError("reuse must be None, 'frames' or 'unchanged'")
+        if int(windows) != windows or windows < 1:
+            raise ValueError("windows must be an integer >= 1")
         self.reuse = reuse
         self.T, self.h, self.w, self.scale = T, h, w, scale
+        self.windows = W = int(windows)
         self.M = 3 * T - 1
         self.centre = T // 2
         self.device = torch.device(device)
@@ -99,58 +110,107 @@ class WarpFusePipeline:
         self.sr = sr if sr is not None else SRProjectionModule(num_maps=self.M)
         if self.sr.num_maps != self.M:
             raise ValueError(f"SRProjectionModule.num_maps={self.sr.num_maps}, window needs {self.M}")
-        self.stack = torch.empty((self.M, 3, h, w), dtype=torch.float32, device=self.device)
-        self.centre_flows = torch.empty((T - 1, h, w, 2), dtype=torch.float32, device=self.device)
+        lead = (W,) if W > 1 else ()
+        self.stack = torch.empty(lead + (self.M, 3, h, w), dtype=torch.float32, device=self.device)
+        self.centre_flows = torch.empty(lead + (T - 1, h, w, 2), dtype=torch.float32, device=self.device)
+        self._stack = self.stack.view(W, self.M, 3, h, w)          # window-major views of the same storage
+        self._centre_flows = self.centre_flows.view(W, T - 1, h, w, 2)
 
     def chain_flows(self, proj, flows):
-        """Fills self.centre_flows (T-1,h,w,2): neighbour order = frame order with the centre left out."""
-        T, c, G = self.T, self.centre, self.centre_flows
-        ops.compose_flow(None, proj[c - 1], out=G[c - 1])
+        """Fills self.centre_flows ([W,]T-1,h,w,2): neighbour order = frame order with the centre left out.
+        proj / flows: ([W,]T-1,h,w,2).  One launch per link for all windows."""
+        T, c, G, W = self.T, self.centre, self._centre_flows, self.windows
+        proj = proj.reshape(W, T - 1, self.h, self.w, 2)
+        flows = flows.reshape(W, T - 1, self.h, self.w, 2)
+        ops.compose_flow_windows(None, proj[:, c - 1], out=G[:, c - 1])
         for t in range(c - 2, -1, -1):
-            ops.compose_flow(G[t + 1], proj[t], out=G[t])
+            ops.compose_flow_windows(G[:, t + 1], proj[:, t], out=G[:, t])
         if c + 1 < T:
-            ops.compose_flow(None, flows[c], out=G[c])               # frame c+1 is neighbour index c
+            ops.compose_flow_windows(None, flows[:, c], out=G[:, c])         # frame c+1 is neighbour index c
             for t in range(c + 2, T):
-                ops.compose_flow(G[t - 2], flows[t - 1], out=G[t - 1])
-        return G
+                ops.compose_flow_windows(G[:, t - 2], flows[:, t - 1], out=G[:, t - 1])
+        return self.centre_flows
 
-    def project_and_warp(self, frames, flows, inv_depth, logits_a, logits_b, estimate=None, estimate_hr=None):
-        """a1-a5 + a7: fills self.stack; returns the intermediate results (for tests).
-        estimate: (3,h,w) LR estimate | None; estimate_hr: (3,s*h,s*w) the previous output frame, downsized here
-        (video_super_resolution.py:35-37); neither: LR frame 0 (:38)."""
-        T, c = self.T, self.centre
-        proj_f, _, cnt_f, hole_f = ops.project_flow(flows, None, self.max_disp)
-        proj_d, wsum, cnt_d, hole_d = ops.project_depth_flow(flows, inv_depth, self.max_disp)
-        G = self.chain_flows(proj_d, flows)
-        warped, resid = ops.warp_window(frames, G, c, 2)          # fast fp32 blend (north star: <= 1e-3)
-        mask = ops.vos_threshold(logits_a, logits_b)
-        mask_w = ops.warp_labels(mask.unsqueeze(0), G[c - 1].unsqueeze(0))[0]
-        ops.assemble_stack(warped, frames[c], proj_f, resid, wsum, estimate, c, out=self.stack, fallback=frames[0])
+    def _batched(self, frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr):
+        """The inputs as window-major (W,...) tensors; raises ValueError on a shape that fits neither form."""
+        W, T, h, w, s = self.windows, self.T, self.h, self.w, self.scale
+        single = W == 1 and frames.dim() == 4
+        lead = () if single else (W,)
+        want = {"frames": (T, h, w, 3), "flows": (T - 1, h, w, 2), "inv_depth": (T - 1, h, w), "logits_a": (h, w),
+                "logits_b": (h, w), "estimate": (3, h, w), "estimate_hr": (3, s * h, s * w)}
+        got = {"frames": frames, "flows": flows, "inv_depth": inv_depth, "logits_a": logits_a, "logits_b": logits_b,
+               "estimate": estimate, "estimate_hr": estimate_hr}
+        for k, t in got.items():
+            if t is not None and tuple(t.shape) != lead + want[k]:
+                raise ValueError(f"WarpFusePipeline: {k} must be {lead + want[k]}, got {tuple(t.shape)}")
+            if t is not None and not t.is_contiguous():
+                raise ValueError(f"WarpFusePipeline: {k}: tensor must be contiguous")
+        return {k: (t.unsqueeze(0) if single and t is not None else t) for k, t in got.items()}, single
+
+    def project_and_warp(self, frames, flows, inv_depth, logits_a, logits_b, estimate=None, estimate_hr=None,
+                         estimate_hr_windows=None):
+        """a1-a5 + a7: fills self.stack; returns the intermediate results (for tests), with the leading window
+        dimension when the inputs have it.
+        estimate: ([W,]3,h,w) LR estimate | None; estimate_hr: ([W,]3,s*h,s*w) the previous output frame, downsized here
+        (video_super_resolution.py:35-37); neither: LR frame 0 (:38).  estimate_hr_windows: the windows that take
+        estimate_hr (default all); the others keep LR frame 0."""
+        x, single = self._batched(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr)
+        W, T, c, h, w = self.windows, self.T, self.centre, self.h, self.w
+        fl = x["flows"].reshape(W * (T - 1), h, w, 2)
+        proj_f, _, cnt_f, hole_f = ops.project_flow(fl, None, self.max_disp)
+        proj_d, wsum, cnt_d, hole_d = ops.project_depth_flow(fl, x["inv_depth"].reshape(W * (T - 1), h, w),
+                                                             self.max_disp)
+        self.chain_flows(proj_d, fl)
+        G = self._centre_flows
+        warped, resid = ops.warp_windows(x["frames"], G, c, 2)     # fast fp32 blend (north star: <= 1e-3)
+        mask = ops.vos_threshold_windows(x["logits_a"], x["logits_b"])
+        mask_w = ops.warp_labels_windows(mask, G[:, c - 1])
+        ops.assemble_stacks(warped, x["frames"], proj_f.view(W, T - 1, h, w, 2), resid, wsum.view(W, T - 1, h, w),
+                            x["estimate"], c, out=self._stack)
         if estimate is None and estimate_hr is not None:
-            ops.estimate_slot(estimate_hr, None, self.stack[self.M - 1], self.scale)
-        return {"proj_flow": proj_f, "count_flow": cnt_f, "hole_flow": hole_f, "proj_depth": proj_d, "wsum": wsum,
-                "count_depth": cnt_d, "hole_depth": hole_d, "warped": warped, "resid": resid, "mask": mask,
-                "mask_warped": mask_w, "centre_flows": G}
+            sel = range(W) if estimate_hr_windows is None else sorted(set(estimate_hr_windows))
+            for a, b in _runs(sel):                                    # one launch per run of consecutive windows
+                ops.estimate_slots(x["estimate_hr"][a:b], None, self._stack[a:b], self.scale)
+        r = {"proj_flow": proj_f, "count_flow": cnt_f, "hole_flow": hole_f, "proj_depth": proj_d, "wsum": wsum,
+             "count_depth": cnt_d, "hole_depth": hole_d}
+        r = {k: v.view((W, T - 1) + tuple(v.shape[1:])) for k, v in r.items()}
+        r.update({"warped": warped, "resid": resid, "mask": mask, "mask_warped": mask_w, "centre_flows": G})
+        return {k: v[0] for k, v in r.items()} if single else r
 
     def step(self, frames, flows, inv_depth, logits_a, logits_b, estimate=None, estimate_hr=None, out_u8=None,
-             want_f32=True):
+             want_f32=True, estimate_hr_windows=None):
         """frames (T,h,w,3) 0..255, flows (T-1,h,w,2), inv_depth (T-1,h,w), logits (h,w) x2,
         estimate (3,h,w)|None -> SR frame (1,3,s*h,s*w) fp32 [and / or out_u8 (s*h,s*w,3) u8].
+        With W windows: the same with a leading W (class docstring) -> (W,3,s*h,s*w) [and / or out_u8 (W,s*h,s*w,3)].
         Every kernel between the first and the last launch of a step is this library's."""
-        r = self.project_and_warp(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr)
+        r = self.project_and_warp(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr,
+                                  estimate_hr_windows)
         if not self.run_fusion:
             return self.stack
         out1 = self.sr(self.stack)                                             # pass 1
-        ops.estimate_slot(out1[0], r["mask_warped"], self.stack[self.M - 1], self.scale)
+        mask_w = r["mask_warped"]
+        ops.estimate_slots(out1, mask_w.view(self.windows, self.h, self.w), self._stack, self.scale)
         changed_from = {None: None, "frames": self.T, "unchanged": self.M - 1}[self.reuse]
         return self.sr(self.stack, out_u8=out_u8, want_f32=want_f32, changed_from=changed_from)   # pass 2 (fuse)
+
+
+def _runs(sel):
+    """[a, b) ranges of consecutive integers in the sorted sequence sel."""
+    out = []
+    for k in sel:
+        if out and out[-1][1] == k:
+            out[-1][1] = k + 1
+        else:
+            out.append([k, k + 1])
+    return [tuple(r) for r in out]
 
 
 class GraphedStep:
     """The per-frame sequence of WarpFusePipeline.step captured once into a CUDA graph (SURVEY.md 7 step 6) and replayed:
     ~190 launches (projection stages, flow chains, warps, stack, two conv-stack passes) become one graph launch.
     Inputs live in static device buffers (`inputs`: copy -- or H2D-copy -- each window into them, then `replay()`);
-    outputs are the static `frame_u8` (s*h, s*w, 3) and, with want_f32, `frame` (1,3,s*h,s*w).
+    outputs are the static `frame_u8` (s*h, s*w, 3) and, with want_f32, `frame` (1,3,s*h,s*w); for a pipeline of W > 1
+    windows the inputs and `frame_u8` have a leading W and `frame` is (W,3,s*h,s*w).
     The step is GPU-bound (100 ms of kernels against ~1 ms of launch calls), so this buys little at C2; it matters for
     small frames, where the front's 40 launches of 5-10 us each are launch-latency bound.
     The graph holds whichever projection path torch.are_deterministic_algorithms_enabled() selected at capture time
@@ -160,10 +220,11 @@ class GraphedStep:
         T, h, w, s, dev = pipe.T, pipe.h, pipe.w, pipe.scale, pipe.device
         f32 = dict(dtype=torch.float32, device=dev)
         self.pipe = pipe
-        self.inputs = {"frames": torch.zeros((T, h, w, 3), **f32), "flows": torch.zeros((T - 1, h, w, 2), **f32),
-                       "inv_depth": torch.ones((T - 1, h, w), **f32), "logits_a": torch.zeros((h, w), **f32),
-                       "logits_b": torch.zeros((h, w), **f32)}
-        self.frame_u8 = torch.empty((s * h, s * w, 3), dtype=torch.uint8, device=dev)
+        n = (pipe.windows,) if pipe.windows > 1 else ()       # a W-window pipeline: every buffer has a leading W
+        self.inputs = {"frames": torch.zeros(n + (T, h, w, 3), **f32), "flows": torch.zeros(n + (T - 1, h, w, 2), **f32),
+                       "inv_depth": torch.ones(n + (T - 1, h, w), **f32), "logits_a": torch.zeros(n + (h, w), **f32),
+                       "logits_b": torch.zeros(n + (h, w), **f32)}
+        self.frame_u8 = torch.empty(n + (s * h, s * w, 3), dtype=torch.uint8, device=dev)
         self.frame = None
         i = self.inputs
         side = torch.cuda.Stream(device=dev)
@@ -232,13 +293,20 @@ def gather_frames_ragged(local_frames: torch.Tensor, group=None) -> torch.Tensor
     return torch.cat([allf[r, :counts[r]] for r in range(world)])
 
 
-def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tensor | None = None):
+def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tensor | None = None, windows: int = 1):
     """The reference's loop over a video (main.py:190-203) on this rank's chunks.
 
     frames (N,h,w,3) fp32 0..255, flows (N-1,h,w,2), inv_depth (N-1,h,w) on the device; logits: callable
     k -> (logits_a, logits_b) for window k; chunks: list of ranges of window indices (shard_chunks).
     Within a chunk window k+1 receives window k's output as its estimate; every chunk starts with
-    estimated_image = None.  Returns (u8 frames (n_local,H,W,3), list of window indices)."""
+    estimated_image = None.  Returns (u8 frames (n_local,H,W,3), list of window indices).
+    windows=W > 1: up to W chunks advance in lockstep, one window of each per step of a W-window pipeline
+    (WarpFusePipeline(windows=W)), each with its own recurrence; a slot whose chunk ends takes the next chunk.  The
+    frames, and their order, are those of the one-window loop."""
+    if int(windows) != windows or windows < 1:
+        raise ValueError("windows must be an integer >= 1")
+    if windows > 1:
+        return _run_lockstep(vsr, frames, flows, inv_depth, logits, chunks, out, int(windows))
     T = vsr.window
     idx = [k for c in chunks for k in c]
     s = vsr.model.upscale_factor
@@ -256,4 +324,60 @@ def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tenso
             est = pipe.step(frames[k:k + T], flows[k:k + T - 1], inv_depth[k:k + T - 1], la, lb,
                             estimate_hr=None if est is None else est[0], out_u8=out[i])
             i += 1
+    return out, idx
+
+
+def _run_lockstep(vsr, frames, flows, inv_depth, logits, chunks, out, W):
+    """run_sequence with W chunk slots.  Each step gathers one window per slot into the pipeline's (W,...) inputs (device
+    copies), runs one batched step and copies the live slots' u8 frames to their places in `out`.  Slot j's estimate
+    is frame j of the previous step's fp32 output unless its chunk just started (then LR frame 0, as the one-window
+    loop).  A slot without a chunk left (the tail) repeats a live slot's inputs and its frame is dropped."""
+    T = vsr.window
+    chunks = [c for c in chunks if len(c) > 0]
+    idx = [k for c in chunks for k in c]
+    s = vsr.model.upscale_factor
+    h, w = frames.shape[1:3]
+    dev = frames.device
+    if out is None:
+        out = torch.empty((len(idx), s * h, s * w, 3), dtype=torch.uint8, device=dev)
+    if not chunks:
+        return out, idx
+    pipe = vsr._pipe(h, w, dev, windows=W)
+    f32 = dict(dtype=torch.float32, device=dev)
+    fb, flb = torch.empty((W, T, h, w, 3), **f32), torch.empty((W, T - 1, h, w, 2), **f32)
+    db, lab, lbb = torch.empty((W, T - 1, h, w), **f32), torch.empty((W, h, w), **f32), torch.empty((W, h, w), **f32)
+    ub = torch.empty((W, s * h, s * w, 3), dtype=torch.uint8, device=dev)
+    starts, acc = [], 0                                  # position of each chunk's first frame in `out`
+    for c in chunks:
+        starts.append(acc)
+        acc += len(c)
+    nxt = 0
+    slots = []                                           # per slot: [chunk number, position in the chunk] or None
+    for _ in range(W):
+        slots.append([nxt, 0] if nxt < len(chunks) else None)
+        nxt += 1 if nxt < len(chunks) else 0
+    prev = None
+    while any(sl is not None for sl in slots):
+        live = [j for j, sl in enumerate(slots) if sl is not None]
+        for j in range(W):
+            ci, pos = slots[j] if slots[j] is not None else slots[live[0]]
+            k = chunks[ci][pos]
+            fb[j].copy_(frames[k:k + T])
+            flb[j].copy_(flows[k:k + T - 1])
+            db[j].copy_(inv_depth[k:k + T - 1])
+            la, lb = logits(k)
+            lab[j].copy_(la)
+            lbb[j].copy_(lb)
+        est = [j for j in live if slots[j][1] > 0]
+        prev = pipe.step(fb, flb, db, lab, lbb, estimate_hr=prev if est else None, estimate_hr_windows=est, out_u8=ub)
+        for j in live:
+            ci, pos = slots[j]
+            out[starts[ci] + pos].copy_(ub[j])
+            if pos + 1 < len(chunks[ci]):
+                slots[j][1] = pos + 1
+            elif nxt < len(chunks):
+                slots[j] = [nxt, 0]                      # the next chunk starts in this slot: recurrence reset
+                nxt += 1
+            else:
+                slots[j] = None
     return out, idx
