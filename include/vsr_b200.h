@@ -379,6 +379,39 @@ int vsr_srfbn_forward_u8(vsr_srfbn_plan* plan, const float* x, float* y, uint8_t
 int vsr_srfbn_prepare_refresh(vsr_srfbn_plan* plan, int first_map);
 int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* plan, const float* x, float* y, uint8_t* y_u8, int first_map,
                                  vsr_stream_t stream);
+/* Map-parallel forward: one frame over G GPUs, bit-identical to vsr_srfbn_forward_u8 on one (DESIGN.md 11).  The maps go
+ * through the conv stack independently until the per-pixel fc, and the fc needs all M maps of a pixel but nothing of
+ * any other pixel, so rank r sweeps the maps [m_r, m_{r+1}), the ranks exchange row bands of the per-map images, and
+ * each rank fuses the rows of its band with the same kernel and the same additions as the one-GPU forward.
+ * vsr_srfbn_plan_set_map_range (before bind, like set_windows / set_workspace_cap): the plan sweeps the stack maps
+ *   [m0, m1) only and lays out the per-map images of m1-m0 maps; x stays the full (M,3,h,w) stack and the fc in-features
+ *   stay M.  A workspace cap chunks inside the range (chunk_maps divides m1-m0).  VSR_ERR_UNSUPPORTED with windows > 1
+ *   (either order); VSR_ERR_WORKSPACE as set_workspace_cap (the plan is then unchanged).  vsr_srfbn_forward[_u8] and
+ *   vsr_srfbn_forward_refresh_u8 return VSR_ERR_UNSUPPORTED on a plan whose range is not all maps.
+ * vsr_srfbn_forward_maps: sweeps the range of x; the per-map images stay in the workspace (no fc).
+ * vsr_srfbn_forward_maps_refresh: after vsr_srfbn_prepare_refresh(plan, first_map) and a forward_maps of the same plan,
+ *   re-sweeps only [max(first_map, m0), m1) -- nothing when that is empty -- for a stack that changed only in the maps
+ *   [first_map, M) (the fuse pass).  windows must be 1.
+ * vsr_srfbn_pack_bands: lr_bounds (host, bands+1 ints) 0 = l_0 < l_1 < ... < l_bands = h, bands 1..64; band p is the HR
+ *   rows [s*l_p, s*l_{p+1}).  Copies the range's per-map images into send (bands, m1-m0, 3, rows_p, s*w) f32, band-major
+ *   and back to back (band p starts (m1-m0)*3*s*l_p*s*w floats in), the send buffer of one all_to_all with split sizes
+ *   (m1-m0)*3*rows_p*s*w.  Maps partitioned contiguously in rank order make each rank's receive buffer (M,3,rows,s*w).
+ * vsr_srfbn_fuse_band: maps (M,3,rows,s*w) f32 (16-byte aligned) -> y_band (3,rows,s*w) f32 (16-byte aligned) and / or
+ *   y_u8_band (rows,s*w,3) u8 -- for band p, the frame's (H,W,3) u8 buffer + s*l_p*W*3 bytes.  rows a multiple of s.
+ *   The fc_fuse kernel of vsr_srfbn_forward_u8 with the band as the frame: every output is bit-identical.
+ * vsr_unpack_bands: the reorder after a gather of bands.  src: `bands` bands band_stride elements apart (0: back to back
+ *   as above), band p holding `planes` planes of bounds[p+1]-bounds[p] rows of `row` elements; dst (planes,
+ *   bounds[bands], row) receives band p's rows at [bounds[p], bounds[p+1]) of every plane.  elem_bytes 1 or 4 (4-byte
+ *   aligned pointers).  E.g. the fp32 frame from (G,3,rows_max,W) padded bands, the (H,W,3) u8 frame (planes 1, row
+ *   W*3 bytes), the (3,h,w) LR estimate slot. */
+int vsr_srfbn_plan_set_map_range(vsr_srfbn_plan* plan, int m0, int m1);
+int vsr_srfbn_forward_maps(vsr_srfbn_plan* plan, const float* x, vsr_stream_t stream);
+int vsr_srfbn_forward_maps_refresh(vsr_srfbn_plan* plan, const float* x, int first_map, vsr_stream_t stream);
+int vsr_srfbn_pack_bands(const vsr_srfbn_plan* plan, const int* lr_bounds, int bands, float* send, vsr_stream_t stream);
+int vsr_srfbn_fuse_band(vsr_srfbn_plan* plan, const float* maps, int rows, float* y_band, uint8_t* y_u8_band,
+                        vsr_stream_t stream);
+int vsr_unpack_bands(const void* src, void* dst, int elem_bytes, int64_t planes, int64_t row, const int* bounds,
+                     int bands, int64_t band_stride, vsr_stream_t stream);
 /* Per-launch accounting for bench.py: with profiling enabled, vsr_srfbn_forward brackets every
  * kernel launch with CUDA events on the caller's stream; vsr_srfbn_profile_read waits for the last
  * forward and returns, per kernel class, the summed device time (ms), the number of launches, and

@@ -95,7 +95,14 @@ SIGNATURES = {
     "vsr_srfbn_forward_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vsr_srfbn_prepare_refresh": (c_int, [c_void_p, c_int]),
     "vsr_srfbn_forward_refresh_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
-    "vsr_srfbn_kernel_class_name": (ctypes.c_char_p, [c_int]),
+    "vsr_srfbn_plan_set_map_range": (c_int, [c_void_p, c_int, c_int]),
+    "vsr_srfbn_forward_maps": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "vsr_srfbn_forward_maps_refresh": (c_int, [c_void_p, c_void_p, c_int, c_void_p]),
+    "vsr_srfbn_pack_bands": (c_int, [c_void_p, ctypes.POINTER(c_int), c_int, c_void_p, c_void_p]),
+    "vsr_srfbn_fuse_band": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
+    "vsr_unpack_bands": (c_int, [c_void_p, c_void_p, c_int, c_i64, c_i64, ctypes.POINTER(c_int), c_int, c_i64,
+                                 c_void_p]),
+    "vsr_srfbn_kernel_class_name":(ctypes.c_char_p, [c_int]),
     "vsr_srfbn_profile_enable": (c_int, [c_void_p, c_int]),
     "vsr_srfbn_profile_read": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vsr_srfbn_profile_launches": (c_int, [c_void_p, c_void_p, c_void_p, c_int]),

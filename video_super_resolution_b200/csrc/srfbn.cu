@@ -29,6 +29,7 @@
 
 #include <string.h>
 
+#include <algorithm>
 #include <new>
 #include <vector>
 
@@ -813,6 +814,34 @@ fc_fuse_kernel(const float* __restrict__ maps, const float* __restrict__ fcw, fl
   }
 }
 
+// Row bands of a stack of `planes` images of `rows` rows (bounds[bands]) x `row` elements each.  Band p holds the rows
+// [bounds[p], bounds[p+1]) of every plane, planes one after another (plane stride (bounds[p+1]-bounds[p])*row).  Bands sit
+// at band_stride elements apart, or, with band_stride == 0, back to back (band p at bounds[p]*planes*row: the layout of
+// the send buffer of an all_to_all with split sizes).
+constexpr int kMaxBands = kMaxMaps;
+struct BandGeom {
+  int bands;
+  int bounds[kMaxBands + 1];
+  int64_t planes, row, band_stride;
+};
+
+// to_bands: image stack -> bands (the exchange's pack); else bands -> image stack (the reorder after a gather).
+// blockIdx.y is the band.
+template <typename T>
+__global__ void __launch_bounds__(256)
+band_copy_kernel(const T* __restrict__ src, T* __restrict__ dst, const BandGeom g, int to_bands) {
+  const int p = blockIdx.y;
+  const int64_t y0 = g.bounds[p], plane_band = (g.bounds[p + 1] - y0) * g.row, plane_img = (int64_t)g.bounds[g.bands] * g.row;
+  const int64_t base = g.band_stride ? p * g.band_stride : y0 * g.planes * g.row;
+  const int64_t n = g.planes * plane_band;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t k = i / plane_band, r = i - k * plane_band;
+    const int64_t img = k * plane_img + y0 * g.row + r;
+    if (to_bands) dst[base + i] = __ldg(src + img);
+    else dst[img] = __ldg(src + base + i);
+  }
+}
+
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 }  // namespace
@@ -844,6 +873,7 @@ struct vsr_srfbn_plan {
   int chunk_maps;         // maps processed per sweep over the layer list (a divisor of num_maps; == num_maps: no chunking)
   size_t ws_cap;          // caller's workspace cap in bytes (0 = none)
   int windows;            // frame windows per forward: the sweeps run over windows * num_maps maps
+  int map0, map1;         // the stack maps this plan sweeps (vsr_srfbn_plan_set_map_range; default [0, num_maps))
   bool bound;
   const uint8_t* dev_w;
   uint8_t* ws;
@@ -886,6 +916,9 @@ static void layout_weights(vsr_srfbn_plan* pl) {
   pl->weight_bytes = off;
 }
 
+// maps one forward sweeps: all maps of every window, or the plan's map range (one window)
+static int swept_maps(const vsr_srfbn_plan* pl) { return pl->windows * (pl->map1 - pl->map0); }
+
 // Activations are laid out for `chunk_maps` maps at a time (the maps are independent until the fc fuse, so the layer
 // list is swept once per chunk); only the per-map SR images in front of the fc fuse exist for all windows * num_maps.
 static void layout_workspace(vsr_srfbn_plan* pl) {
@@ -911,7 +944,7 @@ static void layout_workspace(vsr_srfbn_plan* pl) {
   pl->o_hb = put(P * s2 * 64);   // plain-NHWC result of the `out` deconv
   pl->o_ht = put(x2 ? P * s2 * 64 : 0);   // x2: downtran result (the x4 path keeps it on chip)
   pl->o_acc = put(x2 ? 0 : P * 512);   // fp32 partial slots of the fused down kernel
-  pl->o_premix = put((size_t)pl->windows * c.num_maps * c.h * c.w * s2 * 3 * 4);
+  pl->o_premix = put((size_t)swept_maps(pl) * c.h * c.w * s2 * 3 * 4);
   pl->ws_bytes = off;
 }
 
@@ -938,15 +971,17 @@ extern "C" int vsr_srfbn_plan_create(const vsr_srfbn_config* cfg, vsr_srfbn_plan
   pl->chunk_maps = cfg->num_maps;
   pl->ws_cap = 0;
   pl->windows = 1;
+  pl->map0 = 0;
+  pl->map1 = cfg->num_maps;
   layout_weights(pl);
   layout_workspace(pl);
   *out_plan = pl;
   return VSR_OK;
 }
 
-// the largest divisor of windows * num_maps whose workspace fits under the cap (no ragged tail chunk: one layer list)
+// the largest divisor of the swept maps whose workspace fits under the cap (no ragged tail chunk: one layer list)
 static int choose_chunk(vsr_srfbn_plan* pl, size_t cap_bytes) {
-  const int M = pl->windows * pl->cfg.num_maps;
+  const int M = swept_maps(pl);
   for (int mc = M; mc >= 1; --mc) {
     if (M % mc) continue;
     pl->chunk_maps = mc;
@@ -966,11 +1001,28 @@ extern "C" int vsr_srfbn_plan_set_workspace_cap(vsr_srfbn_plan* pl, size_t cap_b
 extern "C" int vsr_srfbn_plan_set_windows(vsr_srfbn_plan* pl, int windows) {
   if (!pl || windows < 1 || windows > 65535) return VSR_ERR_INVALID_ARG;   // fc_fuse_kernel: one grid row per window
   if (pl->bound) return VSR_ERR_STATE;                // buffers and layer list are sized for the window count
+  if (windows > 1 && pl->map1 - pl->map0 != pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;   // not with a map range
   const int old = pl->windows;
   pl->windows = windows;
   const int rc = choose_chunk(pl, pl->ws_cap);
   if (rc) {                                            // leave the plan as it was
     pl->windows = old;
+    choose_chunk(pl, pl->ws_cap);
+  }
+  return rc;
+}
+
+extern "C" int vsr_srfbn_plan_set_map_range(vsr_srfbn_plan* pl, int m0, int m1) {
+  if (!pl || m0 < 0 || m1 > pl->cfg.num_maps || m0 >= m1) return VSR_ERR_INVALID_ARG;
+  if (pl->bound) return VSR_ERR_STATE;
+  if (pl->windows > 1) return VSR_ERR_UNSUPPORTED;
+  const int old0 = pl->map0, old1 = pl->map1;
+  pl->map0 = m0;
+  pl->map1 = m1;
+  const int rc = choose_chunk(pl, pl->ws_cap);
+  if (rc) {
+    pl->map0 = old0;
+    pl->map1 = old1;
     choose_chunk(pl, pl->ws_cap);
   }
   return rc;
@@ -1167,16 +1219,21 @@ static int build_layer_list(vsr_srfbn_plan* pl, int M, std::vector<Layer>& layer
   return VSR_OK;
 }
 
-// Prepares vsr_srfbn_forward_refresh_u8 for the maps [first_map, num_maps).
+// Prepares vsr_srfbn_forward_refresh_u8 / vsr_srfbn_forward_maps_refresh for the maps [first_map, num_maps), of which a
+// plan with a map range sweeps [max(first_map, map0), map1) -- possibly none.
 extern "C" int vsr_srfbn_prepare_refresh(vsr_srfbn_plan* pl, int first_map) {
   if (!pl) return VSR_ERR_INVALID_ARG;
   if (!pl->bound) return VSR_ERR_STATE;
   if (first_map < 1 || first_map >= pl->cfg.num_maps) return VSR_ERR_INVALID_ARG;
-  if (pl->chunk_maps != pl->windows * pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;   // not with chunked sweeps
+  if (pl->chunk_maps != swept_maps(pl)) return VSR_ERR_UNSUPPORTED;   // not with chunked sweeps
   if (pl->refresh_first == first_map) return VSR_OK;
   pl->refresh_first = -1;
-  const int rc = build_layer_list(pl, pl->cfg.num_maps - first_map, pl->refresh_layers, pl->refresh_conv_out_layer);
-  if (rc) return rc;
+  pl->refresh_layers.clear();
+  const int count = pl->map1 - std::max(first_map, pl->map0);
+  if (count > 0) {
+    const int rc = build_layer_list(pl, count, pl->refresh_layers, pl->refresh_conv_out_layer);
+    if (rc) return rc;
+  }
   pl->refresh_first = first_map;
   return VSR_OK;
 }
@@ -1206,7 +1263,7 @@ static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_o
   {   // the last layer reads the network input (bilinear skip) and writes these maps of the premix buffer
     IgemmParams& cp = layers[conv_out_layer].p;
     cp.skip_src = xc;
-    cp.out = reinterpret_cast<float*>(pl->ws + pl->o_premix) + (int64_t)m0 * 3 * c.upscale * c.upscale * c.h * c.w;
+    cp.out = reinterpret_cast<float*>(pl->ws + pl->o_premix) + (int64_t)(m0 - pl->map0) * 3 * c.upscale * c.upscale * c.h * c.w;
   }
   for (const Layer& L : layers) {
     mark();
@@ -1216,20 +1273,27 @@ static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_o
   return VSR_OK;
 }
 
+// the per-pixel fc across num_maps images of n floats each (maps (windows*num_maps, n)), one window per grid row
+static int launch_fc(vsr_srfbn_plan* pl, const float* maps, float* y, uint8_t* y_u8, int64_t n, int windows,
+                     cudaStream_t st) {
+  int64_t blocks = ceil_div64(ceil_div64(n, 4), 256);
+  if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
+  fc_fuse_kernel<<<dim3((unsigned)blocks, (unsigned)windows), 256, 0, st>>>(
+      maps, reinterpret_cast<const float*>(pl->dev_w + pl->fc_off), y, y_u8, pl->cfg.num_maps, n);
+  return after_launch();
+}
+
 // the per-pixel fc across the num_maps per-map images of each window (SRProjectionModule.py:146), one window per grid row
 static int fuse_maps(vsr_srfbn_plan* pl, float* y, uint8_t* y_u8, cudaStream_t st) {
   const vsr_srfbn_config& c = pl->cfg;
   const int64_t n = (int64_t)3 * c.upscale * c.upscale * c.h * c.w;
-  int64_t blocks = ceil_div64(ceil_div64(n, 4), 256);
-  if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
-  fc_fuse_kernel<<<dim3((unsigned)blocks, (unsigned)pl->windows), 256, 0, st>>>(reinterpret_cast<const float*>(pl->ws + pl->o_premix),
-                                              reinterpret_cast<const float*>(pl->dev_w + pl->fc_off), y, y_u8, c.num_maps, n);
-  return after_launch();
+  return launch_fc(pl, reinterpret_cast<const float*>(pl->ws + pl->o_premix), y, y_u8, n, pl->windows, st);
 }
 
 extern "C" int vsr_srfbn_forward_u8(vsr_srfbn_plan* pl, const float* x, float* y, uint8_t* y_u8, vsr_stream_t stream) {
   if (!pl || !x || (!y && !y_u8)) return VSR_ERR_INVALID_ARG;
   if (!pl->bound) return VSR_ERR_STATE;
+  if (swept_maps(pl) != pl->windows * pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;   // a map range fuses by bands
   cudaStream_t st = as_stream(stream);
   const vsr_srfbn_config& c = pl->cfg;
   const int Mc = pl->chunk_maps;
@@ -1258,6 +1322,7 @@ extern "C" int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* pl, const float* x, 
                                             vsr_stream_t stream) {
   if (!pl || !x || (!y && !y_u8)) return VSR_ERR_INVALID_ARG;
   if (!pl->bound || !pl->premix_valid || pl->refresh_first != first_map || first_map < 1) return VSR_ERR_STATE;
+  if (swept_maps(pl) != pl->windows * pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;
   cudaStream_t st = as_stream(stream);
   const int M = pl->cfg.num_maps;
   for (int b = 0; b < pl->windows; ++b) {
@@ -1266,6 +1331,100 @@ extern "C" int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* pl, const float* x, 
     if (rc) return rc;
   }
   return fuse_maps(pl, y, y_u8, st);
+}
+
+// ---- map-parallel forward: the plan's map range, row bands, band fuse ----
+
+extern "C" int vsr_srfbn_forward_maps(vsr_srfbn_plan* pl, const float* x, vsr_stream_t stream) {
+  if (!pl || !x) return VSR_ERR_INVALID_ARG;
+  if (!pl->bound) return VSR_ERR_STATE;
+  cudaStream_t st = as_stream(stream);
+  const int Mc = pl->chunk_maps;
+  for (int m0 = pl->map0; m0 < pl->map0 + swept_maps(pl); m0 += Mc) {
+    int rc = sweep_maps(pl, pl->layers, pl->conv_out_layer, x, m0, Mc, st, nullptr);
+    if (rc) return rc;
+  }
+  pl->premix_valid = true;
+  return VSR_OK;
+}
+
+extern "C" int vsr_srfbn_forward_maps_refresh(vsr_srfbn_plan* pl, const float* x, int first_map, vsr_stream_t stream) {
+  if (!pl || !x) return VSR_ERR_INVALID_ARG;
+  if (!pl->bound || !pl->premix_valid || pl->refresh_first != first_map || first_map < 1) return VSR_ERR_STATE;
+  if (pl->windows > 1) return VSR_ERR_UNSUPPORTED;
+  const int m0 = std::max(first_map, pl->map0);
+  if (m0 >= pl->map1) return VSR_OK;                   // none of this range's maps changed
+  return sweep_maps(pl, pl->refresh_layers, pl->refresh_conv_out_layer, x, m0, pl->map1 - m0, as_stream(stream),
+                    nullptr);
+}
+
+// bounds[0] == 0 < bounds[1] < ... < bounds[bands] == total, 1 <= bands <= kMaxBands
+static bool bands_ok(const int* bounds, int bands, int total) {
+  if (!bounds || bands < 1 || bands > kMaxBands || bounds[0] != 0 || bounds[bands] != total) return false;
+  for (int p = 0; p < bands; ++p)
+    if (bounds[p + 1] <= bounds[p]) return false;
+  return true;
+}
+
+static int launch_band_copy(const void* src, void* dst, int elem_bytes, const BandGeom& g, int to_bands,
+                            cudaStream_t st) {
+  int max_rows = 0;
+  for (int p = 0; p < g.bands; ++p) max_rows = std::max(max_rows, g.bounds[p + 1] - g.bounds[p]);
+  int64_t blocks = ceil_div64(g.planes * max_rows * g.row, 256);
+  if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
+  const dim3 grid((unsigned)blocks, (unsigned)g.bands);
+  if (elem_bytes == 4)
+    band_copy_kernel<uint32_t><<<grid, 256, 0, st>>>(reinterpret_cast<const uint32_t*>(src),
+                                                     reinterpret_cast<uint32_t*>(dst), g, to_bands);
+  else
+    band_copy_kernel<uint8_t><<<grid, 256, 0, st>>>(reinterpret_cast<const uint8_t*>(src),
+                                                    reinterpret_cast<uint8_t*>(dst), g, to_bands);
+  return after_launch();
+}
+
+extern "C" int vsr_srfbn_pack_bands(const vsr_srfbn_plan* pl, const int* lr_bounds, int bands, float* send,
+                                    vsr_stream_t stream) {
+  if (!pl || !send || !bands_ok(lr_bounds, bands, pl->cfg.h)) return VSR_ERR_INVALID_ARG;
+  if (!pl->bound) return VSR_ERR_STATE;
+  if (pl->windows > 1) return VSR_ERR_UNSUPPORTED;
+  const vsr_srfbn_config& c = pl->cfg;
+  BandGeom g;
+  g.bands = bands;
+  for (int p = 0; p <= bands; ++p) g.bounds[p] = lr_bounds[p] * c.upscale;
+  g.planes = (int64_t)(pl->map1 - pl->map0) * 3;
+  g.row = (int64_t)c.upscale * c.w;
+  g.band_stride = 0;
+  return launch_band_copy(pl->ws + pl->o_premix, send, 4, g, 1, as_stream(stream));
+}
+
+extern "C" int vsr_srfbn_fuse_band(vsr_srfbn_plan* pl, const float* maps, int rows, float* y_band, uint8_t* y_u8_band,
+                                   vsr_stream_t stream) {
+  if (!pl || !maps || (!y_band && !y_u8_band)) return VSR_ERR_INVALID_ARG;
+  if (!pl->bound) return VSR_ERR_STATE;
+  const vsr_srfbn_config& c = pl->cfg;
+  // whole LR rows: every map plane of the band is a multiple of 16 bytes and 4 consecutive outputs share a channel
+  if (rows < 1 || rows % c.upscale || rows > c.upscale * c.h) return VSR_ERR_INVALID_ARG;
+  if (reinterpret_cast<uintptr_t>(maps) % 16 || reinterpret_cast<uintptr_t>(y_band) % 16) return VSR_ERR_INVALID_ARG;
+  return launch_fc(pl, maps, y_band, y_u8_band, (int64_t)3 * rows * c.upscale * c.w, 1, as_stream(stream));
+}
+
+extern "C" int vsr_unpack_bands(const void* bands_src, void* dst, int elem_bytes, int64_t planes, int64_t row,
+                                const int* bounds, int bands, int64_t band_stride, vsr_stream_t stream) {
+  if (!bands_src || !dst || (elem_bytes != 1 && elem_bytes != 4) || planes < 1 || row < 1 || band_stride < 0 ||
+      !bounds || bands < 1 || bands > kMaxBands || !bands_ok(bounds, bands, bounds[bands]))
+    return VSR_ERR_INVALID_ARG;
+  if (elem_bytes == 4 && (reinterpret_cast<uintptr_t>(bands_src) % 4 || reinterpret_cast<uintptr_t>(dst) % 4))
+    return VSR_ERR_INVALID_ARG;
+  BandGeom g;
+  g.bands = bands;
+  for (int p = 0; p <= bands; ++p) {
+    g.bounds[p] = bounds[p];
+    if (p < bands && band_stride && planes * (bounds[p + 1] - bounds[p]) * row > band_stride) return VSR_ERR_INVALID_ARG;
+  }
+  g.planes = planes;
+  g.row = row;
+  g.band_stride = band_stride;
+  return launch_band_copy(bands_src, dst, elem_bytes, g, 0, as_stream(stream));
 }
 
 extern "C" const char* vsr_srfbn_kernel_class_name(int k) {
@@ -1280,7 +1439,7 @@ extern "C" int vsr_srfbn_profile_enable(vsr_srfbn_plan* pl, int enable) {
   if (!pl->bound) return VSR_ERR_STATE;
   pl->profile = enable != 0;
   if (pl->profile && pl->events.empty()) {
-    pl->events.resize((pl->layers.size() + 1) * (size_t)(pl->windows * pl->cfg.num_maps / pl->chunk_maps) + 2);
+    pl->events.resize((pl->layers.size() + 1) * (size_t)(swept_maps(pl) / pl->chunk_maps) + 2);
     for (cudaEvent_t& e : pl->events) {
       cudaError_t r = cudaEventCreate(&e);
       if (r != cudaSuccess) return cuda_status(r);
@@ -1330,7 +1489,7 @@ extern "C" int vsr_srfbn_debug_premix(const vsr_srfbn_plan* pl, float* out_maps,
   if (!pl || !out_maps) return VSR_ERR_INVALID_ARG;
   if (!pl->bound) return VSR_ERR_STATE;
   const vsr_srfbn_config& c = pl->cfg;
-  size_t bytes = (size_t)pl->windows * c.num_maps * 3 * c.upscale * c.upscale * c.h * c.w * 4;
+  size_t bytes = (size_t)swept_maps(pl) * 3 * c.upscale * c.upscale * c.h * c.w * 4;
   return cuda_status(cudaMemcpyAsync(out_maps, pl->ws + pl->o_premix, bytes, cudaMemcpyDeviceToDevice, as_stream(stream)));
 }
 

@@ -7,6 +7,8 @@ maps) with the reference's surface:
     ref: my_packages/SRProjection/SRProjectionModule.py:96-150
     .forward(x (W*M,3,h,w) or (W,M,3,h,w)) -> (W,3,s*h,s*w): W frame windows in one pass of the plan, frame b
     bit-identical to a forward of window b alone
+    SRProjectionModule(..., map_group=pg): one window over the G GPUs of an NCCL process group (DESIGN.md 11), every
+    frame bit-identical to the one-GPU forward; forward(..., gather=False) returns only this rank's row band
 
 Parameters carry the reference's state-dict names and shapes (SURVEY.md Appendix C), so a
 checkpoint written by the reference's main.py:233-237 loads with load_state_dict unchanged; the only
@@ -24,7 +26,8 @@ import ctypes
 import torch
 import torch.nn as nn
 
-from ... import _lib
+from ... import _lib, ops
+from ...map_parallel import as_map_group, band_bounds, exchange_splits, map_ranges
 
 RGB_MEAN = (0.4488, 0.4371, 0.4040)   # SRProjectionModule.py:105
 # (kernel, stride, padding) of the up/down projection units.  x4 is the reference's hard-wired geometry
@@ -64,7 +67,7 @@ class _FeedbackParams(nn.Module):
 
 class SRProjectionModule(nn.Module):
     def __init__(self, in_channels=3, out_channels=3, num_features=32, upscale_factor=4, num_steps=3, num_groups=6,
-                 act_type='prelu', norm_type=None, num_maps=8, workspace_cap_bytes=None):
+                 act_type='prelu', norm_type=None, num_maps=8, workspace_cap_bytes=None, map_group=None):
         super(SRProjectionModule, self).__init__()
         if (in_channels, out_channels, num_features, num_groups) != (3, 3, 32, 6) \
                 or upscale_factor not in GEOMETRY or act_type != 'prelu' or norm_type is not None:
@@ -86,7 +89,12 @@ class SRProjectionModule(nn.Module):
         self.conv_out = _block(nn.Conv2d(nf, out_channels, 3, padding=1), act=False)
         self.add_mean = _MeanShift(RGB_MEAN, 1)
         self.fc = nn.Sequential(nn.Linear(num_maps, 32), nn.ReLU(), nn.Linear(32, 1), nn.ReLU())
-        self._plans = {}          # (M, h, w, device[, W if W > 1]) -> dict(plan, weights, workspace, version)
+        # map_group: an NCCL process group (or a map_parallel.MapGroup); rank r convolves map_ranges(M, G)[r] and fuses
+        # the HR rows of band r
+        self.map_group = as_map_group(map_group)
+        if self.map_group is not None:
+            map_ranges(num_maps, self.map_group.size)          # ValueError for G > M
+        self._plans = {}          # (M, h, w, device[, W if W > 1][, map range]) -> dict(plan, weights, workspace, version)
         self._keep = []
 
     # -- C ABI plumbing ---------------------------------------------------------------------------
@@ -129,9 +137,9 @@ class SRProjectionModule(nn.Module):
     def _version(self):
         return tuple((p.data_ptr(), p._version) for p in self.parameters())
 
-    def _plan_for(self, M, h, w, device, windows=1):
-        # one plan per window count; a one-window plan keeps the key it has always had
-        key = (M, h, w, device.index) + ((windows,) if windows > 1 else ())
+    def _plan_for(self, M, h, w, device, windows=1, map_range=None):
+        # one plan per window count and map range; a one-window plan of all maps keeps the key it has always had
+        key = (M, h, w, device.index) + ((windows,) if windows > 1 else ()) + ((map_range,) if map_range else ())
         ent = self._plans.get(key)
         ver = self._version()
         L = _lib.lib()
@@ -144,6 +152,11 @@ class SRProjectionModule(nn.Module):
                 if rc:
                     L.vsr_srfbn_plan_destroy(plan)
                     _lib.check(rc, "srfbn_plan_set_windows")
+            if map_range:
+                rc = L.vsr_srfbn_plan_set_map_range(plan, *map_range)
+                if rc:
+                    L.vsr_srfbn_plan_destroy(plan)
+                    _lib.check(rc, "srfbn_plan_set_map_range")
             if self.workspace_cap_bytes:
                 _lib.check(L.vsr_srfbn_plan_set_workspace_cap(plan, int(self.workspace_cap_bytes)), "srfbn_plan_set_workspace_cap")
             ent = {"plan": plan, "version": None, "chunk_maps": int(L.vsr_srfbn_chunk_maps(plan)),
@@ -174,7 +187,7 @@ class SRProjectionModule(nn.Module):
         raise ValueError(f"SRProjectionModule: expected ({M},3,h,w), (W*{M},3,h,w) or (W,{M},3,h,w), "
                          f"got {tuple(x.shape)}")
 
-    def forward(self, x, out_u8=None, want_f32=True, changed_from=None):
+    def forward(self, x, out_u8=None, want_f32=True, changed_from=None, gather=True):
         """x: (M,3,h,w), or W frame windows as (W*M,3,h,w) / (W,M,3,h,w) -> (W,3,s*h,s*w) (W = 1: (1,3,s*h,s*w)).
         out_u8: optional (W,s*h,s*w,3) (W = 1: also (s*h,s*w,3)) u8 CUDA tensor that additionally receives the frames as
         clamp(y,0,255) rounded half to even (the loader's pixel format, utils/video_utils.py:23), written by the fc-fuse
@@ -182,9 +195,18 @@ class SRProjectionModule(nn.Module):
         changed_from=k: the caller states that, since the previous forward of this module on a stack of this shape, only
         the maps [k, M) of each window changed (the fuse pass, network/video_super_resolution.py:62, feeds the frames
         unchanged): the maps are independent until the per-pixel fc, so only those go through the conv stack again and
-        the per-map images of the others are reused -- bit-identical to a full forward."""
+        the per-map images of the others are reused -- bit-identical to a full forward.
+        With a map group (one window: x (M,3,h,w) or (1,M,3,h,w)): gather=True returns the full frame on every rank (the
+        u8 frame all-gathered into out_u8, the fp32 frame (1,3,s*h,s*w) gathered when want_f32); gather=False returns
+        this rank's band (1,3,rows,s*w) of the fp32 frame (when want_f32) and writes only the band's rows of out_u8;
+        gather="u8" all-gathers the u8 frame into out_u8 and returns the fp32 band (a recurrence that passes the frame
+        on as its next estimate needs only its own rows).  Without a map group gather must be True."""
         if not x.is_cuda:
             raise RuntimeError("SRProjectionModule: CUDA tensors only (no CPU fallback)")
+        if self.map_group is not None:
+            return self._forward_group(x, out_u8, want_f32, changed_from, gather)
+        if gather is not True:
+            raise ValueError("SRProjectionModule: gather applies to a map group only")
         nw = self._windows_of(x)
         x = x.reshape(nw * self.num_maps, *x.shape[-3:])
         if x.dtype != torch.float32 or not x.is_contiguous():
@@ -204,18 +226,92 @@ class SRProjectionModule(nn.Module):
             yp = y.data_ptr() if y is not None else None
             up = out_u8.data_ptr() if out_u8 is not None else None
             st = torch.cuda.current_stream().cuda_stream
-            if changed_from is None or changed_from <= 0:
-                _lib.check(L.vsr_srfbn_forward_u8(ent["plan"], x.data_ptr(), yp, up, st), "srfbn_forward")
-                ent["have_premix"] = True
-            else:
-                if not ent.get("have_premix"):
-                    raise RuntimeError("SRProjectionModule: changed_from needs a preceding full forward on this shape")
-                if ent.get("refresh_first") != int(changed_from):
-                    _lib.check(L.vsr_srfbn_prepare_refresh(ent["plan"], int(changed_from)), "srfbn_prepare_refresh")
-                    ent["refresh_first"] = int(changed_from)
-                _lib.check(L.vsr_srfbn_forward_refresh_u8(ent["plan"], x.data_ptr(), yp, up, int(changed_from), st),
-                           "srfbn_forward_refresh")
+            self._sweep(ent, x, changed_from, lambda: L.vsr_srfbn_forward_u8(ent["plan"], x.data_ptr(), yp, up, st),
+                        lambda k: L.vsr_srfbn_forward_refresh_u8(ent["plan"], x.data_ptr(), yp, up, k, st))
         return y if want_f32 else out_u8
+
+    def band_geometry(self, h):
+        """(this rank's map range, LR band bounds, HR band bounds) of a map-group forward on LR height h."""
+        G, r, s = self.map_group.size, self.map_group.rank, self.upscale_factor
+        lb = band_bounds(h, G)
+        return map_ranges(self.num_maps, G)[r], lb, [s * b for b in lb]
+
+    def _sweep(self, ent, x, changed_from, full, refresh):
+        """The conv stack over this plan's maps: `full` (all maps) or, for changed_from=k, `refresh` (the maps >= k)."""
+        L = _lib.lib()
+        if changed_from is None or changed_from <= 0:
+            _lib.check(full(), "srfbn_forward")
+            ent["have_premix"] = True
+            return
+        if not ent.get("have_premix"):
+            raise RuntimeError("SRProjectionModule: changed_from needs a preceding full forward on this shape")
+        if ent.get("refresh_first") != int(changed_from):
+            _lib.check(L.vsr_srfbn_prepare_refresh(ent["plan"], int(changed_from)), "srfbn_prepare_refresh")
+            ent["refresh_first"] = int(changed_from)
+        _lib.check(refresh(int(changed_from)), "srfbn_forward_refresh")
+
+    def _forward_group(self, x, out_u8, want_f32, changed_from, gather):
+        """One window over the map group: sweep this rank's maps, pack their row bands, one all_to_all, fuse this rank's
+        band, and (gather) all-gather the bands.  Every kernel is the one-GPU forward's, on the same values."""
+        mg, M, s = self.map_group, self.num_maps, self.upscale_factor
+        if self._windows_of(x) != 1:
+            raise ValueError("SRProjectionModule: a map group runs one frame window per forward (windows > 1 is not "
+                             "supported with map_group)")
+        x = x.reshape(M, *x.shape[-3:])
+        if x.dtype != torch.float32 or not x.is_contiguous():
+            x = x.to(torch.float32).contiguous()
+        h, w = x.shape[2], x.shape[3]
+        H, W = s * h, s * w
+        if out_u8 is not None and (not out_u8.is_cuda or out_u8.dtype != torch.uint8 or not out_u8.is_contiguous()
+                                   or tuple(out_u8.shape) not in ((1, H, W, 3), (H, W, 3))):
+            raise ValueError(f"SRProjectionModule: out_u8 must be a contiguous CUDA u8 tensor of shape {(H, W, 3)}")
+        if out_u8 is None and not want_f32:
+            raise ValueError("SRProjectionModule: nothing to compute")
+        if gather not in (True, False, "u8"):
+            raise ValueError("SRProjectionModule: gather must be True, False or 'u8'")
+        G, r = mg.size, mg.rank
+        (m0, m1), lb, hb = self.band_geometry(h)
+        ent = self._plan_for(M, h, w, x.device, 1, (m0, m1))
+        rows = [hb[p + 1] - hb[p] for p in range(G)]
+        rmax = max(rows)
+        if "send" not in ent:          # exchange buffers, sized once per plan
+            dev = x.device
+            ent["send"] = torch.empty((m1 - m0) * 3 * H * W, dtype=torch.float32, device=dev)
+            ent["recv"] = torch.empty(M * 3 * rows[r] * W, dtype=torch.float32, device=dev)
+            ent["u8_band"] = torch.empty(rmax * W * 3, dtype=torch.uint8, device=dev)
+            ent["u8_all"] = torch.empty(G * rmax * W * 3, dtype=torch.uint8, device=dev)
+            ent["splits"] = exchange_splits(M, h, w, s, G, r)
+            ent["lb"] = (ctypes.c_int * (G + 1))(*lb)
+        L = _lib.lib()
+        plan = ent["plan"]
+        with torch.cuda.device(x.device):
+            st = torch.cuda.current_stream().cuda_stream
+            self._sweep(ent, x, changed_from, lambda: L.vsr_srfbn_forward_maps(plan, x.data_ptr(), st),
+                        lambda k: L.vsr_srfbn_forward_maps_refresh(plan, x.data_ptr(), k, st))
+            _lib.check(L.vsr_srfbn_pack_bands(plan, ent["lb"], G, ent["send"].data_ptr(), st), "srfbn_pack_bands")
+            send_splits, recv_splits = ent["splits"]
+            mg.all_to_all(ent["recv"], ent["send"], recv_splits, send_splits)
+            yb = torch.empty(3 * rmax * W, dtype=torch.float32, device=x.device) if want_f32 else None
+            band = yb[:3 * rows[r] * W].view(1, 3, rows[r], W) if want_f32 else None
+            if out_u8 is None:
+                u8p = None
+            elif gather:
+                u8p = ent["u8_band"].data_ptr()
+            else:
+                u8p = out_u8.data_ptr() + hb[r] * W * 3           # this band's rows of the caller's (H,W,3) frame
+            _lib.check(L.vsr_srfbn_fuse_band(plan, ent["recv"].data_ptr(), rows[r], yb.data_ptr() if want_f32 else None,
+                                             u8p, st), "srfbn_fuse_band")
+            if out_u8 is not None and gather:
+                mg.all_gather(ent["u8_all"], ent["u8_band"])
+                ops.unpack_bands(ent["u8_all"], out_u8, hb, 1, W * 3, rmax * W * 3)
+            if gather is not True:
+                return band if want_f32 else out_u8
+            if not want_f32:
+                return out_u8
+            y_all = torch.empty(G * yb.numel(), dtype=torch.float32, device=x.device)
+            mg.all_gather(y_all, yb)
+            y = torch.empty((1, 3, H, W), dtype=torch.float32, device=x.device)
+            return ops.unpack_bands(y_all, y, hb, 3, W, yb.numel())
 
     def premix(self, x):
         """Test hook: per-map outputs before the fc fuse, (W*M,3,s*h,s*w) (SRProjectionModule.py:143)."""

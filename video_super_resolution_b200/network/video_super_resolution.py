@@ -13,6 +13,8 @@ VOS-masked first-pass output and runs them again (:43-64).  Differences, all for
     benchmarks and tests use;
   * the window is T frames (the reference hard-wires 3), M = 3T-1 maps;
   * losses (loss_function.py) are out of scope: `train=True` raises.
+`map_group=pg` (an NCCL process group) runs every window over the group's GPUs (pipeline.WarpFusePipeline,
+DESIGN.md 11); every rank of the group calls forward with the same inputs and gets the same frame.
 """
 import torch
 
@@ -25,10 +27,10 @@ from ..utils.tools import transpose1312
 
 
 class VSR(torch.nn.Module):
-    def __init__(self, window=3, flow_estimator=None, depth_estimator=None, vos_estimator=None):
+    def __init__(self, window=3, flow_estimator=None, depth_estimator=None, vos_estimator=None, map_group=None):
         super(VSR, self).__init__()
         self.window = window
-        self.model = SRProjectionModule(num_maps=3 * window - 1)
+        self.model = SRProjectionModule(num_maps=3 * window - 1, map_group=map_group)
         self.FlowModule = FlowProjectionModule(estimator=flow_estimator).eval()
         self.DepthModule = DepthProjectionModule(estimator=depth_estimator).eval()
         self.VOSModule = VOSProjectionModule(estimator=vos_estimator).eval()
@@ -38,7 +40,7 @@ class VSR(torch.nn.Module):
         key = (h, w, device.index) + ((windows,) if windows > 1 else ())
         if key not in self._pipes:
             self._pipes[key] = WarpFusePipeline(self.window, h, w, self.model, self.model.upscale_factor, device=device,
-                                                windows=windows)
+                                                windows=windows, map_group=self.model.map_group)
         return self._pipes[key]
 
     def forward_geometry(self, data, flows, inv_depth, logits_a, logits_b, estimated_image=None):

@@ -6,6 +6,8 @@ CPU path: a non-CUDA tensor raises.
 """
 from __future__ import annotations
 
+import ctypes
+
 import torch
 
 from . import _lib
@@ -511,16 +513,39 @@ def compose_flow_windows(g: torch.Tensor | None, f: torch.Tensor, out: torch.Ten
     return out
 
 
-def warp_labels_windows(labels: torch.Tensor, flow: torch.Tensor) -> torch.Tensor:
+def warp_labels_windows(labels: torch.Tensor, flow: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
     """warp_labels over W windows: labels (W,H,W) u8, flow (W,H,W,2) with each window's field contiguous (a view such
-    as x[:, n] of a (W,T-1,H,W,2) array is fine) -> (W,H,W) u8."""
+    as x[:, n] of a (W,T-1,H,W,2) array is fine) -> (W,H,W) u8 (written into `out` when given)."""
     _req(labels, torch.uint8, "labels")
     _req(flow.select(0, 0), torch.float32, "flow")
     nw, H, W = labels.shape
     if tuple(flow.shape) != (nw, H, W, 2):
         raise ValueError("warp_labels_windows: flow must be (W,H,W,2)")
-    dst = torch.empty_like(labels)
+    if out is not None:
+        _req(out, torch.uint8, "out")
+        if out.shape != labels.shape:
+            raise ValueError("warp_labels_windows: out must be (W,H,W)")
+    dst = torch.empty_like(labels) if out is None else out
     with torch.cuda.device(labels.device):
         _lib.check(_lib.lib().vsr_warp_labels_u8_windows(labels.data_ptr(), flow.data_ptr(), dst.data_ptr(), nw,
                                                          flow.stride(0), H, W, _stream()), "warp_labels_windows")
+    return dst
+
+
+def unpack_bands(src: torch.Tensor, dst: torch.Tensor, bounds, planes: int, row: int, band_stride: int) -> torch.Tensor:
+    """The reorder after a gather of row bands (vsr_unpack_bands): src holds len(bounds)-1 bands band_stride elements
+    apart (0: back to back), band p `planes` planes of bounds[p+1]-bounds[p] rows of `row` elements; dst (planes,
+    bounds[-1], row) receives band p at rows [bounds[p], bounds[p+1]) of every plane.  fp32 or u8 tensors; returns dst."""
+    if src.dtype != dst.dtype or src.dtype not in (torch.float32, torch.uint8):
+        raise TypeError("unpack_bands: src and dst must both be float32 or both uint8")
+    _req(src, src.dtype, "src")
+    _req(dst, dst.dtype, "dst")
+    G = len(bounds) - 1
+    need = band_stride * (G - 1) + planes * (bounds[-1] - bounds[-2]) * row if band_stride else dst.numel()
+    if dst.numel() != planes * bounds[-1] * row or src.numel() < need:
+        raise ValueError("unpack_bands: buffer sizes do not match the band geometry")
+    b = (ctypes.c_int * (G + 1))(*bounds)
+    with torch.cuda.device(dst.device):
+        _lib.check(_lib.lib().vsr_unpack_bands(src.data_ptr(), dst.data_ptr(), src.element_size(), int(planes), int(row),
+                                               b, G, int(band_stride), _stream()), "unpack_bands")
     return dst

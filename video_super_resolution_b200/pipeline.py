@@ -19,12 +19,16 @@ Sharding (SURVEY.md 8e): windows are independent once the recurrence is reset at
 Window batching: `WarpFusePipeline(..., windows=W)` runs W independent windows per step with one launch per stage,
 and `run_sequence(..., windows=W)` uses it to advance W of a rank's chunks in lockstep.
 `gather_frames` is the one collective: an all-gather of the u8-quantised output frames.
+Map groups (DESIGN.md 11): `WarpFusePipeline(..., map_group=pg)` runs ONE window over the G GPUs of an NCCL group --
+rank 0 builds the stack and broadcasts it, each rank convolves its share of the maps and fuses its row band -- with
+frames bit-identical to one GPU, so `run_sequence(..., map_group=pg)` runs one recurrence on G GPUs.
 """
 from __future__ import annotations
 
 import torch
 
 from . import ops
+from .map_parallel import as_map_group
 from .my_packages.SRProjection.SRProjectionModule import SRProjectionModule
 
 
@@ -88,11 +92,17 @@ class WarpFusePipeline:
     b's results are bit-identical to a one-window step on it.  With W > 1 the inputs and outputs carry a leading window
     dimension: frames (W,T,h,w,3), flows (W,T-1,h,w,2), inv_depth (W,T-1,h,w), logits (W,h,w), estimate (W,3,h,w),
     estimate_hr (W,3,s*h,s*w); the stack is (W,M,3,h,w) and the SR frames (W,3,s*h,s*w).  With W = 1 the one-window
-    shapes are taken as before (and the batched ones with a leading 1)."""
+    shapes are taken as before (and the batched ones with a leading 1).
+    map_group: an NCCL process group of G ranks (one GPU each) that runs each step together, one window (windows must
+    be 1).  Rank 0 builds the stack and VOS mask (a1-a5, a7) and broadcasts them -- with the default atomic projection
+    their fp32 sums can differ in the last bits from rank to rank, and the frame must be fused from maps of ONE stack;
+    the ranks then split the conv stack by maps and the fc by row bands (SRProjectionModule(map_group=...), which `sr`
+    must be, with the same group).  The estimate slot is written band by band (vsr_estimate_slot on each rank's rows)
+    and all-gathered.  Every rank passes the same inputs; rank 0's are the ones used."""
 
     def __init__(self, T: int, h: int, w: int, sr: SRProjectionModule | None = None, scale: int = 4,
                  device="cuda:0", run_fusion: bool = True, max_disp: float | None = None, reuse: str | None = None,
-                 windows: int = 1):
+                 windows: int = 1, map_group=None):
         if T < 2:
             raise ValueError("window must hold at least 2 frames")
         if reuse not in (None, "frames", "unchanged"):
@@ -107,11 +117,29 @@ class WarpFusePipeline:
         self.device = torch.device(device)
         self.run_fusion = run_fusion
         self.max_disp = max_disp
-        self.sr = sr if sr is not None else SRProjectionModule(num_maps=self.M)
+        self.map_group = mg = as_map_group(map_group)
+        if mg is not None and W > 1:
+            raise ValueError("WarpFusePipeline: windows > 1 is not supported with a map group")
+        if sr is not None and getattr(sr.map_group, "pg", sr.map_group) is not getattr(mg, "pg", mg):
+            raise ValueError("WarpFusePipeline: sr must be an SRProjectionModule built with the same map_group")
+        self.sr = sr if sr is not None else SRProjectionModule(num_maps=self.M, map_group=mg)
         if self.sr.num_maps != self.M:
             raise ValueError(f"SRProjectionModule.num_maps={self.sr.num_maps}, window needs {self.M}")
         lead = (W,) if W > 1 else ()
-        self.stack = torch.empty(lead + (self.M, 3, h, w), dtype=torch.float32, device=self.device)
+        self._mask_w = None
+        if mg is None:
+            self.stack = torch.empty(lead + (self.M, 3, h, w), dtype=torch.float32, device=self.device)
+        else:
+            self.map_group = mg = self.sr.map_group
+            (_, _), lb, _ = self.sr.band_geometry(h)        # ValueError for fewer LR rows than ranks
+            # stack and warped VOS mask in one buffer: one broadcast from rank 0
+            nst = self.M * 3 * h * w
+            self._bcast = torch.empty(nst * 4 + h * w, dtype=torch.uint8, device=self.device)
+            self.stack = self._bcast[:nst * 4].view(torch.float32).view(self.M, 3, h, w)
+            self._mask_w = self._bcast[nst * 4:].view(1, h, w)
+            hmax = max(lb[p + 1] - lb[p] for p in range(mg.size))
+            self._slot_send = torch.empty(3 * hmax * w, dtype=torch.float32, device=self.device)
+            self._slot_all = torch.empty(mg.size * 3 * hmax * w, dtype=torch.float32, device=self.device)
         self.centre_flows = torch.empty(lead + (T - 1, h, w, 2), dtype=torch.float32, device=self.device)
         self._stack = self.stack.view(W, self.M, 3, h, w)          # window-major views of the same storage
         self._centre_flows = self.centre_flows.view(W, T - 1, h, w, 2)
@@ -164,7 +192,7 @@ class WarpFusePipeline:
         G = self._centre_flows
         warped, resid = ops.warp_windows(x["frames"], G, c, 2)     # fast fp32 blend (north star: <= 1e-3)
         mask = ops.vos_threshold_windows(x["logits_a"], x["logits_b"])
-        mask_w = ops.warp_labels_windows(mask, G[:, c - 1])
+        mask_w = ops.warp_labels_windows(mask, G[:, c - 1], out=self._mask_w)
         ops.assemble_stacks(warped, x["frames"], proj_f.view(W, T - 1, h, w, 2), resid, wsum.view(W, T - 1, h, w),
                             x["estimate"], c, out=self._stack)
         if estimate is None and estimate_hr is not None:
@@ -178,11 +206,20 @@ class WarpFusePipeline:
         return {k: v[0] for k, v in r.items()} if single else r
 
     def step(self, frames, flows, inv_depth, logits_a, logits_b, estimate=None, estimate_hr=None, out_u8=None,
-             want_f32=True, estimate_hr_windows=None):
+             want_f32=True, estimate_hr_windows=None, estimate_hr_band=None, gather=True):
         """frames (T,h,w,3) 0..255, flows (T-1,h,w,2), inv_depth (T-1,h,w), logits (h,w) x2,
         estimate (3,h,w)|None -> SR frame (1,3,s*h,s*w) fp32 [and / or out_u8 (s*h,s*w,3) u8].
         With W windows: the same with a leading W (class docstring) -> (W,3,s*h,s*w) [and / or out_u8 (W,s*h,s*w,3)].
-        Every kernel between the first and the last launch of a step is this library's."""
+        With a map group: estimate_hr_band = this rank's row band (1,3,rows,s*w) of the previous output frame (what a step
+        with gather="u8" or False returns), the recurrence without a gathered fp32 frame; `gather` as
+        SRProjectionModule.forward (True: full frames on every rank; "u8": out_u8 gathered, this rank's fp32 band
+        returned; False: this rank's band only).
+        Every kernel between the first and the last launch of a step is this library's (and, with a map group, NCCL's)."""
+        if self.map_group is not None:
+            return self._step_group(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr,
+                                    estimate_hr_band, out_u8, want_f32, gather)
+        if estimate_hr_band is not None or gather is not True:
+            raise ValueError("WarpFusePipeline: estimate_hr_band and gather need a map group")
         r = self.project_and_warp(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr,
                                   estimate_hr_windows)
         if not self.run_fusion:
@@ -192,6 +229,35 @@ class WarpFusePipeline:
         ops.estimate_slots(out1, mask_w.view(self.windows, self.h, self.w), self._stack, self.scale)
         changed_from = {None: None, "frames": self.T, "unchanged": self.M - 1}[self.reuse]
         return self.sr(self.stack, out_u8=out_u8, want_f32=want_f32, changed_from=changed_from)   # pass 2 (fuse)
+
+    def _step_group(self, frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr, estimate_hr_band, out_u8,
+                    want_f32, gather):
+        mg = self.map_group
+        if mg.rank == 0:
+            self.project_and_warp(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr)
+        mg.broadcast(self._bcast, 0)                       # the stack and mask every rank convolves
+        if not self.run_fusion:
+            return self.stack
+        if estimate_hr_band is not None:
+            self._slot_from_band(estimate_hr_band, None)
+        band = self.sr(self.stack, gather=False)           # pass 1: this rank's band of the frame
+        self._slot_from_band(band, self._mask_w[0])
+        changed_from = {None: None, "frames": self.T, "unchanged": self.M - 1}[self.reuse]
+        return self.sr(self.stack, out_u8=out_u8, want_f32=want_f32, changed_from=changed_from, gather=gather)
+
+    def _slot_from_band(self, band, mask):
+        """The estimate slot from the frame's row bands: each rank downsizes its band into its LR rows of the slot
+        (vsr_estimate_slot with the band as the frame), and an all-gather assembles the (3,h,w) slot on every rank."""
+        mg, s, w = self.map_group, self.scale, self.w
+        _, lb, hb = self.sr.band_geometry(self.h)
+        r = mg.rank
+        rows, lrows = hb[r + 1] - hb[r], lb[r + 1] - lb[r]
+        if band.numel() != 3 * rows * s * w:
+            raise ValueError(f"WarpFusePipeline: estimate band must be (1,3,{rows},{s * w}), got {tuple(band.shape)}")
+        slot = self._slot_send[:3 * lrows * w].view(3, lrows, w)
+        ops.estimate_slot(band.reshape(3, rows, s * w), None if mask is None else mask[lb[r]:lb[r + 1]], slot, s)
+        mg.all_gather(self._slot_all, self._slot_send)
+        ops.unpack_bands(self._slot_all, self.stack[self.M - 1], lb, 3, w, self._slot_send.numel())
 
 
 def _runs(sel):
@@ -293,7 +359,8 @@ def gather_frames_ragged(local_frames: torch.Tensor, group=None) -> torch.Tensor
     return torch.cat([allf[r, :counts[r]] for r in range(world)])
 
 
-def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tensor | None = None, windows: int = 1):
+def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tensor | None = None, windows: int = 1,
+                 map_group=None):
     """The reference's loop over a video (main.py:190-203) on this rank's chunks.
 
     frames (N,h,w,3) fp32 0..255, flows (N-1,h,w,2), inv_depth (N-1,h,w) on the device; logits: callable
@@ -302,9 +369,19 @@ def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tenso
     estimated_image = None.  Returns (u8 frames (n_local,H,W,3), list of window indices).
     windows=W > 1: up to W chunks advance in lockstep, one window of each per step of a W-window pipeline
     (WarpFusePipeline(windows=W)), each with its own recurrence; a slot whose chunk ends takes the next chunk.  The
-    frames, and their order, are those of the one-window loop."""
+    frames, and their order, are those of the one-window loop.
+    map_group=pg: one recurrence on the G GPUs of the group (vsr = VSR(..., map_group=pg)); every rank of the group
+    calls this with the same chunks and receives the same u8 frames, bit-identical to the one-GPU loop.  Each step
+    passes only this rank's fp32 row band of its output on as the next estimate.  With a world of groups x G ranks
+    (map_parallel.new_map_groups) each group runs its shard_chunks(chunks, num_groups, group index)."""
     if int(windows) != windows or windows < 1:
         raise ValueError("windows must be an integer >= 1")
+    if map_group is not None:
+        own = vsr.model.map_group
+        if own is None or getattr(own, "pg", own) is not getattr(map_group, "pg", map_group):
+            raise ValueError("run_sequence: map_group must be the group the VSR was built with (VSR(map_group=...))")
+        if windows > 1:
+            raise ValueError("run_sequence: windows > 1 is not supported with a map group")
     if windows > 1:
         return _run_lockstep(vsr, frames, flows, inv_depth, logits, chunks, out, int(windows))
     T = vsr.window
@@ -314,6 +391,8 @@ def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tenso
     if out is None:
         out = torch.empty((len(idx), s * h, s * w, 3), dtype=torch.uint8, device=frames.device)
     pipe = vsr._pipe(h, w, frames.device)
+    if pipe.map_group is not None:
+        return _run_group(pipe, frames, flows, inv_depth, logits, chunks, out, idx, T)
     i = 0
     for c in chunks:
         est = None                                                   # recurrence reset at every chunk start (main.py:196)
@@ -323,6 +402,19 @@ def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tenso
             # vsr_estimate_slot; the u8 frame (utils/video_utils.py:23) is written by the fc-fuse kernel itself
             est = pipe.step(frames[k:k + T], flows[k:k + T - 1], inv_depth[k:k + T - 1], la, lb,
                             estimate_hr=None if est is None else est[0], out_u8=out[i])
+            i += 1
+    return out, idx
+
+
+def _run_group(pipe, frames, flows, inv_depth, logits, chunks, out, idx, T):
+    """run_sequence on a map group: the u8 frame of each step is all-gathered, the fp32 estimate stays banded."""
+    i = 0
+    for c in chunks:
+        band = None                                                  # recurrence reset at every chunk start
+        for k in c:
+            la, lb = logits(k)
+            band = pipe.step(frames[k:k + T], flows[k:k + T - 1], inv_depth[k:k + T - 1], la, lb,
+                             estimate_hr_band=band, out_u8=out[i], gather="u8")
             i += 1
     return out, idx
 
