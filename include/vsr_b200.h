@@ -343,7 +343,8 @@ void vsr_srfbn_plan_destroy(vsr_srfbn_plan* plan);
 /* Optional, before vsr_srfbn_bind: cap the activation workspace.  The M stacked maps are independent until the per-pixel
  * fc fuse, so the plan then sweeps its layers over chunks of `vsr_srfbn_chunk_maps` maps (the largest divisor of M whose
  * workspace fits under the cap); results are bit-identical to the unchunked plan.  cap_bytes == 0 removes the cap.
- * VSR_ERR_WORKSPACE if not even one map at a time fits; VSR_ERR_STATE after bind.  (Config C4 unchunked: 89 GB.) */
+ * VSR_ERR_WORKSPACE if not even one map at a time fits (the chunk and workspace are then unchanged, but the cap stays
+ * set and holds for the setters after it); VSR_ERR_STATE after bind.  (Config C4 unchunked: 89 GB.) */
 int vsr_srfbn_plan_set_workspace_cap(vsr_srfbn_plan* plan, size_t cap_bytes);
 int vsr_srfbn_chunk_maps(const vsr_srfbn_plan* plan);
 /* Optional, before vsr_srfbn_bind: the number of frame windows W (1..65535, default 1) one forward fuses.  x is then

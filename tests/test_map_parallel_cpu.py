@@ -102,6 +102,11 @@ def test_plan_map_range_arguments():
         one = L.vsr_srfbn_workspace_bytes(plan)
         assert L.vsr_srfbn_plan_set_workspace_cap(plan, one - 1) == 0
         assert L.vsr_srfbn_chunk_maps(plan) == 1
+        # a range no chunk fits under the cap (the per-map images of 20 maps, not 3) leaves the plan as it was
+        capped = L.vsr_srfbn_workspace_bytes(plan)
+        assert L.vsr_srfbn_plan_set_workspace_cap(plan, capped) == 0
+        assert L.vsr_srfbn_plan_set_map_range(plan, 0, 20) == 3
+        assert L.vsr_srfbn_chunk_maps(plan) == 1 and L.vsr_srfbn_workspace_bytes(plan) == capped
         # host-side checks of the band entry points run before any CUDA call; an unbound plan is a state error
         b = (ctypes.c_int * 3)(0, 5, 9)
         assert L.vsr_srfbn_pack_bands(plan, b, 2, 1, None) == 4

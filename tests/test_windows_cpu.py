@@ -58,11 +58,12 @@ def test_plan_windows_scale_the_workspace_and_chunking():
         assert L.vsr_srfbn_plan_set_windows(two, 3) == 0
         c3 = L.vsr_srfbn_chunk_maps(two)
         assert (3 * M) % c3 == 0 and L.vsr_srfbn_workspace_bytes(two) <= b1
-        # a cap no chunk fits under leaves the plan as it was
+        # a cap no chunk fits under leaves the plan as it was, and the setters after it are held to it
         assert L.vsr_srfbn_plan_set_workspace_cap(two, 0) == 0 and L.vsr_srfbn_chunk_maps(two) == 3 * M
+        b3 = L.vsr_srfbn_workspace_bytes(two)
         assert L.vsr_srfbn_plan_set_workspace_cap(two, 1) == WORKSPACE
         assert L.vsr_srfbn_plan_set_windows(two, 2) == WORKSPACE
-        assert L.vsr_srfbn_chunk_maps(two) > 0
+        assert L.vsr_srfbn_chunk_maps(two) == 3 * M and L.vsr_srfbn_workspace_bytes(two) == b3
         # refresh and forward before bind
         assert L.vsr_srfbn_prepare_refresh(two, 3) == STATE
     finally:

@@ -919,12 +919,15 @@ static void layout_weights(vsr_srfbn_plan* pl) {
 // maps one forward sweeps: all maps of every window, or the plan's map range (one window)
 static int swept_maps(const vsr_srfbn_plan* pl) { return pl->windows * (pl->map1 - pl->map0); }
 
-// Activations are laid out for `chunk_maps` maps at a time (the maps are independent until the fc fuse, so the layer
-// list is swept once per chunk); only the per-map SR images in front of the fc fuse exist for all windows * num_maps.
-static void layout_workspace(vsr_srfbn_plan* pl) {
+// the plan's range is all maps (no map range set): the only kind of plan that fuses whole frames or has several windows
+static bool all_maps(const vsr_srfbn_plan* pl) { return pl->map1 - pl->map0 == pl->cfg.num_maps; }
+
+// Activations are laid out for `chunk` maps at a time (the maps are independent until the fc fuse, so the layer list is
+// swept once per chunk); only the per-map SR images in front of the fc fuse exist for all `swept` maps.
+static void layout_workspace(vsr_srfbn_plan* pl, int chunk, int swept) {
   const vsr_srfbn_config& c = pl->cfg;
-  const size_t P = (size_t)pl->chunk_maps * c.h * c.w;
-  const size_t Rb = (size_t)pl->chunk_maps * (c.h + 1) * (c.w + 1) * 16;
+  const size_t P = (size_t)chunk * c.h * c.w;
+  const size_t Rb = (size_t)chunk * (c.h + 1) * (c.w + 1) * 16;
   size_t off = 0;
   auto put = [&](size_t bytes) {
     size_t o = off;
@@ -944,8 +947,29 @@ static void layout_workspace(vsr_srfbn_plan* pl) {
   pl->o_hb = put(P * s2 * 64);   // plain-NHWC result of the `out` deconv
   pl->o_ht = put(x2 ? P * s2 * 64 : 0);   // x2: downtran result (the x4 path keeps it on chip)
   pl->o_acc = put(x2 ? 0 : P * 512);   // fp32 partial slots of the fused down kernel
-  pl->o_premix = put((size_t)swept_maps(pl) * c.h * c.w * s2 * 3 * 4);
+  pl->o_premix = put((size_t)swept * c.h * c.w * s2 * 3 * 4);
   pl->ws_bytes = off;
+}
+
+// The one place a plan's shape changes: `windows` windows of the maps [m0, m1), in chunks of the largest divisor of
+// the swept maps whose workspace fits under ws_cap (no ragged tail chunk: one layer list).  Several windows need the
+// range of all maps.  The plan changes only when this returns VSR_OK.
+static int set_shape(vsr_srfbn_plan* pl, int windows, int m0, int m1) {
+  if (windows > 1 && m1 - m0 != pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;
+  const int swept = windows * (m1 - m0);
+  for (int mc = swept; mc >= 1; --mc) {
+    if (swept % mc) continue;
+    layout_workspace(pl, mc, swept);
+    if (pl->ws_cap == 0 || pl->ws_bytes <= pl->ws_cap) {
+      pl->windows = windows;
+      pl->map0 = m0;
+      pl->map1 = m1;
+      pl->chunk_maps = mc;
+      return VSR_OK;
+    }
+  }
+  layout_workspace(pl, pl->chunk_maps, swept_maps(pl));   // not even one map at a time fits: back to the plan's layout
+  return VSR_ERR_WORKSPACE;
 }
 
 extern "C" int vsr_srfbn_plan_create(const vsr_srfbn_config* cfg, vsr_srfbn_plan** out_plan) {
@@ -968,64 +992,32 @@ extern "C" int vsr_srfbn_plan_create(const vsr_srfbn_config* cfg, vsr_srfbn_plan
   pl->refresh_conv_out_layer = -1;
   pl->premix_valid = false;
   pl->profile = false;
-  pl->chunk_maps = cfg->num_maps;
   pl->ws_cap = 0;
-  pl->windows = 1;
-  pl->map0 = 0;
-  pl->map1 = cfg->num_maps;
   layout_weights(pl);
-  layout_workspace(pl);
+  set_shape(pl, 1, 0, cfg->num_maps);                  // no cap: always fits unchunked
   *out_plan = pl;
   return VSR_OK;
 }
 
-// the largest divisor of the swept maps whose workspace fits under the cap (no ragged tail chunk: one layer list)
-static int choose_chunk(vsr_srfbn_plan* pl, size_t cap_bytes) {
-  const int M = swept_maps(pl);
-  for (int mc = M; mc >= 1; --mc) {
-    if (M % mc) continue;
-    pl->chunk_maps = mc;
-    layout_workspace(pl);
-    if (cap_bytes == 0 || pl->ws_bytes <= cap_bytes) return VSR_OK;
-  }
-  return VSR_ERR_WORKSPACE;                            // not even one map at a time fits
-}
-
+// The cap stays set even when no chunk fits under it, so the setters after it are held to it too.
 extern "C" int vsr_srfbn_plan_set_workspace_cap(vsr_srfbn_plan* pl, size_t cap_bytes) {
   if (!pl) return VSR_ERR_INVALID_ARG;
   if (pl->bound) return VSR_ERR_STATE;                // the layer list is built for a chunk size: set the cap before bind
   pl->ws_cap = cap_bytes;
-  return choose_chunk(pl, cap_bytes);
+  return set_shape(pl, pl->windows, pl->map0, pl->map1);
 }
 
 extern "C" int vsr_srfbn_plan_set_windows(vsr_srfbn_plan* pl, int windows) {
   if (!pl || windows < 1 || windows > 65535) return VSR_ERR_INVALID_ARG;   // fc_fuse_kernel: one grid row per window
   if (pl->bound) return VSR_ERR_STATE;                // buffers and layer list are sized for the window count
-  if (windows > 1 && pl->map1 - pl->map0 != pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;   // not with a map range
-  const int old = pl->windows;
-  pl->windows = windows;
-  const int rc = choose_chunk(pl, pl->ws_cap);
-  if (rc) {                                            // leave the plan as it was
-    pl->windows = old;
-    choose_chunk(pl, pl->ws_cap);
-  }
-  return rc;
+  return set_shape(pl, windows, pl->map0, pl->map1);
 }
 
 extern "C" int vsr_srfbn_plan_set_map_range(vsr_srfbn_plan* pl, int m0, int m1) {
   if (!pl || m0 < 0 || m1 > pl->cfg.num_maps || m0 >= m1) return VSR_ERR_INVALID_ARG;
   if (pl->bound) return VSR_ERR_STATE;
-  if (pl->windows > 1) return VSR_ERR_UNSUPPORTED;
-  const int old0 = pl->map0, old1 = pl->map1;
-  pl->map0 = m0;
-  pl->map1 = m1;
-  const int rc = choose_chunk(pl, pl->ws_cap);
-  if (rc) {
-    pl->map0 = old0;
-    pl->map1 = old1;
-    choose_chunk(pl, pl->ws_cap);
-  }
-  return rc;
+  if (pl->windows > 1) return VSR_ERR_UNSUPPORTED;     // even the range of all maps
+  return set_shape(pl, pl->windows, m0, m1);
 }
 
 extern "C" int vsr_srfbn_chunk_maps(const vsr_srfbn_plan* pl) { return pl ? pl->chunk_maps : 0; }
@@ -1242,7 +1234,8 @@ extern "C" int vsr_srfbn_forward(vsr_srfbn_plan* pl, const float* x, float* y, v
   return vsr_srfbn_forward_u8(pl, x, y, nullptr, stream);
 }
 
-// One sweep of a layer list over the maps [m0, m0 + Mc) of the stack x; the per-map images land in the premix buffer.
+// One sweep of a layer list over the maps [m0, m0 + Mc) of the stack x; the per-map image of map m lands in premix slot
+// m - map0 (several windows imply map0 == 0, so window b's map m lands in slot b*M + m).
 static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_out_layer, const float* x, int m0, int Mc,
                       cudaStream_t st, size_t* ev) {
   const vsr_srfbn_config& c = pl->cfg;
@@ -1273,6 +1266,29 @@ static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_o
   return VSR_OK;
 }
 
+// The full forward's sweeps: the plan's maps [map0, map0 + swept_maps) in chunks of chunk_maps.
+static int sweep_all(vsr_srfbn_plan* pl, const float* x, cudaStream_t st, size_t* ev) {
+  for (int m0 = pl->map0; m0 < pl->map0 + swept_maps(pl); m0 += pl->chunk_maps) {
+    int rc = sweep_maps(pl, pl->layers, pl->conv_out_layer, x, m0, pl->chunk_maps, st, ev);
+    if (rc) return rc;
+  }
+  return VSR_OK;
+}
+
+// The refresh forward's sweeps: the maps of window b that changed since the last forward and lie in the plan's range,
+// [b*M + max(first_map, map0), b*M + map1), one sweep of the refresh layer list per window -- none when that range is
+// empty.  The stack keeps the caller's window-major layout, so no map is copied or reordered to make the changed maps
+// of all windows contiguous; the price is windows sweeps instead of one, which only matters where launches dominate.
+static int sweep_changed(vsr_srfbn_plan* pl, int first_map, const float* x, cudaStream_t st) {
+  const int M = pl->cfg.num_maps, m0 = std::max(first_map, pl->map0);
+  if (m0 >= pl->map1) return VSR_OK;
+  for (int b = 0; b < pl->windows; ++b) {
+    int rc = sweep_maps(pl, pl->refresh_layers, pl->refresh_conv_out_layer, x, b * M + m0, pl->map1 - m0, st, nullptr);
+    if (rc) return rc;
+  }
+  return VSR_OK;
+}
+
 // the per-pixel fc across num_maps images of n floats each (maps (windows*num_maps, n)), one window per grid row
 static int launch_fc(vsr_srfbn_plan* pl, const float* maps, float* y, uint8_t* y_u8, int64_t n, int windows,
                      cudaStream_t st) {
@@ -1293,17 +1309,13 @@ static int fuse_maps(vsr_srfbn_plan* pl, float* y, uint8_t* y_u8, cudaStream_t s
 extern "C" int vsr_srfbn_forward_u8(vsr_srfbn_plan* pl, const float* x, float* y, uint8_t* y_u8, vsr_stream_t stream) {
   if (!pl || !x || (!y && !y_u8)) return VSR_ERR_INVALID_ARG;
   if (!pl->bound) return VSR_ERR_STATE;
-  if (swept_maps(pl) != pl->windows * pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;   // a map range fuses by bands
+  if (!all_maps(pl)) return VSR_ERR_UNSUPPORTED;      // a map range fuses by bands
   cudaStream_t st = as_stream(stream);
-  const vsr_srfbn_config& c = pl->cfg;
-  const int Mc = pl->chunk_maps;
   size_t ev = 0;
-  for (int m0 = 0; m0 < pl->windows * c.num_maps; m0 += Mc) {   // one sweep over the layer list per chunk of maps
-    int rc = sweep_maps(pl, pl->layers, pl->conv_out_layer, x, m0, Mc, st, &ev);
-    if (rc) return rc;
-  }
+  int rc = sweep_all(pl, x, st, &ev);
+  if (rc) return rc;
   if (pl->profile && ev < pl->events.size()) cudaEventRecord(pl->events[ev++], st);
-  int rc = fuse_maps(pl, y, y_u8, st);
+  rc = fuse_maps(pl, y, y_u8, st);
   if (rc) return rc;
   if (pl->profile && ev < pl->events.size()) cudaEventRecord(pl->events[ev++], st);
   pl->premix_valid = true;
@@ -1315,21 +1327,14 @@ extern "C" int vsr_srfbn_forward_u8(vsr_srfbn_plan* pl, const float* x, float* y
 // independent until the per-pixel fc, so the per-map images of the unchanged maps are still in the workspace and only
 // the changed ones are swept again -- bit-identical to a full forward on the same stack.  Needs
 // vsr_srfbn_prepare_refresh(plan, first_map) and a preceding vsr_srfbn_forward[_u8] on the same stream.
-// With several windows the changed maps of window b are [b*M + first_map, (b+1)*M): one sweep of the refresh layer list
-// per window.  The stack keeps the caller's window-major layout, so no map is copied or reordered to make the changed
-// maps contiguous; the price is windows sweeps instead of one, which only matters where launches dominate.
 extern "C" int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* pl, const float* x, float* y, uint8_t* y_u8, int first_map,
                                             vsr_stream_t stream) {
   if (!pl || !x || (!y && !y_u8)) return VSR_ERR_INVALID_ARG;
   if (!pl->bound || !pl->premix_valid || pl->refresh_first != first_map || first_map < 1) return VSR_ERR_STATE;
-  if (swept_maps(pl) != pl->windows * pl->cfg.num_maps) return VSR_ERR_UNSUPPORTED;
+  if (!all_maps(pl)) return VSR_ERR_UNSUPPORTED;
   cudaStream_t st = as_stream(stream);
-  const int M = pl->cfg.num_maps;
-  for (int b = 0; b < pl->windows; ++b) {
-    int rc = sweep_maps(pl, pl->refresh_layers, pl->refresh_conv_out_layer, x, b * M + first_map, M - first_map, st,
-                        nullptr);
-    if (rc) return rc;
-  }
+  int rc = sweep_changed(pl, first_map, x, st);
+  if (rc) return rc;
   return fuse_maps(pl, y, y_u8, st);
 }
 
@@ -1338,12 +1343,8 @@ extern "C" int vsr_srfbn_forward_refresh_u8(vsr_srfbn_plan* pl, const float* x, 
 extern "C" int vsr_srfbn_forward_maps(vsr_srfbn_plan* pl, const float* x, vsr_stream_t stream) {
   if (!pl || !x) return VSR_ERR_INVALID_ARG;
   if (!pl->bound) return VSR_ERR_STATE;
-  cudaStream_t st = as_stream(stream);
-  const int Mc = pl->chunk_maps;
-  for (int m0 = pl->map0; m0 < pl->map0 + swept_maps(pl); m0 += Mc) {
-    int rc = sweep_maps(pl, pl->layers, pl->conv_out_layer, x, m0, Mc, st, nullptr);
-    if (rc) return rc;
-  }
+  int rc = sweep_all(pl, x, as_stream(stream), nullptr);
+  if (rc) return rc;
   pl->premix_valid = true;
   return VSR_OK;
 }
@@ -1352,10 +1353,7 @@ extern "C" int vsr_srfbn_forward_maps_refresh(vsr_srfbn_plan* pl, const float* x
   if (!pl || !x) return VSR_ERR_INVALID_ARG;
   if (!pl->bound || !pl->premix_valid || pl->refresh_first != first_map || first_map < 1) return VSR_ERR_STATE;
   if (pl->windows > 1) return VSR_ERR_UNSUPPORTED;
-  const int m0 = std::max(first_map, pl->map0);
-  if (m0 >= pl->map1) return VSR_OK;                   // none of this range's maps changed
-  return sweep_maps(pl, pl->refresh_layers, pl->refresh_conv_out_layer, x, m0, pl->map1 - m0, as_stream(stream),
-                    nullptr);
+  return sweep_changed(pl, first_map, x, as_stream(stream));
 }
 
 // bounds[0] == 0 < bounds[1] < ... < bounds[bands] == total, 1 <= bands <= kMaxBands
@@ -1448,25 +1446,38 @@ extern "C" int vsr_srfbn_profile_enable(vsr_srfbn_plan* pl, int enable) {
   return VSR_OK;
 }
 
+struct ProfiledLaunch {
+  int kclass;
+  double flops, bytes;
+};
+
+// The launch between events i and i + 1 of a profiled vsr_srfbn_forward_u8: per chunk sweep an im2col and the layer
+// list, then the fc fuse in the last interval.
+static ProfiledLaunch profiled_launch(const vsr_srfbn_plan* pl, size_t i) {
+  const vsr_srfbn_config& c = pl->cfg;
+  const size_t per = pl->layers.size() + 1;   // launches per chunk sweep
+  if (i == pl->events.size() - 2) {
+    const double s2 = (double)c.upscale * c.upscale, Pall = (double)pl->windows * c.num_maps * c.h * c.w;
+    return {KC_FC, s2 * Pall / c.num_maps * 3 * 2.0 * (32.0 * c.num_maps + 32.0),
+            s2 * Pall * 12.0 + s2 * Pall / c.num_maps * 12.0};
+  }
+  if (i % per == 0) return {KC_IM2COL, 0, (double)pl->chunk_maps * c.h * c.w * (12.0 + 64.0)};
+  const Layer& L = pl->layers[i % per - 1];
+  return {L.kclass, L.flops, L.bytes};
+}
+
 extern "C" int vsr_srfbn_profile_read(vsr_srfbn_plan* pl, double* ms, int32_t* launches, double* flops, double* bytes) {
   if (!pl || !ms || !launches || !flops || !bytes) return VSR_ERR_INVALID_ARG;
   if (!pl->bound || pl->events.empty()) return VSR_ERR_STATE;
   for (int k = 0; k < VSR_SRFBN_KERNEL_CLASSES; ++k) { ms[k] = 0; launches[k] = 0; flops[k] = 0; bytes[k] = 0; }
   cudaError_t r = cudaEventSynchronize(pl->events.back());
   if (r != cudaSuccess) return cuda_status(r);
-  const vsr_srfbn_config& c = pl->cfg;
-  const double Pc = (double)pl->chunk_maps * c.h * c.w, Pall = (double)pl->windows * c.num_maps * c.h * c.w;
-  const size_t per = pl->layers.size() + 1, n = pl->events.size() - 1;     // launches per chunk sweep; intervals
-  for (size_t i = 0; i < n; ++i) {
+  for (size_t i = 0; i + 1 < pl->events.size(); ++i) {
     float t = 0;
     r = cudaEventElapsedTime(&t, pl->events[i], pl->events[i + 1]);
     if (r != cudaSuccess) return cuda_status(r);
-    int k;
-    double f, b;
-    if (i == n - 1) { const double s2 = (double)c.upscale * c.upscale; k = KC_FC; f = s2 * Pall / c.num_maps * 3 * 2.0 * (32.0 * c.num_maps + 32.0); b = s2 * Pall * 12.0 + s2 * Pall / c.num_maps * 12.0; }
-    else if (i % per == 0) { k = KC_IM2COL; f = 0; b = Pc * (12.0 + 64.0); }
-    else { const Layer& L = pl->layers[i % per - 1]; k = L.kclass; f = L.flops; b = L.bytes; }
-    ms[k] += t; launches[k] += 1; flops[k] += f; bytes[k] += b;
+    const ProfiledLaunch l = profiled_launch(pl, i);
+    ms[l.kclass] += t; launches[l.kclass] += 1; flops[l.kclass] += l.flops; bytes[l.kclass] += l.bytes;
   }
   return VSR_OK;
 }
@@ -1475,12 +1486,12 @@ extern "C" int vsr_srfbn_profile_launches(vsr_srfbn_plan* pl, float* ms, int32_t
   if (!pl || !ms || !kclass) return -1;
   if (!pl->bound || pl->events.empty()) return -1;
   if (cudaEventSynchronize(pl->events.back()) != cudaSuccess) return -1;
-  const size_t per = pl->layers.size() + 1, n = pl->events.size() - 1;
+  const size_t n = pl->events.size() - 1;
   for (size_t i = 0; i < n && (int32_t)i < capacity; ++i) {
     float t = 0;
     cudaEventElapsedTime(&t, pl->events[i], pl->events[i + 1]);
     ms[i] = t;
-    kclass[i] = i == n - 1 ? KC_FC : (i % per == 0 ? KC_IM2COL : pl->layers[i % per - 1].kclass);
+    kclass[i] = profiled_launch(pl, i).kclass;
   }
   return (int)n;
 }

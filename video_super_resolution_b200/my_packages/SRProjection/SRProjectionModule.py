@@ -203,11 +203,15 @@ class SRProjectionModule(nn.Module):
         on as its next estimate needs only its own rows).  Without a map group gather must be True."""
         if not x.is_cuda:
             raise RuntimeError("SRProjectionModule: CUDA tensors only (no CPU fallback)")
-        if self.map_group is not None:
-            return self._forward_group(x, out_u8, want_f32, changed_from, gather)
-        if gather is not True:
+        mg = self.map_group
+        if mg is None and gather is not True:
             raise ValueError("SRProjectionModule: gather applies to a map group only")
+        if gather not in (True, False, "u8"):
+            raise ValueError("SRProjectionModule: gather must be True, False or 'u8'")
         nw = self._windows_of(x)
+        if mg is not None and nw != 1:
+            raise ValueError("SRProjectionModule: a map group runs one frame window per forward (windows > 1 is not "
+                             "supported with map_group)")
         x = x.reshape(nw * self.num_maps, *x.shape[-3:])
         if x.dtype != torch.float32 or not x.is_contiguous():
             x = x.to(torch.float32).contiguous()
@@ -219,6 +223,8 @@ class SRProjectionModule(nn.Module):
             raise ValueError(f"SRProjectionModule: out_u8 must be a contiguous CUDA u8 tensor of shape {shapes[-1]}")
         if out_u8 is None and not want_f32:
             raise ValueError("SRProjectionModule: nothing to compute")
+        if mg is not None:
+            return self._forward_group(x, out_u8, want_f32, changed_from, gather)
         ent = self._plan_for(M, h, w, x.device, nw)
         y = torch.empty((nw, 3, s * h, s * w), dtype=torch.float32, device=x.device) if want_f32 else None
         L = _lib.lib()
@@ -251,24 +257,12 @@ class SRProjectionModule(nn.Module):
         _lib.check(refresh(int(changed_from)), "srfbn_forward_refresh")
 
     def _forward_group(self, x, out_u8, want_f32, changed_from, gather):
-        """One window over the map group: sweep this rank's maps, pack their row bands, one all_to_all, fuse this rank's
-        band, and (gather) all-gather the bands.  Every kernel is the one-GPU forward's, on the same values."""
+        """forward of one window x (M,3,h,w), checked by forward, over the map group: sweep this rank's maps, pack their
+        row bands, one all_to_all, fuse this rank's band, and (gather) all-gather the bands.  Every kernel is the one-GPU
+        forward's, on the same values."""
         mg, M, s = self.map_group, self.num_maps, self.upscale_factor
-        if self._windows_of(x) != 1:
-            raise ValueError("SRProjectionModule: a map group runs one frame window per forward (windows > 1 is not "
-                             "supported with map_group)")
-        x = x.reshape(M, *x.shape[-3:])
-        if x.dtype != torch.float32 or not x.is_contiguous():
-            x = x.to(torch.float32).contiguous()
         h, w = x.shape[2], x.shape[3]
         H, W = s * h, s * w
-        if out_u8 is not None and (not out_u8.is_cuda or out_u8.dtype != torch.uint8 or not out_u8.is_contiguous()
-                                   or tuple(out_u8.shape) not in ((1, H, W, 3), (H, W, 3))):
-            raise ValueError(f"SRProjectionModule: out_u8 must be a contiguous CUDA u8 tensor of shape {(H, W, 3)}")
-        if out_u8 is None and not want_f32:
-            raise ValueError("SRProjectionModule: nothing to compute")
-        if gather not in (True, False, "u8"):
-            raise ValueError("SRProjectionModule: gather must be True, False or 'u8'")
         G, r = mg.size, mg.rank
         (m0, m1), lb, hb = self.band_geometry(h)
         ent = self._plan_for(M, h, w, x.device, 1, (m0, m1))

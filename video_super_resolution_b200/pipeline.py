@@ -113,6 +113,7 @@ class WarpFusePipeline:
         self.T, self.h, self.w, self.scale = T, h, w, scale
         self.windows = W = int(windows)
         self.M = 3 * T - 1
+        self._changed_from = {None: None, "frames": T, "unchanged": self.M - 1}[reuse]   # pass 2 convolves maps >= it
         self.centre = T // 2
         self.device = torch.device(device)
         self.run_fusion = run_fusion
@@ -126,9 +127,9 @@ class WarpFusePipeline:
         if self.sr.num_maps != self.M:
             raise ValueError(f"SRProjectionModule.num_maps={self.sr.num_maps}, window needs {self.M}")
         lead = (W,) if W > 1 else ()
-        self._mask_w = None
         if mg is None:
             self.stack = torch.empty(lead + (self.M, 3, h, w), dtype=torch.float32, device=self.device)
+            self._mask_w = torch.empty((W, h, w), dtype=torch.uint8, device=self.device)
         else:
             self.map_group = mg = self.sr.map_group
             (_, _), lb, _ = self.sr.band_geometry(h)        # ValueError for fewer LR rows than ranks
@@ -215,35 +216,24 @@ class WarpFusePipeline:
         SRProjectionModule.forward (True: full frames on every rank; "u8": out_u8 gathered, this rank's fp32 band
         returned; False: this rank's band only).
         Every kernel between the first and the last launch of a step is this library's (and, with a map group, NCCL's)."""
-        if self.map_group is not None:
-            return self._step_group(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr,
-                                    estimate_hr_band, out_u8, want_f32, gather)
-        if estimate_hr_band is not None or gather is not True:
-            raise ValueError("WarpFusePipeline: estimate_hr_band and gather need a map group")
-        r = self.project_and_warp(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr,
-                                  estimate_hr_windows)
-        if not self.run_fusion:
-            return self.stack
-        out1 = self.sr(self.stack)                                             # pass 1
-        mask_w = r["mask_warped"]
-        ops.estimate_slots(out1, mask_w.view(self.windows, self.h, self.w), self._stack, self.scale)
-        changed_from = {None: None, "frames": self.T, "unchanged": self.M - 1}[self.reuse]
-        return self.sr(self.stack, out_u8=out_u8, want_f32=want_f32, changed_from=changed_from)   # pass 2 (fuse)
-
-    def _step_group(self, frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr, estimate_hr_band, out_u8,
-                    want_f32, gather):
         mg = self.map_group
-        if mg.rank == 0:
-            self.project_and_warp(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr)
-        mg.broadcast(self._bcast, 0)                       # the stack and mask every rank convolves
+        if mg is None and (estimate_hr_band is not None or gather is not True):
+            raise ValueError("WarpFusePipeline: estimate_hr_band and gather need a map group")
+        if mg is None or mg.rank == 0:
+            self.project_and_warp(frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr,
+                                  estimate_hr_windows)
+        if mg is not None:
+            mg.broadcast(self._bcast, 0)                   # the stack and mask every rank convolves
         if not self.run_fusion:
             return self.stack
-        if estimate_hr_band is not None:
-            self._slot_from_band(estimate_hr_band, None)
-        band = self.sr(self.stack, gather=False)           # pass 1: this rank's band of the frame
-        self._slot_from_band(band, self._mask_w[0])
-        changed_from = {None: None, "frames": self.T, "unchanged": self.M - 1}[self.reuse]
-        return self.sr(self.stack, out_u8=out_u8, want_f32=want_f32, changed_from=changed_from, gather=gather)
+        if mg is None:
+            ops.estimate_slots(self.sr(self.stack), self._mask_w, self._stack, self.scale)     # pass 1
+        else:
+            if estimate_hr_band is not None:
+                self._slot_from_band(estimate_hr_band, None)
+            self._slot_from_band(self.sr(self.stack, gather=False), self._mask_w[0])    # pass 1: this rank's band
+        return self.sr(self.stack, out_u8=out_u8, want_f32=want_f32, changed_from=self._changed_from,   # pass 2 (fuse)
+                       gather=gather)
 
     def _slot_from_band(self, band, mask):
         """The estimate slot from the frame's row bands: each rank downsizes its band into its LR rows of the slot
@@ -391,30 +381,20 @@ def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tenso
     if out is None:
         out = torch.empty((len(idx), s * h, s * w, 3), dtype=torch.uint8, device=frames.device)
     pipe = vsr._pipe(h, w, frames.device)
-    if pipe.map_group is not None:
-        return _run_group(pipe, frames, flows, inv_depth, logits, chunks, out, idx, T)
+    group = pipe.map_group is not None
     i = 0
     for c in chunks:
         est = None                                                   # recurrence reset at every chunk start (main.py:196)
         for k in c:
             la, lb = logits(k)
             # the previous output frame stays planar fp32 on the device and is downsized into the estimate slot by
-            # vsr_estimate_slot; the u8 frame (utils/video_utils.py:23) is written by the fc-fuse kernel itself
-            est = pipe.step(frames[k:k + T], flows[k:k + T - 1], inv_depth[k:k + T - 1], la, lb,
-                            estimate_hr=None if est is None else est[0], out_u8=out[i])
-            i += 1
-    return out, idx
-
-
-def _run_group(pipe, frames, flows, inv_depth, logits, chunks, out, idx, T):
-    """run_sequence on a map group: the u8 frame of each step is all-gathered, the fp32 estimate stays banded."""
-    i = 0
-    for c in chunks:
-        band = None                                                  # recurrence reset at every chunk start
-        for k in c:
-            la, lb = logits(k)
-            band = pipe.step(frames[k:k + T], flows[k:k + T - 1], inv_depth[k:k + T - 1], la, lb,
-                             estimate_hr_band=band, out_u8=out[i], gather="u8")
+            # vsr_estimate_slot (a map group keeps only this rank's row band of it and all-gathers the u8 frame); the
+            # u8 frame (utils/video_utils.py:23) is written by the fc-fuse kernel itself
+            if group:
+                nxt = {"estimate_hr_band": est, "gather": "u8"}
+            else:
+                nxt = {"estimate_hr": None if est is None else est[0]}
+            est = pipe.step(frames[k:k + T], flows[k:k + T - 1], inv_depth[k:k + T - 1], la, lb, out_u8=out[i], **nxt)
             i += 1
     return out, idx
 
