@@ -68,27 +68,21 @@ int vsr_warp_nhwc_f32(const float* src, const float* flow, float* dst,
                       const float* ref, float* norm_out,
                       int B, int H, int W, int C, int bilinear, vsr_stream_t stream);
 
-/* The neighbour warp of one frame window in a single launch, without a gathered copy of the frames:
- * frames (T,H,W,3) f32 NHWC; flows (T-1,H,W,2) f32, one field per NEIGHBOUR in frame order with the centre
- * frame left out, each mapping centre coordinates to that neighbour; warped (T-1,H,W,3); resid (T-1,H,W) or
- * NULL = per-pixel L2 norm of (frames[centre] - warped[n]) (models.py:86-88 fused).  Arithmetic and
- * `bilinear` modes as vsr_warp_nhwc_f32. */
-int vsr_warp_window_nhwc3(const float* frames, const float* flows, float* warped, float* resid,
-                          int T, int centre, int H, int W, int bilinear, vsr_stream_t stream);
-/* The same for `windows` independent frame windows in one launch (1..65535): frames (windows,T,H,W,3), flows
- * (windows,T-1,H,W,2), warped (windows,T-1,H,W,3), resid (windows,T-1,H,W) or NULL; window b is warped to its own
- * centre frame, bit-identical to a one-window call on it.  vsr_warp_window_nhwc3 is this with windows = 1. */
+/* The neighbour warp of `windows` independent frame windows in a single launch (1..65535; one window is windows = 1),
+ * without a gathered copy of the frames: frames (windows,T,H,W,3) f32 NHWC; flows (windows,T-1,H,W,2) f32, one field
+ * per NEIGHBOUR in frame order with the centre frame left out, each mapping centre coordinates to that neighbour;
+ * warped (windows,T-1,H,W,3); resid (windows,T-1,H,W) or NULL = per-pixel L2 norm of (frames[centre] - warped[n])
+ * (models.py:86-88 fused).  Window b is warped to its own centre frame, bit-identical to a call on it alone.
+ * Arithmetic and `bilinear` modes as vsr_warp_nhwc_f32. */
 int vsr_warp_windows_nhwc3(const float* frames, const float* flows, float* warped, float* resid, int windows,
                            int T, int centre, int H, int W, int bilinear, vsr_stream_t stream);
 
 /* Flow composition out(p) = g(p) + f(p + g(p)) with f sampled bilinearly (the warp's taps and border rule,
- * fp32 blend): if g maps image A to B and f maps B to C, out maps A to C.  g, f, out (B,H,W,2) f32.  Used to chain
- * adjacent-pair flows into centre -> neighbour flows for windows longer than 3 frames.  g == NULL is the identity
- * field: out = f (the first link of a chain, placed into the caller's contiguous (T-1,H,W,2) array). */
-int vsr_compose_flow(const float* g, const float* f, float* out, int B, int H, int W, vsr_stream_t stream);
-/* One link of the chains of `windows` frame windows in one launch (1..65535): window b composes the (H,W,2) fields at
- * g + b*stride and f + b*stride into out + b*stride (stride in floats, even).  The centre -> neighbour fields of a
- * (windows,T-1,H,W,2) array are (T-1)*H*W*2 floats apart. */
+ * fp32 blend): if g maps image A to B and f maps B to C, out maps A to C.  Used to chain adjacent-pair flows into
+ * centre -> neighbour flows for windows longer than 3 frames.  One link of the chains of `windows` frame windows in one
+ * launch (1..65535): window b composes the (H,W,2) f32 fields at g + b*stride and f + b*stride into out + b*stride
+ * (stride in floats, even; it may be 0 when windows = 1).  The centre -> neighbour fields of a (windows,T-1,H,W,2)
+ * array are (T-1)*H*W*2 floats apart.  g == NULL is the identity field: out = f (the first link of a chain). */
 int vsr_compose_flow_windows(const float* g, const float* f, float* out, int windows, int64_t stride, int H, int W,
                              vsr_stream_t stream);
 
@@ -98,7 +92,7 @@ int vsr_compose_flow_windows(const float* g, const float* f, float* out, int win
 int vsr_warp_labels_u8(const uint8_t* labels, const float* flow, uint8_t* dst,
                        int B, int H, int W, vsr_stream_t stream);
 /* `windows` label images (windows,H,W) -> dst (windows,H,W) in one launch (1..65535); window b is warped along the
- * (H,W,2) field at flow + b*flow_stride (floats, even). */
+ * (H,W,2) field at flow + b*flow_stride (floats, even; it may be 0 when windows = 1). */
 int vsr_warp_labels_u8_windows(const uint8_t* labels, const float* flow, uint8_t* dst, int windows,
                                int64_t flow_stride, int H, int W, vsr_stream_t stream);
 
@@ -217,13 +211,10 @@ int vsr_flow_projection_forward_deterministic(const float* flow, const float* in
  * a5: VOS mask arithmetic.  ref: VOSProjectionModule.py:22-25 (sigmoid(a)+sigmoid(b) > 0.7),
  * utils/tools.py:76-77 (maskprocess) and network/video_super_resolution.py:58-60
  * (MaskedArray(img, mask, fill_value=0).filled()).
- * logits_a/logits_b (h,w) f32 -> mask (h,w) u8 in {0,1}.
- * image (C,h,w) f32 -> masked (C,h,w) f32 = image where mask==0 else 0.
+ * vsr_vos_threshold_windows: `windows` logit pairs in one launch (one window is windows = 1):
+ * logits_a/logits_b (windows,h,w) f32 -> mask (windows,h,w) u8 in {0,1}.
+ * vsr_mask_fill: image (C,h,w) f32 -> masked (C,h,w) f32 = image where mask==0 else 0.
  * ---------------------------------------------------------------------------------------- */
-int vsr_vos_threshold(const float* logits_a, const float* logits_b, uint8_t* mask,
-                      int h, int w, vsr_stream_t stream);
-/* `windows` logit pairs in one launch: logits_a/logits_b (windows,h,w) -> mask (windows,h,w).
- * vsr_vos_threshold is this with windows = 1. */
 int vsr_vos_threshold_windows(const float* logits_a, const float* logits_b, uint8_t* mask,
                               int windows, int h, int w, vsr_stream_t stream);
 int vsr_mask_fill(const float* image, const uint8_t* mask, float* masked,
@@ -236,25 +227,19 @@ int vsr_mask_fill(const float* image, const uint8_t* mask, float* masked,
  * (video_super_resolution.py:40 generalised to T frames): T frames (warped neighbours, the centre
  * frame at centre_idx), T-1 flow maps (projected fx, projected fy, warp-residual norm), T-1 depth
  * maps tiled x3 (utils/tools.py:76-77), 1 estimate.
- * warped (T-1,h,w,3) NHWC, centre (h,w,3), proj (T-1,h,w,2), resid (T-1,h,w), depth (T-1,h,w),
- * estimate (3,h,w) NCHW, or NULL: the slot then receives `fallback` (h,w,3) NHWC, which the caller sets to LR
- * frame 0 of the window (video_super_resolution.py:37-38 `else data_clone[0:1]`); stack (M,3,h,w).
- * vsr_estimate_slot: slot (3,h,w) = mask ? 0 : hr[:, y*scale, x*scale] for hr (3,h*scale,w*scale);
- * mask (h,w) u8 or NULL.
+ * Both entry points take `windows` frame windows in one launch (1..65535; one window is windows = 1), window b
+ * bit-identical to a call on it alone.
+ * vsr_assemble_stack_windows: warped (windows,T-1,h,w,3) NHWC, proj (windows,T-1,h,w,2), resid / depth
+ * (windows,T-1,h,w), estimate (windows,3,h,w) NCHW or NULL, stack (windows,M,3,h,w).  The centre frame and the
+ * fallback frame of window b are the (h,w,3) NHWC images at centre + b*frame_stride and fallback + b*frame_stride
+ * (floats; it may be 0 when windows = 1).  For frames (windows,T,h,w,3), frame_stride = T*h*w*3, and centre / fallback
+ * point at frame centre_idx / 0 of window 0.  Without an estimate the slot receives the fallback frame: LR frame 0 of
+ * the window (video_super_resolution.py:37-38 `else data_clone[0:1]`).
+ * vsr_estimate_slot_windows: slot (3,h,w) = mask ? 0 : hr[:, y*scale, x*scale] for hr (windows,3,h*scale,w*scale) and
+ * mask (windows,h,w) u8 or NULL.  The slot of window b is the (3,h,w) image at slot + b*slot_stride (floats; it may be
+ * 0 when windows = 1).  For the estimate slots of a (windows,M,3,h,w) stack, slot = map M-1 of window 0 and
+ * slot_stride = M*3*h*w.
  * ---------------------------------------------------------------------------------------- */
-int vsr_assemble_stack(const float* warped, const float* centre, const float* proj, const float* resid,
-                       const float* depth, const float* estimate, const float* fallback, float* stack,
-                       int T, int centre_idx, int h, int w, vsr_stream_t stream);
-int vsr_estimate_slot(const float* hr, const uint8_t* mask, float* slot, int h, int w, int scale,
-                      vsr_stream_t stream);
-/* `windows` frame windows in one launch each (1..65535), window b bit-identical to a one-window call on it:
- * vsr_assemble_stack_windows: warped (windows,T-1,h,w,3), proj (windows,T-1,h,w,2), resid / depth (windows,T-1,h,w),
- * estimate (windows,3,h,w) or NULL, stack (windows,M,3,h,w); the centre frame and the fallback frame of window b are
- * the (h,w,3) images at centre + b*frame_stride and fallback + b*frame_stride (floats; for frames (windows,T,h,w,3)
- * frame_stride = T*h*w*3 and centre / fallback point at frame centre_idx / 0 of window 0).
- * vsr_estimate_slot_windows: hr (windows,3,h*scale,w*scale), mask (windows,h,w) or NULL; the slot of window b is the
- * (3,h,w) image at slot + b*slot_stride (floats; the estimate slots of a (windows,M,3,h,w) stack: slot = map M-1 of
- * window 0, slot_stride = M*3*h*w).  The one-window entry points above are these with windows = 1. */
 int vsr_assemble_stack_windows(const float* warped, const float* centre, const float* proj, const float* resid,
                                const float* depth, const float* estimate, const float* fallback, float* stack,
                                int windows, int64_t frame_stride, int T, int centre_idx, int h, int w,

@@ -35,7 +35,7 @@ def test_front_entry_points_refuse_bad_window_counts():
     assert L.vsr_estimate_slot_windows(p, None, p, 2, -3, 8, 8, 4, None) == INVALID
     assert L.vsr_compose_flow_windows(p, p, p, 2, 3, 8, 8, None) == INVALID
     assert L.vsr_warp_labels_u8_windows(p, p, p, 2, 7, 8, 8, None) == INVALID
-    # the per-window limits of the one-window entry points still hold
+    # the per-window limits hold as well
     assert L.vsr_warp_windows_nhwc3(p, p, p, p, 2, 3, 3, 8, 8, 2, None) == INVALID      # centre outside 0..T-1
 
 

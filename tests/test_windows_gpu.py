@@ -178,9 +178,9 @@ def test_argument_errors_launch_nothing():
     with pytest.raises(ValueError):
         pipe.sr(pipe.stack, out_u8=torch.zeros((4 * h, 4 * w, 3), dtype=torch.uint8, device=DEV))
     with pytest.raises(ValueError):
-        ops.warp_windows(good[0], good[1][:1], 1)
+        ops.warp_window(good[0], good[1][:1], 1)
     with pytest.raises(ValueError):
-        ops.assemble_stacks(*[torch.zeros(1, device=DEV)] * 5, None, 1)
+        ops.assemble_stack(*[torch.zeros(1, device=DEV)] * 5, None, 1)
     assert _lib.launch_count() == 0
     # the setter after bind
     ent = pipe.sr._plans[(3 * T - 1, h, w, 0, W)]

@@ -53,9 +53,7 @@ SIGNATURES = {
     "vsr_error_string": (ctypes.c_char_p, [c_int]),
     "vsr_resample2d_forward": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "vsr_warp_nhwc_f32": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
-    "vsr_warp_window_nhwc3": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "vsr_warp_windows_nhwc3": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p] + [c_int] * 6 + [c_void_p]),
-    "vsr_compose_flow": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "vsr_compose_flow_windows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_i64, c_int, c_int, c_void_p]),
     "vsr_warp_labels_u8": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "vsr_warp_labels_u8_windows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_i64, c_int, c_int, c_void_p]),
@@ -74,12 +72,9 @@ SIGNATURES = {
     "vsr_flow_projection_forward_bounded": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_float, c_void_p]),
     "vsr_flow_projection_deterministic_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "vsr_flow_projection_forward_deterministic": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_int, c_int, c_int, c_void_p]),
-    "vsr_vos_threshold": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "vsr_vos_threshold_windows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "vsr_flow_to_image": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "vsr_mask_fill": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
-    "vsr_assemble_stack": (c_int, [c_void_p] * 8 + [c_int, c_int, c_int, c_int, c_void_p]),
-    "vsr_estimate_slot": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "vsr_assemble_stack_windows": (c_int, [c_void_p] * 8 + [c_int, c_i64, c_int, c_int, c_int, c_int, c_void_p]),
     "vsr_estimate_slot_windows": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_i64, c_int, c_int, c_int, c_void_p]),
     "vsr_srfbn_plan_create": (c_int, [ctypes.POINTER(SrfbnConfig), ctypes.POINTER(c_void_p)]),

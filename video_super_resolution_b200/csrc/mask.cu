@@ -53,11 +53,6 @@ extern "C" int vsr_vos_threshold_windows(const float* logits_a, const float* log
   return after_launch();
 }
 
-extern "C" int vsr_vos_threshold(const float* logits_a, const float* logits_b, uint8_t* mask, int h, int w,
-                                 vsr_stream_t stream) {
-  return vsr_vos_threshold_windows(logits_a, logits_b, mask, 1, h, w, stream);
-}
-
 extern "C" int vsr_mask_fill(const float* image, const uint8_t* mask, float* masked, int C, int h, int w,
                              vsr_stream_t stream) {
   if (!image || !mask || !masked || C <= 0 || h <= 0 || w <= 0) return VSR_ERR_INVALID_ARG;

@@ -112,13 +112,6 @@ extern "C" int vsr_assemble_stack_windows(const float* warped, const float* cent
   return after_launch();
 }
 
-extern "C" int vsr_assemble_stack(const float* warped, const float* centre, const float* proj, const float* resid,
-                                  const float* depth, const float* estimate, const float* fallback, float* stack, int T,
-                                  int centre_idx, int h, int w, vsr_stream_t stream) {
-  return vsr_assemble_stack_windows(warped, centre, proj, resid, depth, estimate, fallback, stack, 1, 0, T, centre_idx, h,
-                                    w, stream);
-}
-
 extern "C" int vsr_estimate_slot_windows(const float* hr, const uint8_t* mask, float* slot, int windows,
                                          int64_t slot_stride, int h, int w, int scale, vsr_stream_t stream) {
   if (!hr || !slot || windows < 1 || windows > 65535 || slot_stride < 0 || h <= 0 || w <= 0 || scale < 1)
@@ -126,9 +119,4 @@ extern "C" int vsr_estimate_slot_windows(const float* hr, const uint8_t* mask, f
   estimate_slot_kernel<<<dim3(grid_for((int64_t)h * w), windows), kThreads, 0, as_stream(stream)>>>(hr, mask, slot, h, w,
                                                                                                    scale, slot_stride);
   return after_launch();
-}
-
-extern "C" int vsr_estimate_slot(const float* hr, const uint8_t* mask, float* slot, int h, int w, int scale,
-                                 vsr_stream_t stream) {
-  return vsr_estimate_slot_windows(hr, mask, slot, 1, 0, h, w, scale, stream);
 }

@@ -591,22 +591,6 @@ extern "C" int vsr_warp_windows_nhwc3(const float* frames, const float* flows, f
   return after_launch();
 }
 
-extern "C" int vsr_warp_window_nhwc3(const float* frames, const float* flows, float* warped, float* resid, int T,
-                                     int centre, int H, int W, int bilinear, vsr_stream_t stream) {
-  return vsr_warp_windows_nhwc3(frames, flows, warped, resid, 1, T, centre, H, W, bilinear, stream);
-}
-
-extern "C" int vsr_compose_flow(const float* g, const float* f, float* out, int B, int H, int W, vsr_stream_t stream) {
-  if (!f || !out || B <= 0 || H <= 0 || W <= 0) return VSR_ERR_INVALID_ARG;
-  if (!aligned(g, 8) || !aligned(f, 8) || !aligned(out, 8)) return VSR_ERR_INVALID_ARG;
-  const int64_t n_pix = (int64_t)B * H * W;
-  if (n_pix >= ((int64_t)1 << 32)) return VSR_ERR_UNSUPPORTED;
-  compose_flow_kernel<<<grid_for(n_pix, kThreads), kThreads, 0, as_stream(stream)>>>(
-      reinterpret_cast<const float2*>(g), reinterpret_cast<const float2*>(f), reinterpret_cast<float2*>(out), n_pix, H, W,
-      make_pixdecode(H, W), 0);
-  return after_launch();
-}
-
 extern "C" int vsr_compose_flow_windows(const float* g, const float* f, float* out, int windows, int64_t stride, int H,
                                         int W, vsr_stream_t stream) {
   if (!f || !out || windows < 1 || windows > 65535 || stride < 0 || (stride & 1) || H <= 0 || W <= 0)

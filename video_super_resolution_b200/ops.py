@@ -32,6 +32,16 @@ def _req(t: torch.Tensor, dtype, name: str) -> torch.Tensor:
     return t
 
 
+def _lead(t: torch.Tensor, nd: int, what: str):
+    """(lead, windows) of an argument with nd dimensions per window: ((), 1) for one window without a leading
+    dimension, ((W,), W) for W >= 1 windows along dim 0."""
+    if t.dim() == nd:
+        return (), 1
+    if t.dim() != nd + 1 or t.shape[0] < 1:
+        raise ValueError(what)
+    return (t.shape[0],), t.shape[0]
+
+
 def _workspace(nbytes: int, device) -> torch.Tensor:
     """Caller-side workspace cache (the library itself owns no memory)."""
     key = (device.index, torch.cuda.current_stream().cuda_stream)
@@ -181,58 +191,71 @@ def warp(src: torch.Tensor, flow: torch.Tensor, bilinear: bool | int = True, ref
 
 
 def warp_window(frames: torch.Tensor, flows: torch.Tensor, centre: int, bilinear: bool | int = 2, want_resid: bool = True):
-    """The neighbour warp of one window in one launch: frames (T,H,W,3), flows (T-1,H,W,2) = one centre -> neighbour
-    field per neighbour (frame order, centre left out) -> warped (T-1,H,W,3) and, with want_resid, the per-pixel L2
-    norm of (frames[centre] - warped[n]) (T-1,H,W).  No gathered copy of the neighbours, no expanded reference."""
+    """The neighbour warp of a frame window in one launch: frames ([W,]T,H,W,3), flows ([W,]T-1,H,W,2) = one centre ->
+    neighbour field per neighbour (frame order, centre left out) -> warped ([W,]T-1,H,W,3) and, with want_resid, the
+    per-pixel L2 norm of (frames[centre] - warped[n]) ([W,]T-1,H,W).  With a leading W the one launch warps W windows,
+    each to its own centre frame.  No gathered copy of the neighbours, no expanded reference."""
     _req(frames, torch.float32, "frames")
     _req(flows, torch.float32, "flows")
-    T, H, W, C = frames.shape
-    if C != 3 or tuple(flows.shape) != (T - 1, H, W, 2) or not 0 <= centre < T:
-        raise ValueError("warp_window: frames (T,H,W,3), flows (T-1,H,W,2), 0 <= centre < T expected")
-    warped = torch.empty((T - 1, H, W, 3), dtype=torch.float32, device=frames.device)
-    resid = torch.empty((T - 1, H, W), dtype=torch.float32, device=frames.device) if want_resid else None
+    lead, nw = _lead(frames, 4, "warp_window: frames ([W,]T,H,W,3) expected")
+    T, H, W, C = frames.shape[-4:]
+    if C != 3 or tuple(flows.shape) != lead + (T - 1, H, W, 2) or not 0 <= centre < T:
+        raise ValueError("warp_window: frames ([W,]T,H,W,3), flows ([W,]T-1,H,W,2), 0 <= centre < T expected")
+    warped = torch.empty(lead + (T - 1, H, W, 3), dtype=torch.float32, device=frames.device)
+    resid = torch.empty(lead + (T - 1, H, W), dtype=torch.float32, device=frames.device) if want_resid else None
     with torch.cuda.device(frames.device):
-        _lib.check(_lib.lib().vsr_warp_window_nhwc3(frames.data_ptr(), flows.data_ptr(), warped.data_ptr(),
-                                                    resid.data_ptr() if resid is not None else None, T, int(centre), H, W,
-                                                    int(bilinear), _stream()), "warp_window")
+        _lib.check(_lib.lib().vsr_warp_windows_nhwc3(frames.data_ptr(), flows.data_ptr(), warped.data_ptr(),
+                                                     resid.data_ptr() if resid is not None else None, nw, T,
+                                                     int(centre), H, W, int(bilinear), _stream()), "warp_window")
     return warped, resid
 
 
-def compose_flow(g: torch.Tensor, f: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+def compose_flow(g: torch.Tensor | None, f: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
     """out(p) = g(p) + f(p + g(p)), f sampled bilinearly (border-clamped taps): g maps image A to B, f maps B to C,
-    out maps A to C.  g, f (B,H,W,2) or (H,W,2); g=None is the identity field (out = f, a copy by our own kernel)."""
-    _req(f, torch.float32, "f")
-    if g is not None:
-        _req(g, torch.float32, "g")
-    if (g is not None and g.shape != f.shape) or f.shape[-1] != 2 or f.dim() not in (3, 4):
-        raise ValueError("compose_flow: two (B,H,W,2) or (H,W,2) fields of the same shape expected")
-    B = f.shape[0] if f.dim() == 4 else 1
-    H, W = f.shape[-3], f.shape[-2]
+    out maps A to C.  g, f, out ([W,]H,W,2); g=None is the identity field (out = f, a copy by our own kernel).  A
+    W-window argument may be a view such as x[:, n] of a (W,T-1,H,W,2) array: each window's field is contiguous, and g,
+    f and out have one window stride (out=None allocates it with f's strides).  One launch for all windows."""
+    lead, nw = _lead(f, 3, "compose_flow: (H,W,2) or (W,H,W,2) fields expected")
+    if f.shape[-1] != 2:
+        raise ValueError("compose_flow: (H,W,2) or (W,H,W,2) fields expected")
     if out is None:
-        out = torch.empty_like(f)
-    else:
-        _req(out, torch.float32, "out")
-        if out.shape != f.shape:
-            raise ValueError("compose_flow: out must have the shape of f")
+        out = torch.empty_strided(f.shape, f.stride(), dtype=torch.float32, device=f.device)
+    for t, n in ((f, "f"), (g, "g"), (out, "out")):
+        if t is not None:
+            _req(t[0] if lead else t, torch.float32, n)
+            if t.shape != f.shape or (nw > 1 and t.stride(0) != f.stride(0)):
+                raise ValueError(f"compose_flow: {n} must have the shape and window stride of f")
+    H, W = f.shape[-3:-1]
     with torch.cuda.device(f.device):
-        _lib.check(_lib.lib().vsr_compose_flow(g.data_ptr() if g is not None else None, f.data_ptr(), out.data_ptr(),
-                                               B, H, W, _stream()), "compose_flow")
+        _lib.check(_lib.lib().vsr_compose_flow_windows(g.data_ptr() if g is not None else None, f.data_ptr(),
+                                                       out.data_ptr(), nw, f.stride(0) if nw > 1 else 0, H, W,
+                                                       _stream()), "compose_flow")
     return out
 
 
-def warp_labels(labels: torch.Tensor, flow: torch.Tensor) -> torch.Tensor:
-    """Nearest label warp: labels (B,H,W) u8, flow (B,H,W,2) -> (B,H,W) u8, bit-exact."""
+def warp_labels(labels: torch.Tensor, flow: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
+    """Nearest label warp, bit-exact: labels (B,H,W) u8, flow (B,H,W,2) -> (B,H,W) u8 (written into `out` when
+    given).  A contiguous flow is one flat launch over the B images; a view such as x[:, n] of a (B,T-1,H,W,2) array,
+    each image's field contiguous, is warped with the image index on the grid."""
     _req(labels, torch.uint8, "labels")
-    _req(flow, torch.float32, "flow")
+    if labels.dim() != 3 or labels.shape[0] < 1 or tuple(flow.shape) != tuple(labels.shape) + (2,):
+        raise ValueError("warp_labels: labels (B,H,W) and flow (B,H,W,2) expected")
+    _req(flow[0], torch.float32, "flow")
     B, H, W = labels.shape
-    if tuple(flow.shape) != (B, H, W, 2):
-        raise ValueError("warp_labels: flow must be (B,H,W,2)")
-    dst = torch.empty_like(labels)
+    if out is not None:
+        _req(out, torch.uint8, "out")
+        if out.shape != labels.shape:
+            raise ValueError("warp_labels: out must be (B,H,W)")
+    dst = torch.empty_like(labels) if out is None else out
+    L = _lib.lib()
     with torch.cuda.device(labels.device):
-        _lib.check(_lib.lib().vsr_warp_labels_u8(labels.data_ptr(), flow.data_ptr(), dst.data_ptr(), B, H, W,
-                                                 _stream()), "warp_labels")
+        if flow.is_contiguous():
+            _lib.check(L.vsr_warp_labels_u8(labels.data_ptr(), flow.data_ptr(), dst.data_ptr(), B, H, W, _stream()),
+                       "warp_labels")
+        else:
+            _lib.check(L.vsr_warp_labels_u8_windows(labels.data_ptr(), flow.data_ptr(), dst.data_ptr(), B,
+                                                    flow.stride(0), H, W, _stream()), "warp_labels")
     return dst
-
 
 _DTYPES = {torch.float32: 0, torch.float16: 1, torch.float64: 2}     # VSR_DTYPE_*
 
@@ -323,16 +346,18 @@ def flow_to_image(flow: torch.Tensor, out_size=None, want_u8: bool = True):
 
 
 def vos_threshold(logits_a: torch.Tensor, logits_b: torch.Tensor) -> torch.Tensor:
-    """sigmoid(a)+sigmoid(b) > 0.7 -> u8 {0,1}.  ref: VOSProjectionModule.py:22-25."""
+    """sigmoid(a)+sigmoid(b) > 0.7 -> u8 {0,1}: logits ([W,]h,w) x2 -> mask ([W,]h,w), one launch for all windows.
+    ref: VOSProjectionModule.py:22-25."""
     _req(logits_a, torch.float32, "logits_a")
     _req(logits_b, torch.float32, "logits_b")
-    if logits_a.shape != logits_b.shape or logits_a.dim() != 2:
-        raise ValueError("vos_threshold: two (h,w) tensors expected")
-    h, w = logits_a.shape
-    mask = torch.empty((h, w), dtype=torch.uint8, device=logits_a.device)
+    _, nw = _lead(logits_a, 2, "vos_threshold: two ([W,]h,w) tensors expected")
+    if logits_b.shape != logits_a.shape:
+        raise ValueError("vos_threshold: two ([W,]h,w) tensors expected")
+    h, w = logits_a.shape[-2:]
+    mask = torch.empty(logits_a.shape, dtype=torch.uint8, device=logits_a.device)
     with torch.cuda.device(logits_a.device):
-        _lib.check(_lib.lib().vsr_vos_threshold(logits_a.data_ptr(), logits_b.data_ptr(), mask.data_ptr(), h, w,
-                                                _stream()), "vos_threshold")
+        _lib.check(_lib.lib().vsr_vos_threshold_windows(logits_a.data_ptr(), logits_b.data_ptr(), mask.data_ptr(), nw,
+                                                        h, w, _stream()), "vos_threshold")
     return mask
 
 
@@ -351,185 +376,58 @@ def mask_fill(image: torch.Tensor, mask: torch.Tensor) -> torch.Tensor:
     return out
 
 
-def assemble_stack(warped: torch.Tensor, centre: torch.Tensor, proj: torch.Tensor, resid: torch.Tensor,
+def assemble_stack(warped: torch.Tensor, frames: torch.Tensor, proj: torch.Tensor, resid: torch.Tensor,
                    depth: torch.Tensor, estimate: torch.Tensor | None, centre_idx: int,
-                   out: torch.Tensor | None = None, fallback: torch.Tensor | None = None) -> torch.Tensor:
-    """One-pass assembly of the (3T-1,3,h,w) map stack (video_super_resolution.py:33-40).
-    warped (T-1,h,w,3), centre (h,w,3), proj (T-1,h,w,2), resid/depth (T-1,h,w), estimate (3,h,w)|None.
-    Without an estimate the last slot receives `fallback` (h,w,3): LR frame 0 of the window, as the reference's
-    `else data_clone[0:1]` (:37-38); `fallback=None` keeps the centre frame there."""
-    for t, n in ((warped, "warped"), (centre, "centre"), (proj, "proj"), (resid, "resid"), (depth, "depth")):
+                   out: torch.Tensor | None = None) -> torch.Tensor:
+    """One-pass assembly of the ([W,]3T-1,3,h,w) map stack (video_super_resolution.py:33-40), one launch for all
+    windows.  warped ([W,]T-1,h,w,3), frames ([W,]T,h,w,3), proj ([W,]T-1,h,w,2), resid / depth ([W,]T-1,h,w),
+    estimate ([W,]3,h,w) | None.  The centre frame and, without an estimate, LR frame 0 of each window (the
+    reference's `else data_clone[0:1]`, :37-38) are read from frames in place."""
+    for t, n in ((warped, "warped"), (frames, "frames"), (proj, "proj"), (resid, "resid"), (depth, "depth")):
         _req(t, torch.float32, n)
-    Tm1, h, w, _ = warped.shape
-    T = Tm1 + 1
-    if tuple(centre.shape) != (h, w, 3) or tuple(proj.shape) != (Tm1, h, w, 2) or \
-            tuple(resid.shape) != (Tm1, h, w) or tuple(depth.shape) != (Tm1, h, w):
+    lead, nw = _lead(frames, 4, "assemble_stack: frames ([W,]T,h,w,3) expected")
+    T, h, w, C = frames.shape[-4:]
+    if C != 3 or tuple(warped.shape) != lead + (T - 1, h, w, 3) or tuple(proj.shape) != lead + (T - 1, h, w, 2) or \
+            tuple(resid.shape) != lead + (T - 1, h, w) or tuple(depth.shape) != lead + (T - 1, h, w) or \
+            not 0 <= centre_idx < T:
         raise ValueError("assemble_stack: inconsistent shapes")
     if estimate is not None:
         _req(estimate, torch.float32, "estimate")
-        if tuple(estimate.shape) != (3, h, w):
-            raise ValueError("assemble_stack: estimate must be (3,h,w)")
-    if fallback is None:
-        fallback = centre
-    _req(fallback, torch.float32, "fallback")
-    if tuple(fallback.shape) != (h, w, 3):
-        raise ValueError("assemble_stack: fallback must be (h,w,3)")
+        if tuple(estimate.shape) != lead + (3, h, w):
+            raise ValueError("assemble_stack: estimate must be ([W,]3,h,w)")
     if out is None:
-        out = torch.empty((3 * T - 1, 3, h, w), dtype=torch.float32, device=warped.device)
+        out = torch.empty(lead + (3 * T - 1, 3, h, w), dtype=torch.float32, device=warped.device)
+    else:
+        _req(out, torch.float32, "out")
+        if tuple(out.shape) != lead + (3 * T - 1, 3, h, w):
+            raise ValueError("assemble_stack: out must be ([W,]3T-1,3,h,w)")
     with torch.cuda.device(warped.device):
-        _lib.check(_lib.lib().vsr_assemble_stack(warped.data_ptr(), centre.data_ptr(), proj.data_ptr(), resid.data_ptr(),
-                                                 depth.data_ptr(), estimate.data_ptr() if estimate is not None else None,
-                                                 fallback.data_ptr(), out.data_ptr(), T, int(centre_idx), h, w, _stream()),
-                   "assemble_stack")
+        _lib.check(_lib.lib().vsr_assemble_stack_windows(
+            warped.data_ptr(), frames.select(-4, centre_idx).data_ptr(), proj.data_ptr(), resid.data_ptr(),
+            depth.data_ptr(), estimate.data_ptr() if estimate is not None else None, frames.data_ptr(), out.data_ptr(),
+            nw, T * h * w * 3, T, int(centre_idx), h, w, _stream()), "assemble_stack")
     return out
 
 
 def estimate_slot(hr: torch.Tensor, mask: torch.Tensor | None, slot: torch.Tensor, scale: int = 4) -> torch.Tensor:
-    """slot (3,h,w) <- nearest-downsized hr (3,h*scale,w*scale) with masked pixels zeroed
-    (video_super_resolution.py:44,58-60).  `slot` is written in place (a view of the stack)."""
+    """slot ([W,]3,h,w) <- nearest-downsized hr ([W,]3,h*scale,w*scale) with the pixels of mask ([W,]h,w) zeroed
+    (video_super_resolution.py:44,58-60), one launch for all windows.  `slot` is written in place: a view of the
+    stack, such as stack[:, M-1] of a (W,M,3,h,w) stack, with each window's slot contiguous."""
     _req(hr, torch.float32, "hr")
-    _req(slot, torch.float32, "slot")
-    _, h, w = slot.shape
-    if tuple(hr.shape) != (3, h * scale, w * scale):
-        raise ValueError("estimate_slot: hr must be (3,h*scale,w*scale)")
+    lead, nw = _lead(slot, 3, "estimate_slot: slot ([W,]3,h,w) expected")
+    _req(slot[0] if lead else slot, torch.float32, "slot")
+    c, h, w = slot.shape[-3:]
+    if c != 3 or tuple(hr.shape) != lead + (3, h * scale, w * scale):
+        raise ValueError("estimate_slot: slot ([W,]3,h,w) and hr ([W,]3,h*scale,w*scale) expected")
     if mask is not None:
         _req(mask, torch.uint8, "mask")
-        if tuple(mask.shape) != (h, w):
-            raise ValueError("estimate_slot: mask must be (h,w)")
-    with torch.cuda.device(hr.device):
-        _lib.check(_lib.lib().vsr_estimate_slot(hr.data_ptr(), mask.data_ptr() if mask is not None else None,
-                                                slot.data_ptr(), h, w, int(scale), _stream()), "estimate_slot")
-    return slot
-
-
-# -- several frame windows per launch ------------------------------------------------------------------------------
-# The per-window stages above with a leading window dimension W: one launch per stage for all W windows, window b
-# bit-identical to the one-window call on it (the one-window entry points are the same kernels with W = 1).
-
-def warp_windows(frames: torch.Tensor, flows: torch.Tensor, centre: int, bilinear: bool | int = 2,
-                 want_resid: bool = True):
-    """warp_window over W windows: frames (W,T,H,W,3), flows (W,T-1,H,W,2) -> warped (W,T-1,H,W,3) and, with
-    want_resid, resid (W,T-1,H,W)."""
-    _req(frames, torch.float32, "frames")
-    _req(flows, torch.float32, "flows")
-    if frames.dim() != 5:
-        raise ValueError("warp_windows: frames (W,T,H,W,3) expected")
-    nw, T, H, W, C = frames.shape
-    if nw < 1 or C != 3 or tuple(flows.shape) != (nw, T - 1, H, W, 2) or not 0 <= centre < T:
-        raise ValueError("warp_windows: frames (W,T,H,W,3), flows (W,T-1,H,W,2), 0 <= centre < T expected")
-    warped = torch.empty((nw, T - 1, H, W, 3), dtype=torch.float32, device=frames.device)
-    resid = torch.empty((nw, T - 1, H, W), dtype=torch.float32, device=frames.device) if want_resid else None
-    with torch.cuda.device(frames.device):
-        _lib.check(_lib.lib().vsr_warp_windows_nhwc3(frames.data_ptr(), flows.data_ptr(), warped.data_ptr(),
-                                                     resid.data_ptr() if resid is not None else None, nw, T,
-                                                     int(centre), H, W, int(bilinear), _stream()), "warp_windows")
-    return warped, resid
-
-
-def vos_threshold_windows(logits_a: torch.Tensor, logits_b: torch.Tensor) -> torch.Tensor:
-    """vos_threshold over W windows: logits (W,h,w) x2 -> mask (W,h,w) u8."""
-    _req(logits_a, torch.float32, "logits_a")
-    _req(logits_b, torch.float32, "logits_b")
-    if logits_a.shape != logits_b.shape or logits_a.dim() != 3 or logits_a.shape[0] < 1:
-        raise ValueError("vos_threshold_windows: two (W,h,w) tensors expected")
-    nw, h, w = logits_a.shape
-    mask = torch.empty((nw, h, w), dtype=torch.uint8, device=logits_a.device)
-    with torch.cuda.device(logits_a.device):
-        _lib.check(_lib.lib().vsr_vos_threshold_windows(logits_a.data_ptr(), logits_b.data_ptr(), mask.data_ptr(), nw,
-                                                        h, w, _stream()), "vos_threshold_windows")
-    return mask
-
-
-def assemble_stacks(warped: torch.Tensor, frames: torch.Tensor, proj: torch.Tensor, resid: torch.Tensor,
-                    depth: torch.Tensor, estimate: torch.Tensor | None, centre_idx: int,
-                    out: torch.Tensor | None = None) -> torch.Tensor:
-    """assemble_stack over W windows -> (W,3T-1,3,h,w).  warped (W,T-1,h,w,3), frames (W,T,h,w,3) (the centre frame
-    and, without an estimate, the fallback LR frame 0 of each window are read from it in place), proj (W,T-1,h,w,2),
-    resid / depth (W,T-1,h,w), estimate (W,3,h,w) | None."""
-    for t, n in ((warped, "warped"), (frames, "frames"), (proj, "proj"), (resid, "resid"), (depth, "depth")):
-        _req(t, torch.float32, n)
-    if frames.dim() != 5:
-        raise ValueError("assemble_stacks: frames (W,T,h,w,3) expected")
-    nw, T, h, w, _ = frames.shape
-    if nw < 1 or frames.shape[4] != 3 or tuple(warped.shape) != (nw, T - 1, h, w, 3) or \
-            tuple(proj.shape) != (nw, T - 1, h, w, 2) or tuple(resid.shape) != (nw, T - 1, h, w) or \
-            tuple(depth.shape) != (nw, T - 1, h, w) or not 0 <= centre_idx < T:
-        raise ValueError("assemble_stacks: inconsistent shapes")
-    if estimate is not None:
-        _req(estimate, torch.float32, "estimate")
-        if tuple(estimate.shape) != (nw, 3, h, w):
-            raise ValueError("assemble_stacks: estimate must be (W,3,h,w)")
-    if out is None:
-        out = torch.empty((nw, 3 * T - 1, 3, h, w), dtype=torch.float32, device=warped.device)
-    else:
-        _req(out, torch.float32, "out")
-        if tuple(out.shape) != (nw, 3 * T - 1, 3, h, w):
-            raise ValueError("assemble_stacks: out must be (W,3T-1,3,h,w)")
-    with torch.cuda.device(warped.device):
-        _lib.check(_lib.lib().vsr_assemble_stack_windows(
-            warped.data_ptr(), frames[0, centre_idx].data_ptr(), proj.data_ptr(), resid.data_ptr(), depth.data_ptr(),
-            estimate.data_ptr() if estimate is not None else None, frames.data_ptr(), out.data_ptr(), nw,
-            T * h * w * 3, T, int(centre_idx), h, w, _stream()), "assemble_stacks")
-    return out
-
-
-def estimate_slots(hr: torch.Tensor, mask: torch.Tensor | None, stack: torch.Tensor, scale: int = 4) -> torch.Tensor:
-    """estimate_slot over W windows: the last map of each window of stack (W,M,3,h,w) <- nearest-downsized hr
-    (W,3,h*scale,w*scale) with the pixels of mask (W,h,w) zeroed.  Written in place; returns stack."""
-    _req(hr, torch.float32, "hr")
-    _req(stack, torch.float32, "stack")
-    if stack.dim() != 5 or stack.shape[2] != 3:
-        raise ValueError("estimate_slots: stack must be (W,M,3,h,w)")
-    nw, M, _, h, w = stack.shape
-    if nw < 1 or tuple(hr.shape) != (nw, 3, h * scale, w * scale):
-        raise ValueError("estimate_slots: hr must be (W,3,h*scale,w*scale)")
-    if mask is not None:
-        _req(mask, torch.uint8, "mask")
-        if tuple(mask.shape) != (nw, h, w):
-            raise ValueError("estimate_slots: mask must be (W,h,w)")
+        if tuple(mask.shape) != lead + (h, w):
+            raise ValueError("estimate_slot: mask must be ([W,]h,w)")
     with torch.cuda.device(hr.device):
         _lib.check(_lib.lib().vsr_estimate_slot_windows(hr.data_ptr(), mask.data_ptr() if mask is not None else None,
-                                                        stack[0, M - 1].data_ptr(), nw, M * 3 * h * w, h, w,
-                                                        int(scale), _stream()), "estimate_slots")
-    return stack
-
-
-def compose_flow_windows(g: torch.Tensor | None, f: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
-    """compose_flow over W windows on strided views: g, f, out (W,H,W,2) with the same stride between windows (e.g.
-    neighbour n of a (W,T-1,H,W,2) array, x[:, n]), each window's field contiguous.  g=None: out = f."""
-    _req(f.select(0, 0), torch.float32, "f")
-    for t, n in ((g, "g"), (out, "out")):
-        if t is not None:
-            _req(t.select(0, 0), torch.float32, n)
-            if t.shape != f.shape or t.stride(0) != f.stride(0):
-                raise ValueError(f"compose_flow_windows: {n} must have the shape and window stride of f")
-    if f.dim() != 4 or f.shape[3] != 2 or f.shape[0] < 1:
-        raise ValueError("compose_flow_windows: (W,H,W,2) fields expected")
-    nw, H, W, _ = f.shape
-    with torch.cuda.device(f.device):
-        _lib.check(_lib.lib().vsr_compose_flow_windows(g.data_ptr() if g is not None else None, f.data_ptr(),
-                                                       out.data_ptr(), nw, f.stride(0), H, W, _stream()),
-                   "compose_flow_windows")
-    return out
-
-
-def warp_labels_windows(labels: torch.Tensor, flow: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
-    """warp_labels over W windows: labels (W,H,W) u8, flow (W,H,W,2) with each window's field contiguous (a view such
-    as x[:, n] of a (W,T-1,H,W,2) array is fine) -> (W,H,W) u8 (written into `out` when given)."""
-    _req(labels, torch.uint8, "labels")
-    _req(flow.select(0, 0), torch.float32, "flow")
-    nw, H, W = labels.shape
-    if tuple(flow.shape) != (nw, H, W, 2):
-        raise ValueError("warp_labels_windows: flow must be (W,H,W,2)")
-    if out is not None:
-        _req(out, torch.uint8, "out")
-        if out.shape != labels.shape:
-            raise ValueError("warp_labels_windows: out must be (W,H,W)")
-    dst = torch.empty_like(labels) if out is None else out
-    with torch.cuda.device(labels.device):
-        _lib.check(_lib.lib().vsr_warp_labels_u8_windows(labels.data_ptr(), flow.data_ptr(), dst.data_ptr(), nw,
-                                                         flow.stride(0), H, W, _stream()), "warp_labels_windows")
-    return dst
+                                                        slot.data_ptr(), nw, slot.stride(0) if nw > 1 else 0, h, w,
+                                                        int(scale), _stream()), "estimate_slot")
+    return slot
 
 
 def unpack_bands(src: torch.Tensor, dst: torch.Tensor, bounds, planes: int, row: int, band_stride: int) -> torch.Tensor:

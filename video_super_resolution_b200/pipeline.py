@@ -97,8 +97,8 @@ class WarpFusePipeline:
     be 1).  Rank 0 builds the stack and VOS mask (a1-a5, a7) and broadcasts them -- with the default atomic projection
     their fp32 sums can differ in the last bits from rank to rank, and the frame must be fused from maps of ONE stack;
     the ranks then split the conv stack by maps and the fc by row bands (SRProjectionModule(map_group=...), which `sr`
-    must be, with the same group).  The estimate slot is written band by band (vsr_estimate_slot on each rank's rows)
-    and all-gathered.  Every rank passes the same inputs; rank 0's are the ones used."""
+    must be, with the same group).  The estimate slot is written band by band (vsr_estimate_slot_windows on each rank's
+    rows) and all-gathered.  Every rank passes the same inputs; rank 0's are the ones used."""
 
     def __init__(self, T: int, h: int, w: int, sr: SRProjectionModule | None = None, scale: int = 4,
                  device="cuda:0", run_fusion: bool = True, max_disp: float | None = None, reuse: str | None = None,
@@ -151,13 +151,13 @@ class WarpFusePipeline:
         T, c, G, W = self.T, self.centre, self._centre_flows, self.windows
         proj = proj.reshape(W, T - 1, self.h, self.w, 2)
         flows = flows.reshape(W, T - 1, self.h, self.w, 2)
-        ops.compose_flow_windows(None, proj[:, c - 1], out=G[:, c - 1])
+        ops.compose_flow(None, proj[:, c - 1], out=G[:, c - 1])
         for t in range(c - 2, -1, -1):
-            ops.compose_flow_windows(G[:, t + 1], proj[:, t], out=G[:, t])
+            ops.compose_flow(G[:, t + 1], proj[:, t], out=G[:, t])
         if c + 1 < T:
-            ops.compose_flow_windows(None, flows[:, c], out=G[:, c])         # frame c+1 is neighbour index c
+            ops.compose_flow(None, flows[:, c], out=G[:, c])     # frame c+1 is neighbour index c
             for t in range(c + 2, T):
-                ops.compose_flow_windows(G[:, t - 2], flows[:, t - 1], out=G[:, t - 1])
+                ops.compose_flow(G[:, t - 2], flows[:, t - 1], out=G[:, t - 1])
         return self.centre_flows
 
     def _batched(self, frames, flows, inv_depth, logits_a, logits_b, estimate, estimate_hr):
@@ -191,15 +191,15 @@ class WarpFusePipeline:
                                                              self.max_disp)
         self.chain_flows(proj_d, fl)
         G = self._centre_flows
-        warped, resid = ops.warp_windows(x["frames"], G, c, 2)     # fast fp32 blend (north star: <= 1e-3)
-        mask = ops.vos_threshold_windows(x["logits_a"], x["logits_b"])
-        mask_w = ops.warp_labels_windows(mask, G[:, c - 1], out=self._mask_w)
-        ops.assemble_stacks(warped, x["frames"], proj_f.view(W, T - 1, h, w, 2), resid, wsum.view(W, T - 1, h, w),
-                            x["estimate"], c, out=self._stack)
+        warped, resid = ops.warp_window(x["frames"], G, c, 2)      # fast fp32 blend (north star: <= 1e-3)
+        mask = ops.vos_threshold(x["logits_a"], x["logits_b"])
+        mask_w = ops.warp_labels(mask, G[:, c - 1], out=self._mask_w)
+        ops.assemble_stack(warped, x["frames"], proj_f.view(W, T - 1, h, w, 2), resid, wsum.view(W, T - 1, h, w),
+                           x["estimate"], c, out=self._stack)
         if estimate is None and estimate_hr is not None:
             sel = range(W) if estimate_hr_windows is None else sorted(set(estimate_hr_windows))
             for a, b in _runs(sel):                                    # one launch per run of consecutive windows
-                ops.estimate_slots(x["estimate_hr"][a:b], None, self._stack[a:b], self.scale)
+                ops.estimate_slot(x["estimate_hr"][a:b], None, self._stack[a:b, self.M - 1], self.scale)
         r = {"proj_flow": proj_f, "count_flow": cnt_f, "hole_flow": hole_f, "proj_depth": proj_d, "wsum": wsum,
              "count_depth": cnt_d, "hole_depth": hole_d}
         r = {k: v.view((W, T - 1) + tuple(v.shape[1:])) for k, v in r.items()}
@@ -227,7 +227,7 @@ class WarpFusePipeline:
         if not self.run_fusion:
             return self.stack
         if mg is None:
-            ops.estimate_slots(self.sr(self.stack), self._mask_w, self._stack, self.scale)     # pass 1
+            ops.estimate_slot(self.sr(self.stack), self._mask_w, self._stack[:, self.M - 1], self.scale)   # pass 1
         else:
             if estimate_hr_band is not None:
                 self._slot_from_band(estimate_hr_band, None)
@@ -237,7 +237,8 @@ class WarpFusePipeline:
 
     def _slot_from_band(self, band, mask):
         """The estimate slot from the frame's row bands: each rank downsizes its band into its LR rows of the slot
-        (vsr_estimate_slot with the band as the frame), and an all-gather assembles the (3,h,w) slot on every rank."""
+        (vsr_estimate_slot_windows with the band as the frame), and an all-gather assembles the (3,h,w) slot on every
+        rank."""
         mg, s, w = self.map_group, self.scale, self.w
         _, lb, hb = self.sr.band_geometry(self.h)
         r = mg.rank
@@ -388,8 +389,8 @@ def run_sequence(vsr, frames, flows, inv_depth, logits, chunks, out: torch.Tenso
         for k in c:
             la, lb = logits(k)
             # the previous output frame stays planar fp32 on the device and is downsized into the estimate slot by
-            # vsr_estimate_slot (a map group keeps only this rank's row band of it and all-gathers the u8 frame); the
-            # u8 frame (utils/video_utils.py:23) is written by the fc-fuse kernel itself
+            # vsr_estimate_slot_windows (a map group keeps only this rank's row band of it and all-gathers the u8
+            # frame); the u8 frame (utils/video_utils.py:23) is written by the fc-fuse kernel itself
             if group:
                 nxt = {"estimate_hr_band": est, "gather": "u8"}
             else:
