@@ -458,6 +458,19 @@ int vsr_test_fused_updown(const void* lr_bf16, void* hr_bf16, int nsrc, int stor
                           const float* bt_host, float slope_t, const float* wd_host, const float* bd_host,
                           float slope_d, void* y_bf16, void* workspace, size_t workspace_bytes,
                           vsr_stream_t stream);
+/*   conv_in  : the stack's first layer as the plan runs it: sub_mean (sub_bias), Conv2d(3,128,3,p1) zero-padding the
+ *              SHIFTED image, + PReLU.  x (B,3,h,w) f32 -> y (B,h,w,128) bf16; w (128,3,3,3), b (128), sub_bias (3)
+ *              fp32 host.  workspace: vsr_test_workspace_bytes + B*h*w*64 bytes (the im2col operand). */
+int vsr_test_conv_in(const float* x, int B, int h, int w, const float* w_host, const float* b_host, float slope,
+                     const float* sub_bias_host, void* y_bf16, void* workspace, size_t workspace_bytes,
+                     vsr_stream_t stream);
+/*   conv_out : the stack's last layer as the plan runs it: Conv2d(32,3,3,p1) of hb (B,s*h,s*w,32) bf16 + bilinear
+ *              upsampling (align_corners=False) of x (B,3,h,w) f32 + sub_bias, + add_bias -> y (B,3,s*h,s*w) f32;
+ *              scale s 2 or 4.  w (3,32,3,3), b (3), sub_bias (3), add_bias (3) fp32 host.
+ *              workspace: vsr_test_workspace_bytes bytes. */
+int vsr_test_conv_out(const void* hb_bf16, const float* x, int scale, int B, int h, int w, const float* w_host,
+                      const float* b_host, const float* sub_bias_host, const float* add_bias_host, float* y,
+                      void* workspace, size_t workspace_bytes, vsr_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -158,3 +158,71 @@ def fused_updown(lr_bf16, hr_bf16, store, wu, bu, slope_u, wt, bt, slope_t, wd, 
     assert torch.equal(hr[:nsrc - 1].view(torch.int16), hr_bf16[:nsrc - 1].view(torch.int16)), \
         "fused_updown wrote into a source slot it only reads"
     return y.clone(), hr.clone()
+
+
+def conv_in(x, w, b, slope, sub_bias):
+    """x (B,3,h,w) f32 cuda; w (128,3,3,3), b (128), sub_bias (3) f32 cpu -> (B,h,w,128) bf16 (vsr_test_conv_in).  y
+    starts as NaN between two guard bands that must come back untouched; the workspace starts as 0xFF bytes."""
+    B, _, h, w_ = x.shape
+    ybuf, y, G = _guarded((B, h, w_, 128), x.device)
+    y.fill_(float("nan"))
+    n = int(_lib.lib().vsr_test_workspace_bytes(B, h, w_)) + B * h * w_ * 64
+    ws = torch.full((n,), 0xFF, dtype=torch.uint8, device=x.device)
+    x = x.contiguous().float()
+    w, b, sub_bias = (t.contiguous().float() for t in (w, b, sub_bias))
+    _lib.check(_lib.lib().vsr_test_conv_in(x.data_ptr(), B, h, w_, _fp(w), _fp(b), float(slope), _fp(sub_bias),
+                                           y.data_ptr(), ws.data_ptr(), ws.numel(),
+                                           torch.cuda.current_stream().cuda_stream), "test_conv_in")
+    assert _guards_intact(ybuf, G), "conv_in wrote outside y"
+    return y.clone()
+
+
+F32_GUARD = 1234.5           # value of the fp32 guard bands around conv_out's output
+
+
+def conv_out(hb_bf16, x, scale, w, b, sub_bias, add_bias):
+    """hb (B,s*h,s*w,32) bf16 cuda; x (B,3,h,w) f32 cuda; w (3,32,3,3), b (3), sub_bias (3), add_bias (3) f32 cpu ->
+    (B,3,s*h,s*w) f32 (vsr_test_conv_out).  y starts as NaN between two fp32 guard bands that must come back
+    untouched."""
+    B, _, h, w_ = x.shape
+    assert tuple(hb_bf16.shape) == (B, scale * h, scale * w_, 32)
+    n = B * 3 * scale * h * scale * w_
+    G = 1 << 15                                   # 128 KB on each side: more than one output row of a tile
+    buf = torch.full((n + 2 * G,), F32_GUARD, dtype=torch.float32, device=x.device)
+    y = buf[G:G + n].view(B, 3, scale * h, scale * w_)
+    y.fill_(float("nan"))
+    ws = _ws(x.device)
+    x = x.contiguous().float()
+    w, b, sub_bias, add_bias = (t.contiguous().float() for t in (w, b, sub_bias, add_bias))
+    _lib.check(_lib.lib().vsr_test_conv_out(hb_bf16.data_ptr(), x.data_ptr(), int(scale), B, h, w_, _fp(w), _fp(b),
+                                            _fp(sub_bias), _fp(add_bias), y.data_ptr(), ws.data_ptr(), ws.numel(),
+                                            torch.cuda.current_stream().cuda_stream), "test_conv_out")
+    assert bool((buf[:G] == F32_GUARD).all()) and bool((buf[G + n:] == F32_GUARD).all()), "conv_out wrote outside y"
+    return y.clone()
+
+
+def faithful_bf16(got, want, absdot, what, c=16.0, max_frac=None, ulps=1, extra=0.0):
+    """BF16 outputs of one layer fed the restatement's own BF16 inputs: |got - want| <= ulps * ulp_bf16(want) +
+    c * 2^-24 * absdot + extra per element, absdot = sum |w * x| (the fp32 accumulation error, cancellation included);
+    and the fraction of elements that differ at all <= max_frac.  ulps is 1, or 2 where a second BF16 rounding follows
+    the first (the negative side of the packed PReLU: bf16(s * bf16(x)), so one ulp of x may become two of the
+    output); extra covers an intermediate BF16 value that rounds the other way (see the fused down tests).  Returns
+    (fraction that differs, worst err / tolerance)."""
+    got, want, absdot = (t.double().cpu() for t in (got, want, absdot))
+    ulps = ulps.double().cpu() if torch.is_tensor(ulps) else ulps
+    extra = extra.double().cpu() if torch.is_tensor(extra) else extra
+    assert torch.isfinite(got).all(), f"{what}: non-finite output"
+    ulp = torch.exp2(torch.floor(torch.log2(want.abs().clamp_min(2.0 ** -126))) - 7)
+    tol = ulps * ulp + c * 2.0 ** -24 * absdot + extra
+    err = (got - want).abs()
+    bad = (err > tol).nonzero()
+    if bad.numel():
+        first = [tuple(i.tolist()) for i in bad[:6]]
+        raise AssertionError(f"{what}: {bad.shape[0]}/{err.numel()} outside the faithful bound; first got/want/tol: "
+                             + ", ".join(f"{i}: {got[i].item():.6g}/{want[i].item():.6g}/{tol[i].item():.3g}"
+                                         for i in first))
+    frac = (got != want).double().mean().item()
+    print(f"[measure] {what}: differ {frac:.6f}, worst err/tol {(err / tol).max().item():.3f}")
+    if max_frac is not None:
+        assert frac <= max_frac, f"{what}: {frac:.4%} of the elements differ (bound {max_frac:.4%})"
+    return frac, (err / tol).max().item()

@@ -111,6 +111,10 @@ SIGNATURES = {
                                       c_size_t, c_void_p]),
     "vsr_test_x2_layer": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_size_t, c_void_p]),
     "vsr_test_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "vsr_test_conv_in": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_void_p,
+                                 c_size_t, c_void_p]),
+    "vsr_test_conv_out": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_void_p, c_void_p, c_size_t, c_void_p]),
 }
 
 _lib = None

@@ -726,6 +726,14 @@ im2col_kernel(const float* __restrict__ x, const float* __restrict__ sub_bias, u
   }
 }
 
+// conv_in's A operand for the maps x (M,3,h,w): a0 [M*h*w][32] BF16 (the plan's sweeps and vsr_test_conv_in)
+int launch_im2col(const float* x, const float* sub_bias_dev, void* a0, int M, int h, int w, cudaStream_t st) {
+  int64_t blocks = ceil_div64((int64_t)M * h * w, 256);
+  if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
+  im2col_kernel<<<(int)blocks, 256, 0, st>>>(x, sub_bias_dev, reinterpret_cast<uint4*>(a0), M, h, w);
+  return after_launch();
+}
+
 // fc over the map axis per (channel, HR pixel): Linear(M,32)-ReLU-Linear(32,1)-ReLU
 // (SRProjectionModule.py:126-131,146).  maps (W*M,3,H,W) f32 -> y (W,3,H,W) f32: window b = blockIdx.y fuses the
 // maps [b*M, (b+1)*M) into frame b with the same per-pixel arithmetic as a one-window launch.
@@ -1239,18 +1247,14 @@ extern "C" int vsr_srfbn_forward(vsr_srfbn_plan* pl, const float* x, float* y, v
 static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_out_layer, const float* x, int m0, int Mc,
                       cudaStream_t st, size_t* ev) {
   const vsr_srfbn_config& c = pl->cfg;
-  const int64_t P = (int64_t)Mc * c.h * c.w;
   auto mark = [&]() {
     if (ev && pl->profile && *ev < pl->events.size()) cudaEventRecord(pl->events[(*ev)++], st);
   };
   const float* xc = x + (int64_t)m0 * 3 * c.h * c.w;
   mark();
   {
-    int64_t blocks = ceil_div64(P, 256);
-    if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
-    im2col_kernel<<<(int)blocks, 256, 0, st>>>(xc, reinterpret_cast<const float*>(pl->dev_w + pl->misc_off),
-                                               reinterpret_cast<uint4*>(pl->ws + pl->o_a0), Mc, c.h, c.w);
-    int rc = after_launch();
+    int rc = launch_im2col(xc, reinterpret_cast<const float*>(pl->dev_w + pl->misc_off), pl->ws + pl->o_a0, Mc, c.h,
+                           c.w, st);
     if (rc) return rc;
   }
   {   // the last layer reads the network input (bilinear skip) and writes these maps of the premix buffer
@@ -1703,6 +1707,72 @@ extern "C" int vsr_test_fused_updown(const void* lr_bf16, void* hr_bf16, int nsr
   if (rc) return rc;
   rc = build_finalize(L, acc, bd_dev, y_bf16, (int64_t)B * h * w, h, w);
   if (rc) return rc;
+  rc = launch_layer(L, st);
+  if (rc) return rc;
+  return cuda_status(cudaStreamSynchronize(st));
+}
+
+// conv_in (3x3 p1, 3 -> 128) + PReLU as the plan runs it: im2col_kernel (sub_mean, zero padding of the shifted image,
+// K padded 27 -> 32), then the N = 128 pointwise GEMM.  x (B,3,h,w) f32, w_host (128,3,3,3), b_host (128), sub_bias_host
+// (3) -> y (B,h,w,128) bf16.  Workspace: packed weights [0, 8K), bias + slope at 256K, sub_mean bias at 257K, then the
+// A0 operand: vsr_test_workspace_bytes(B,h,w) + B*h*w*64 bytes.
+extern "C" int vsr_test_conv_in(const float* x, int B, int h, int w, const float* w_host, const float* b_host, float slope,
+                                const float* sub_bias_host, void* y_bf16, void* workspace, size_t workspace_bytes,
+                                vsr_stream_t stream) {
+  if (!x || !w_host || !b_host || !sub_bias_host || !y_bf16 || !workspace || B <= 0 || h <= 0 || w <= 0)
+    return VSR_ERR_INVALID_ARG;
+  const size_t base_bytes = vsr_test_workspace_bytes(B, h, w);
+  const int64_t P = (int64_t)B * h * w;
+  if (workspace_bytes < base_bytes + (size_t)P * 64) return VSR_ERR_WORKSPACE;
+  cudaStream_t st = as_stream(stream);
+  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
+  std::vector<uint16_t> wp((size_t)128 * 32);
+  pack_conv_in(w_host, wp.data());
+  float bias[129];
+  memcpy(bias, b_host, 128 * 4);
+  bias[128] = slope;
+  int rc = upload(ws, wp.data(), wp.size() * 2, st);
+  if (!rc) rc = upload(ws + 256 * 1024, bias, sizeof(bias), st);
+  if (!rc) rc = upload(ws + 257 * 1024, sub_bias_host, 3 * 4, st);
+  if (rc) return rc;
+  uint8_t* a0 = ws + base_bytes;
+  rc = launch_im2col(x, reinterpret_cast<const float*>(ws + 257 * 1024), a0, B, h, w, st);
+  if (rc) return rc;
+  Layer L;
+  Src s{a0, 32, 0, 32};
+  rc = build_pointwise(L, &s, 1, P, ws, reinterpret_cast<const float*>(ws + 256 * 1024), 128, 1, y_bf16, 256, 0, 0, h, w);
+  if (rc) return rc;
+  rc = launch_layer(L, st);
+  if (rc) return rc;
+  return cuda_status(cudaStreamSynchronize(st));
+}
+
+// conv_out (3x3 p1, 32 -> 3) + bilinear skip of sub_mean(x) + add_mean as the plan runs it (EPI_CONV_OUT).  hb (B,s*h,
+// s*w,32) bf16 (the `out` transposed conv's NHWC map), x (B,3,h,w) f32, scale 2 or 4, w_host (3,32,3,3), b_host (3),
+// sub_bias_host / add_bias_host (3) -> y (B,3,s*h,s*w) f32.  Workspace: vsr_test_workspace_bytes(B,h,w) bytes.
+extern "C" int vsr_test_conv_out(const void* hb_bf16, const float* x, int scale, int B, int h, int w, const float* w_host,
+                                 const float* b_host, const float* sub_bias_host, const float* add_bias_host, float* y,
+                                 void* workspace, size_t workspace_bytes, vsr_stream_t stream) {
+  if (!hb_bf16 || !x || !w_host || !b_host || !sub_bias_host || !add_bias_host || !y || !workspace || B <= 0 || h <= 0 ||
+      w <= 0)
+    return VSR_ERR_INVALID_ARG;
+  if (scale != 2 && scale != 4) return VSR_ERR_UNSUPPORTED;
+  if (workspace_bytes < vsr_test_workspace_bytes(B, h, w)) return VSR_ERR_WORKSPACE;
+  cudaStream_t st = as_stream(stream);
+  uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
+  std::vector<uint16_t> wp((size_t)32 * 32);
+  pack_conv_out(w_host, wp.data());
+  float bias[16 + 7] = {};   // the plan's layout (vsr_srfbn_pack_weights): conv_out bias, slope slot, sub / add mean
+  memcpy(bias, b_host, 3 * 4);
+  memcpy(bias + 17, sub_bias_host, 3 * 4);
+  memcpy(bias + 20, add_bias_host, 3 * 4);
+  int rc = upload(ws, wp.data(), wp.size() * 2, st);
+  if (!rc) rc = upload(ws + 256 * 1024, bias, sizeof(bias), st);
+  if (rc) return rc;
+  Layer L;
+  rc = build_conv_out(L, hb_bf16, B, h, w, scale, ws, reinterpret_cast<const float*>(ws + 256 * 1024), y);
+  if (rc) return rc;
+  L.p.skip_src = x;
   rc = launch_layer(L, st);
   if (rc) return rc;
   return cuda_status(cudaStreamSynchronize(st));
