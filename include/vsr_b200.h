@@ -414,6 +414,32 @@ int vsr_srfbn_profile_launches(vsr_srfbn_plan* plan, float* ms, int32_t* kclass,
 /* Test hook: per-map network output before the fc fuse, (M,3,s*h,s*w) f32 (SRProjectionModule.py:143);
  * valid after vsr_srfbn_forward on the same stream. */
 int vsr_srfbn_debug_premix(const vsr_srfbn_plan* plan, float* out_maps, vsr_stream_t stream);
+/* Test hook: runs the layers [first, first + count) of a bound plan's layer list (count >= 1) over the plan's first chunk
+ * of maps of x, exactly as a forward's sweep launches them: the im2col of those maps first when first == 0, and the last
+ * layer (conv_out) reads x for its skip and writes the chunk's premix slot.  The layer list is the one a profiled forward
+ * of an unchunked plan reports through vsr_srfbn_profile_launches, without its first (im2col) and last (fc) launch.
+ * VSR_ERR_INVALID_ARG for a null plan or x or a range outside the list, VSR_ERR_STATE for an unbound plan; no CUDA call
+ * before these checks. */
+int vsr_srfbn_debug_run_layers(vsr_srfbn_plan* plan, const float* x, int first, int count, vsr_stream_t stream);
+/* Test hook (host only, valid once the plan is created, bound or not): byte offset and size of one activation buffer in
+ * the plan's workspace layout.  LR takes index 0..6 and HR 0..5, every other id index 0.  Sizes for chunk_maps maps
+ * (P = chunk_maps*h*w LR pixels): A0, XFEAT, HIDDEN, LR, U P*64 (BF16 (P,32)); C128 P*256; HR x4 chunk_maps*(h+1)*(w+1)*
+ * 16*64 (HR block layout), x2 4P*64 (NHWC); HB s*s*P*64; HT (x2) 4P*64; ACC (x4) P*512 (fp32 partial slots); PREMIX the
+ * per-map images of every swept map.  VSR_ERR_UNSUPPORTED for a buffer the plan does not have (x4: HR index 5, kept on
+ * chip by the merged kernel, and HT; x2: ACC); VSR_ERR_INVALID_ARG for a null pointer or an id / index out of range. */
+#define VSR_SRFBN_BUF_A0 0
+#define VSR_SRFBN_BUF_C128 1
+#define VSR_SRFBN_BUF_XFEAT 2
+#define VSR_SRFBN_BUF_HIDDEN 3
+#define VSR_SRFBN_BUF_LR 4
+#define VSR_SRFBN_BUF_U 5
+#define VSR_SRFBN_BUF_HR 6
+#define VSR_SRFBN_BUF_HB 7
+#define VSR_SRFBN_BUF_HT 8
+#define VSR_SRFBN_BUF_ACC 9
+#define VSR_SRFBN_BUF_PREMIX 10
+#define VSR_SRFBN_BUFFERS 11
+int vsr_srfbn_debug_buffer(const vsr_srfbn_plan* plan, int id, int index, size_t* offset, size_t* bytes);
 
 /* Single-layer test hooks: run ONE layer of the stack through the same tcgen05 kernels the plan
  * uses, on BF16 channels-last operands, so tests can compare layer by layer with torch.nn fp32

@@ -1,10 +1,16 @@
-"""Python front-ends of the single-layer test hooks of the C ABI (vsr_test_*) and the HR block
-layout helpers.  Test support only."""
+"""Python front-ends of the single-layer test hooks of the C ABI (vsr_test_*), the plan walk hooks
+(vsr_srfbn_debug_run_layers / vsr_srfbn_debug_buffer), the HR block layout helpers and the float64 expectations the
+layer tests share.  Test support only."""
 import ctypes
 
 import torch
+import torch.nn.functional as F
 
+from oracle import srfbn_bf16 as sb
 from video_super_resolution_b200 import _lib
+
+# activation buffer ids of vsr_srfbn_debug_buffer (include/vsr_b200.h VSR_SRFBN_BUF_*)
+BUF_A0, BUF_C128, BUF_XFEAT, BUF_HIDDEN, BUF_LR, BUF_U, BUF_HR, BUF_HB, BUF_HT, BUF_ACC, BUF_PREMIX = range(11)
 
 
 def _fp(t):
@@ -226,3 +232,105 @@ def faithful_bf16(got, want, absdot, what, c=16.0, max_frac=None, ulps=1, extra=
     if max_frac is not None:
         assert frac <= max_frac, f"{what}: {frac:.4%} of the elements differ (bound {max_frac:.4%})"
     return frac, (err / tol).max().item()
+
+
+def act(pre, slope, packed=True):
+    """Expected BF16 layer output from the float64 pre-activation acc + bias: bf16 then the packed-BF16 PReLU of
+    igemm.cuh, or (packed=False, the x4 strided conv of fused_down.cuh) the fp32 PReLU with the fp32 slope, rounded
+    once."""
+    s32 = float(torch.tensor(slope, dtype=torch.float32))
+    if packed:
+        return sb.prelu_packed(sb.round_bf16(pre), s32, float(sb.round_bf16(torch.tensor(s32))))
+    return sb.round_bf16(torch.where(pre >= 0, pre, pre * s32))
+
+
+def ulps(want, packed=True, pre=None):
+    """Output ulps a one-ulp difference of the rounded pre-activation can become: two on the negative side of the
+    packed PReLU (bf16(s_b * x_b) rounds a second time), one elsewhere.  The side is the pre-activation's: `pre` where
+    given; else the sign of `want`, which is the pre-activation's only for slopes >= 0 (a negative slope maps negative
+    pre-activations to positive outputs)."""
+    if not packed:
+        return 1.0
+    return torch.where((want if pre is None else pre) < 0, 2.0, 1.0)
+
+
+def down_faithful(srcs, wt, bt, slope_t, wd, bd, slope_d):
+    """The HR half of a feedback group in float64 with the kernels' rounding points (oracle/srfbn_bf16.py): srcs = nsrc
+    pairs (map (B,4h,4w,32) of BF16 values, its own sum |w * x| or None) -> (want (B,h,w,32), sum |w * x| through both
+    layers, extra tolerance).  H = packed-PReLU(bf16(downtran)) for nsrc > 1; lr = bf16(fp32-PReLU(conv)).  The
+    accumulation error of H reaches the output through |wd|, so H's sum |w * x| is carried into the conv's.  H is
+    rounded on chip: where its fp32 sum lies next to a BF16 rounding boundary, an element of H (or, in the merged
+    kernel, of U before it) rounds the other way, and that one element moves the output by up to 2 ulp(H) * |wd| --
+    measured on a B200 at 1 to 8 outputs in a million, 2 to 7 output ulps each.  The extra tolerance allows two such
+    elements in each output's 8x8 window.  The maps' device is the computation's."""
+    dev = srcs[0][0].device
+
+    def d(t):
+        return t.to(dev, torch.float64)
+
+    x = torch.cat([m.permute(0, 3, 1, 2) for m, _ in srcs], dim=1)
+    ax = torch.cat([(a if a is not None else torch.zeros_like(m)).permute(0, 3, 1, 2) for m, a in srcs], dim=1)
+    if len(srcs) > 1:
+        w1 = d(wt).view(32, 32 * len(srcs), 1, 1)
+        pre = F.conv2d(x, w1, d(bt))
+        ax = F.conv2d(x.abs() + ax, w1.abs(), d(bt).abs())
+        x = act(pre, slope_t)
+    pre = F.conv2d(x, d(wd), d(bd), stride=4, padding=2)
+    absdot = F.conv2d(x.abs() + ax, d(wd).abs(), d(bd).abs(), stride=4, padding=2)
+    extra = torch.zeros_like(pre)
+    if len(srcs) > 1:
+        ulp_h = torch.exp2(torch.floor(torch.log2(x.abs().amax(dim=1, keepdim=True).clamp_min(2.0 ** -126))) - 7)
+        win = F.max_pool2d(F.pad(ulp_h, (2, 2, 2, 2)), 8, stride=4)          # the window of each output pixel
+        extra = 2 * 2 * win * d(wd).abs().amax(dim=(1, 2, 3)).view(1, 32, 1, 1)
+    return (act(pre, slope_d, packed=False).permute(0, 2, 3, 1), absdot.permute(0, 2, 3, 1),
+            extra.permute(0, 2, 3, 1))
+
+
+def bits_equal(got, want, what, dims="b,y,x,c"):
+    """Raw-bit equality of two BF16 tensors (-0 and +0 differ); on failure names the first differing elements."""
+    a, b = got.view(torch.int16), want.view(torch.int16)
+    if torch.equal(a, b):
+        return
+    idx = (a != b).nonzero().cpu()
+    first = [tuple(i.tolist()) for i in idx[:8]]
+    pairs = [(got[i].item(), want[i].item()) for i in first]
+    raise AssertionError(f"{what}: {idx.shape[0]}/{a.numel()} elements differ; first ({dims}) got/want: "
+                         + ", ".join(f"{i}: {g}/{w}" for i, (g, w) in zip(first, pairs)))
+
+
+def conv_out_abs(hb, x, sd, scale):
+    """sum of |terms| of one conv_out output: the conv's |w * x|, |bias|, the skip's |taps| and |add_mean|.  hb (B,32,
+    sH,sW) float64 on the computation's device, x (B,3,h,w) and sd anywhere."""
+    dev = hb.device
+
+    def d(t):
+        return t.to(dev, torch.float64)
+
+    R = sb.Restatement()
+    conv = F.conv2d(hb.abs(), R.rb(d(sd["conv_out.0.weight"])).abs(), d(sd["conv_out.0.bias"]).abs(), padding=1)
+    xs = (d(x) + d(sd["sub_mean.bias"]).view(1, 3, 1, 1)).abs()
+    skip = F.interpolate(xs, scale_factor=scale, mode="bilinear", align_corners=False)
+    return conv + skip + d(sd["add_mean.bias"]).abs().view(1, 3, 1, 1)
+
+
+# ---- the bound plan, one layer range at a time ------------------------------------------------------------------------
+def plan_buffer(ent, id, index, shape, dtype):
+    """A typed view of activation buffer `id` (BUF_*, `index` of LR / HR) in the workspace of a plan entry of
+    SRProjectionModule (ent["plan"], ent["workspace"]); its size must be exactly the shape's."""
+    off, n = ctypes.c_size_t(), ctypes.c_size_t()
+    _lib.check(_lib.lib().vsr_srfbn_debug_buffer(ent["plan"], id, index, ctypes.byref(off), ctypes.byref(n)),
+               f"srfbn_debug_buffer({id}, {index})")
+    elems = 1
+    for s in shape:
+        elems *= s
+    itemsize = torch.empty((), dtype=dtype).element_size()
+    assert n.value == elems * itemsize, (id, index, n.value, shape, dtype)
+    return ent["workspace"][off.value:off.value + n.value].view(dtype).view(shape)
+
+
+def run_layers(ent, x, first, count):
+    """Layers [first, first + count) of the bound plan over its first chunk of the maps x (vsr_srfbn_debug_run_layers),
+    on the current stream."""
+    _lib.check(_lib.lib().vsr_srfbn_debug_run_layers(ent["plan"], x.data_ptr(), int(first), int(count),
+                                                     torch.cuda.current_stream().cuda_stream),
+               f"srfbn_debug_run_layers({first}, {count})")

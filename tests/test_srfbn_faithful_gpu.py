@@ -73,15 +73,6 @@ def _conv_out_operands(B, h, w, scale, seed):
     return hb, x, sd
 
 
-def _conv_out_abs(hb, x, sd, scale):
-    """sum of |terms| of one conv_out output: the conv's |w * x|, |bias|, the skip's |taps| and |add_mean|."""
-    R = sb.Restatement()
-    conv = F.conv2d(hb.abs(), R.rb(_d(sd["conv_out.0.weight"])).abs(), _d(sd["conv_out.0.bias"]).abs(), padding=1)
-    xs = (_d(x) + _d(sd["sub_mean.bias"]).view(1, 3, 1, 1)).abs()
-    skip = F.interpolate(xs, scale_factor=scale, mode="bilinear", align_corners=False)
-    return conv + skip + _d(sd["add_mean.bias"]).abs().view(1, 3, 1, 1)
-
-
 @pytest.mark.parametrize("B,h,w,scale", _CONV_OUT_CASES)
 def test_conv_out_against_fp64(B, h, w, scale):
     """conv_out's fp32 output against float64 on the same BF16 operands: |got - want| <= 16 * 2^-24 * sum |terms| per
@@ -92,7 +83,7 @@ def test_conv_out_against_fp64(B, h, w, scale):
     assert torch.isfinite(got).all()
     hbd = _d(hb).permute(0, 3, 1, 2)
     want = sb.Restatement().conv_out(hbd, _d(x), sd, scale)
-    tol = 16 * 2.0 ** -24 * _conv_out_abs(hbd, x, sd, scale)
+    tol = 16 * 2.0 ** -24 * hk.conv_out_abs(hbd, x, sd, scale)
     err = (got - want).abs()
     bad = (err > tol).nonzero()
     assert bad.numel() == 0, f"{bad.shape[0]} pixels outside, first (b,c,y,x) {[tuple(i.tolist()) for i in bad[:6]]}"
@@ -328,7 +319,7 @@ def test_bounds_reject_a_perturbed_restatement(kind, scale):
         got_l = hk.conv_out(hb.to(DEV), xl.to(DEV), scale, lsd["conv_out.0.weight"], lsd["conv_out.0.bias"],
                             lsd["sub_mean.bias"], lsd["add_mean.bias"]).double()
         hbd = _d(hb).permute(0, 3, 1, 2)
-        tol = 16 * 2.0 ** -24 * _conv_out_abs(hbd, xl, lsd, scale)
+        tol = 16 * 2.0 ** -24 * hk.conv_out_abs(hbd, xl, lsd, scale)
         assert ((got_l - sb.Restatement().conv_out(hbd, _d(xl), ysd, scale)).abs() > tol).any()
     else:                                 # one layer at slope -0.2 against the restatement with the fp32 slope
         g = torch.Generator().manual_seed(scale)

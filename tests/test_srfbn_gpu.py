@@ -13,7 +13,6 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from oracle import srfbn_bf16 as sb
 from oracle import srfbn_oracle as so
 from tests import srfbn_hooks as hk
 from video_super_resolution_b200.my_packages.SRProjection.SRProjectionModule import SRProjectionModule
@@ -32,22 +31,6 @@ def _bf(t):
 # rounds once more before the strided conv.
 _MAX_DIFF_FRAC = 0.002
 _MAX_DIFF_FRAC_FUSED = 0.025
-
-
-def _act(pre, slope, packed=True):
-    """Expected BF16 layer output from the float64 pre-activation acc + bias: bf16 then the packed-BF16 PReLU of
-    igemm.cuh, or (packed=False, the x4 strided conv of fused_down.cuh) the fp32 PReLU with the fp32 slope, rounded
-    once."""
-    s32 = float(torch.tensor(slope, dtype=torch.float32))
-    if packed:
-        return sb.prelu_packed(sb.round_bf16(pre), s32, float(sb.round_bf16(torch.tensor(s32))))
-    return sb.round_bf16(torch.where(pre >= 0, pre, pre * s32))
-
-
-def _ulps(want, packed=True):
-    """Output ulps a one-ulp difference of the rounded pre-activation can become: two on the negative side of the
-    packed PReLU (bf16(s_b * x_b) rounds a second time), one elsewhere."""
-    return torch.where(want < 0, 2.0, 1.0) if packed else 1.0
 
 
 def _d(t):
@@ -74,9 +57,9 @@ def test_pointwise_layer(rows, K):
     want = F.prelu(x.float() @ w.t() + b, torch.tensor([0.2]))
     _close(got, want, f"pointwise rows={rows} K={K}")
     pre, absdot = _d(x) @ _d(w).t() + _d(b), _d(x).abs() @ _d(w).abs().t() + _d(b).abs()
-    want = _act(pre, 0.2)
+    want = hk.act(pre, 0.2)
     hk.faithful_bf16(got, want, absdot, f"pointwise rows={rows} K={K} faithful", max_frac=_MAX_DIFF_FRAC,
-                     ulps=_ulps(want))
+                     ulps=hk.ulps(want))
 
 
 @pytest.mark.parametrize("slope", [0.0, 1.0, 1.7, -0.3])
@@ -90,9 +73,9 @@ def test_pointwise_prelu_slope_forms(slope):
     want = F.prelu(x.float() @ w.t() + b, torch.tensor([slope]))
     _close(got, want, f"pointwise slope={slope}")
     pre, absdot = _d(x) @ _d(w).t() + _d(b), _d(x).abs() @ _d(w).abs().t() + _d(b).abs()
-    want = _act(pre, slope)
+    want = hk.act(pre, slope)
     hk.faithful_bf16(got, want, absdot, f"pointwise slope={slope} faithful", max_frac=_MAX_DIFF_FRAC,
-                     ulps=_ulps(want))
+                     ulps=hk.ulps(want))
 
 
 @pytest.mark.parametrize("B,h,w", [(1, 8, 16), (2, 5, 7), (1, 19, 33)])
@@ -115,9 +98,9 @@ def test_deconv_layer(B, h, w, block):
     xc = _d(x).permute(0, 3, 1, 2)
     pre = F.conv_transpose2d(xc, _d(wt), _d(b), stride=4, padding=2).permute(0, 2, 3, 1)
     absdot = F.conv_transpose2d(xc.abs(), _d(wt).abs(), _d(b).abs(), stride=4, padding=2).permute(0, 2, 3, 1)
-    want = _act(pre, 0.25)
+    want = hk.act(pre, 0.25)
     hk.faithful_bf16(got, want, absdot, f"deconv B={B} {h}x{w} block={block} faithful", max_frac=_MAX_DIFF_FRAC,
-                     ulps=_ulps(want))
+                     ulps=hk.ulps(want))
 
 
 @pytest.mark.parametrize("nsrc,B,h,w", [(1, 1, 8, 16), (2, 2, 5, 7), (3, 1, 19, 33), (6, 1, 9, 17)])
@@ -133,7 +116,7 @@ def test_fused_downtran_downconv(nsrc, B, h, w):
     got = hk.fused_down(hrb.to(DEV), wt, bt, 0.3, wd, bd, 0.15)
     want = _down_reference([hr[j].float() for j in range(nsrc)], wt, bt, 0.3, wd, bd, 0.15)
     _close(got, want, f"fused_down nsrc={nsrc} B={B} {h}x{w}")
-    want, absdot, extra = _down_faithful([(_d(hr[j]), None) for j in range(nsrc)], wt, bt, 0.3, wd, bd, 0.15)
+    want, absdot, extra = hk.down_faithful([(_d(hr[j]), None) for j in range(nsrc)], wt, bt, 0.3, wd, bd, 0.15)
     hk.faithful_bf16(got, want, absdot, f"fused_down nsrc={nsrc} B={B} {h}x{w} faithful", max_frac=_MAX_DIFF_FRAC_FUSED,
                      extra=extra)
 
@@ -146,45 +129,6 @@ def _down_reference(srcs, wt, bt, slope_t, wd, bd, slope_d):
         x = F.prelu(F.conv2d(x, wt.view(32, 32 * len(srcs), 1, 1), bt), torch.tensor([slope_t]))
         x = _bf(x).float()
     return F.prelu(F.conv2d(x, wd, bd, stride=4, padding=2), torch.tensor([slope_d])).permute(0, 2, 3, 1)
-
-
-def _down_faithful(srcs, wt, bt, slope_t, wd, bd, slope_d):
-    """The HR half of a feedback group in float64 with the kernels' rounding points (oracle/srfbn_bf16.py): srcs = nsrc
-    pairs (map (B,4h,4w,32) of BF16 values, its own sum |w * x| or None) -> (want (B,h,w,32), sum |w * x| through both
-    layers, extra tolerance).  H = packed-PReLU(bf16(downtran)) for nsrc > 1; lr = bf16(fp32-PReLU(conv)).  The
-    accumulation error of H reaches the output through |wd|, so H's sum |w * x| is carried into the conv's.  H is
-    rounded on chip: where its fp32 sum lies next to a BF16 rounding boundary, an element of H (or, in the merged
-    kernel, of U before it) rounds the other way, and that one element moves the output by up to 2 ulp(H) * |wd| --
-    measured on a B200 at 1 to 8 outputs in a million, 2 to 7 output ulps each.  The extra tolerance allows two such
-    elements in each output's 8x8 window."""
-    x = torch.cat([m.permute(0, 3, 1, 2) for m, _ in srcs], dim=1)
-    ax = torch.cat([(a if a is not None else torch.zeros_like(m)).permute(0, 3, 1, 2) for m, a in srcs], dim=1)
-    if len(srcs) > 1:
-        w1 = _d(wt).view(32, 32 * len(srcs), 1, 1)
-        pre = F.conv2d(x, w1, _d(bt))
-        ax = F.conv2d(x.abs() + ax, w1.abs(), _d(bt).abs())
-        x = _act(pre, slope_t)
-    pre = F.conv2d(x, _d(wd), _d(bd), stride=4, padding=2)
-    absdot = F.conv2d(x.abs() + ax, _d(wd).abs(), _d(bd).abs(), stride=4, padding=2)
-    extra = torch.zeros_like(pre)
-    if len(srcs) > 1:
-        ulp_h = torch.exp2(torch.floor(torch.log2(x.abs().amax(dim=1, keepdim=True).clamp_min(2.0 ** -126))) - 7)
-        win = F.max_pool2d(F.pad(ulp_h, (2, 2, 2, 2)), 8, stride=4)          # the window of each output pixel
-        extra = 2 * 2 * win * _d(wd).abs().amax(dim=(1, 2, 3)).view(1, 32, 1, 1)
-    return (_act(pre, slope_d, packed=False).permute(0, 2, 3, 1), absdot.permute(0, 2, 3, 1),
-            extra.permute(0, 2, 3, 1))
-
-
-def _bits_equal(got, want, what, dims="b,y,x,c"):
-    """Raw-bit equality of two BF16 tensors (-0 and +0 differ); on failure names the first differing elements."""
-    a, b = got.view(torch.int16), want.view(torch.int16)
-    if torch.equal(a, b):
-        return
-    idx = (a != b).nonzero().cpu()
-    first = [tuple(i.tolist()) for i in idx[:8]]
-    pairs = [(got[i].item(), want[i].item()) for i in first]
-    raise AssertionError(f"{what}: {idx.shape[0]}/{a.numel()} elements differ; first ({dims}) got/want: "
-                         + ", ".join(f"{i}: {g}/{w}" for i, (g, w) in zip(first, pairs)))
 
 
 def _group_operands(nsrc, B, h, w, seed):
@@ -217,10 +161,10 @@ def _check_fused_updown(nsrc, store, B, h, w, slope_u, seed):
 
     y, hr_after = hk.fused_updown(lr_d, hr, store, wu, bu, slope_u, wt, bt, slope_t, wd, bd, slope_d)
     # y of the merged kernel is the layered pair's, bit for bit (LR tile: 16 x 8 blocks -> tile (x // 16, y // 8))
-    _bits_equal(y, want_y, f"fused_updown y vs layered pair, {where}")
+    hk.bits_equal(y, want_y, f"fused_updown y vs layered pair, {where}")
     if store:   # the stored hr map is the standalone transposed conv's, zero ring included
-        _bits_equal(hr_after[nsrc - 1], u_blk, f"fused_updown hr[{nsrc - 1}] vs transposed conv, {where}",
-                    dims="b,pair,Yb,Xb,el")
+        hk.bits_equal(hr_after[nsrc - 1], u_blk, f"fused_updown hr[{nsrc - 1}] vs transposed conv, {where}",
+                      dims="b,pair,Yb,Xb,el")
     else:       # the merged kernel keeps U on chip and leaves the slot alone
         assert bool((hr_after[nsrc - 1].view(torch.int16) == hk.SENTINEL_BITS).all()), \
             f"fused_updown wrote hr[{nsrc - 1}] with store=0, {where}"
@@ -233,8 +177,8 @@ def _check_fused_updown(nsrc, store, B, h, w, slope_u, seed):
     lc = _d(lr).permute(0, 3, 1, 2)
     pre_u = F.conv_transpose2d(lc, _d(wu), _d(bu), stride=4, padding=2).permute(0, 2, 3, 1)
     abs_u = F.conv_transpose2d(lc.abs(), _d(wu).abs(), _d(bu).abs(), stride=4, padding=2).permute(0, 2, 3, 1)
-    want, absdot, extra = _down_faithful([(_d(prev[j]), None) for j in range(nsrc - 1)]
-                                         + [(_act(pre_u, slope_u), abs_u)], wt, bt, slope_t, wd, bd, slope_d)
+    want, absdot, extra = hk.down_faithful([(_d(prev[j]), None) for j in range(nsrc - 1)]
+                                           + [(hk.act(pre_u, slope_u), abs_u)], wt, bt, slope_t, wd, bd, slope_d)
     hk.faithful_bf16(y, want, absdot, f"fused_updown faithful, {where}", max_frac=_MAX_DIFF_FRAC_FUSED,
                      extra=extra)
 
@@ -281,9 +225,9 @@ def test_x2_transposed_conv_layer(B, h, w):
     xc = _d(x).permute(0, 3, 1, 2)
     pre = F.conv_transpose2d(xc, _d(wt), _d(b), stride=2, padding=2).permute(0, 2, 3, 1)
     absdot = F.conv_transpose2d(xc.abs(), _d(wt).abs(), _d(b).abs(), stride=2, padding=2).permute(0, 2, 3, 1)
-    want = _act(pre, 0.25)
+    want = hk.act(pre, 0.25)
     hk.faithful_bf16(got, want, absdot, f"deconv2 B={B} {h}x{w} faithful", max_frac=_MAX_DIFF_FRAC,
-                     ulps=_ulps(want))
+                     ulps=hk.ulps(want))
 
 
 @pytest.mark.parametrize("B,h,w", [(1, 8, 16), (2, 5, 7), (1, 19, 33), (1, 9, 14), (1, 9, 15), (1, 17, 28), (1, 17, 29),
@@ -302,9 +246,9 @@ def test_x2_strided_conv_layer(B, h, w):
     xc = _d(x).permute(0, 3, 1, 2)
     pre = F.conv2d(xc, _d(wd), _d(b), stride=2, padding=2).permute(0, 2, 3, 1)
     absdot = F.conv2d(xc.abs(), _d(wd).abs(), _d(b).abs(), stride=2, padding=2).permute(0, 2, 3, 1)
-    want = _act(pre, 0.15)
+    want = hk.act(pre, 0.15)
     hk.faithful_bf16(got, want, absdot, f"downconv2 B={B} {h}x{w} faithful", max_frac=_MAX_DIFF_FRAC,
-                     ulps=_ulps(want))
+                     ulps=hk.ulps(want))
 
 
 def _psnr(a, b):

@@ -102,6 +102,8 @@ SIGNATURES = {
     "vsr_srfbn_profile_read": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "vsr_srfbn_profile_launches": (c_int, [c_void_p, c_void_p, c_void_p, c_int]),
     "vsr_srfbn_debug_premix": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "vsr_srfbn_debug_run_layers": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "vsr_srfbn_debug_buffer": (c_int, [c_void_p, c_int, c_int, ctypes.POINTER(c_size_t), ctypes.POINTER(c_size_t)]),
     "vsr_test_pointwise": (c_int, [c_void_p, c_i64, c_int, c_void_p, c_void_p, c_float, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "vsr_test_deconv": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "vsr_test_fused_down": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_float, c_void_p, c_void_p,

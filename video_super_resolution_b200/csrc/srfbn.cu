@@ -930,32 +930,45 @@ static int swept_maps(const vsr_srfbn_plan* pl) { return pl->windows * (pl->map1
 // the plan's range is all maps (no map range set): the only kind of plan that fuses whole frames or has several windows
 static bool all_maps(const vsr_srfbn_plan* pl) { return pl->map1 - pl->map0 == pl->cfg.num_maps; }
 
+// Bytes of activation buffer `id` (VSR_SRFBN_BUF_*; `index` of LR / HR) with the layers over `chunk` maps at a time and
+// the per-map images of `swept` maps; 0: the plan has no such buffer.
+static size_t buffer_bytes(const vsr_srfbn_config& c, int chunk, int swept, int id, int index) {
+  const size_t P = (size_t)chunk * c.h * c.w;
+  const size_t s2 = (size_t)c.upscale * c.upscale;
+  const bool x2 = c.upscale == 2;
+  switch (id) {
+    case VSR_SRFBN_BUF_C128: return P * 256;
+    // x2: plain NHWC.  x4: hr[5] exists only when its group runs layered (the merged kernel keeps it on chip)
+    case VSR_SRFBN_BUF_HR:
+      return x2 ? P * s2 * 64 : (index == 5 && updown_merged(6)) ? 0 : (size_t)chunk * (c.h + 1) * (c.w + 1) * 16 * 64;
+    case VSR_SRFBN_BUF_HB: return P * s2 * 64;             // plain-NHWC result of the `out` deconv
+    case VSR_SRFBN_BUF_HT: return x2 ? P * s2 * 64 : 0;    // x2: downtran result (the x4 path keeps it on chip)
+    case VSR_SRFBN_BUF_ACC: return x2 ? 0 : P * 512;       // fp32 partial slots of the fused down kernel
+    case VSR_SRFBN_BUF_PREMIX: return (size_t)swept * c.h * c.w * s2 * 3 * 4;
+    default: return P * 64;                                // A0, XFEAT, HIDDEN, LR, U
+  }
+}
+
 // Activations are laid out for `chunk` maps at a time (the maps are independent until the fc fuse, so the layer list is
 // swept once per chunk); only the per-map SR images in front of the fc fuse exist for all `swept` maps.
 static void layout_workspace(vsr_srfbn_plan* pl, int chunk, int swept) {
-  const vsr_srfbn_config& c = pl->cfg;
-  const size_t P = (size_t)chunk * c.h * c.w;
-  const size_t Rb = (size_t)chunk * (c.h + 1) * (c.w + 1) * 16;
   size_t off = 0;
-  auto put = [&](size_t bytes) {
+  auto put = [&](int id, int index) {
     size_t o = off;
-    off = align_up(off + bytes, 1024);
+    off = align_up(off + buffer_bytes(pl->cfg, chunk, swept, id, index), 1024);
     return o;
   };
-  pl->o_a0 = put(P * 64);
-  pl->o_c128 = put(P * 256);
-  pl->o_xfeat = put(P * 64);
-  pl->o_hidden = put(P * 64);
-  for (int i = 0; i < 7; ++i) pl->o_lr[i] = put(P * 64);
-  pl->o_u = put(P * 64);
-  const size_t s2 = (size_t)c.upscale * c.upscale;
-  const bool x2 = c.upscale == 2;
-  // x2: plain NHWC.  x4: hr[5] exists only when its group runs layered (the merged kernel keeps it on chip)
-  for (int i = 0; i < 6; ++i) pl->o_hr[i] = put(x2 ? P * s2 * 64 : (i == 5 && updown_merged(6)) ? 0 : Rb * 64);
-  pl->o_hb = put(P * s2 * 64);   // plain-NHWC result of the `out` deconv
-  pl->o_ht = put(x2 ? P * s2 * 64 : 0);   // x2: downtran result (the x4 path keeps it on chip)
-  pl->o_acc = put(x2 ? 0 : P * 512);   // fp32 partial slots of the fused down kernel
-  pl->o_premix = put((size_t)swept * c.h * c.w * s2 * 3 * 4);
+  pl->o_a0 = put(VSR_SRFBN_BUF_A0, 0);
+  pl->o_c128 = put(VSR_SRFBN_BUF_C128, 0);
+  pl->o_xfeat = put(VSR_SRFBN_BUF_XFEAT, 0);
+  pl->o_hidden = put(VSR_SRFBN_BUF_HIDDEN, 0);
+  for (int i = 0; i < 7; ++i) pl->o_lr[i] = put(VSR_SRFBN_BUF_LR, i);
+  pl->o_u = put(VSR_SRFBN_BUF_U, 0);
+  for (int i = 0; i < 6; ++i) pl->o_hr[i] = put(VSR_SRFBN_BUF_HR, i);
+  pl->o_hb = put(VSR_SRFBN_BUF_HB, 0);
+  pl->o_ht = put(VSR_SRFBN_BUF_HT, 0);
+  pl->o_acc = put(VSR_SRFBN_BUF_ACC, 0);
+  pl->o_premix = put(VSR_SRFBN_BUF_PREMIX, 0);
   pl->ws_bytes = off;
 }
 
@@ -1242,17 +1255,18 @@ extern "C" int vsr_srfbn_forward(vsr_srfbn_plan* pl, const float* x, float* y, v
   return vsr_srfbn_forward_u8(pl, x, y, nullptr, stream);
 }
 
-// One sweep of a layer list over the maps [m0, m0 + Mc) of the stack x; the per-map image of map m lands in premix slot
-// m - map0 (several windows imply map0 == 0, so window b's map m lands in slot b*M + m).
-static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_out_layer, const float* x, int m0, int Mc,
-                      cudaStream_t st, size_t* ev) {
+// The layers [first, first + count) of a layer list over the maps [m0, m0 + Mc) of the stack x, preceded by their im2col
+// when first == 0; the per-map image of map m lands in premix slot m - map0 (several windows imply map0 == 0, so window
+// b's map m lands in slot b*M + m).  A sweep is the whole list; vsr_srfbn_debug_run_layers runs any range of it.
+static int run_layers(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_out_layer, const float* x, int m0, int Mc,
+                      int first, int count, cudaStream_t st, size_t* ev) {
   const vsr_srfbn_config& c = pl->cfg;
   auto mark = [&]() {
     if (ev && pl->profile && *ev < pl->events.size()) cudaEventRecord(pl->events[(*ev)++], st);
   };
   const float* xc = x + (int64_t)m0 * 3 * c.h * c.w;
-  mark();
-  {
+  if (first == 0) {
+    mark();
     int rc = launch_im2col(xc, reinterpret_cast<const float*>(pl->dev_w + pl->misc_off), pl->ws + pl->o_a0, Mc, c.h,
                            c.w, st);
     if (rc) return rc;
@@ -1262,12 +1276,18 @@ static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_o
     cp.skip_src = xc;
     cp.out = reinterpret_cast<float*>(pl->ws + pl->o_premix) + (int64_t)(m0 - pl->map0) * 3 * c.upscale * c.upscale * c.h * c.w;
   }
-  for (const Layer& L : layers) {
+  for (int i = first; i < first + count; ++i) {
     mark();
-    int rc = launch_layer(L, st);
+    int rc = launch_layer(layers[i], st);
     if (rc) return rc;
   }
   return VSR_OK;
+}
+
+// One sweep of a layer list over the maps [m0, m0 + Mc) of the stack x.
+static int sweep_maps(vsr_srfbn_plan* pl, std::vector<Layer>& layers, int conv_out_layer, const float* x, int m0, int Mc,
+                      cudaStream_t st, size_t* ev) {
+  return run_layers(pl, layers, conv_out_layer, x, m0, Mc, 0, (int)layers.size(), st, ev);
 }
 
 // The full forward's sweeps: the plan's maps [map0, map0 + swept_maps) in chunks of chunk_maps.
@@ -1506,6 +1526,28 @@ extern "C" int vsr_srfbn_debug_premix(const vsr_srfbn_plan* pl, float* out_maps,
   const vsr_srfbn_config& c = pl->cfg;
   size_t bytes = (size_t)swept_maps(pl) * 3 * c.upscale * c.upscale * c.h * c.w * 4;
   return cuda_status(cudaMemcpyAsync(out_maps, pl->ws + pl->o_premix, bytes, cudaMemcpyDeviceToDevice, as_stream(stream)));
+}
+
+extern "C" int vsr_srfbn_debug_run_layers(vsr_srfbn_plan* pl, const float* x, int first, int count, vsr_stream_t stream) {
+  if (!pl || !x) return VSR_ERR_INVALID_ARG;
+  if (!pl->bound) return VSR_ERR_STATE;
+  const int n = (int)pl->layers.size();
+  if (first < 0 || count < 1 || first >= n || count > n - first) return VSR_ERR_INVALID_ARG;
+  return run_layers(pl, pl->layers, pl->conv_out_layer, x, pl->map0, pl->chunk_maps, first, count, as_stream(stream),
+                    nullptr);
+}
+
+extern "C" int vsr_srfbn_debug_buffer(const vsr_srfbn_plan* pl, int id, int index, size_t* offset, size_t* bytes) {
+  if (!pl || !offset || !bytes || id < 0 || id >= VSR_SRFBN_BUFFERS) return VSR_ERR_INVALID_ARG;
+  const int n = id == VSR_SRFBN_BUF_LR ? 7 : id == VSR_SRFBN_BUF_HR ? 6 : 1;
+  if (index < 0 || index >= n) return VSR_ERR_INVALID_ARG;
+  const size_t b = buffer_bytes(pl->cfg, pl->chunk_maps, swept_maps(pl), id, index);
+  if (b == 0) return VSR_ERR_UNSUPPORTED;
+  const size_t off[VSR_SRFBN_BUFFERS] = {pl->o_a0, pl->o_c128, pl->o_xfeat, pl->o_hidden, pl->o_lr[index % 7], pl->o_u,
+                                         pl->o_hr[index % 6], pl->o_hb, pl->o_ht, pl->o_acc, pl->o_premix};
+  *offset = off[id];
+  *bytes = b;
+  return VSR_OK;
 }
 
 // ------------------------------------------------------------------------------------------------
