@@ -1,16 +1,108 @@
 """Python front-ends of the single-layer test hooks of the C ABI (vsr_test_*), the plan walk hooks
-(vsr_srfbn_debug_run_layers / vsr_srfbn_debug_buffer), the HR block layout helpers and the float64 expectations the
-layer tests share.  Test support only."""
+(vsr_srfbn_debug_run_layers / vsr_srfbn_debug_buffer), the HR block layout helpers, the float64 expectations the
+layer tests share, and the full-size cases, state dict and per-region error measures of the whole-stack tests.  Test
+support only."""
 import ctypes
 
 import torch
 import torch.nn.functional as F
 
 from oracle import srfbn_bf16 as sb
+from oracle import srfbn_oracle as so
 from video_super_resolution_b200 import _lib
 
 # activation buffer ids of vsr_srfbn_debug_buffer (include/vsr_b200.h VSR_SRFBN_BUF_*)
 BUF_A0, BUF_C128, BUF_XFEAT, BUF_HIDDEN, BUF_LR, BUF_U, BUF_HR, BUF_HB, BUF_HT, BUF_ACC, BUF_PREMIX = range(11)
+
+# The full-size plans of test_srfbn_faithful_gpu.py::test_full_size_maps_against_restatement and
+# test_fullsize_gpu.py::test_full_size_windows_bit_identical: name -> (M, h, w, scale, windows, workspace cap in bytes or
+# None).  tests/test_srfbn_plan_buffers_cpu.py checks that each still reaches the size it exists for.
+FULL_SIZE_PLANS = {
+    "C2": (20, 270, 480, 4, 1, None),                 # bench C2: the HR ring over 2^31 bytes
+    "C5": (8, 360, 720, 4, 1, None),                  # bench C5: every map restated, so the fused frame is too
+    "C4": (14, 1080, 1920, 2, 1, None),               # bench C4, uncapped: buffers over 2^31 BF16 elements
+    "C5-W3": (8, 360, 720, 4, 3, None),               # 24 maps in one chunk: the HR ring over 2^32 bytes
+    "C5-W3-capped": (8, 360, 720, 4, 3, 14 << 30),    # chunks of 6 maps that straddle the window boundaries
+    "C2-W2": (20, 270, 480, 4, 2, None),              # 40 maps in one chunk: the HR ring over 2^32 bytes
+}
+
+
+def stack_state(M, h, scale):
+    """The state dict of test_full_stack_against_oracle with distinct slopes, plus one layer at slope 1.3 and one at
+    -0.2, so the stack runs all three packed-PReLU forms (and the fp32 PReLU of the x4 strided convs)."""
+    sd = so.init_state_dict(num_maps=M, seed=M + h, gain=2.3, upscale=scale)
+    gs = torch.Generator().manual_seed(99)
+    for k in sd:
+        if k.endswith(".1.weight"):
+            sd[k] = torch.rand(1, generator=gs) * 0.4 + 0.05
+    sd["block.upBlocks.2.1.weight"] = torch.tensor([1.3])
+    sd["block.compress_in.1.weight"] = torch.tensor([-0.2])
+    sd["fc.2.weight"] = sd["fc.2.weight"].abs()          # a fused frame the final ReLU does not zero
+    return sd
+
+
+def fc_fuse_bound(maps, sd):
+    """Per-element error bound of the fused frame against an fp64 fc (sb.fc_fuse) over the same per-map images maps
+    (M,3,H,W): twice the error bound of the kernel's fp32 FMA chains (hid_j: M + 1 terms, o: 33 terms), on the maps'
+    device, (1,3,H,W) float64.  Elementwise, so it may be taken over any slice of the channels, rows or columns."""
+    dev, M = maps.device, maps.shape[0]
+
+    def d(t):
+        return t.to(dev, torch.float64)
+
+    w0, b0, w2, b2 = (d(sd[k]) for k in ("fc.0.weight", "fc.0.bias", "fc.2.weight", "fc.2.bias"))
+    t = maps.double().permute(1, 2, 3, 0)
+    hid = F.relu(F.linear(t, w0, b0))
+    u = 2.0 ** -24
+    bound = 33 * u * F.linear(hid, w2.abs(), b2.abs())
+    del hid
+    bound += F.linear((M + 1) * u * F.linear(t.abs(), w0.abs(), b0.abs()), w2.abs())
+    return 2 * bound.permute(3, 0, 1, 2) + 1e-30
+
+
+# ---- per-region errors of whole maps ------------------------------------------------------------------------------
+def regions(H, W, scale):
+    """The regions region_errors reports on an H x W HR map, as (name, y0, y1, x0, x1) in HR pixels: the outermost
+    2 * scale HR rows and columns on each side as four bands (the (h+1) x (w+1) block ring and the ragged last tiles
+    meet there), then a grid of tiles over 32 x 32 LR blocks (ragged at the bottom and right), named in LR pixels."""
+    e, t = 2 * scale, 32 * scale
+    out = [("top band", 0, e, 0, W), ("bottom band", H - e, H, 0, W), ("left band", 0, H, 0, e),
+           ("right band", 0, H, W - e, W)]
+    for y0 in range(0, H, t):
+        for x0 in range(0, W, t):
+            y1, x1 = min(y0 + t, H), min(x0 + t, W)
+            out.append((f"tile LR y {y0 // scale}:{y1 // scale} x {x0 // scale}:{x1 // scale}", y0, y1, x0, x1))
+    return out
+
+
+def region_errors(got, want, scale):
+    """Per-map, per-region max-abs and RMS of got - want, maps (n,3,H,W) on any devices (computed in float64 on got's):
+    -> (regions(H, W, scale), max (n, R), RMS (n, R)), the two on the CPU."""
+    err = got.double() - want.to(got.device, torch.float64)
+    n, _, H, W = err.shape
+    regs = regions(H, W, scale)
+    t = 32 * scale
+    ty, tx = -(-H // t), -(-W // t)
+    pad = (0, tx * t - W, 0, ty * t - H)
+    mx, ss, cnt = [], [], []
+    for _, y0, y1, x0, x1 in regs[:4]:
+        band = err[:, :, y0:y1, x0:x1]
+        mx.append(band.abs().amax(dim=(1, 2, 3)))
+        ss.append(band.square().sum(dim=(1, 2, 3)))
+    tiles = F.pad(err, pad).view(n, 3, ty, t, tx, t)
+    mx = torch.cat([torch.stack(mx, 1), tiles.abs().amax(dim=(1, 3, 5)).flatten(1)], 1)
+    ss = torch.cat([torch.stack(ss, 1), tiles.square().sum(dim=(1, 3, 5)).flatten(1)], 1)
+    cnt = torch.tensor([3.0 * (y1 - y0) * (x1 - x0) for _, y0, y1, x0, x1 in regs], dtype=torch.float64,
+                       device=err.device)
+    return regs, mx.cpu(), (ss / cnt).sqrt().cpu()
+
+
+def region_failures(regs, mx, rms, b_max, b_rms, maps):
+    """One line per (map, region) of region_errors whose max-abs exceeds b_max or whose RMS exceeds b_rms; maps names
+    the rows of mx and rms."""
+    bad = ((mx > b_max) | (rms > b_rms)).nonzero().tolist()
+    return [f"map {maps[i]} {regs[r][0]}: max {mx[i, r].item():.4g} (bound {b_max}) rms {rms[i, r].item():.4g} "
+            f"(bound {b_rms})" for i, r in bad]
 
 
 def _fp(t):

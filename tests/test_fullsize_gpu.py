@@ -5,6 +5,7 @@ import pytest
 import torch
 
 from oracle import oracle as orc
+from tests import srfbn_hooks as hk
 from video_super_resolution_b200 import ops, synthetic as syn
 from video_super_resolution_b200.my_packages.SRProjection.SRProjectionModule import SRProjectionModule
 from video_super_resolution_b200.network.video_super_resolution import VSR
@@ -242,6 +243,41 @@ def test_c4_2x_4k_conv_stack_full_size_is_deterministic_and_tiling_consistent():
     del cap, fresh, y1, y3, x
     gc.collect()
     torch.cuda.empty_cache()
+
+
+@pytest.mark.parametrize("name", ["C5-W3", "C5-W3-capped", "C2-W2"])
+def test_full_size_windows_bit_identical(name):
+    """W frame windows in one forward of the window-batched plan, at full size, against W one-window forwards of the
+    same module: the fp32 frames, the u8 frames and all W * M per-map images are bit-identical.  Uncapped, C5 W = 3
+    and C2 W = 2 sweep 24 and 40 maps in one chunk (HR ring over 2^32 bytes); under the cap, C5 W = 3 sweeps chunks of
+    6 maps, two of which straddle a window boundary."""
+    import gc
+    M, h, w, s, W, cap = hk.FULL_SIZE_PLANS[name]
+    gc.collect()
+    torch.cuda.empty_cache()
+    mod = SRProjectionModule(num_maps=M, upscale_factor=s, workspace_cap_bytes=cap)
+    try:
+        mod.load_state_dict(hk.stack_state(M, h, s))
+        x = (torch.rand((W, M, 3, h, w), generator=torch.Generator().manual_seed(W)) * 255).to(DEV)
+        u8 = torch.empty((W, s * h, s * w, 3), dtype=torch.uint8, device=DEV)
+        pre = mod.premix(x)
+        y = mod(x, out_u8=u8)
+        chunk = mod._plans[(M, h, w, 0, W)]["chunk_maps"]
+        assert chunk == (W * M if cap is None else 6), chunk
+        if cap is not None:
+            assert chunk % M and M % chunk, chunk                # a chunk straddles the windows
+        assert y.shape == (W, 3, s * h, s * w) and torch.isfinite(y).all() and y.mean().item() > 1.0
+        for b in range(W):
+            u1 = torch.empty((s * h, s * w, 3), dtype=torch.uint8, device=DEV)
+            pre1 = mod.premix(x[b])
+            y1 = mod(x[b], out_u8=u1)
+            assert torch.equal(pre[b * M:(b + 1) * M], pre1), (name, b, "premix")
+            assert torch.equal(y[b:b + 1], y1), (name, b, "fp32 frame")
+            assert torch.equal(u8[b], u1), (name, b, "u8 frame")
+    finally:
+        del mod                                   # both plans' workspaces: 65 GB at C5 W = 3
+        gc.collect()
+        torch.cuda.empty_cache()
 
 
 def test_unsupported_geometry_is_rejected_loudly():

@@ -9,7 +9,11 @@ feedback steps carry these flips on.  Measured on a B200, the per-map difference
 times smaller than to the fp32 oracle (e.g. C2 maps: max 0.108, RMS 0.0145 on the 0..255 scale).  The whole-stack
 bounds below are still set per case at about 4x the measured values -- an order of magnitude under the fp32 criteria
 of test_srfbn_gpu.py -- and reject a border or padding error of the conv_in / skip kind; errors as small as one
-conv_out tap off by 1 % or one PReLU slope left unrounded are rejected by the single-layer checks instead."""
+conv_out tap off by 1 % or one PReLU slope left unrounded are rejected by the single-layer checks instead.
+
+At the benchmark's sizes a whole-map max and RMS cannot see an error confined to a few rows or one corner of a map,
+so there every region of a map -- its border bands and its tiles of 32 x 32 LR blocks -- is held to a bound too."""
+import gc
 import math
 import time
 
@@ -104,15 +108,8 @@ def test_fc_fuse_teacher_forced(M):
     x = (torch.rand((M, 3, h, w), generator=torch.Generator().manual_seed(M + 1)) * 255).to(DEV)
     maps = mod.premix(x).double()
     got = mod(x).double()
-    w0, b0 = _d(sd["fc.0.weight"]), _d(sd["fc.0.bias"])
-    w2, b2 = _d(sd["fc.2.weight"]), _d(sd["fc.2.bias"])
-    t = maps.permute(1, 2, 3, 0)
-    hid = F.linear(t, w0, b0)
-    hid_abs = F.linear(t.abs(), w0.abs(), b0.abs())
-    want = F.relu(F.linear(F.relu(hid), w2, b2)).permute(3, 0, 1, 2)
-    u = 2.0 ** -24
-    bound = (33 * u * F.linear(F.relu(hid), w2.abs(), b2.abs()) + F.linear((M + 1) * u * hid_abs, w2.abs()))
-    bound = 2 * bound.permute(3, 0, 1, 2) + 1e-30
+    want = sb.fc_fuse(maps, sd)
+    bound = hk.fc_fuse_bound(maps, sd)
     err = (got - want).abs()
     assert (err <= bound).all(), \
         f"M={M}: max err {err.max().item():.3g}, worst err/bound {(err / bound).max().item():.3f}"
@@ -185,22 +182,8 @@ STACK_BOUNDS = {
 C2_BOUNDS = (0.43, 0.058)                             # maps 0 and 19: 0.108, 0.0145 (restatement 1.0 s)
 
 
-def _stack_state(M, h, scale):
-    """The state dict of test_full_stack_against_oracle with distinct slopes, plus one layer at slope 1.3 and one at
-    -0.2, so the stack runs all three packed-PReLU forms (and the fp32 PReLU of the x4 strided convs)."""
-    sd = so.init_state_dict(num_maps=M, seed=M + h, gain=2.3, upscale=scale)
-    gs = torch.Generator().manual_seed(99)
-    for k in sd:
-        if k.endswith(".1.weight"):
-            sd[k] = torch.rand(1, generator=gs) * 0.4 + 0.05
-    sd["block.upBlocks.2.1.weight"] = torch.tensor([1.3])
-    sd["block.compress_in.1.weight"] = torch.tensor([-0.2])
-    sd["fc.2.weight"] = sd["fc.2.weight"].abs()          # a fused frame the final ReLU does not zero
-    return sd
-
-
 def _stack_run(M, h, w, steps, scale):
-    sd = _stack_state(M, h, scale)
+    sd = hk.stack_state(M, h, scale)
     mod = SRProjectionModule(num_steps=steps, num_maps=M, upscale_factor=scale)
     mod.load_state_dict(sd)
     x = torch.rand((M, 3, h, w), generator=torch.Generator().manual_seed(5)) * 255
@@ -252,6 +235,150 @@ def test_full_stack_c2_maps_against_restatement():
     print(f"[measure] stack C2 maps 0,19: max {mx.max().item():.4g} rms {rms.max().item():.4g} "
           f"(restatement {time.time() - t0:.1f} s)")
     assert mx.max().item() <= C2_BOUNDS[0] and rms.max().item() <= C2_BOUNDS[1], (mx.tolist(), rms.tolist())
+
+
+# ---- the stack at the benchmark's sizes ---------------------------------------------------------------------------
+# hk.FULL_SIZE_PLANS cases, their restated maps and bounds on |premix - restatement| (0..255 scale): whole-map max-abs,
+# which every region's max-abs must meet too; whole-map RMS; every region's RMS (hk.region_errors: the 2*scale-pixel
+# border bands and the tiles over 32 x 32 LR blocks); and, where every map is restated, max-abs of |fused frame -
+# fc(restatement)|.  About 4x the values measured on one NVIDIA B200 (1000 W power limit), given in the comments as
+# (max, RMS, region RMS, fused).  In the same run the restatement, one map at a time, peaked at 9.8 (C2), 20.6 (C5) and
+# 43.0 GiB (C4) allocated, and in the whole suite the three cases took 1.5, 8.0 and 8.5 s.
+FULL_SIZE_MAPS = {"C2": (0, 19), "C5": tuple(range(8)), "C4": (0, 13)}
+FULL_SIZE_BOUNDS = {
+    "C2": (0.58, 0.086, 0.089, None),                 # maps 0, 19: 0.1435, 0.02135, 0.02209
+    "C5": (0.33, 0.046, 0.048, 0.068),                # maps 0..7: 0.08289, 0.01135, 0.01183, 0.01699
+    "C4": (2.3, 0.37, 0.39, None),                    # maps 0, 13: 0.565, 0.092, 0.09638
+}
+
+
+def _teacher_forced_fuse(maps, got, sd, what):
+    """The fused frame got (1,3,H,W) against sb.fc_fuse over the stack's own per-map images maps (M,3,H,W), within
+    hk.fc_fuse_bound, one colour channel at a time (C4's float64 hidden layer is 2 GB per channel).  Returns the worst
+    err / bound."""
+    worst = 0.0
+    for c in range(3):
+        m = maps[:, c:c + 1]
+        want = sb.fc_fuse(m, sd)
+        err = (got[:, c:c + 1].double() - want).abs()
+        ratio = (err / hk.fc_fuse_bound(m, sd)).max().item()
+        assert ratio <= 1.0, f"{what}: channel {c} max err {err.max().item():.3g}, worst err/bound {ratio:.3f}"
+        assert want.abs().mean().item() > 1.0                 # the fc carries signal
+        worst = max(worst, ratio)
+    return worst
+
+
+def _full_size_run(name):
+    """One plan forward of case `name` on stack_state weights and fp32 frames: (state dict, x, premix, fused frame)."""
+    M, h, w, scale, _, _ = hk.FULL_SIZE_PLANS[name]
+    sd = hk.stack_state(M, h, scale)
+    mod = SRProjectionModule(num_maps=M, upscale_factor=scale)
+    mod.load_state_dict(sd)
+    x = (torch.rand((M, 3, h, w), generator=torch.Generator().manual_seed(4)) * 255).to(DEV)
+    premix = mod.premix(x)
+    got = mod(x)
+    assert torch.isfinite(premix).all() and torch.isfinite(got).all()
+    del mod                                               # the plan's workspace: 89 GB at C4
+    gc.collect()
+    torch.cuda.empty_cache()
+    return sd, x, premix, got
+
+
+@pytest.mark.parametrize("name", ["C2", "C5", "C4"])
+def test_full_size_maps_against_restatement(name):
+    """The conv stack at the benchmark's sizes, where 32-bit offsets, TMA coordinates and the last rows of the last map
+    are exercised: C2 (M = 20, 270 x 480, x4; the HR ring over 2^31 bytes), C5 (M = 8, 360 x 720, x4) and C4 (M = 14,
+    1080 x 1920, x2, uncapped as bench.py runs it; buffers over 2^31 BF16 elements).  The maps are independent until
+    the fc fuse, so the first and last maps are restated (all of them at C5), one at a time in CUDA float64, and held to
+    whole-map and per-region bounds; the fused frame is checked teacher-forced over all M maps, and at C5 also against
+    the fc over the restated maps."""
+    M, h, w, scale, _, _ = hk.FULL_SIZE_PLANS[name]
+    maps = FULL_SIZE_MAPS[name]
+    b_max, b_rms, b_region_rms, b_fused = FULL_SIZE_BOUNDS[name]
+    gc.collect()
+    torch.cuda.empty_cache()
+    t0 = time.time()
+    sd, x, premix, got = _full_size_run(name)
+    tf = _teacher_forced_fuse(premix, got, sd, f"{name} teacher-forced fc fuse")
+    got_maps = premix[list(maps)].clone()
+    del premix
+    torch.cuda.empty_cache()
+    t1 = time.time()
+    torch.cuda.reset_peak_memory_stats()
+    held = torch.cuda.memory_allocated()
+    mx, rms, region_mx, region_rms, fails, wants = [], [], 0.0, 0.0, [], []
+    for i, m in enumerate(maps):
+        want = sb.forward_maps(x[m:m + 1], sd, upscale=scale)
+        if i == 0:                                        # the conv branch carries signal: not blind
+            skip = F.interpolate(x[m:m + 1].double(), scale_factor=scale, mode="bilinear", align_corners=False)
+            assert (want - skip).abs().mean().item() > 0.05
+            del skip
+        d = got_maps[i:i + 1].double() - want
+        mx.append(d.abs().max().item())
+        rms.append(d.square().mean().sqrt().item())
+        del d
+        regs, rmx, rrms = hk.region_errors(got_maps[i:i + 1], want, scale)
+        region_mx, region_rms = max(region_mx, rmx.max().item()), max(region_rms, rrms.max().item())
+        fails += hk.region_failures(regs, rmx, rrms, b_max, b_region_rms, [m])
+        if b_fused is not None:
+            wants.append(want)
+        del want
+    torch.cuda.synchronize()
+    t2 = time.time()
+    peak = torch.cuda.max_memory_allocated()
+    fused = None
+    if b_fused is not None:
+        fused = (got.double() - sb.fc_fuse(torch.cat(wants), sd)).abs().max().item()
+    print(f"[measure] full-size {name} maps {maps[0]}..{maps[-1]}: max {max(mx):.4g} rms {max(rms):.4g} region max "
+          f"{region_mx:.4g} region rms {region_rms:.4g} fused {fused if fused is None else f'{fused:.4g}'}; "
+          f"teacher-forced fc worst err/bound {tf:.3f}; forward + fc check {t1 - t0:.1f} s, restatement "
+          f"{t2 - t1:.1f} s, restatement peak {peak / 2**30:.1f} GiB allocated ({(peak - held) / 2**30:.1f} GiB over "
+          f"the {held / 2**30:.2f} GiB held)")
+    assert max(mx) <= b_max and max(rms) <= b_rms, (name, mx, rms)
+    assert not fails, f"{name}: {len(fails)} regions outside: " + "; ".join(fails[:12])
+    if b_fused is not None:
+        assert fused <= b_fused, (name, fused)
+
+
+# C5's last map restated with its input raised by this much (0..255 scale) in the bottom-right 8 x 8 LR pixels
+CORNER_DELTA = 0.1
+
+
+def test_region_bounds_see_an_error_in_the_last_corner():
+    """A deliberate error on the expected side: C5's last map restated from an input raised by CORNER_DELTA in its
+    bottom-right 8 x 8 LR pixels (the kernels are untouched) -- an error where the addresses are highest, in 0.025 % of
+    the map's pixels.  Some region must exceed the C5 bounds, and only regions within the x4 receptive field of that
+    corner (48 LR px) may.  Measured on one NVIDIA B200 (1000 W power limit), whole map / corner tile (LR y 352:360
+    x 704:720):
+      clean           max 0.0829  RMS 0.0114    corner tile RMS 0.0115
+      +0.05           max 0.110   RMS 0.0114    0.0370
+      +0.1 (used)     max 0.160   RMS 0.0114    0.0706   -> whole-map bounds (0.33, 0.046) pass it; the region RMS
+                                                            bound 0.048 rejects the corner tile, and no other region
+      +0.2            max 0.269   RMS 0.0118    0.139
+      +0.3            max 0.366   RMS 0.0122    0.208    -> the whole-map max rejects it from here on
+    Every region outside the receptive field stays at max 0.0829, RMS 0.0117 at every size of the change."""
+    name = "C5"
+    M, h, w, scale, _, _ = hk.FULL_SIZE_PLANS[name]
+    b_max, b_rms, b_region_rms, _ = FULL_SIZE_BOUNDS[name]
+    gc.collect()
+    torch.cuda.empty_cache()
+    sd, x, premix, _ = _full_size_run(name)
+    got = premix[M - 1:M].clone()
+    del premix
+    xp = x[M - 1:M].clone()
+    xp[:, :, -8:, -8:] += CORNER_DELTA
+    want = sb.forward_maps(xp, sd, upscale=scale)
+    d = got.double() - want
+    mx, rms = d.abs().max().item(), d.square().mean().sqrt().item()
+    regs, rmx, rrms = hk.region_errors(got, want, scale)
+    flagged = [regs[r] for r in ((rmx[0] > b_max) | (rrms[0] > b_region_rms)).nonzero().flatten().tolist()]
+    H, W, reach = scale * h, scale * w, scale * (8 + 48)
+    far = [r[0] for r in flagged if r[2] <= H - reach or r[4] <= W - reach]
+    print(f"[measure] corner +{CORNER_DELTA}: whole-map max {mx:.4g} rms {rms:.4g}, rejected by the whole-map bounds "
+          f"alone: {mx > b_max or rms > b_rms}; region max {rmx.max().item():.4g} rms {rrms.max().item():.4g}, "
+          f"flagged {[r[0] for r in flagged]}")
+    assert flagged, "the region bounds miss an error in the last map's bottom-right corner"
+    assert not far, f"regions outside the corner's receptive field flagged: {far}"
 
 
 # ---- sensitivity --------------------------------------------------------------------------------------------------

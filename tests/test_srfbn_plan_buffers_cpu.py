@@ -74,6 +74,39 @@ def test_buffers_lie_in_the_workspace_disjoint_and_sized_by_the_chunk(scale, cap
         L.vsr_srfbn_plan_destroy(plan)
 
 
+# What each full-size case of hk.FULL_SIZE_PLANS exists to reach: its largest activation buffer over 2^k bytes, or over
+# 2^k BF16 elements (2^(k+1) bytes)
+_REACH = {"C2": ("bytes", 31), "C4": ("BF16 elements", 31), "C5-W3": ("bytes", 32), "C2-W2": ("bytes", 32)}
+
+
+@pytest.mark.parametrize("name", list(hk.FULL_SIZE_PLANS))
+def test_full_size_cases_reach_their_sizes(name):
+    """The plans of the full-size GPU tests, created as those tests create them, still reach the sizes they exist for:
+    a buffer past 2^31 bytes (C2), 2^31 BF16 elements (C4) or 2^32 bytes (the uncapped window-batched cases), and for
+    the capped C5 W = 3 case a chunk of maps that straddles window boundaries."""
+    M, h, w, scale, W, cap = hk.FULL_SIZE_PLANS[name]
+    L = _lib.lib()
+    plan = _plan(M, h, w, scale)
+    try:
+        if W > 1:
+            _lib.check(L.vsr_srfbn_plan_set_windows(plan, W), "set_windows")
+        if cap is not None:
+            _lib.check(L.vsr_srfbn_plan_set_workspace_cap(plan, cap), "set_workspace_cap")
+        chunk = L.vsr_srfbn_chunk_maps(plan)
+        largest = max(_buffer(plan, id, 0)[2] for id in range(len(NAMES)))
+        print(f"[measure] {name}: chunk {chunk}, workspace {L.vsr_srfbn_workspace_bytes(plan) / 2**30:.2f} GiB, "
+              f"largest buffer {largest / 2**30:.2f} GiB")
+        if cap is None:
+            assert chunk == W * M, chunk
+        else:
+            assert chunk % M and M % chunk and chunk < W * M, chunk             # a chunk straddles the windows
+        if name in _REACH:
+            unit, k = _REACH[name]
+            assert largest > 2 ** (k + (unit != "bytes")), (name, largest, unit, k)
+    finally:
+        L.vsr_srfbn_plan_destroy(plan)
+
+
 def test_argument_errors():
     L = _lib.lib()
     plan = _plan(3, 5, 7, 4)

@@ -31,7 +31,7 @@ from oracle import srfbn_bf16 as sb
 from tests import srfbn_hooks as hk
 from tests.srfbn_hooks import (BUF_A0, BUF_ACC, BUF_C128, BUF_HB, BUF_HIDDEN, BUF_HR, BUF_HT, BUF_LR, BUF_PREMIX, BUF_U,
                                BUF_XFEAT)
-from tests.test_srfbn_faithful_gpu import MAX_DIFF_FRAC, STACK_BOUNDS, _map_errors, _stack_state
+from tests.test_srfbn_faithful_gpu import MAX_DIFF_FRAC, STACK_BOUNDS, _map_errors
 from tests.test_srfbn_gpu import _MAX_DIFF_FRAC_FUSED
 from video_super_resolution_b200 import _lib
 from video_super_resolution_b200.my_packages.SRProjection.SRProjectionModule import SRProjectionModule
@@ -371,7 +371,7 @@ def test_plan_walk(M, h, w, steps, scale):
     """Every layer of the bound plan: hook identity, restatement agreement and no stray writes; the layer sequence is
     the graph's; after the walk the per-map images are the whole forward's, bit for bit."""
     t0 = time.time()
-    sd = _stack_state(M, h, scale)
+    sd = hk.stack_state(M, h, scale)
     plan = _Plan(sd, M, h, w, steps, scale)
     n = _walk(plan, sd, _plan_steps(scale, steps), sb.Restatement())
     assert torch.equal(plan.views[PREMIX].view(torch.int32), plan.premix.view(torch.int32)), "premix after the walk"
@@ -425,7 +425,7 @@ def test_walk_rejects_a_perturbed_expectation_at_its_layer(scale):
     x4 / x2); the other three leave the whole stack within its bounds (max 0.064 to 0.072 at x4, 0.28 to 0.42 at x2, the
     size of the clean divergence)."""
     M, h, w, steps = 3, 9, 21, 2
-    sd = _stack_state(M, h, scale)
+    sd = hk.stack_state(M, h, scale)
     plan = _Plan(sd, M, h, w, steps, scale)
     b_max, b_rms, b_fused = STACK_BOUNDS[(M, h, w, steps, scale)]
     for kind, layer in _PERTURBATIONS.items():
