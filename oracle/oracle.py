@@ -40,6 +40,10 @@ def lib():
         I = ctypes.c_int
         _lib.or_resample2d.argtypes = [_f32p, _f32p, _f32p, I, I, I, I] + [L] * 12 + [I, I, I, I]
         _lib.or_resample2d.restype = None
+        _lib.or_warp_nhwc_fast.argtypes = [_f32p] * 5 + [I] * 6
+        _lib.or_warp_nhwc_fast.restype = None
+        _lib.or_compose_flow_fast.argtypes = [_f32p] * 3 + [I] * 4
+        _lib.or_compose_flow_fast.restype = None
         _lib.or_warp_labels.argtypes = [_u8p, _f32p, _u8p, I, I, I]
         _lib.or_warp_labels.restype = None
         _lib.or_channelnorm.argtypes = [_f32p, _f32p, I, I, I, I, L, L, L, L]
@@ -103,22 +107,39 @@ def resample2d_nchw(input1, flow, kernel_size=1, bilinear=True, threads=1):
     return out
 
 
-def warp_nhwc(src, flow, bilinear=True, threads=1):
-    """Pipeline layout: src (B,H,W,C), flow (B,H,W,2) -> (B,H,W,C); same arithmetic."""
+def warp_nhwc(src, flow, bilinear=True, threads=1, ref=None):
+    """Pipeline layout: src (B,H,W,C), flow (B,H,W,2) -> (B,H,W,C).  bilinear: False/0 nearest, True/1 the reference
+    arithmetic, 2 the fast mode (or_warp_nhwc_fast: fp32 FMA blend).  With ref (B,H,W,C) also returns the per-pixel
+    L2 norm of (ref - warped), (B,H,W), as ops.warp(..., ref=ref)."""
     src = _c(src, np.float32)
     flow = _c(flow, np.float32)
     B, H, W, C = src.shape
     assert flow.shape == (B, H, W, 2)
     out = np.zeros((B, H, W, C), np.float32)
     L = lib()
+    mode = int(bilinear)
+    if mode == 2:
+        if ref is not None:
+            ref = _c(ref, np.float32)
+            assert ref.shape == src.shape
+        norm = np.zeros((B, H, W), np.float32) if ref is not None else None
+
+        def run(y0, y1):
+            L.or_warp_nhwc_fast(_p(src, _f32p), _p(flow, _f32p), _p(out, _f32p),
+                                _p(ref, _f32p) if ref is not None else None,
+                                _p(norm, _f32p) if ref is not None else None, B, H, W, C, y0, y1)
+
+        _fan_rows(run, H, threads)
+        return out if ref is None else (out, norm)
+    assert mode in (0, 1), bilinear
 
     def run(y0, y1):
         L.or_resample2d(_p(src, _f32p), _p(flow, _f32p), _p(out, _f32p), B, C, H, W,
                         H * W * C, 1, W * C, C, H * W * 2, 1, W * 2, 2, H * W * C, 1, W * C, C,
-                        1, int(bool(bilinear)), y0, y1)
+                        1, mode, y0, y1)
 
     _fan_rows(run, H, threads)
-    return out
+    return out if ref is None else (out, channelnorm_nhwc(_c(ref, np.float32) - out))
 
 
 def warp_labels(labels, flow):
@@ -264,28 +285,45 @@ def assemble_stack(warped, centre, proj, resid, depth, estimate, centre_idx, fal
     return out
 
 
-def compose_flow(g, f):
+def compose_flow(g, f, fast=False, threads=1):
     """out(p) = g(p) + f(p + g(p)), f (h,w,2) sampled with the Resample2d taps and border rule (Appendix A);
-    g maps image A to B, f maps B to C, the result maps A to C."""
-    g = _c(g, np.float32)
+    g maps image A to B, f maps B to C, the result maps A to C.  fast=True: the arithmetic of ops.compose_flow
+    (compose_flow_kernel: fast-mode blend, fp32 add of g), g=None the identity field; fast=False: the exact blend."""
     f = _c(f, np.float32)
-    return (g + warp_nhwc(f[None], g[None], True)[0]).astype(np.float32)
+    if not fast:
+        g = _c(g, np.float32)
+        return (g + warp_nhwc(f[None], g[None], True)[0]).astype(np.float32)
+    H, W, two = f.shape
+    assert two == 2
+    if g is not None:
+        g = _c(g, np.float32)
+        assert g.shape == f.shape
+    out = np.zeros_like(f)
+    L = lib()
+    _fan_rows(lambda y0, y1: L.or_compose_flow_fast(_p(g, _f32p) if g is not None else None, _p(f, _f32p),
+                                                    _p(out, _f32p), H, W, y0, y1), H, threads)
+    return out
 
 
-def chain_flows(proj, flows, centre):
+def chain_flows(proj, flows, centre, fast=False, threads=1):
     """Centre -> neighbour flows (T-1,h,w,2), frame order with the centre left out (WarpFusePipeline docstring):
     past frames chain the PROJECTED flows (they live in the later frame's coordinates), future frames the forward
-    flows (they live in the earlier frame's)."""
+    flows (they live in the earlier frame's).  fast=True restates WarpFusePipeline.chain_flows link for link, the
+    first link of each side included (compose_flow(None, .), a copy up to the sign of zero)."""
     Tm1 = flows.shape[0]
     T, c = Tm1 + 1, centre
     G = np.zeros_like(flows)
-    G[c - 1] = proj[c - 1]
+
+    def link(g, f):
+        return compose_flow(g, f, fast=fast, threads=threads)
+
+    G[c - 1] = link(None, proj[c - 1]) if fast else proj[c - 1]
     for t in range(c - 2, -1, -1):
-        G[t] = compose_flow(G[t + 1], proj[t])
+        G[t] = link(G[t + 1], proj[t])
     if c + 1 < T:
-        G[c] = flows[c]
+        G[c] = link(None, flows[c]) if fast else flows[c]
         for t in range(c + 2, T):
-            G[t - 1] = compose_flow(G[t - 2], flows[t - 1])
+            G[t - 1] = link(G[t - 2], flows[t - 1])
     return G
 
 
@@ -298,17 +336,33 @@ def estimate_slot(hr, mask, scale=4):
     return lo.astype(np.float32)
 
 
-def warp_fuse_front(frames, flows, inv_depth, logits_a, logits_b, estimate=None, threads=1):
+def warp_fuse_front(frames, flows, inv_depth, logits_a, logits_b, estimate=None, threads=1, fast=False, projected=None):
     """CPU restatement of WarpFusePipeline.project_and_warp (a1-a5 + a7): returns the map stack and
-    the intermediates.  frames (T,h,w,3), flows (T-1,h,w,2), inv_depth (T-1,h,w), logits (h,w) x2."""
+    the intermediates.  frames (T,h,w,3), flows (T-1,h,w,2), inv_depth (T-1,h,w), logits (h,w) x2.
+    fast=False: the warps and the flow chain in the reference's exact arithmetic; fast=True: in the arithmetic the
+    pipeline runs (mode 2 warp with the fused residual, compose_flow_kernel), so that with the deterministic projection
+    every output is restated bit for bit.
+    projected: (proj_flow, proj_depth, wsum) taken as given instead of this restatement's projections -- the chain,
+    warps, label warp and assembly downstream of them are restated from those arrays.
+    W windows: frames (W,T,h,w,3) and every other input with the same leading W (estimate (W,3,h,w) | None,
+    projected arrays (W,T-1,...)): one restatement per window, results stacked along a leading W."""
+    frames = np.asarray(frames)
+    if frames.ndim == 5:
+        outs = [warp_fuse_front(frames[b], flows[b], inv_depth[b], logits_a[b], logits_b[b],
+                                None if estimate is None else estimate[b], threads, fast,
+                                None if projected is None else tuple(p[b] for p in projected))
+                for b in range(frames.shape[0])]
+        return (np.stack([o[0] for o in outs]), {k: np.stack([o[1][k] for o in outs]) for k in outs[0][1]})
     T = frames.shape[0]
     c = T // 2
     proj_f, _, cnt_f, hole_f = flow_projection(flows, None, threads=threads)
     proj_d, wsum, cnt_d, hole_d = flow_projection(flows, inv_depth, threads=threads)
-    G = chain_flows(proj_d, flows, c)
+    if projected is not None:
+        proj_f, proj_d, wsum = (_c(p, np.float32) for p in projected)
+    G = chain_flows(proj_d, flows, c, fast=fast, threads=threads)
     neigh = np.ascontiguousarray(frames[[t for t in range(T) if t != c]])
-    warped = warp_nhwc(neigh, G, True, threads=threads)
-    resid = channelnorm_nhwc(frames[c][None] - warped)
+    centre = np.broadcast_to(frames[c], neigh.shape)
+    warped, resid = warp_nhwc(neigh, G, 2 if fast else True, threads=threads, ref=centre)
     mask = vos_threshold(logits_a, logits_b)
     mask_w = warp_labels(mask[None], G[c - 1][None])[0]
     stack = assemble_stack(warped, frames[c], proj_f, resid, wsum, estimate, c, fallback=frames[0])

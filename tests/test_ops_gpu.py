@@ -90,13 +90,21 @@ def test_huge_and_nan_flow_take_the_exact_fallback():
 
 
 def test_warp_unaligned_views_and_ragged_tail():
-    # 1 pixel short of a vector multiple, and an output carved at a non-16-byte offset
+    # 1 pixel short of a vector multiple, and an output carved at a non-16-byte offset (through the C ABI: ops.warp
+    # allocates its output aligned), which the C = 3 kernel must store element by element
+    from tests.front_hooks import warp_carved
     B, H, W = 1, 17, 19
     g = torch.Generator().manual_seed(5)
     src = torch.rand((B, H, W, 3), generator=g)
     flow = (torch.rand((B, H, W, 2), generator=g) - 0.5) * 5
+    ref = torch.rand((B, H, W, 3), generator=g)
     got = _np(ops.warp(src.to(DEV), flow.to(DEV)))
     assert np.array_equal(got, orc.warp_nhwc(src.numpy(), flow.numpy()))
+    for mode in (0, 1, 2):
+        for offset in (1, 2, 3):
+            carved, norm = warp_carved(src.to(DEV), flow.to(DEV), mode, ref.to(DEV), offset_floats=offset)
+            want, want_n = orc.warp_nhwc(src.numpy(), flow.numpy(), mode, ref=ref.numpy())
+            assert np.array_equal(_np(carved), want) and np.array_equal(_np(norm), want_n), (mode, offset)
 
 
 @pytest.mark.parametrize("shape", [(1, 64, 64), (3, 31, 45), (2, 8, 1023)])

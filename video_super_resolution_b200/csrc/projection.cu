@@ -469,7 +469,7 @@ constexpr size_t kTileSmem = (size_t)(kNC + 32) * 16 + (size_t)kColWords * kTW *
 
 struct TileRect {      // the tile's cells as bounds on the target position (x2, y2), and the tile's first cell
   float xa, xb, ya, yb;
-  float cx0f, cy0f;
+  int cx0, cy0;
 };
 
 // One claim round for two sources per lane, as one block of PTX on 32-bit shared addresses (the compiler's version
@@ -543,8 +543,10 @@ __device__ __forceinline__ void add_sources(const float (&fx)[U], const float (&
     // "lands in one of the tile's cells and inside the image" (Appendix B step 2; NaN fails every compare)
     const bool in = x2 >= R.xa && x2 <= R.xb && y2 >= R.ya && y2 <= R.yb;
     pend[u] = in ? 1u : 0u;
-    // local cell: x2 - cx0 is exact (an integer below 2^11 off a float below 2^24) and >= 0 where it matters
-    const int ix = (int)(x2 - R.cx0f), iy = (int)(y2 - R.cy0f);
+    // local cell: Appendix B's cell int(x2) less the tile's first cell.  Not int(x2 - cx0) in fp32: in the first tile
+    // column / row cx0 = -1, and x2 + 1 rounds up to the next integer for an x2 within an ulp below a power of two
+    // (31.999998f + 1 = 33.0f), which put such a source one cell to the right
+    const int ix = (int)x2 - R.cx0, iy = (int)y2 - R.cy0;
     cell_a[u] = cells_sa + 16u * (uint32_t)(iy * kCW + ix);
     claim_a[u] = in ? claim_sa + (uint32_t)(iy * kClaimPitch + ix) : scr_claim;
     vx[u] = __fmul_rn(-fx[u], dd[u]);
@@ -785,8 +787,8 @@ projection_tiled_kernel(const ProjArgs a) {
       R.xb = gcx_hi <= w - 1 ? nextafterf((float)gcx_hi, 0.0f) : xmax;
       R.ya = (float)max(ty0 - 1, 0);
       R.yb = gcy_hi <= h - 1 ? nextafterf((float)gcy_hi, 0.0f) : ymax;
-      R.cx0f = (float)(tx0 - 1);
-      R.cy0f = (float)(ty0 - 1);
+      R.cx0 = tx0 - 1;
+      R.cy0 = ty0 - 1;
     }
     __syncthreads();
 
