@@ -146,10 +146,14 @@ int vsr_resample2d_backward_deterministic(const float* input1, const float* flow
  * correlation_cuda_kernel.cu:46-147.  input1/input2 (B,C,H,W) f32 NCHW; output (B, D*D, outH, outW)
  * f32 with D = 2*(max_displacement/stride2)+1 and outH/outW from vsr_correlation_output_shape (the
  * reference resizes `output` itself; here the caller allocates, as everywhere in this ABI).  No
- * padded NHWC copies (`rInput1/2`) are needed.  fp32 results agree with the reference to fp32
- * summation order (tested <= 1e-5 relative).  Positions outside the image are zeros for any pad_size;
- * the reference is only defined for pad_size >= max_displacement + (kernel_size-1)/2 (with less it
- * indexes outside its padded copies). */
+ * padded NHWC copies (`rInput1/2`) are needed.  Arithmetic, the same on both kernels: one fp32 fmaf
+ * chain per output over the window taps (j, i) and then the channels, then acc / (k*k*C) rounded to
+ * nearest; bit-identical to oracle.c::or_correlation (padded = 1) and within fp32 summation order of
+ * the reference, which sums 32 strided partials.  Positions outside the image are zeros and their
+ * products are taken, as in the reference's zero-padded copies: an Inf or NaN that meets padding
+ * gives NaN.  That holds for any pad_size; the reference is only defined for pad_size >=
+ * max_displacement + (kernel_size-1)/2 (with less it indexes outside its padded copies).
+ * VSR_ERR_UNSUPPORTED for more than 21 displacements per axis, with nothing launched. */
 int vsr_correlation_output_shape(int C, int H, int W, int pad_size, int kernel_size, int max_displacement,
                                  int stride1, int stride2, int* out_channels, int* out_h, int* out_w);
 int vsr_correlation_forward(const float* input1, const float* input2, float* output, int B, int C, int H, int W,
@@ -159,7 +163,10 @@ int vsr_correlation_forward(const float* input1, const float* input2, float* out
  * correlation_cuda.backward = correlation_backward_cuda(input1, input2, rInput1, rInput2, gradOutput, gradInput1,
  * gradInput2, ...) correlation_cuda.cc:89-166 -> correlation_cuda_kernel.cu:148-333.  grad_output (B, D*D, outH, outW),
  * grad_input1/2 (B,C,H,W), all f32; every element of the gradients is written (no pre-zeroing needed).  stride1 must
- * be 1 (VSR_ERR_UNSUPPORTED otherwise: the reference's kernels write out of bounds for stride1 > 1). */
+ * be 1 (VSR_ERR_UNSUPPORTED otherwise: the reference's kernels write out of bounds for stride1 > 1).  One fp32 fmaf
+ * chain per element over the displacements (tj, then ti) and the window of outputs that covers it (rows, then
+ * columns), then acc / (k*k*C): bit-identical to oracle.c::or_correlation_backward_chain.  The other image is zero
+ * outside itself and those products are taken, so an Inf or NaN of grad_output that meets padding gives NaN. */
 int vsr_correlation_backward(const float* input1, const float* input2, const float* grad_output,
                              float* grad_input1, float* grad_input2, int B, int C, int H, int W, int pad_size,
                              int kernel_size, int max_displacement, int stride1, int stride2, int corr_multiply,

@@ -58,10 +58,12 @@ def lib():
         _lib.or_resample2d_backward.restype = None
         _lib.or_channelnorm_backward.argtypes = [_f32p] * 4 + [I, I, L]
         _lib.or_channelnorm_backward.restype = None
-        _lib.or_correlation.argtypes = [_f32p] * 3 + [I] * 11
+        _lib.or_correlation.argtypes = [_f32p] * 3 + [I] * 14
         _lib.or_correlation.restype = None
         _lib.or_correlation_backward.argtypes = [_f32p] * 3 + [I] * 11
         _lib.or_correlation_backward.restype = None
+        _lib.or_correlation_backward_chain.argtypes = [_f32p] * 3 + [I] * 13
+        _lib.or_correlation_backward_chain.restype = None
         _lib.or_flow2img.argtypes = [_f32p, _u8p, I, I]
         _lib.or_flow2img.restype = None
         _lib.or_resize_nearest_planar.argtypes = [_u8p, _f32p, I, I, I, I]
@@ -194,18 +196,26 @@ def channelnorm_backward(x, out, grad_output):
     return g
 
 
-def correlation(input1, input2, pad_size=3, kernel_size=3, max_displacement=20, stride1=1, stride2=2):
-    """FlowNetC cost volume, NCHW.  ref: correlation_cuda.cc:25-42, correlation_cuda_kernel.cu:73-147."""
+def correlation(input1, input2, pad_size=3, kernel_size=3, max_displacement=20, stride1=1, stride2=2, padded=False,
+                items=None, threads=1):
+    """FlowNetC cost volume, NCHW.  ref: correlation_cuda.cc:25-42, correlation_cuda_kernel.cu:73-147.
+    padded=True: the reference's zero padding with every product taken (the kernels' rule, NaN from 0 * Inf);
+    padded=False: taps with a position outside the image skipped.  items=(n0, n1) restates batch items n0..n1-1 only
+    (the result has n1 - n0 items); threads fans the output rows out."""
     input1 = _c(input1, np.float32)
     input2 = _c(input2, np.float32)
+    if items is not None:
+        input1, input2 = input1[items[0]:items[1]], input2[items[0]:items[1]]
     B, C, H, W = input1.shape
     border = (kernel_size - 1) // 2 + max_displacement
     outH = -(-(H + 2 * pad_size - 2 * border) // stride1)
     outW = -(-(W + 2 * pad_size - 2 * border) // stride1)
     D = 2 * (max_displacement // stride2) + 1
     out = np.zeros((B, D * D, outH, outW), np.float32)
-    lib().or_correlation(_p(input1, _f32p), _p(input2, _f32p), _p(out, _f32p), B, C, H, W, pad_size, kernel_size,
-                         max_displacement, stride1, stride2, outH, outW)
+    L = lib()
+    _fan_rows(lambda y0, y1: L.or_correlation(_p(input1, _f32p), _p(input2, _f32p), _p(out, _f32p), B, C, H, W, pad_size,
+                                              kernel_size, max_displacement, stride1, stride2, outH, outW, int(padded),
+                                              y0, y1), outH, threads)
     return out
 
 
@@ -400,3 +410,26 @@ def correlation_backward(input1, input2, grad_output, pad_size, kernel_size, max
     lib().or_correlation_backward(_p(a, _f32p), _p(g, _f32p), _p(g2, _f32p), 1, B, C, H, W, pad_size, kernel_size,
                                   max_displacement, stride2, oh, ow)
     return g1, g2
+
+
+def correlation_backward_chain(input1, input2, grad_output, pad_size, kernel_size, max_displacement, stride2,
+                               items=None, channels=None, threads=1):
+    """(grad_input1, grad_input2) in the order of correlation_backward_kernel: one fmaf chain per element over (tj, ti,
+    j, i), padded values zero with their products taken.  items=(n0, n1) / channels=(c0, c1) restate that block only
+    (the results are (n1 - n0, c1 - c0, H, W)); threads fans the channels out."""
+    a, b, g = _c(input1, np.float32), _c(input2, np.float32), _c(grad_output, np.float32)
+    if items is not None:
+        a, b, g = a[items[0]:items[1]], b[items[0]:items[1]], g[items[0]:items[1]]
+    B, C, H, W = a.shape
+    oh, ow = g.shape[2], g.shape[3]
+    c0, c1 = channels if channels is not None else (0, C)
+    g1, g2 = np.zeros_like(a), np.zeros_like(a)
+    L = lib()
+
+    def run(k0, k1):
+        for which, other, gin in ((0, b, g1), (1, a, g2)):
+            L.or_correlation_backward_chain(_p(other, _f32p), _p(g, _f32p), _p(gin, _f32p), which, B, C, H, W, pad_size,
+                                            kernel_size, max_displacement, stride2, oh, ow, c0 + k0, c0 + k1)
+
+    _fan_rows(run, c1 - c0, threads)
+    return np.ascontiguousarray(g1[:, c0:c1]), np.ascontiguousarray(g2[:, c0:c1])

@@ -13,8 +13,12 @@
 // through a warp-shuffle reduction.  Here a warp owns 32 consecutive output x of one (n, y, tj):
 // lane = x keeps the D accumulators of its pixel in registers, in1 is read once per channel and the D
 // shifted in2 values are coalesced, L1-resident loads; no repack, no padding copy, no reduction.
-// fp32 FMA accumulation in channel order (the reference sums 32 strided partials and tree-reduces,
-// so results agree to fp32 rounding, not bit for bit).
+//
+// Arithmetic contract (both forward kernels, restated by oracle.c::or_correlation with padded = 1): one fp32 fmaf
+// chain per output over the window taps (j, i) and then the channels c, then __fdiv_rn(acc, k*k*C).  A position
+// outside the image reads as zero and its products are taken, as in the reference's zero-padded copies: an Inf or NaN
+// that meets padding makes NaN.  (The reference sums 32 strided partials and tree-reduces them, so it agrees to fp32
+// rounding, not bit for bit.)
 #include "common.cuh"
 
 #include <stdlib.h>
@@ -51,15 +55,16 @@ correlation_forward_kernel(const float* __restrict__ in1, const float* __restric
     for (int t = 0; t < kMaxD; ++t) acc[t] = 0.0f;
     const float* p1 = in1 + (int64_t)n * C * HW;
     const float* p2 = in2 + (int64_t)n * C * HW;
+    const bool lane_ok = x < outW;
     for (int j = -krad; j <= krad; ++j) {
       const int y1 = ya + j, y2 = yb + j;
-      const bool row1 = (y1 >= 0) && (y1 < H), row2 = (y2 >= 0) && (y2 < H);
-      if (!(row1 && row2)) continue;                 // a zero-padded row on either side contributes nothing
+      // a zero-padded row still takes its products: 0 * Inf on the other side is NaN, as in the reference
+      const bool row1 = lane_ok && (y1 >= 0) && (y1 < H), row2 = lane_ok && (y2 >= 0) && (y2 < H);
       for (int i = -krad; i <= krad; ++i) {
         const int x1 = xa + i;
-        const bool in_a = (x < outW) && (x1 >= 0) && (x1 < W);
-        const float* a_ptr = p1 + (int64_t)y1 * W + (in_a ? x1 : 0);
-        const float* b_row = p2 + (int64_t)y2 * W;
+        const bool in_a = row1 && (x1 >= 0) && (x1 < W);
+        const float* a_ptr = p1 + (in_a ? (int64_t)y1 * W + x1 : 0);
+        const float* b_row = p2 + (row2 ? (int64_t)y2 * W : 0);
         for (int c = 0; c < C; ++c) {
           const float a = in_a ? __ldg(a_ptr + (int64_t)c * HW) : 0.0f;
           const float* b_c = b_row + (int64_t)c * HW;
@@ -67,7 +72,7 @@ correlation_forward_kernel(const float* __restrict__ in1, const float* __restric
           for (int t = 0; t < kMaxD; ++t) {
             if (t < D) {
               const int x2 = x1 + (t - R) * s2;
-              const float b = (in_a && x2 >= 0 && x2 < W) ? __ldg(b_c + x2) : 0.0f;
+              const float b = (row2 && x2 >= 0 && x2 < W) ? __ldg(b_c + x2) : 0.0f;
               acc[t] = fmaf(a, b, acc[t]);
             }
           }
@@ -92,7 +97,13 @@ correlation_forward_kernel(const float* __restrict__ in1, const float* __restric
 // row segments DE-INTERLEAVED BY COLUMN PARITY, because every displacement is even: a thread that owns the four
 // same-parity columns x, x+2, x+4, x+6 then needs 4 contiguous A values and 24 contiguous B values per channel --
 // 7 16-byte shared loads for 84 FMAs, against one global load per FMA in the generic kernel above (which was
-// L1-bound at 2 TFLOP/s).  Same fp32 FMA chain in channel order as the generic kernel: identical bits.
+// L1-bound at 2 TFLOP/s).  Same fp32 FMA chain in channel order and the same padding rule as the generic kernel:
+// identical bits, non-finite inputs included.
+// Padding follows the reference: a padded row is staged as zeros and its products are taken (0 * Inf is NaN).  A task
+// whose in2 row is padding and in1 row is not (about 8 % of FlowNetC's) would run the chain fmaf(a, 0, acc) over the
+// channels, the same for every displacement ti of its row: +0, or NaN where a column of in1 holds an Inf or NaN.  The
+// zero-displacement task of the same (n, y, x-tile) reads that in1 row anyway; it runs this chain beside its own (one
+// fmaf per staged value) and writes those tasks' outputs, which are skipped.
 // ---------------------------------------------------------------------------------------------------------
 constexpr int kCorrCc = 8;                     // channels per staging round
 constexpr int kCorrXT = 128;                   // output columns per warp task
@@ -122,64 +133,67 @@ correlation_s2_kernel(const float* __restrict__ in1, const float* __restrict__ i
     const int x0 = xt * kCorrXT;
     const int ya = y + off, yb = ya + (tjw - R) * 2;
     const int xs = x0 + off;                      // in1 column of output column x0
-    const bool rows_ok = ya >= 0 && ya < H && yb >= 0 && yb < H;   // a zero-padded row contributes nothing
+    const bool row_a = ya >= 0 && ya < H, row_b = yb >= 0 && yb < H;
+    if (row_a && !row_b) continue;                // written by the task with tjw == R (below)
     float acc[4][kMaxD];
+    float chk[kCorrXT / 32] = {};                 // slot j: fmaf(a, 0, .) over the channels
 #pragma unroll
     for (int k = 0; k < 4; ++k)
 #pragma unroll
       for (int t = 0; t < kMaxD; ++t) acc[k][t] = 0.0f;
-    if (rows_ok) {
-      const float* p1 = in1 + (int64_t)n * C * HW + (int64_t)ya * W;
-      const float* p2 = in2 + (int64_t)n * C * HW + (int64_t)yb * W;
-      // column validity of this lane's staging slots, once per task (bit j: slot lane + 32 j)
-      uint32_t okA = 0, okB = 0;
+    const float* p1 = in1 + (int64_t)n * C * HW + (int64_t)(row_a ? ya : 0) * W;
+    const float* p2 = in2 + (int64_t)n * C * HW + (int64_t)(row_b ? yb : 0) * W;
+    // validity of this lane's staging slots, once per task (bit j: slot lane + 32 j); a padded row stages zeros
+    uint32_t okA = 0, okB = 0;
 #pragma unroll
-      for (int j = 0; j < kCorrXT / 32; ++j) {
-        const int xi = lane + 32 * j, gx = xs + xi;
-        okA |= (uint32_t)(gx >= 0 && gx < W && x0 + xi < outW) << j;
-      }
+    for (int j = 0; j < kCorrXT / 32; ++j) {
+      const int xi = lane + 32 * j, gx = xs + xi;
+      okA |= (uint32_t)(row_a && gx >= 0 && gx < W && x0 + xi < outW) << j;
+    }
 #pragma unroll
-      for (int j = 0; j < (kCorrBW + 31) / 32; ++j) {
-        const int xi = lane + 32 * j, gx = xs - 2 * R + xi;
-        okB |= (uint32_t)(xi < kCorrBW && gx >= 0 && gx < W) << j;
-      }
-      const float* q1 = p1 + xs + lane;
-      const float* q2 = p2 + xs - 2 * R + lane;
-      float* dA = &A[0][lane & 1][lane >> 1];            // slot lane + 32 j -> [(lane&1)][(lane>>1) + 16 j]
-      float* dB = &Bs[0][lane & 1][lane >> 1];
-      for (int c0 = 0; c0 < C; c0 += kCorrCc) {
-        const int nc = min(kCorrCc, C - c0);
+    for (int j = 0; j < (kCorrBW + 31) / 32; ++j) {
+      const int xi = lane + 32 * j, gx = xs - 2 * R + xi;
+      okB |= (uint32_t)(row_b && xi < kCorrBW && gx >= 0 && gx < W) << j;
+    }
+    const float* q1 = p1 + xs + lane;
+    const float* q2 = p2 + xs - 2 * R + lane;
+    float* dA = &A[0][lane & 1][lane >> 1];            // slot lane + 32 j -> [(lane&1)][(lane>>1) + 16 j]
+    float* dB = &Bs[0][lane & 1][lane >> 1];
+    for (int c0 = 0; c0 < C; c0 += kCorrCc) {
+      const int nc = min(kCorrCc, C - c0);
 #pragma unroll
-        for (int c = 0; c < kCorrCc; ++c) {
-          const uint32_t mA = c < nc ? okA : 0u, mB = c < nc ? okB : 0u;
-          const float* r1 = q1 + (int64_t)(c0 + c) * HW;
-          const float* r2 = q2 + (int64_t)(c0 + c) * HW;
+      for (int c = 0; c < kCorrCc; ++c) {
+        const uint32_t mA = c < nc ? okA : 0u, mB = c < nc ? okB : 0u;
+        const float* r1 = q1 + (int64_t)(c0 + c) * HW;
+        const float* r2 = q2 + (int64_t)(c0 + c) * HW;
 #pragma unroll
-          for (int j = 0; j < kCorrXT / 32; ++j)
-            dA[c * kCorrXT + 16 * j] = ((mA >> j) & 1u) ? __ldg(r1 + 32 * j) : 0.0f;
-#pragma unroll
-          for (int j = 0; j < (kCorrBW + 31) / 32; ++j)
-            if (lane + 32 * j < kCorrBW) dB[c * kCorrBW + 16 * j] = ((mB >> j) & 1u) ? __ldg(r2 + 32 * j) : 0.0f;
+        for (int j = 0; j < kCorrXT / 32; ++j) {
+          const float v = ((mA >> j) & 1u) ? __ldg(r1 + 32 * j) : 0.0f;
+          dA[c * kCorrXT + 16 * j] = v;
+          chk[j] = fmaf(v, 0.0f, chk[j]);
         }
-        __syncwarp();
+#pragma unroll
+        for (int j = 0; j < (kCorrBW + 31) / 32; ++j)
+          if (lane + 32 * j < kCorrBW) dB[c * kCorrBW + 16 * j] = ((mB >> j) & 1u) ? __ldg(r2 + 32 * j) : 0.0f;
+      }
+      __syncwarp();
 #pragma unroll 2
-        for (int c = 0; c < kCorrCc; ++c) {
-          const float4 a4 = *reinterpret_cast<const float4*>(&A[c][par][4 * q]);
-          const float a[4] = {a4.x, a4.y, a4.z, a4.w};
-          float bb[24];
+      for (int c = 0; c < kCorrCc; ++c) {
+        const float4 a4 = *reinterpret_cast<const float4*>(&A[c][par][4 * q]);
+        const float a[4] = {a4.x, a4.y, a4.z, a4.w};
+        float bb[24];
 #pragma unroll
-          for (int j = 0; j < 6; ++j) {
-            const float4 b4 = *reinterpret_cast<const float4*>(&Bs[c][par][4 * q + 4 * j]);
-            bb[4 * j] = b4.x; bb[4 * j + 1] = b4.y; bb[4 * j + 2] = b4.z; bb[4 * j + 3] = b4.w;
-          }
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-#pragma unroll
-            for (int t = 0; t < kMaxD; ++t)
-              if (t < D) acc[k][t] = fmaf(a[k], bb[k + t], acc[k][t]);
+        for (int j = 0; j < 6; ++j) {
+          const float4 b4 = *reinterpret_cast<const float4*>(&Bs[c][par][4 * q + 4 * j]);
+          bb[4 * j] = b4.x; bb[4 * j + 1] = b4.y; bb[4 * j + 2] = b4.z; bb[4 * j + 3] = b4.w;
         }
-        __syncwarp();
+#pragma unroll
+        for (int k = 0; k < 4; ++k)
+#pragma unroll
+          for (int t = 0; t < kMaxD; ++t)
+            if (t < D) acc[k][t] = fmaf(a[k], bb[k + t], acc[k][t]);
       }
+      __syncwarp();
     }
     // transpose through shared memory so that the stores are 128 contiguous floats per displacement
     const float nelems = (float)C;
@@ -199,6 +213,22 @@ correlation_s2_kernel(const float* __restrict__ in1, const float* __restrict__ i
         __syncwarp();
       }
     }
+    if (tjw == R && row_a) {                      // the skipped tasks of this in1 row whose in2 row is padding
+      float z[kCorrXT / 32];
+#pragma unroll
+      for (int j = 0; j < kCorrXT / 32; ++j) z[j] = __fdiv_rn(chk[j], nelems);   // column lane + 32 j
+      for (int tp = 0; tp < D; ++tp) {
+        const int yp = ya + (tp - R) * 2;
+        if (yp >= 0 && yp < H) continue;
+        float* op = out + (((int64_t)n * D * D + (int64_t)tp * D) * outH + y) * outW + x0;
+        for (int t = 0; t < D; ++t)
+#pragma unroll
+          for (int j = 0; j < kCorrXT / 32; ++j) {
+            const int xi = lane + 32 * j;
+            if (x0 + xi < outW) op[(int64_t)t * outH * outW + xi] = z[j];
+          }
+      }
+    }
   }
 }
 
@@ -209,8 +239,11 @@ correlation_s2_kernel(const float* __restrict__ in1, const float* __restrict__ i
 //   gradInput1[n,c,Y,X] = 1/(k*k*C) * sum_tc in2[n,c,Y + j2, X + i2] * sum_window gradOutput[n,tc,.,.]
 //   gradInput2[n,c,Y,X] = 1/(k*k*C) * sum_tc in1[n,c,Y - j2, X - i2] * sum_{window shifted by (j2,i2)} gradOutput[n,tc,.,.]
 // the window being the outputs whose kernel footprint covers the pixel (one output for kernel_size 1).  Both the
-// gradOutput and the shifted-image loads are coalesced along X.  fp32 FMA chain over tc in order (the reference
-// sums 32 strided partials and reduces them: equal to fp32 rounding, not bit for bit).
+// gradOutput and the shifted-image loads are coalesced along X.  One fp32 fmaf chain per element over tj, ti and the
+// clamped window rows j and columns i, then __fdiv_rn(acc, k*k*C) (restated by
+// oracle.c::or_correlation_backward_chain).  The other image is zero outside itself and those products are taken, so
+// an Inf or NaN of gradOutput that meets padding makes NaN, as in the reference (which sums 32 strided partials and
+// reduces them: equal to fp32 rounding, not bit for bit).
 // ---------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(kThreads)
 correlation_backward_kernel(const float* __restrict__ other, const float* __restrict__ gout, float* __restrict__ gin,
@@ -232,7 +265,7 @@ correlation_backward_kernel(const float* __restrict__ other, const float* __rest
     for (int tj = 0; tj < D; ++tj) {
       const int j2 = (tj - R) * s2;
       const int oy = (which ? y - j2 : y + j2) - pad;
-      if (oy < 0 || oy >= H) continue;                       // the other image's row is zero padding
+      const bool row_in = oy >= 0 && oy < H;                 // else the other image's row is zero padding
       int ymin = y - krad - maxdisp - (which ? j2 : 0), ymax = ymin + 2 * krad;
       if (ymax < 0 || ymin >= outH) continue;
       ymin = max(ymin, 0);
@@ -241,10 +274,10 @@ correlation_backward_kernel(const float* __restrict__ other, const float* __rest
         const int i2 = (ti - R) * s2;
         const int ox = (which ? x - i2 : x + i2) - pad;
         int xmin = x - krad - maxdisp - (which ? i2 : 0), xmax = xmin + 2 * krad;
-        if (ox < 0 || ox >= W || xmax < 0 || xmin >= outW) continue;
+        if (xmax < 0 || xmin >= outW) continue;
         xmin = max(xmin, 0);
         xmax = min(xmax, outW - 1);
-        const float val = __ldg(img + (int64_t)oy * W + ox);
+        const float val = (row_in && ox >= 0 && ox < W) ? __ldg(img + (int64_t)oy * W + ox) : 0.0f;
         const float* gt = g + (int64_t)(tj * D + ti) * OHW;
         for (int j = ymin; j <= ymax; ++j)
           for (int i = xmin; i <= xmax; ++i) acc = fmaf(__ldg(gt + (int64_t)j * outW + i), val, acc);
